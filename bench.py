@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- headline benchmark of the region-merging hot path (BASELINE.json metric).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference] [--dump-outputs DIR]
 
 A step = one end-to-end pass (RAG + band pooling -> point pooling -> L2 edge scoring ->
 iterative union-find merge -> relabel) over the synthetic scene of SURVEY.md section 8(d).
@@ -181,11 +181,43 @@ def cpu_baseline_record(cfg, side, steps=3, warmup=1):
     return {"value": mpx, "unit": "Mpx/s", "cores": procs, "kind": "port", "sample": sample}, sec, merges * procs
 
 
+DUMP_MAX_ELEMS = 1 << 19        # per array: the 13 files written for a MergeResult stay below 64 MB in all
+
+
+def dump_outputs(path, res, seed=0):
+    """Writes every field of a MergeResult as path/<field>.npy so that two builds can be compared output for output:
+    integers as float64 (exact below 2**53), floats as float32.  An array of more than DUMP_MAX_ELEMS elements is
+    replaced by a sample of its flattened elements at seeded positions, the same in every run of the same workload.
+    A float field holds NaN by design where a region has no sample points (its mean is NaN, its edges score NaN and are
+    never selected): such values are written as 0, and path/<field>_finite.npy holds 1 where the value is finite and 0
+    where it is not, so every file holds finite numbers and nothing is lost."""
+    import dataclasses
+    import torch
+    os.makedirs(path, exist_ok=True)
+    for f in dataclasses.fields(res):
+        v = getattr(res, f.name)
+        if isinstance(v, int):
+            v = torch.tensor(v)
+        if not isinstance(v, torch.Tensor):         # MergeEngine.run leaves the initial graph out (rag is None)
+            continue
+        if v.numel() > DUMP_MAX_ELEMS:
+            idx = np.unique(np.random.default_rng(seed).integers(0, v.numel(), DUMP_MAX_ELEMS))
+            v = v.reshape(-1)[torch.from_numpy(idx).to(v.device)]
+        a = v.cpu().numpy()
+        if a.dtype.kind == "f":
+            ok = np.isfinite(a)
+            np.save(os.path.join(path, f.name + "_finite.npy"), ok.astype(np.float32))
+            a = np.where(ok, a, 0).astype(np.float32)
+        else:
+            a = a.astype(np.float64)
+        np.save(os.path.join(path, f.name + ".npy"), a)
+
+
 def reference_arm(args):
     rank = int(os.environ.get("RANK", "0"))
     if rank != 0:
         return
-    steps, warmup = max(1, min(args.steps, 3)), min(max(args.warmup, 0), 1)
+    steps, warmup = args.steps, max(args.warmup, 0)
     rec, sec, merges = cpu_baseline_record(CFG, args.cpu_side, steps=steps, warmup=warmup)
     line = {
         "impl": "reference", "metric": "megapixels/sec end-to-end (RAG+pool+score+merge+relabel)", "value": rec["value"],
@@ -269,6 +301,8 @@ def b200_arm(args):
     ms = ev0.elapsed_time(ev1) / args.steps
     launches = (L.dm_launch_count() - launches0)
     mpx = H * W / ms / 1e3
+    if args.dump_outputs:               # res holds views of the engine's buffers: write them before anything else runs
+        dump_outputs(args.dump_outputs, res)
 
     # ---- the dominant kernel alone (fused RAG + band pooling raster pass), CUDA events -------------
     s = _stream()
@@ -584,7 +618,15 @@ def main():
     ap.add_argument("--config2", action="store_true",
                     help="N > 1 only: run BASELINE.json configs[2] (ONE 40k x 40k scene, ~1M segments, split over the ranks) "
                          "instead of the weak-scaling stack of configs[1] tiles")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="single GPU: write the result of the last timed step as DIR/<field>.npy (float32 / float64; "
+                         "fields above %d elements as a fixed, seeded sample; non-finite floats as 0, flagged in "
+                         "DIR/<field>_finite.npy)" % DUMP_MAX_ELEMS)
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.impl != "b200" or int(os.environ.get("WORLD_SIZE", "1")) > 1):
+        ap.error("--dump-outputs needs the single-GPU b200 run")
     if args.impl == "reference":
         reference_arm(args)
     else:

@@ -18,7 +18,7 @@ import tempfile
 import numpy as np
 import torch
 
-from . import ref_shim
+from . import golden, ref_shim
 
 OUT = os.path.join(os.path.dirname(os.path.dirname(os.path.abspath(__file__))), "tests", "golden")
 
@@ -90,7 +90,7 @@ def golden_mlp(ref, rng):
     with torch.no_grad():
         fc3, fc2 = m(x)
     sd = {k: v.numpy() for k, v in m.state_dict().items()}
-    np.savez(os.path.join(OUT, "mlp784.npz"), x=x.numpy(), fc3=fc3.numpy(), fc2=fc2.numpy(),
+    golden.save(os.path.join(OUT, "mlp784.npz"), x=x.numpy(), fc3=fc3.numpy(), fc2=fc2.numpy(),
              **{k.replace(".", "_"): v for k, v in sd.items()})
     # pair-MLP: the same class and forward code (Nets.py:28-35) with fc1/fc3 re-dimensioned
     torch.manual_seed(1)
@@ -250,7 +250,7 @@ def golden_pair_dataset(ref, rng):
             for k, patch in enumerate(meta[2]):
                 out[f"{side}{i}_patch{k}"] = patch
         out[f"flag{i}"] = np.int64(flag)
-    np.savez_compressed(os.path.join(OUT, "pair_dataset.npz"), arr=arr, gt=np.array(gt), fields=np.array(fields), attr=attr,
+    golden.save(os.path.join(OUT, "pair_dataset.npz"), compressed=True, arr=arr, gt=np.array(gt), fields=np.array(fields), attr=attr,
                         inner=inner, obj=obj, X=X, Y=Y, pos_pairs=pos_pairs, neg_pairs=neg_pairs, seed=11, n=len(ds),
                         counts=np.array([ds.positive_number, ds.positive_pair_number, ds.negative_number,
                                          ds.negative_pair_number]),

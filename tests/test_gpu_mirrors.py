@@ -4,6 +4,7 @@ import os
 import numpy as np
 import pytest
 
+from oracle import golden
 from oracle import oracle_np as o
 
 pytestmark = pytest.mark.gpu
@@ -124,7 +125,7 @@ def test_pair_dataset_items_equal_the_executed_reference(cuda, golden_dir, tmp_p
     import torch
     from deepmerge_b200 import MyUtils1
     from test_mirrors_cpu import _pair_dataset_fixture
-    g = np.load(os.path.join(golden_dir, "pair_dataset.npz"))
+    g = golden.load(os.path.join(golden_dir, "pair_dataset.npz"))
     pos, neg, open_vector, open_image = _pair_dataset_fixture(g, tmp_path)
     random.seed(int(g["seed"]))
     ds = MyUtils1.MergingSegmensPairDataset("IF", "PF", "QF", pos, neg, open_vector=open_vector, open_image=open_image,

@@ -14,6 +14,7 @@ import os
 import numpy as np
 import pytest
 
+from oracle import golden
 from oracle import oracle_np as o
 
 pytestmark = pytest.mark.gpu
@@ -34,7 +35,7 @@ def close(got, want, tol):
 def test_mlp_forward_against_reference_golden(cuda, golden_dir, name):
     from deepmerge_b200.Nets import MLP
     import torch
-    m = np.load(os.path.join(golden_dir, name))
+    m = golden.load(os.path.join(golden_dir, name))
     n_in, hidden, n_out = m["fc1_weight"].shape[1], m["fc1_weight"].shape[0], m["fc3_weight"].shape[0]
     net = MLP((n_in, hidden, n_out)).to(cuda)
     net.load_state_dict({k: torch.from_numpy(m[k.replace(".", "_")]) for k in

@@ -7,6 +7,7 @@ import numpy as np
 import pytest
 
 from deepmerge_b200 import MyUtils1, MyUtils2
+from oracle import golden
 from oracle.ref_shim import FakeFeature, FakeLayer, FakeRaster
 
 
@@ -248,7 +249,7 @@ def _pair_dataset_fixture(g, tmp_path):
 def test_pair_dataset_class_builds_the_reference_item_list(golden_dir, tmp_path):
     """MergingSegmensPairDataset(image_folder, polygon_folder, point_folder, positive_folder, negative_folder): same
     attributes and, under the same seed, the item list of the executed reference (MyUtils1.py:20-38, :236-295)."""
-    g = np.load(os.path.join(golden_dir, "pair_dataset.npz"))
+    g = golden.load(os.path.join(golden_dir, "pair_dataset.npz"))
     pos, neg, open_vector, open_image = _pair_dataset_fixture(g, tmp_path)
     random.seed(int(g["seed"]))
     ds = MyUtils1.MergingSegmensPairDataset("IF", "PF", "QF", pos, neg, open_vector=open_vector, open_image=open_image)

@@ -6,11 +6,12 @@ import os
 import numpy as np
 import pytest
 
+from oracle import golden
 from oracle import oracle_np as o
 
 
 def g(golden_dir, name):
-    return np.load(os.path.join(golden_dir, name))
+    return golden.load(os.path.join(golden_dir, name))
 
 
 def test_euclidean_distance_matches_reference(golden_dir):
@@ -40,6 +41,22 @@ def test_pooling_is_bit_exact_with_reference_loop(golden_dir):
     keys = (p["left"].astype(np.uint64) << np.uint64(32)) | p["right"].astype(np.uint64)
     sc = o.score_l2(m, keys)
     assert np.max(np.abs(sc - p["simi"]) / np.maximum(p["simi"], 1e-6)) < 1e-5
+
+
+def test_golden_archives_split_into_parts_below_the_size_limit(golden_dir, tmp_path, monkeypatch):
+    for f in os.listdir(golden_dir):
+        assert os.path.getsize(os.path.join(golden_dir, f)) < golden.MAX_BYTES, f
+    monkeypatch.setattr(golden, "MAX_BYTES", 3000)
+    arrays = {f"a{i}": np.arange(500, dtype=np.float32) + i for i in range(3)}     # ~2.1 kB each: one per part
+    path = str(tmp_path / "x.npz")
+    golden.save(path, **arrays)
+    assert sorted(os.listdir(tmp_path)) == ["x.1.npz", "x.2.npz", "x.npz"]
+    back = golden.load(path)
+    assert list(back) == list(arrays) and all(np.array_equal(back[k], arrays[k]) for k in arrays)
+    golden.save(path, a0=arrays["a0"])                                             # stale parts go
+    assert os.listdir(tmp_path) == ["x.npz"] and list(golden.load(path)) == ["a0"]
+    with pytest.raises(ValueError, match="alone exceeds"):
+        golden.save(path, big=np.zeros(1000, np.float32))
 
 
 @pytest.mark.parametrize("name", ["mlp784.npz", "mlp_pair.npz"])
