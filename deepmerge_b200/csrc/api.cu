@@ -48,14 +48,14 @@ extern "C" int dm_num_sms(void) {
     return n;
 }
 
-extern "C" size_t dm_sort_edges_workspace_bytes(int64_t capacity) { return prims::sort_ws_bytes(capacity); }
+extern "C" size_t dm_sort_edges_workspace_bytes(int64_t capacity) { return prims::ws_bytes(capacity, false); }
 
 extern "C" int dm_sort_edges(uint64_t* keys, uint32_t* vals, const int64_t* n_dev, int64_t capacity, int64_t n_regions,
                              void* ws, size_t ws_bytes, dm_stream_t stream) {
     if (capacity < 0 || n_regions < 1) return DM_ERR_BAD_ARG;
     if (capacity == 0) return DM_OK;
     if (!keys || !n_dev || !ws) return DM_ERR_BAD_ARG;
-    if (ws_bytes < prims::sort_ws_bytes(capacity)) return DM_ERR_WORKSPACE;
+    if (ws_bytes < prims::ws_bytes(capacity, false)) return DM_ERR_WORKSPACE;
     const int b = bits_for(n_regions);
     return prims::sort_pairs(keys, vals, n_dev, capacity, b, 2 * b, ws, S(stream));
 }

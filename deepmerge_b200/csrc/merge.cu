@@ -775,7 +775,7 @@ extern "C" int dm_uf_compress(int32_t* parent, int64_t R, dm_stream_t stream) {
 
 extern "C" size_t dm_merge_apply_workspace_bytes(int64_t R) {
     const int64_t cap = R < 1 ? 1 : R;
-    return align_up((size_t)cap * 8, 256) + prims::sort_ws_bytes(cap) + 512;
+    return align_up((size_t)cap * 8, 256) + prims::ws_bytes(cap, false) + 512;
 }
 
 extern "C" size_t dm_merge_apply_workspace_bytes(int64_t R);
@@ -791,7 +791,7 @@ extern "C" int dm_merge_apply_masked(const int32_t* parent, uint8_t* alive, uint
     if (ws_bytes < dm_merge_apply_workspace_bytes(R)) return DM_ERR_WORKSPACE;
     Carver c(ws);
     uint64_t* list = c.take<uint64_t>(R);
-    void* sws = c.take<char>(prims::sort_ws_bytes(R));
+    void* sws = c.take<char>(prims::ws_bytes(R, false));
     int64_t* n_list = c.take<int64_t>(1);
     DM_CUDA(cudaMemsetAsync(changed, 0, (size_t)R, s));
     DM_CUDA(cudaMemsetAsync(n_list, 0, sizeof(int64_t), s));
@@ -800,7 +800,7 @@ extern "C" int dm_merge_apply_masked(const int32_t* parent, uint8_t* alive, uint
                                                               (unsigned long long*)n_list, (unsigned long long*)n_merged,
                                                               root_mask);
     const int b = bits_for(R);
-    DM_TRY(prims::sort_pairs(list, nullptr, n_list, R, b, 2 * b, sws, s, prims::sort_fused_mode() >= 2, R));
+    DM_TRY(prims::sort_pairs(list, nullptr, n_list, R, b, 2 * b, sws, s, R));
     DM_COUNT_LAUNCH(); merge::merge_sums_kernel<<<grid_for(R * 32), 256, 0, s>>>(list, n_list, sum, (int)D);
     DM_LAUNCH_CHECK();
     return DM_OK;
@@ -815,8 +815,7 @@ extern "C" int dm_merge_apply(const int32_t* parent, uint8_t* alive, uint8_t* ch
 
 extern "C" size_t dm_edges_rekey_workspace_bytes(int64_t capacity) {
     const int64_t cap = capacity < 1 ? 1 : capacity;
-    return 2 * align_up((size_t)cap * 8, 256) + 3 * align_up((size_t)cap * 4, 256) + prims::sort_ws_bytes(cap) +
-           prims::unique_ws_bytes(cap) + 256;
+    return 2 * align_up((size_t)cap * 8, 256) + 3 * align_up((size_t)cap * 4, 256) + prims::ws_bytes(cap, true) + 256;
 }
 
 extern "C" int dm_edges_rekey(const int32_t* parent, uint64_t* keys, uint32_t* lens, float* scores, int64_t* n_dev,
@@ -833,15 +832,14 @@ extern "C" int dm_edges_rekey(const int32_t* parent, uint64_t* keys, uint32_t* l
     uint32_t* perm = c.take<uint32_t>(capacity);
     uint32_t* ol = c.take<uint32_t>(capacity);
     float* os = c.take<float>(capacity);
-    void* sws = c.take<char>(prims::sort_ws_bytes(capacity));
-    void* uws = c.take<char>(prims::unique_ws_bytes(capacity));
+    void* sws = c.take<char>(prims::ws_bytes(capacity, true));
     const uint64_t sentinel = ((uint64_t)R << 32) | (uint64_t)R;
     DM_COUNT_LAUNCH(); merge::rekey_kernel<<<grid_for(capacity), 256, 0, s>>>(parent, keys, lens, n_dev, sentinel,
                                                            (unsigned long long*)perimeter, nk, perm);
     const int b = bits_for(R + 1);
     int64_t* n_new = c.take<int64_t>(1);
     DM_TRY(prims::sort_unique(nk, perm, n_dev, capacity, b, 2 * b, sws, lens, scores, sentinel, ok, ol, scores ? os : nullptr,
-                              n_new, uws, keys, lens, scores, n_dev, s, R));
+                              n_new, keys, lens, scores, n_dev, s, R));
     DM_LAUNCH_CHECK();
     return DM_OK;
 }

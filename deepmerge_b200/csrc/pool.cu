@@ -28,24 +28,6 @@ __global__ void csr_keys_kernel(const int32_t* __restrict__ rop, int64_t n, int6
     }
 }
 
-// offsets[r] = first sorted position whose key >= r, for r in [0, R]: one binary search per region (region ids
-// with no points -- e.g. every region of the other row tiles -- cost the same as any other)
-__global__ void csr_offsets_kernel(const uint64_t* __restrict__ keys, const uint32_t* __restrict__ vals, int64_t n,
-                                   int64_t n_regions, int64_t* __restrict__ offsets, int32_t* __restrict__ point_ids) {
-    const int64_t stride = (int64_t)gridDim.x * blockDim.x, t0 = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
-    for (int64_t r = t0; r <= n_regions; r += stride) {
-        int64_t lo = 0, hi = n;
-        while (lo < hi) {
-            const int64_t mid = (lo + hi) >> 1;
-            if ((int64_t)keys[mid] < r) lo = mid + 1;
-            else hi = mid;
-        }
-        offsets[r] = lo;
-    }
-    for (int64_t i = t0; i < n; i += stride)
-        if ((int64_t)keys[i] < n_regions) point_ids[i] = (int32_t)vals[i];
-}
-
 // One warp per region, lanes over the feature dimension, points visited in membership
 // order: sum = ((f0 + f1) + f2) + ...  exactly like np.mean's row-by-row reduction
 // (ExtractFeatures.py:211-212).  K*32 feature columns per pass starting at d_base.
@@ -389,14 +371,15 @@ extern "C" int dm_points_region(const int32_t* labels, int64_t H, int64_t W, int
 }
 
 extern "C" size_t dm_csr_workspace_bytes(int64_t n_points, int64_t n_regions) {
-    (void)n_regions;
     const int64_t cap = n_points < 1 ? 1 : n_points;
-    return align_up((size_t)cap * 8, 256) + align_up((size_t)cap * 4, 256) + 256 + prims::sort_ws_bytes(cap);
+    // the bucket sort keeps per-id arrays for the n_regions + 1 keys (region ids and the "no region" key)
+    return align_up((size_t)cap * 8, 256) + align_up((size_t)cap * 4, 256) + 256 +
+           prims::ws_bytes(cap, false, n_regions + 1);
 }
 
 extern "C" int dm_csr_build(const int32_t* rop, int64_t n, int64_t R, int64_t* offsets, int32_t* point_ids, void* ws,
                             size_t ws_bytes, dm_stream_t stream) {
-    if (n < 0 || R < 0 || !offsets) return DM_ERR_BAD_ARG;
+    if (n < 0 || n > INT32_MAX || R < 0 || !offsets) return DM_ERR_BAD_ARG;   // point ids are int32
     cudaStream_t s = S(stream);
     if (n == 0) {
         DM_CUDA(cudaMemsetAsync(offsets, 0, (size_t)(R + 1) * sizeof(int64_t), s));
@@ -408,18 +391,13 @@ extern "C" int dm_csr_build(const int32_t* rop, int64_t n, int64_t R, int64_t* o
     uint64_t* keys = c.take<uint64_t>(n);
     uint32_t* vals = c.take<uint32_t>(n);
     int64_t* n_dev = c.take<int64_t>(1);
-    void* sws = c.take<char>(prims::sort_ws_bytes(n));
+    void* sws = c.take<char>(prims::ws_bytes(n, false, R + 1));
     const unsigned g = pool::grid_for(n, 256, 8);
     DM_COUNT_LAUNCH(); pool::csr_keys_kernel<<<g, 256, 0, s>>>(rop, n, R, keys, vals, n_dev);
     // stable sort by region only (input is in ascending point id): low bits_for(R+1) bits
     const int b = bits_for(R + 1);
-    // bucket + rank in one cooperative launch, offsets and point ids included ...
-    const int rc = prims::sort_pairs(keys, vals, n_dev, n, b, b, sws, s, true, R + 1, offsets, point_ids);
-    if (rc == DM_OK) return DM_OK;
-    if (rc != DM_ERR_UNSUPPORTED) return rc;
-    // ... or radix passes, one launch per phase, and a binary search per region
-    DM_TRY(prims::sort_pairs(keys, vals, n_dev, n, b, b, sws, s, false));
-    DM_COUNT_LAUNCH(); pool::csr_offsets_kernel<<<pool::grid_for((n > R ? n : R) + 1, 256, 8), 256, 0, s>>>(keys, vals, n, R, offsets, point_ids);
+    // bucket + rank in one cooperative launch, offsets and point ids included
+    DM_TRY(prims::sort_pairs(keys, vals, n_dev, n, b, b, sws, s, R + 1, offsets, point_ids));
     DM_LAUNCH_CHECK();
     return DM_OK;
 }

@@ -1,8 +1,10 @@
 // Scan / radix sort / run reduction (see prims.cuh).  Hand-written for sm_100a; no CUB.
 #include <cstdio>
 #include "prims.cuh"
+#include <map>
 #include <stdlib.h>
 #include <string.h>
+#include <utility>
 
 namespace dm {
 namespace prims {
@@ -92,13 +94,10 @@ int scan_exclusive_u32(const uint32_t* in, uint32_t* out, const int64_t* n_dev, 
 
 // ------------------------------------------------------------------------------------ //
 // LSD radix sort, 9-bit digits.  Per pass: tile histograms, per-digit offsets over tiles, scatter.
-// Two drivers share the per-tile device code:
-//   * radix_sort_fused: ONE cooperative launch for the whole sort (and, optionally, the run
-//     reduction that follows it); persistent blocks walk their tiles and meet at grid barriers
-//     between the phases.  At the sizes of the graph stages (<= a few million pairs) a pass is
-//     launch/latency bound, so 12 + 6 launches collapse into one.
-//   * radix_hist / radix_offsets / radix_scatter: one launch per phase (no co-residency needed;
-//     used beside the raster kernel, which leaves no room for a co-resident grid).
+// radix_sort_fused runs the whole sort (and, optionally, the run reduction that follows it) as ONE
+// cooperative launch; persistent blocks walk their tiles and meet at grid barriers between the
+// phases.  At the sizes of the graph stages (<= a few million pairs) a pass is launch/latency
+// bound, so the 12 + 6 launches of a one-launch-per-phase driver collapse into one.
 // Buffers written inside the fused kernel are read back with ld.global.cg (L2): L1 is not coherent
 // across blocks and `const __restrict__` loads could take the non-coherent path.
 // ------------------------------------------------------------------------------------ //
@@ -251,40 +250,6 @@ __device__ __forceinline__ void scatter_tile(SortSmem& sm, const uint64_t* kin, 
     __syncthreads();
 }
 
-__global__ void __launch_bounds__(SORT_THREADS) radix_hist(const uint64_t* keys, const int64_t* __restrict__ n_dev,
-                                                           int id_bits, int shift, uint32_t* hist, int tiles_cap) {
-    const int64_t n = *n_dev;
-    if ((int64_t)blockIdx.x * SORT_TILE >= n) return;
-    __shared__ SortSmem sm;
-    hist_tile(sm, keys, n, (int)blockIdx.x, id_bits, shift, hist, tiles_cap);
-}
-
-__global__ void __launch_bounds__(1024) radix_offsets(uint32_t* hist, const int64_t* __restrict__ n_dev, uint32_t* totals,
-                                                      int tiles_cap) {
-    const int64_t n = *n_dev;
-    const int tiles = (int)((n + SORT_TILE - 1) / SORT_TILE);
-    offsets_digit(hist, totals, blockIdx.x * 32 + (threadIdx.x >> 5), tiles, tiles_cap);
-}
-
-__global__ void __launch_bounds__(SORT_THREADS) radix_scatter(const uint64_t* kin, const uint32_t* vin, uint64_t* kout,
-                                                              uint32_t* vout, const int64_t* __restrict__ n_dev, int id_bits,
-                                                              int shift, const uint32_t* hist, const uint32_t* totals,
-                                                              int tiles_cap) {
-    const int64_t n = *n_dev;
-    if ((int64_t)blockIdx.x * SORT_TILE >= n) return;
-    __shared__ SortSmem sm;
-    scatter_tile(sm, kin, vin, kout, vout, n, (int)blockIdx.x, id_bits, shift, hist, totals, tiles_cap);
-}
-
-__global__ void copy_pairs(const uint64_t* __restrict__ kin, const uint32_t* __restrict__ vin, uint64_t* __restrict__ kout,
-                           uint32_t* __restrict__ vout, const int64_t* __restrict__ n_dev) {
-    const int64_t n = *n_dev;
-    for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (int64_t)gridDim.x * blockDim.x) {
-        kout[i] = kin[i];
-        if (vin) vout[i] = vin[i];
-    }
-}
-
 // ---- the fused (single cooperative launch) driver ---------------------------------------
 
 struct FusedArgs {
@@ -294,7 +259,7 @@ struct FusedArgs {
     uint32_t* hist; uint32_t* totals;
     unsigned* bar;                       // [0] arrivals (zeroed before the launch), [1] error flag
     int id_bits, passes, tiles_cap;
-    // run reduction of the sorted pairs (do_unique): see unique_reduce
+    // run reduction of the sorted pairs (do_unique): see sort_unique in prims.cuh
     int do_unique;
     const uint32_t* gather_lens;         // null: the sorted values are the lengths; else lengths / scores are
     const float* gather_scores;          //       gathered through the sorted values (a permutation)
@@ -887,372 +852,151 @@ __global__ void __launch_bounds__(SORT_THREADS, HASH_BLOCKS_PER_SM) bucket_sort_
 }
 
 
+// ------------------------------------------------------------------------------------ //
+// host side: one workspace layout, one cooperative launch per call
+// ------------------------------------------------------------------------------------ //
 namespace {
-size_t legacy_unique_ws_bytes(int64_t cap) {
-    return 2 * align_up((size_t)cap * sizeof(uint32_t), 256) + scan_ws_bytes(cap);
-}
 int ceil_log2_i64(int64_t x) {
     int l = 0;
     while ((1ll << l) < x) ++l;
     return l;
 }
-// ids the hashed run reduction can index with a workspace sized for `cap` entries (more ids: the radix path)
+// ids the per-id arrays of a workspace sized for `cap` entries hold at least
 int64_t hash_ids_cap(int64_t cap) { return 4 * cap + 65536; }
 int hash_tab_log2(int64_t cap) { return ceil_log2_i64(imax64(1024, cap + cap / 2 + 1)); }
 
-struct HashWs {
-    uint4* tab;
-    uint32_t *deg, *off, *cur, *chunk_tot, *hubs;
-    uint4* t_ent;
-    uint2* t_bkt;
-    unsigned* misc;
-    size_t bytes;
-};
-HashWs carve_hash_ws(void* base, int64_t cap, bool with_table = true) {
-    Carver c(base);
-    HashWs w;
-    const size_t ids = (size_t)hash_ids_cap(cap);
-    w.tab = with_table ? c.take<uint4>((size_t)1 << hash_tab_log2(cap)) : nullptr;
-    w.deg = c.take<uint32_t>(ids);
-    w.off = c.take<uint32_t>(ids);
-    w.cur = c.take<uint32_t>(ids);
-    w.chunk_tot = c.take<uint32_t>(HASH_MAX_GRID);
-    w.hubs = c.take<uint32_t>(HUB_CAP);
-    w.t_ent = c.take<uint4>(cap);
-    w.t_bkt = c.take<uint2>(cap);
-    w.misc = c.take<unsigned>(16);
-    w.bytes = c.used();
-    return w;
-}
-int hashed_mode() {                                        // DM_EDGE_HASH=0: always the radix path
-    static int mode = -1;
-    if (mode < 0) {
-        const char* e = getenv("DM_EDGE_HASH");
-        mode = (e && e[0] == '0') ? 0 : 1;
-    }
-    return mode;
-}
-int hashed_grid_limit() {
-    static thread_local int cached_dev = -1, cached = 0;
-    int dev = 0;
-    if (cudaGetDevice(&dev) != cudaSuccess) return 0;
-    if (dev != cached_dev) {
-        int coop = 0, per_sm = 0;
-        cached = 0;
-        if (cudaDeviceGetAttribute(&coop, cudaDevAttrCooperativeLaunch, dev) == cudaSuccess && coop &&
-            cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, edge_unique_hashed, SORT_THREADS, 0) == cudaSuccess)
-            cached = (int)imin64((int64_t)(per_sm < HASH_BLOCKS_PER_SM ? per_sm : HASH_BLOCKS_PER_SM) * num_sms(), HASH_MAX_GRID);
-        cached_dev = dev;
-    }
-    return cached;
-}
-int bucket_sort_grid_limit() {
-    static thread_local int cached_dev = -1, cached = 0;
-    int dev = 0;
-    if (cudaGetDevice(&dev) != cudaSuccess) return 0;
-    if (dev != cached_dev) {
-        int coop = 0, per_sm = 0;
-        cached = 0;
-        if (cudaDeviceGetAttribute(&coop, cudaDevAttrCooperativeLaunch, dev) == cudaSuccess && coop &&
-            cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, bucket_sort_fused, SORT_THREADS, 0) == cudaSuccess)
-            cached = (int)imin64((int64_t)(per_sm < HASH_BLOCKS_PER_SM ? per_sm : HASH_BLOCKS_PER_SM) * num_sms(), HASH_MAX_GRID);
-        cached_dev = dev;
-    }
-    return cached;
-}
-size_t legacy_sort_ws_bytes(int64_t cap) {
-    size_t b = 0;
-    b += align_up((size_t)cap * sizeof(uint64_t), 256);
-    b += align_up((size_t)cap * sizeof(uint32_t), 256);
-    b += align_up((size_t)ceil_div(cap, SORT_TILE) * RADIX * sizeof(uint32_t), 256);
-    b += align_up(RADIX * sizeof(uint32_t), 256);
-    b += 256;                                              // grid barrier words of the fused kernel
-    return b;
-}
-}  // namespace
-
-size_t sort_ws_bytes(int64_t cap) {
-    if (cap < 1) cap = 1;
-    return legacy_sort_ws_bytes(cap) + carve_hash_ws(nullptr, cap, false).bytes;
-}
-
-namespace {
-struct SortWs {
-    uint64_t* k2;
-    uint32_t* v2;
-    uint32_t* hist;
-    uint32_t* totals;
-    unsigned* bar;
-    unsigned tiles;
-};
-SortWs carve_sort_ws(void* ws, int64_t cap) {
+// The layout ws_bytes measures, carved into the workspace pointers of H; returns the bytes it spans.  The per-id
+// arrays hold max(hash_ids_cap(cap), ids) ids; the tile heads and the hash table exist only for the run reduction.
+size_t carve_ws(HashArgs& H, void* ws, int64_t cap, bool unique, int64_t ids) {
+    FusedArgs& A = H.F;
     Carver c(ws);
-    SortWs w;
-    w.k2 = c.take<uint64_t>(cap);
-    w.v2 = c.take<uint32_t>(cap);
-    w.tiles = (unsigned)ceil_div(cap, SORT_TILE);
-    w.hist = c.take<uint32_t>((size_t)w.tiles * RADIX);
-    w.totals = c.take<uint32_t>(RADIX);
-    w.bar = c.take<unsigned>(2);
-    return w;
-}
-
-// DM_SORT_FUSED: 0 = one launch per phase everywhere, 1 = fused kernel for the edge sorts, 2 (default) = also for the
-// member sort of dm_merge_apply, which runs on a side stream beside the edge re-keying.
-int fused_mode() {
-    static int mode = -1;
-    if (mode < 0) {
-        const char* e = getenv("DM_SORT_FUSED");
-        mode = (e && e[0] >= '0' && e[0] <= '9') ? e[0] - '0' : 2;
+    A.k1 = c.take<uint64_t>(cap);
+    A.v1 = c.take<uint32_t>(cap);
+    A.tiles_cap = (int)ceil_div(cap, SORT_TILE);
+    A.hist = c.take<uint32_t>((size_t)A.tiles_cap * RADIX);
+    A.totals = c.take<uint32_t>(RADIX);
+    A.bar = c.take<unsigned>(2);
+    if (unique) {
+        A.tile_heads = c.take<uint32_t>(A.tiles_cap);
+        H.tab_cap_log2 = hash_tab_log2(cap);
+        H.tab = c.take<uint4>((size_t)1 << H.tab_cap_log2);
     }
-    return mode;
+    const size_t n_ids = (size_t)imax64(hash_ids_cap(cap), ids);
+    H.deg = c.take<uint32_t>(n_ids);
+    H.off = c.take<uint32_t>(n_ids);
+    H.cur = c.take<uint32_t>(n_ids);
+    H.chunk_tot = c.take<uint32_t>(HASH_MAX_GRID);
+    H.hubs = c.take<uint32_t>(HUB_CAP);
+    H.t_ent = c.take<uint4>(cap);
+    H.t_bkt = c.take<uint2>(cap);
+    H.misc = c.take<unsigned>(16);
+    return c.used();
 }
 
-// Blocks of the fused kernel that are co-resident on this device (0: cooperative launch unsupported).
-int fused_grid_limit() {
-    static thread_local int cached_dev = -1, cached = 0;
+// Kernel arguments of one call: the carved workspace and the pairs (the run-reduction fields stay zero).
+HashArgs make_args(void* ws, int64_t cap, bool unique, int64_t ws_ids, uint64_t* keys, uint32_t* vals,
+                   const int64_t* n_dev, int id_bits, int key_bits, int64_t n_ids) {
+    HashArgs H;
+    memset(&H, 0, sizeof(H));
+    carve_ws(H, ws, cap, unique, ws_ids);
+    FusedArgs& A = H.F;
+    A.k0 = keys; A.v0 = vals;
+    A.n_dev = n_dev; A.n_max = cap;
+    A.id_bits = id_bits; A.passes = (key_bits + RADIX_BITS - 1) / RADIX_BITS;
+    H.n_ids = n_ids;
+    return H;
+}
+
+// Blocks of `kernel` (SORT_THREADS threads) that are co-resident on the current device, at most per_sm_cap per SM;
+// 0 when the device has no cooperative launch.
+int coop_grid_limit(const void* kernel, int per_sm_cap) {
+    static thread_local std::map<std::pair<int, const void*>, int> cache;
     int dev = 0;
     if (cudaGetDevice(&dev) != cudaSuccess) return 0;
-    if (dev != cached_dev) {
-        int coop = 0, per_sm = 0;
-        cached = 0;
-        if (cudaDeviceGetAttribute(&coop, cudaDevAttrCooperativeLaunch, dev) == cudaSuccess && coop &&
-            cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, radix_sort_fused, SORT_THREADS, 0) == cudaSuccess)
-            cached = (per_sm < 2 ? per_sm : 2) * num_sms();     // measured: a third block per SM costs more in the
-                                                                // barriers than it saves in the phases
-        cached_dev = dev;
-    }
-    return cached;
+    const auto hit = cache.find({dev, kernel});
+    if (hit != cache.end()) return hit->second;
+    int coop = 0, per_sm = 0, limit = 0;
+    if (cudaDeviceGetAttribute(&coop, cudaDevAttrCooperativeLaunch, dev) == cudaSuccess && coop &&
+        cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kernel, SORT_THREADS, 0) == cudaSuccess)
+        limit = (per_sm < per_sm_cap ? per_sm : per_sm_cap) * num_sms();
+    cache[{dev, kernel}] = limit;
+    return limit;
 }
 
-int launch_fused(FusedArgs& A, int64_t cap, cudaStream_t s) {
-    const int limit = fused_grid_limit();
-    if (limit <= 0) return DM_ERR_UNSUPPORTED;
-    const int grid = (int)imax64(1, imin64(ceil_div(cap, SORT_TILE), limit));
-    DM_CUDA(cudaMemsetAsync(A.bar, 0, 2 * sizeof(unsigned), s));
-    void* args[] = {(void*)&A};
+// Zeroes the grid barrier words (and, when given, the hub count and fall-back flag of misc) and launches `kernel`
+// cooperatively on `grid` blocks.  grid < 1 means the device has no cooperative launch: DM_ERR_UNSUPPORTED.  A refused
+// launch is DM_ERR_CUDA with the CUDA error recorded; there is no other path to fall back to.
+int launch_coop(const void* kernel, int64_t grid, void** args, unsigned* bar, unsigned* misc, cudaStream_t s) {
+    if (grid < 1) return DM_ERR_UNSUPPORTED;
+    DM_CUDA(cudaMemsetAsync(bar, 0, 2 * sizeof(unsigned), s));
+    if (misc) DM_CUDA(cudaMemsetAsync(misc, 0, 4 * sizeof(unsigned), s));
     DM_COUNT_LAUNCH();
-    DM_CUDA(cudaLaunchCooperativeKernel((const void*)radix_sort_fused, dim3(grid), dim3(SORT_THREADS), args, 0, s));
+    DM_CUDA(cudaLaunchCooperativeKernel(kernel, dim3((unsigned)grid), dim3(SORT_THREADS), args, 0, s));
     return DM_OK;
 }
+
+int launch_radix(FusedArgs& A, int64_t cap, cudaStream_t s) {
+    // measured: a third block per SM costs more in the barriers than it saves in the phases
+    const int64_t grid = imin64(ceil_div(cap, SORT_TILE), coop_grid_limit((const void*)radix_sort_fused, 2));
+    void* args[] = {(void*)&A};
+    return launch_coop((const void*)radix_sort_fused, grid, args, A.bar, nullptr, s);
+}
 }  // namespace
 
-int sort_fused_mode() { return fused_mode(); }
-bool sort_fused_available() { return fused_mode() != 0 && fused_grid_limit() > 0; }
+size_t ws_bytes(int64_t cap, bool unique, int64_t n_ids) {
+    HashArgs H;
+    return carve_ws(H, nullptr, cap < 1 ? 1 : cap, unique, n_ids);
+}
 
 int sort_pairs(uint64_t* keys, uint32_t* vals, const int64_t* n_dev, int64_t cap, int id_bits, int key_bits, void* ws,
-               cudaStream_t s, bool allow_fused, int64_t n_ids, int64_t* csr_offsets, int32_t* csr_ids) {
+               cudaStream_t s, int64_t n_ids, int64_t* csr_offsets, int32_t* csr_ids) {
     if (cap <= 0) return DM_OK;
     if (id_bits < 1 || id_bits > 32 || key_bits < 1 || key_bits > 2 * id_bits) return DM_ERR_BAD_ARG;
-    const SortWs w = carve_sort_ws(ws, cap);
-    const int passes = (key_bits + RADIX_BITS - 1) / RADIX_BITS;
-    if (csr_offsets && !(allow_fused && sort_fused_available() && n_ids > 0)) return DM_ERR_UNSUPPORTED;
-    if (allow_fused && sort_fused_available()) {
-        FusedArgs A;
-        memset(&A, 0, sizeof(A));
-        A.k0 = keys; A.v0 = vals; A.k1 = w.k2; A.v1 = w.v2;
-        A.n_dev = n_dev; A.n_max = cap;
-        A.hist = w.hist; A.totals = w.totals; A.bar = w.bar;
-        A.id_bits = id_bits; A.passes = passes; A.tiles_cap = (int)w.tiles;
-        // bucket + rank instead of radix passes (small buckets; the kernel takes the radix path itself otherwise)
-        const int blimit = (hashed_mode() || csr_offsets) ? bucket_sort_grid_limit() : 0;
-        if (n_ids > 0 && n_ids <= hash_ids_cap(cap) && (key_bits == 2 * id_bits || key_bits == id_bits) && cap < (1ll << 31)) {
-            if (blimit <= 0) {
-                if (csr_offsets) return DM_ERR_UNSUPPORTED;
-            } else {
-                const HashWs hw = carve_hash_ws((char*)ws + legacy_sort_ws_bytes(cap), cap, false);
-                HashArgs H;
-                memset(&H, 0, sizeof(H));
-                H.F = A;
-                H.deg = hw.deg; H.off = hw.off; H.cur = hw.cur; H.chunk_tot = hw.chunk_tot; H.hubs = hw.hubs; H.misc = hw.misc;
-                H.t_ent = hw.t_ent; H.t_bkt = hw.t_bkt;
-                H.n_ids = n_ids;
-                BucketSortExtra X;
-                X.by_low = key_bits == id_bits ? 1 : 0;
-                X.csr_offsets = csr_offsets; X.csr_ids = csr_ids;
-                // one id-scan tile per block, but not more than ~2.5 blocks per SM: beyond that the barriers cost more than
-                // the shorter phases save (measured: 98 k members 31.6 us at 96 blocks, 20.5 at 383; 392 k points 24.3 us at
-                // 383 blocks, 26.4 at 592)
-                const int grid = (int)imax64(1, imin64(imin64(ceil_div(imax64(cap, n_ids), SORT_THREADS), blimit), 5 * num_sms() / 2));
-                DM_CUDA(cudaMemsetAsync(A.bar, 0, 2 * sizeof(unsigned), s));
-                DM_CUDA(cudaMemsetAsync(H.misc, 0, 4 * sizeof(unsigned), s));
-                void* args[] = {(void*)&H, (void*)&X};
-                DM_COUNT_LAUNCH();
-                if (cudaLaunchCooperativeKernel((const void*)bucket_sort_fused, dim3(grid), dim3(SORT_THREADS), args, 0, s) ==
-                    cudaSuccess)
-                    return DM_OK;
-                (void)cudaGetLastError();
-                if (csr_offsets) return DM_ERR_UNSUPPORTED;
-            }
-        } else if (csr_offsets) {
-            return DM_ERR_UNSUPPORTED;
-        }
-        if (launch_fused(A, cap, s) == DM_OK) return DM_OK;
-        (void)cudaGetLastError();       // the cooperative launch was refused (e.g. no room for a co-resident grid
-                                        // under a profiler or a partitioned GPU): take the one-launch-per-phase path
-    }
-    const unsigned tiles = w.tiles;
-    uint64_t *ka = keys, *kb = w.k2;
-    uint32_t *va = vals, *vb = vals ? w.v2 : nullptr;
-    for (int p = 0; p < passes; ++p) {
-        DM_COUNT_LAUNCH(); radix_hist<<<tiles, SORT_THREADS, 0, s>>>(ka, n_dev, id_bits, RADIX_BITS * p, w.hist, (int)tiles);
-        DM_COUNT_LAUNCH(); radix_offsets<<<RADIX / 32, 1024, 0, s>>>(w.hist, n_dev, w.totals, (int)tiles);
-        DM_COUNT_LAUNCH(); radix_scatter<<<tiles, SORT_THREADS, 0, s>>>(ka, va, kb, vb, n_dev, id_bits, RADIX_BITS * p, w.hist,
-                                                    w.totals, (int)tiles);
-        uint64_t* tk = ka; ka = kb; kb = tk;
-        uint32_t* tv = va; va = vb; vb = tv;
-    }
-    if (ka != keys) {
-        const unsigned g = (unsigned)imin64(ceil_div(cap, 256), 148 * 8);
-        DM_COUNT_LAUNCH(); copy_pairs<<<g, 256, 0, s>>>(ka, va, keys, vals, n_dev);
-    }
-    DM_LAUNCH_CHECK();
-    return DM_OK;
+    HashArgs H = make_args(ws, cap, false, n_ids, keys, vals, n_dev, id_bits, key_bits, n_ids);
+    const bool bucket = n_ids > 0 && (key_bits == 2 * id_bits || key_bits == id_bits) && cap < (1ll << 31);
+    if (!bucket) return csr_offsets ? DM_ERR_BAD_ARG : launch_radix(H.F, cap, s);
+    BucketSortExtra X;
+    X.by_low = key_bits == id_bits ? 1 : 0;
+    X.csr_offsets = csr_offsets; X.csr_ids = csr_ids;
+    // one id-scan tile per block, but not more than ~2.5 blocks per SM: beyond that the barriers cost more than the
+    // shorter phases save (measured: 98 k members 31.6 us at 96 blocks, 20.5 at 383; 392 k points 24.3 us at 383
+    // blocks, 26.4 at 592)
+    const int64_t limit = imin64(coop_grid_limit((const void*)bucket_sort_fused, HASH_BLOCKS_PER_SM), HASH_MAX_GRID);
+    const int64_t grid = imin64(imin64(ceil_div(imax64(cap, n_ids), SORT_THREADS), limit), 5 * num_sms() / 2);
+    void* args[] = {(void*)&H, (void*)&X};
+    return launch_coop((const void*)bucket_sort_fused, grid, args, H.F.bar, H.misc, s);
 }
 
-// ------------------------------------------------------------------------------------ //
-// run reduction on sorted keys
-// ------------------------------------------------------------------------------------ //
-
-__global__ void unique_flags(const uint64_t* __restrict__ keys, const int64_t* __restrict__ n_dev, uint64_t sentinel,
-                             uint32_t* __restrict__ flags) {
-    const int64_t n = *n_dev;
-    for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (int64_t)gridDim.x * blockDim.x) {
-        const uint64_t k = keys[i];
-        flags[i] = (k != sentinel && (i == 0 || keys[i - 1] != k)) ? 1u : 0u;
-    }
-}
-
-__global__ void unique_scatter(const uint64_t* __restrict__ keys, const uint32_t* __restrict__ perm,
-                               const uint32_t* __restrict__ lens_in, const float* __restrict__ scores_in,
-                               const int64_t* __restrict__ n_dev, uint64_t sentinel, const uint32_t* __restrict__ flags,
-                               const uint32_t* __restrict__ excl, uint64_t* __restrict__ out_keys,
-                               uint32_t* __restrict__ out_lens, float* __restrict__ out_scores) {
-    const int64_t n = *n_dev;
-    for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (int64_t)gridDim.x * blockDim.x) {
-        const uint64_t k = keys[i];
-        if (k == sentinel) continue;
-        const uint32_t f = flags[i];
-        const uint32_t run = excl[i] + f - 1;
-        const uint32_t src = perm ? perm[i] : (uint32_t)i;
-        if (f) {
-            out_keys[run] = k;
-            if (scores_in) out_scores[run] = scores_in[src];
-        }
-        atomicAdd(&out_lens[run], lens_in[src]);
-    }
-}
-
-__global__ void clamp_count(const int64_t* n_dev, int64_t cap, int64_t* out) { *out = *n_dev < cap ? *n_dev : cap; }
-
-__global__ void copy_runs(const uint64_t* __restrict__ k, const uint32_t* __restrict__ l, const float* __restrict__ sc,
-                          const int64_t* __restrict__ n_dev, uint64_t* __restrict__ ko, uint32_t* __restrict__ lo,
-                          float* __restrict__ so) {
-    const int64_t n = *n_dev;
-    for (int64_t e = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; e < n; e += (int64_t)gridDim.x * blockDim.x) {
-        ko[e] = k[e];
-        lo[e] = l[e];
-        if (so && sc) so[e] = sc[e];
-    }
-}
-
-size_t unique_ws_bytes(int64_t cap) {
-    if (cap < 1) cap = 1;
-    return align_up(legacy_unique_ws_bytes(cap), 256) + carve_hash_ws(nullptr, cap).bytes;
-}
-
-int unique_reduce(const uint64_t* keys, const uint32_t* perm, const uint32_t* lens_in, const float* scores_in,
-                  const int64_t* n_dev, int64_t cap, uint64_t sentinel, uint64_t* out_keys, uint32_t* out_lens,
-                  float* out_scores, int64_t* n_out_dev, void* ws, cudaStream_t s) {
-    if (cap <= 0) {
-        DM_CUDA(cudaMemsetAsync(n_out_dev, 0, sizeof(int64_t), s));
-        return DM_OK;
-    }
-    Carver c(ws);
-    uint32_t* flags = c.take<uint32_t>(cap);
-    uint32_t* excl = c.take<uint32_t>(cap);
-    void* scan_ws = c.take<char>(scan_ws_bytes(cap));
-    const unsigned g = (unsigned)imin64(ceil_div(cap, 256), 148 * 8);
-    DM_CUDA(cudaMemsetAsync(out_lens, 0, (size_t)cap * sizeof(uint32_t), s));
-    DM_COUNT_LAUNCH(); unique_flags<<<g, 256, 0, s>>>(keys, n_dev, sentinel, flags);
-    DM_TRY(scan_exclusive_u32(flags, excl, n_dev, cap, n_out_dev, scan_ws, s));
-    DM_COUNT_LAUNCH(); unique_scatter<<<g, 256, 0, s>>>(keys, perm, lens_in, scores_in, n_dev, sentinel, flags, excl, out_keys, out_lens,
-                                     out_scores);
-    DM_LAUNCH_CHECK();
-    return DM_OK;
-}
-
-int sort_unique(uint64_t* keys, uint32_t* vals, const int64_t* n_dev, int64_t cap, int id_bits, int key_bits, void* sort_ws,
+int sort_unique(uint64_t* keys, uint32_t* vals, const int64_t* n_dev, int64_t cap, int id_bits, int key_bits, void* ws,
                 const uint32_t* gather_lens, const float* gather_scores, uint64_t sentinel, uint64_t* out_keys,
-                uint32_t* out_lens, float* out_scores, int64_t* n_out_dev, void* unique_ws, uint64_t* back_keys,
-                uint32_t* back_lens, float* back_scores, int64_t* back_n, cudaStream_t s, int64_t n_ids) {
+                uint32_t* out_lens, float* out_scores, int64_t* n_out_dev, uint64_t* back_keys, uint32_t* back_lens,
+                float* back_scores, int64_t* back_n, cudaStream_t s, int64_t n_ids) {
     if (cap <= 0) {
         DM_CUDA(cudaMemsetAsync(n_out_dev, 0, sizeof(int64_t), s));
         if (back_n) DM_CUDA(cudaMemsetAsync(back_n, 0, sizeof(int64_t), s));
         return DM_OK;
     }
     if (!vals || id_bits < 1 || id_bits > 32 || key_bits < 1 || key_bits > 2 * id_bits) return DM_ERR_BAD_ARG;
-    if (sort_fused_available()) {
-        const SortWs w = carve_sort_ws(sort_ws, cap);
-        FusedArgs A;
-        memset(&A, 0, sizeof(A));
-        A.k0 = keys; A.v0 = vals; A.k1 = w.k2; A.v1 = w.v2;
-        A.n_dev = n_dev; A.n_max = cap;
-        A.hist = w.hist; A.totals = w.totals; A.bar = w.bar;
-        A.id_bits = id_bits; A.passes = (key_bits + RADIX_BITS - 1) / RADIX_BITS; A.tiles_cap = (int)w.tiles;
-        A.do_unique = 1;
-        A.gather_lens = gather_lens; A.gather_scores = gather_lens ? gather_scores : nullptr;
-        A.sentinel = sentinel;
-        A.out_keys = out_keys; A.out_lens = out_lens; A.out_scores = out_scores; A.n_out = n_out_dev;
-        A.tile_heads = (uint32_t*)unique_ws;               // unique_ws_bytes(cap) >= tiles words
-        A.back_keys = back_keys; A.back_lens = back_lens; A.back_scores = back_scores; A.back_n = back_n;
-        // the hashed run reduction (no sort of the raw entries); it takes the radix path itself where it does not apply
-        const int hlimit = hashed_mode() ? hashed_grid_limit() : 0;
-        if (hlimit > 0 && n_ids > 0 && n_ids <= hash_ids_cap(cap) && key_bits == 2 * id_bits && cap < (1ll << 31)) {
-            const HashWs hw = carve_hash_ws((char*)unique_ws + align_up(legacy_unique_ws_bytes(cap), 256), cap);
-            HashArgs H;
-            memset(&H, 0, sizeof(H));
-            H.F = A;
-            H.tab = hw.tab; H.tab_cap_log2 = hash_tab_log2(cap);
-            H.deg = hw.deg; H.off = hw.off; H.cur = hw.cur; H.chunk_tot = hw.chunk_tot; H.hubs = hw.hubs; H.misc = hw.misc;
-            H.t_ent = hw.t_ent; H.t_bkt = hw.t_bkt;
-            H.n_ids = n_ids;
-            static const int grid_cap = getenv("DM_HASH_GRID") ? atoi(getenv("DM_HASH_GRID")) : 1 << 30;   // experiments
-            const int grid = (int)imax64(1, imin64(imin64(ceil_div(imax64(cap, n_ids), SORT_THREADS * 4), hlimit), grid_cap));
-            DM_CUDA(cudaMemsetAsync(A.bar, 0, 2 * sizeof(unsigned), s));
-            DM_CUDA(cudaMemsetAsync(H.misc, 0, 4 * sizeof(unsigned), s));
-            void* args[] = {(void*)&H};
-            DM_COUNT_LAUNCH();
-            if (cudaLaunchCooperativeKernel((const void*)edge_unique_hashed, dim3(grid), dim3(SORT_THREADS), args, 0, s) ==
-                cudaSuccess) {
-                static const bool print_ts = getenv("DM_HASH_TS") != nullptr;
-                if (print_ts) {                            // profiling aid: phase boundaries seen by block 0 (ns)
-                    unsigned long long t[6];
-                    cudaStreamSynchronize(s);
-                    cudaMemcpy(t, H.misc + 4, sizeof(t), cudaMemcpyDeviceToHost);
-                    fprintf(stderr, "edge_unique_hashed grid %d: clear %llu insert %llu offsets %llu buckets %llu rank %llu ns\n",
-                            grid, t[1] - t[0], t[2] - t[1], t[3] - t[2], t[4] - t[3], t[5] - t[4]);
-                }
-                return DM_OK;
-            }
-            (void)cudaGetLastError();
-        }
-        if (launch_fused(A, cap, s) == DM_OK) return DM_OK;
-        (void)cudaGetLastError();       // the cooperative launch was refused (e.g. no room for a co-resident grid
-                                        // under a profiler or a partitioned GPU): take the one-launch-per-phase path
-    }
-    // one launch per phase: n = min(*n_dev, cap) like the fused kernel (a raw list may have overflowed its capacity)
-    int64_t* n_clamped = (int64_t*)(carve_sort_ws(sort_ws, cap).bar + 2);
-    DM_COUNT_LAUNCH(); clamp_count<<<1, 1, 0, s>>>(n_dev, cap, n_clamped);
-    DM_TRY(sort_pairs(keys, vals, n_clamped, cap, id_bits, key_bits, sort_ws, s, false));
-    DM_TRY(unique_reduce(keys, gather_lens ? vals : nullptr, gather_lens ? gather_lens : vals,
-                         gather_lens ? gather_scores : nullptr, n_clamped, cap, sentinel, out_keys, out_lens, out_scores,
-                         n_out_dev, unique_ws, s));
-    if (back_keys) {
-        const unsigned g = (unsigned)imax64(1, imin64(ceil_div(cap, 256), (int64_t)num_sms() * 8));
-        DM_COUNT_LAUNCH(); copy_runs<<<g, 256, 0, s>>>(out_keys, out_lens, out_scores, n_out_dev, back_keys, back_lens, back_scores);
-        if (back_n) DM_CUDA(cudaMemcpyAsync(back_n, n_out_dev, sizeof(int64_t), cudaMemcpyDeviceToDevice, s));
-        DM_LAUNCH_CHECK();
+    HashArgs H = make_args(ws, cap, true, 0, keys, vals, n_dev, id_bits, key_bits, n_ids);
+    FusedArgs& A = H.F;
+    A.do_unique = 1;
+    A.gather_lens = gather_lens; A.gather_scores = gather_lens ? gather_scores : nullptr;
+    A.sentinel = sentinel;
+    A.out_keys = out_keys; A.out_lens = out_lens; A.out_scores = out_scores; A.n_out = n_out_dev;
+    A.back_keys = back_keys; A.back_lens = back_lens; A.back_scores = back_scores; A.back_n = back_n;
+    if (!(n_ids > 0 && n_ids <= hash_ids_cap(cap) && key_bits == 2 * id_bits && cap < (1ll << 31)))
+        return launch_radix(A, cap, s);
+    const int64_t limit = imin64(coop_grid_limit((const void*)edge_unique_hashed, HASH_BLOCKS_PER_SM), HASH_MAX_GRID);
+    const int64_t grid = imin64(ceil_div(imax64(cap, n_ids), SORT_THREADS * 4), limit);
+    void* args[] = {(void*)&H};
+    DM_TRY(launch_coop((const void*)edge_unique_hashed, grid, args, A.bar, H.misc, s));
+    static const bool print_ts = getenv("DM_HASH_TS") != nullptr;
+    if (print_ts) {                                        // profiling aid: phase boundaries seen by block 0 (ns)
+        unsigned long long t[6];
+        cudaStreamSynchronize(s);
+        cudaMemcpy(t, H.misc + 4, sizeof(t), cudaMemcpyDeviceToHost);
+        fprintf(stderr, "edge_unique_hashed grid %d: clear %llu insert %llu offsets %llu buckets %llu rank %llu ns\n",
+                (int)grid, t[1] - t[0], t[2] - t[1], t[3] - t[2], t[4] - t[3], t[5] - t[4]);
     }
     return DM_OK;
 }

@@ -19,41 +19,40 @@ size_t scan_ws_bytes(int64_t cap);
 int scan_exclusive_u32(const uint32_t* in, uint32_t* out, const int64_t* n_dev, int64_t cap,
                        int64_t* total_dev, void* ws, cudaStream_t s);
 
-size_t sort_ws_bytes(int64_t cap);
-// Stable sort of (keys, vals) in place by the low key_bits bits of the compacted key
-// ((hi32 << id_bits) | lo32); both 32-bit halves of every key must be < 2^id_bits.
-// key_bits = 2*id_bits sorts by (hi, lo); key_bits = id_bits sorts by lo only.  vals may be null.
-// allow_fused: the whole sort may run as ONE cooperative launch (persistent blocks + grid barriers); callers that
-// sort beside a kernel filling every SM (the pooling chain beside the raster pass) pass false.
-// n_ids > 0 (with key_bits = id_bits or 2 id_bits): the primary half of every key is an id < n_ids, and the sort may
-// run as bucket + rank in one cooperative launch (bucket_sort_fused in prims.cu).  csr_offsets / csr_ids (need
-// n_ids > 0 and a cooperative launch; DM_ERR_UNSUPPORTED otherwise, the caller then takes its own path): also
+// sort_pairs and sort_unique each run as ONE cooperative launch (persistent blocks meeting at grid barriers).  On a
+// device without cooperative launch they return DM_ERR_UNSUPPORTED; a refused launch is DM_ERR_CUDA with the CUDA
+// error recorded.  Which kernel runs depends on the input only.
+
+// Workspace of sort_pairs (unique = false) or sort_unique (unique = true; adds the tile heads and the hash table of
+// the run reduction) over `cap` pairs.  Its per-id arrays hold max(4 cap + 65536, n_ids) ids.
+size_t ws_bytes(int64_t cap, bool unique, int64_t n_ids = 0);
+
+// Stable sort of (keys, vals) in place by the low key_bits bits of the compacted key ((hi32 << id_bits) | lo32); both
+// 32-bit halves of every key must be < 2^id_bits.  key_bits = 2*id_bits sorts by (hi, lo); key_bits = id_bits sorts by
+// lo only.  n = min(*n_dev, cap) pairs; vals may be null; ws holds ws_bytes(cap, false, n_ids) bytes.
+// n_ids > 0 with key_bits = id_bits or 2 id_bits and cap < 2^31: the sort runs as bucket + rank (bucket_sort_fused in
+// prims.cu), one bucket per primary id (the lo half for id_bits, hi for 2 id_bits) below n_ids; it takes the radix
+// path inside the same launch when a bucket is too large or an id is >= n_ids.  Otherwise: the LSD radix sort
+// (radix_sort_fused).  csr_offsets / csr_ids need the bucket sort (DM_ERR_BAD_ARG otherwise): they also receive
 // offsets[id] = first sorted position of primary id `id`, for id < n_ids, and the sorted values as int32.
 int sort_pairs(uint64_t* keys, uint32_t* vals, const int64_t* n_dev, int64_t cap, int id_bits, int key_bits,
-               void* ws, cudaStream_t s, bool allow_fused = true, int64_t n_ids = 0, int64_t* csr_offsets = nullptr,
-               int32_t* csr_ids = nullptr);
-bool sort_fused_available();
-int sort_fused_mode();   // DM_SORT_FUSED: 0 off, 1 edge sorts, 2 (default) also the member sort of dm_merge_apply
+               void* ws, cudaStream_t s, int64_t n_ids = 0, int64_t* csr_offsets = nullptr, int32_t* csr_ids = nullptr);
 
-size_t unique_ws_bytes(int64_t cap);
-// keys sorted.  For every run of equal keys (runs of `sentinel` are dropped):
-//   out_keys[r] = key, out_lens[r] = sum lens_in[perm ? perm[i] : i],
-//   out_scores[r] = scores_in[perm ? perm[i] : i] of the run head (when scores_in != null).
-int unique_reduce(const uint64_t* keys, const uint32_t* perm, const uint32_t* lens_in, const float* scores_in,
-                  const int64_t* n_dev, int64_t cap, uint64_t sentinel, uint64_t* out_keys, uint32_t* out_lens,
-                  float* out_scores, int64_t* n_out_dev, void* ws, cudaStream_t s);
-
-// sort_pairs + unique_reduce (+ an optional copy of the reduced list over back_keys / back_lens / back_scores and
-// its length to back_n) -- one launch when the fused kernel is available.  n = min(*n_dev, cap) pairs are read.
-// gather_lens == null: the (sorted) values are the lengths.  Otherwise the values are a permutation and lengths /
-// scores are gathered through it (gather_lens[vals[i]], gather_scores[vals[i]]).
-int sort_unique(uint64_t* keys, uint32_t* vals, const int64_t* n_dev, int64_t cap, int id_bits, int key_bits, void* sort_ws,
+// Sort + run reduction of n = min(*n_dev, cap) pairs; ws holds ws_bytes(cap, true) bytes.  For every run of equal keys
+// (runs of `sentinel` are dropped), in ascending key order:
+//   out_keys[r] = key, out_lens[r] = sum of the run's lengths, out_scores[r] = score of the run's first pair;
+// *n_out_dev = number of runs.  gather_lens == null: the values are the lengths.  Otherwise the values are a
+// permutation and lengths / scores are gathered through it (gather_lens[vals[i]], gather_scores[vals[i]]; out_scores
+// is written when gather_scores is set).  back_keys / back_lens / back_scores / back_n (nullable): a copy of the
+// reduced list and its length, e.g. over the input arrays.  keys / vals are left sorted or untouched.
+// n_ids in (0, 4 cap + 65536] with key_bits = 2 id_bits and cap < 2^31: both halves of every key that is not the
+// sentinel are ids < n_ids, and the run reduction goes through a hash table + per-id buckets without sorting the raw
+// pairs (edge_unique_hashed in prims.cu), which takes the radix path inside the same launch when a bucket is too large
+// or an id is out of range.  Otherwise: the LSD radix sort of the pairs, then the reduction (radix_sort_fused).
+int sort_unique(uint64_t* keys, uint32_t* vals, const int64_t* n_dev, int64_t cap, int id_bits, int key_bits, void* ws,
                 const uint32_t* gather_lens, const float* gather_scores, uint64_t sentinel, uint64_t* out_keys,
-                uint32_t* out_lens, float* out_scores, int64_t* n_out_dev, void* unique_ws, uint64_t* back_keys,
-                uint32_t* back_lens, float* back_scores, int64_t* back_n, cudaStream_t s, int64_t n_ids = 0);
-// n_ids > 0: both halves of every key that is not the sentinel are ids < n_ids and only the reduced list is wanted
-// (keys / vals keep their contents): the run reduction may then go through a hash table + per-id buckets instead of
-// sorting the raw entries (edge_unique_hashed in prims.cu; DM_EDGE_HASH=0 switches it off).
+                uint32_t* out_lens, float* out_scores, int64_t* n_out_dev, uint64_t* back_keys, uint32_t* back_lens,
+                float* back_scores, int64_t* back_n, cudaStream_t s, int64_t n_ids = 0);
 
 // ---- device helpers -------------------------------------------------------------------
 

@@ -53,10 +53,6 @@ bool make_map_2d(CUtensorMap* m, const void* base, uint64_t dim0, uint64_t dim1,
     return r == CUDA_SUCCESS;
 }
 
-__global__ void clamp_count_kernel(const int64_t* raw, int64_t capacity, int64_t* out) {
-    *out = *raw < capacity ? *raw : capacity;
-}
-
 // DM_RAG_NO_TMA=1 forces the ld.global staging path (tests exercise both).
 static bool allow_tma_env() {
     const char* e = getenv("DM_RAG_NO_TMA");
@@ -75,17 +71,14 @@ extern "C" int dm_rag_last_encode_error(void) { return rag::last_encode_error();
 
 extern "C" size_t dm_rag_workspace_bytes(int64_t capacity) {
     const int64_t cap = capacity < 1 ? 1 : capacity;
-    return align_up((size_t)cap * 8, 256) + align_up((size_t)cap * 4, 256) + 256 + prims::sort_ws_bytes(cap) +
-           prims::unique_ws_bytes(cap);
+    return align_up((size_t)cap * 8, 256) + align_up((size_t)cap * 4, 256) + prims::ws_bytes(cap, true);
 }
 
 namespace {
 struct RagWs {
     uint64_t* raw_keys;
     uint32_t* raw_cnt;
-    int64_t* n_raw;
     void* sws;
-    void* uws;
 };
 RagWs carve_rag_ws(void* ws, int64_t capacity) {
     const int64_t cap = capacity < 1 ? 1 : capacity;
@@ -93,9 +86,7 @@ RagWs carve_rag_ws(void* ws, int64_t capacity) {
     RagWs w;
     w.raw_keys = c.take<uint64_t>(cap);
     w.raw_cnt = c.take<uint32_t>(cap);
-    w.n_raw = c.take<int64_t>(1);
-    w.sws = c.take<char>(prims::sort_ws_bytes(cap));
-    w.uws = c.take<char>(prims::unique_ws_bytes(cap));
+    w.sws = c.take<char>(prims::ws_bytes(cap, true));
     return w;
 }
 }  // namespace
@@ -149,14 +140,9 @@ extern "C" int dm_rag_finish(uint64_t* edge_keys, uint32_t* boundary_len, int64_
     cudaStream_t s = S(stream);
     RagWs w = carve_rag_ws(ws, capacity);
     const int b = bits_for(n_regions);
-    const int64_t* n_raw = counts + 1;                      // the fused kernel clamps to capacity itself
-    if (!prims::sort_fused_available()) {
-        // n_raw = min(raw entries, capacity): what actually sits in the raw list
-        DM_COUNT_LAUNCH(); rag::clamp_count_kernel<<<1, 1, 0, s>>>(counts + 1, capacity, w.n_raw);
-        n_raw = w.n_raw;
-    }
-    DM_TRY(prims::sort_unique(w.raw_keys, w.raw_cnt, n_raw, capacity, b, 2 * b, w.sws, nullptr, nullptr, ~0ull, edge_keys,
-                              boundary_len, nullptr, counts, w.uws, nullptr, nullptr, nullptr, nullptr, s, n_regions));
+    // counts[1] may exceed capacity (an overflowed raw list): sort_unique reads min(counts[1], capacity) entries
+    DM_TRY(prims::sort_unique(w.raw_keys, w.raw_cnt, counts + 1, capacity, b, 2 * b, w.sws, nullptr, nullptr, ~0ull,
+                              edge_keys, boundary_len, nullptr, counts, nullptr, nullptr, nullptr, nullptr, s, n_regions));
     DM_LAUNCH_CHECK();
     return DM_OK;
 }
@@ -225,8 +211,7 @@ extern "C" int dm_edges_concat(const uint64_t* src_keys, const uint32_t* src_len
 
 extern "C" size_t dm_edges_unique_workspace_bytes(int64_t capacity) {
     const int64_t cap = capacity < 1 ? 1 : capacity;
-    return align_up((size_t)cap * 8, 256) + align_up((size_t)cap * 4, 256) + 256 + prims::sort_ws_bytes(cap) +
-           prims::unique_ws_bytes(cap);
+    return align_up((size_t)cap * 8, 256) + align_up((size_t)cap * 4, 256) + 256 + prims::ws_bytes(cap, true);
 }
 
 extern "C" int dm_edges_sort_unique(uint64_t* keys, uint32_t* lens, const int64_t* n_in, int64_t capacity, int64_t n_regions,
@@ -243,10 +228,9 @@ extern "C" int dm_edges_sort_unique(uint64_t* keys, uint32_t* lens, const int64_
     uint64_t* ok = c.take<uint64_t>(capacity);
     uint32_t* ol = c.take<uint32_t>(capacity);
     int64_t* n_new = c.take<int64_t>(1);
-    void* sws = c.take<char>(prims::sort_ws_bytes(capacity));
-    void* uws = c.take<char>(prims::unique_ws_bytes(capacity));
+    void* sws = c.take<char>(prims::ws_bytes(capacity, true));
     const int b = bits_for(n_regions);
-    DM_TRY(prims::sort_unique(keys, lens, n_in, capacity, b, 2 * b, sws, nullptr, nullptr, ~0ull, ok, ol, nullptr, n_new, uws,
+    DM_TRY(prims::sort_unique(keys, lens, n_in, capacity, b, 2 * b, sws, nullptr, nullptr, ~0ull, ok, ol, nullptr, n_new,
                               keys, lens, nullptr, n_out, s, n_regions));
     DM_LAUNCH_CHECK();
     return DM_OK;

@@ -58,8 +58,9 @@ void dm_launch_count_add(int64_t n);  /* a host layer that replays a CUDA graph 
  * ----------------------------------------------------------------------------------- */
 
 /* Stable LSD radix sort of (key,value) pairs on the bit range implied by n_regions
- * (both 32-bit halves of an edge key are < n_regions).  n is read from n_dev[0] on the
- * device, capacity bounds it.  Sorted output is left in keys/vals. */
+ * (both 32-bit halves of an edge key are < n_regions), one cooperative launch.
+ * n = min(n_dev[0], capacity) is read on the device.  Sorted output is left in keys/vals
+ * (vals nullable).  DM_ERR_UNSUPPORTED on a device without cooperative launch. */
 size_t dm_sort_edges_workspace_bytes(int64_t capacity);
 int dm_sort_edges(uint64_t* keys, uint32_t* vals, const int64_t* n_dev, int64_t capacity,
                   int64_t n_regions, void* ws, size_t ws_bytes, dm_stream_t stream);
@@ -102,8 +103,9 @@ int dm_rag_build(const int32_t* labels, int64_t rows_own, int64_t rows_avail, in
  * the HBM-bound part) can be timed and profiled on its own:
  *   dm_rag_scan   zeroes counts, runs the fused raster kernel: accumulators updated, raw
  *                 per-CTA (key,count) entries appended inside the workspace, counts[1..3] set;
- *   dm_rag_finish radix sort + run reduction of the raw entries -> edge_keys/boundary_len,
- *                 counts[0].  Same ws / capacity as the scan call. */
+ *   dm_rag_finish run reduction of the raw entries (one cooperative launch, normally through a
+ *                 hash table and per-region buckets instead of a sort) -> ascending unique
+ *                 edge_keys, summed boundary_len, counts[0].  Same ws / capacity as the scan call. */
 int dm_rag_scan(const int32_t* labels, int64_t rows_own, int64_t rows_avail, int64_t W, int64_t ld,
                 const uint8_t* image, int64_t C, int64_t image_pitch, int64_t n_regions,
                 int top_border, int bottom_border,
@@ -150,6 +152,8 @@ int dm_perimeter(const uint64_t* edge_keys, const uint32_t* boundary_len, const 
  * ----------------------------------------------------------------------------------- */
 int dm_points_region(const int32_t* labels, int64_t H, int64_t W, int64_t ld, const int32_t* xs,
                      const int32_t* ys, int64_t n_points, int32_t* region_of_point, dm_stream_t stream);
+/* Grows with n_regions once n_regions + 1 exceeds 4 n_points + 65536 (per-region arrays of
+ * the bucket sort).  dm_csr_build: n_points <= INT32_MAX (point ids are int32). */
 size_t dm_csr_workspace_bytes(int64_t n_points, int64_t n_regions);
 int dm_csr_build(const int32_t* region_of_point, int64_t n_points, int64_t n_regions, int64_t* offsets,
                  int32_t* point_ids, void* ws, size_t ws_bytes, dm_stream_t stream);

@@ -52,6 +52,7 @@ def test_workspace_queries_are_pure(L):
     assert 0 < a < b
     assert L.dm_edges_rekey_workspace_bytes(1 << 20) > (1 << 20) * 8
     assert L.dm_csr_workspace_bytes(0, 5) > 0 and L.dm_merge_apply_workspace_bytes(0) > 0
+    assert L.dm_csr_workspace_bytes(1000, 10**6) > L.dm_csr_workspace_bytes(1000, 10)    # per-id arrays for every region
     assert L.dm_sort_edges_workspace_bytes(4096) > 4096 * 12
 
 

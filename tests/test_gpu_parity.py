@@ -105,6 +105,21 @@ def test_scan(cuda, n):
     assert int(tot.item()) == int(x.sum())
 
 
+@pytest.mark.parametrize("R,N,hub", [(500, 3000, 0), (200_000, 1_000, 0), (100, 20_000, 5_000)])
+def test_csr_build_matches_oracle(cuda, R, N, hub):
+    """Region -> point CSR (bucket sort with offsets) against the oracle.  The cases: random regions with invalid points;
+    many more regions than points (per-id arrays sized from the region count); one region holding `hub` points, above
+    the bucket sort's hub limit, so the radix path inside the same launch and its binary-search offsets run."""
+    from deepmerge_b200 import csr_from_region_of_point
+    rng = np.random.default_rng(R + N)
+    rop = rng.integers(-1, R, N).astype(np.int32)
+    rop[rng.choice(N, hub, replace=False)] = R // 2
+    off, ids = csr_from_region_of_point(T(rop, cuda), R)
+    ho, hi = o.csr_from_region_of_point(rop, R)
+    assert np.array_equal(off.cpu().numpy(), ho)
+    assert np.array_equal(ids.cpu().numpy()[: hi.size], hi)
+
+
 # ------------------------------------------------------------------------------------------
 # synthetic generator: device == oracle, bit for bit
 # ------------------------------------------------------------------------------------------

@@ -1,4 +1,4 @@
-"""Time the edge sort / sort+unique primitives alone (CUDA events), e.g. under DM_SORT_FUSED=0 and =1."""
+"""Time the edge sort / sort+unique primitives alone (CUDA events): tools/prof_sort.py [n [R [reps]]]."""
 import os, sys
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 import numpy as np
@@ -42,5 +42,4 @@ def timed(fn):
 t_sort = timed(lambda: L.check(L.dm_sort_edges(k.data_ptr(), v.data_ptr(), nd.data_ptr(), cap, R, ws.data_ptr(), wsb, s), "sort"))
 t_uniq = timed(lambda: L.check(L.dm_edges_sort_unique(k.data_ptr(), v.data_ptr(), nd.data_ptr(), cap, R, nout.data_ptr(),
                                                        ws.data_ptr(), wsb, s), "sort_unique"))
-print("DM_SORT_FUSED=%s n=%d R=%d: sort %.1f us, sort+unique %.1f us (%d unique)" % (
-    os.environ.get("DM_SORT_FUSED", "default"), n, R, t_sort, t_uniq, int(nout.item())))
+print("n=%d R=%d: sort %.1f us, sort+unique %.1f us (%d unique)" % (n, R, t_sort, t_uniq, int(nout.item())))
