@@ -628,3 +628,24 @@ def rasterize_polygons(polygons, geotransform, height, width, nodata=-1, ids=Non
         inside = np.cumsum(d, axis=1)[:, :-1] > 0
         out[r0:r1 + 1, c_lo:c_hi][inside] = label
     return out
+
+
+def write_polygonized(path, polys, geotransform, columns=None):
+    """Write the rings of a polygonized label raster (deepmerge_b200.polygonize -> Polygons) as a polygon shapefile:
+    one record per region present, in ascending id order, with the attributes REGION (the label id) and AREA (pixels)
+    and any `columns` = {field name: array indexed by region id} (e.g. MergeResult.perimeter).  A region made of several
+    pieces is one multi-ring record (label = record, as in rasterize_polygons), unlike gdal.Polygonize, which writes one
+    feature per connected piece."""
+    ids, rings = polys.shapes(geotransform)
+    base = path[:-4] if path.lower().endswith(".shp") else path
+    write_polygon_shp(base + ".shp", rings)
+    region = polys.ring_region.cpu().numpy().astype(np.int64)
+    area = np.zeros(int(ids.max()) + 1 if len(ids) else 0, np.int64)
+    np.add.at(area, region, polys.ring_area.cpu().numpy())
+    fields = [FieldDefn("REGION", "N", 11, 0), FieldDefn("AREA", "N", 18, 0)]
+    cols = {"REGION": ids, "AREA": area[ids]}
+    for name, values in (columns or {}).items():
+        a = np.asarray(values.cpu() if hasattr(values, "cpu") else values)[ids]
+        fields.append(FieldDefn(name, "N", 18, 0) if np.issubdtype(a.dtype, np.integer) else FieldDefn(name, OFTReal))
+        cols[name] = a
+    write_dbf(base + ".dbf", fields, cols)

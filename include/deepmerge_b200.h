@@ -388,6 +388,41 @@ int dm_region_bbox(const int32_t* labels, int64_t H, int64_t W, int64_t ld, int6
                    int64_t* bad_label, dm_stream_t stream);
 
 /* ----------------------------------------------------------------------------------- *
+ * Polygonize a label raster: the way back from a merged label map to the polygons of the reference's tile.shp (one
+ * polygon per segment).  Not part of the merge step.
+ *
+ * labels int32 [H, ld] (ld >= W); negative labels are nodata and get no polygon; a label >= n_regions sets status 1.
+ *  - Rings: every region present gets its boundary as closed rings of pixel-corner vertices, int32 (x, y) with
+ *    x in [0, W], y in [0, H].  A boundary side is a pixel side facing another label, nodata or the image border
+ *    (the sides dm_rag_build counts in the perimeter).
+ *  - Connectivity: regions are 4-connected.  At a saddle vertex (a 2 x 2 block with the same label on one diagonal
+ *    only) each region's ring turns so that it stays on its own pixel, so diagonal pixels are never joined.  A ring may
+ *    touch itself or another ring of its region at such a vertex.
+ *  - Orientation: in pixel coordinates (y down) the region lies on the right of the direction of travel: outer rings
+ *    have positive shoelace area 1/2 sum(x_i y_{i+1} - x_{i+1} y_i), holes negative; the sum over a region's rings is
+ *    its pixel count.
+ *  - Vertices: corners only (the direction changes at every vertex), the ring is not explicitly closed; every ring has
+ *    an even number >= 4 of vertices and its edges alternate between horizontal and vertical.
+ *  - Canonical form (deterministic): each ring starts at its smallest vertex in (y, x) order, which a ring passes only
+ *    once; rings are ordered by (region id, start y, start x), a total order.
+ * Outputs (device, caller-owned), with ring_cap = capacity / 4 (a ring has at least 4 boundary sides, and at most one
+ * vertex per side):
+ *    ring_region  int32 [ring_cap]          ring_offsets int64 [ring_cap + 1] (into vertices)
+ *    ring_area    int64 [ring_cap] (signed, pixels)    vertices int32 [capacity, 2]
+ *    region_rings int64 [n_regions + 1]: rings of region r are [region_rings[r], region_rings[r + 1])
+ *    counts int64 [4]: [0] rings, [1] vertices, [2] boundary sides found (exact, also above capacity),
+ *           [3] status: 0 ok, 1 a label >= n_regions, 2 capacity exceeded (outputs invalid; retry with
+ *           capacity >= counts[2]).
+ * capacity bounds the boundary sides, < 2^31.  (H + 1) (W + 1) <= 2^32.  The workspace grows with H W / 4 bytes, the
+ * capacity and n_regions (per-region arrays of the ring sort).  The empty raster writes zero counts (when the outputs
+ * are given) and returns 0.
+ * ----------------------------------------------------------------------------------- */
+size_t dm_polygonize_workspace_bytes(int64_t H, int64_t W, int64_t n_regions, int64_t capacity);
+int dm_polygonize(const int32_t* labels, int64_t H, int64_t W, int64_t ld, int64_t n_regions, int64_t capacity,
+                  int32_t* ring_region, int64_t* ring_offsets, int64_t* ring_area, int32_t* vertices,
+                  int64_t* region_rings, int64_t* counts, void* ws, size_t ws_bytes, dm_stream_t stream);
+
+/* ----------------------------------------------------------------------------------- *
  * R11 Contrastive pair loss forward + backward (Losses.py:34-38):
  *     d = sum_k (a-b)^2 ; L = mean(flag*d + (1-flag)*relu(margin-d)).
  *     loss fp32 [1]; grad_a, grad_b fp32 [B,D] (nullable).  flag int64 as collated.
