@@ -529,14 +529,6 @@ __global__ void slots_word_max_kernel(const unsigned char* __restrict__ slots, i
     if (threadIdx.x == 0) *out = m;
 }
 
-__global__ void any_diff_kernel(const int32_t* __restrict__ a, const int32_t* __restrict__ b, int64_t n,
-                                int64_t* __restrict__ flag) {
-    bool d = false;
-    for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (int64_t)gridDim.x * blockDim.x)
-        d |= a[i] != b[i];
-    if (__any_sync(0xffffffffu, d) && (threadIdx.x & 31) == 0) *flag = 1;
-}
-
 }  // namespace merge
 }  // namespace dm
 
@@ -644,17 +636,6 @@ extern "C" int dm_slots_word_max(const void* slots, int64_t n_slots, int64_t slo
     if (n_slots > 0 && !slots) return DM_ERR_BAD_ARG;
     DM_COUNT_LAUNCH(); merge::slots_word_max_kernel<<<1, 32, 0, S(stream)>>>((const unsigned char*)slots, (int)n_slots, slot_bytes, word_offset,
                                                                        out_dev);
-    DM_LAUNCH_CHECK();
-    return DM_OK;
-}
-
-extern "C" int dm_any_diff_i32(const int32_t* a, const int32_t* b, int64_t n, int64_t* flag_dev, dm_stream_t stream) {
-    if (n < 0 || !flag_dev) return DM_ERR_BAD_ARG;
-    cudaStream_t s = S(stream);
-    DM_CUDA(cudaMemsetAsync(flag_dev, 0, sizeof(int64_t), s));
-    if (n == 0) return DM_OK;
-    if (!a || !b) return DM_ERR_BAD_ARG;
-    DM_COUNT_LAUNCH(); merge::any_diff_kernel<<<grid_for(n), 256, 0, s>>>(a, b, n, flag_dev);
     DM_LAUNCH_CHECK();
     return DM_OK;
 }
@@ -777,8 +758,6 @@ extern "C" size_t dm_merge_apply_workspace_bytes(int64_t R) {
     const int64_t cap = R < 1 ? 1 : R;
     return align_up((size_t)cap * 8, 256) + prims::ws_bytes(cap, false) + 512;
 }
-
-extern "C" size_t dm_merge_apply_workspace_bytes(int64_t R);
 
 extern "C" int dm_merge_apply_masked(const int32_t* parent, uint8_t* alive, uint8_t* changed, float* sum, int32_t* cnt,
                                      int64_t* area, int64_t* perimeter, int64_t R, int64_t D, int64_t* n_merged,

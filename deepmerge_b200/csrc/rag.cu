@@ -53,14 +53,6 @@ bool make_map_2d(CUtensorMap* m, const void* base, uint64_t dim0, uint64_t dim1,
     return r == CUDA_SUCCESS;
 }
 
-// DM_RAG_NO_TMA=1 forces the ld.global staging path (tests exercise both).
-static bool allow_tma_env() {
-    const char* e = getenv("DM_RAG_NO_TMA");
-    return !(e && e[0] == '1');
-}
-
-int run(const Params& P, int C, cudaStream_t s) { return run_blocks(P, C, allow_tma_env(), s); }
-
 }  // namespace rag
 }  // namespace dm
 
@@ -128,7 +120,7 @@ extern "C" int dm_rag_scan(const int32_t* labels, int64_t rows_own, int64_t rows
     P.capacity = capacity;
     P.counters = (unsigned long long*)counts;
     P.tiles_x = P.tiles_y = P.tiles_per_cta = 0;
-    return rag::run(P, (int)C, s);
+    return rag::run_blocks(P, (int)C, s);
 }
 
 extern "C" int dm_rag_finish(uint64_t* edge_keys, uint32_t* boundary_len, int64_t capacity, int64_t n_regions,

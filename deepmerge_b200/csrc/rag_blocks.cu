@@ -335,7 +335,7 @@ rag_blocks_kernel(const __grid_constant__ CUtensorMap mapL, const __grid_constan
 }
 
 template <typename CF>
-static int launch(const Params& Pin, bool allow_tma, cudaStream_t s) {
+static int launch(const Params& Pin, cudaStream_t s) {
     Params P = Pin;
     P.tiles_x = (int)ceil_div(P.W, STRIP_W);            // strips
     P.tiles_y = (int)ceil_div(P.rows_avail, CF::TH);    // units per strip (a halo row below counts)
@@ -352,7 +352,7 @@ static int launch(const Params& Pin, bool allow_tma, cudaStream_t s) {
     memset(&mapL, 0, sizeof(mapL));
     memset(&mapI, 0, sizeof(mapI));
     // TMA needs 16-byte aligned bases and row pitches; anything else takes the ld.global staging path
-    bool tma = allow_tma && ((uintptr_t)P.labels % 16 == 0) && ((P.ld * 4) % 16 == 0) && P.ld >= P.W;
+    bool tma = ((uintptr_t)P.labels % 16 == 0) && ((P.ld * 4) % 16 == 0) && P.ld >= P.W;
     if (CF::C > 0)
         tma = tma && ((uintptr_t)P.image % 16 == 0) && (P.image_pitch % 16 == 0) && (((int64_t)P.W * CF::C) % 4 == 0);
     if (tma)
@@ -377,24 +377,14 @@ static int launch(const Params& Pin, bool allow_tma, cudaStream_t s) {
 }  // namespace blk
 
 // Kernel shapes per band count: <bands, rows per stage, stages, warps per CTA, item capacity>.
-// DM_RAG_CFG selects one of the alternative shapes of the 4-band kernel (measurement only).
-int run_blocks(const Params& P, int C, bool allow_tma, cudaStream_t s) {
+int run_blocks(const Params& P, int C, cudaStream_t s) {
     using namespace blk;
     switch (C) {
-        case 0: return launch<Cfg<0, 8, 2, 14, 48>>(P, allow_tma, s);
-        case 1: return launch<Cfg<1, 4, 2, 16, 48>>(P, allow_tma, s);
-        case 2: return launch<Cfg<2, 4, 2, 14, 48>>(P, allow_tma, s);
-        case 3: return launch<Cfg<3, 4, 2, 12, 48>>(P, allow_tma, s);
-        case 4: {
-            const char* e = getenv("DM_RAG_CFG");
-            const int v = e ? atoi(e) : 0;
-            switch (v) {
-                case 1: return launch<Cfg<4, 4, 2, 10, 64>>(P, allow_tma, s);
-                case 2: return launch<Cfg<4, 4, 3, 9, 48>>(P, allow_tma, s);
-                case 3: return launch<Cfg<4, 8, 2, 8, 48>>(P, allow_tma, s);
-                default: return launch<Cfg<4, 4, 2, 12, 48>>(P, allow_tma, s);
-            }
-        }
+        case 0: return launch<Cfg<0, 8, 2, 14, 48>>(P, s);
+        case 1: return launch<Cfg<1, 4, 2, 16, 48>>(P, s);
+        case 2: return launch<Cfg<2, 4, 2, 14, 48>>(P, s);
+        case 3: return launch<Cfg<3, 4, 2, 12, 48>>(P, s);
+        case 4: return launch<Cfg<4, 4, 2, 12, 48>>(P, s);
         default: return DM_ERR_BAD_ARG;
     }
 }

@@ -83,7 +83,7 @@ __device__ __forceinline__ void tma_load_2d(void* dst, const CUtensorMap* map, i
 bool make_map_2d(CUtensorMap* m, const void* base, uint64_t dim0, uint64_t dim1, uint64_t pitch_bytes, uint32_t box0,
                  uint32_t box1);
 void set_last_path(int path);
-int run_blocks(const Params& P, int C, bool allow_tma, cudaStream_t s);   // rag_blocks.cu
+int run_blocks(const Params& P, int C, cudaStream_t s);   // rag_blocks.cu
 
 }  // namespace rag
 }  // namespace dm

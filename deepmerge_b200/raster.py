@@ -9,7 +9,6 @@ signed view orders like the unsigned key).
 """
 from __future__ import annotations
 
-import os
 from dataclasses import dataclass
 from typing import Optional, Sequence
 
@@ -357,6 +356,11 @@ class PackedMLP:
             raise RuntimeError("pair-MLP kernel: a bounded wait expired (lost TMA / tensor-core signal); outputs are invalid")
 
 
+def _check_pair_mlp(mlp, D):
+    if mlp is not None and mlp.in_features != 2 * D:
+        raise ValueError("the pair-MLP takes concat(mean[lo], mean[hi]): in_features must be 2 D")
+
+
 def score_mlp(mean, edge_keys, mlp: PackedMLP, want_h2=False, n_edges_dev=None, out=None, check=False):
     """Pair-MLP scores of every edge: x_e = concat(mean[lo], mean[hi]) through the three
     Linear + leaky_relu layers of Nets.MLP.forward (Nets.py:28-35), bf16 operands / fp32
@@ -367,8 +371,7 @@ def score_mlp(mean, edge_keys, mlp: PackedMLP, want_h2=False, n_edges_dev=None, 
     if mean.dtype != _F32 or not mean.is_contiguous():
         raise ValueError("mean must be a contiguous float32 [R, D] tensor")
     R, D = mean.shape
-    if mlp.in_features != 2 * D:
-        raise ValueError("the pair-MLP takes concat(mean[lo], mean[hi]): in_features must be 2 D")
+    _check_pair_mlp(mlp, D)
     dev = mean.device
     E = edge_keys.shape[0]
     o = out if out is not None else torch.empty((E, mlp.n_out), dtype=_F32, device=dev)
@@ -456,15 +459,13 @@ class MergeEngine:
         self.H, self.W, self.R, self.D, self.C, self.N = int(H), int(W), int(n_regions), int(D), int(C), int(n_points)
         self.cap = default_edge_capacity(n_regions, H, W) if edge_capacity is None else int(edge_capacity)
         self.logits = None
-        self._means_fresh = self._init_fresh = False     # run() prepares both beside the raster pass
-        self.use_graphs = os.environ.get("DM_GRAPHS", "1") != "0"
-        self._round_graphs = {}
+        self.use_graphs = True                           # False once a capture was refused: plain launches from then on
         self.pool_id_range, self.id_range = False, None  # a row tile's engine (sharded.py) pools only the id interval of its points
         self._alloc()
 
     def _alloc(self):
         L, dev, R, D, C, N, cap = self.L, self.dev, self.R, self.D, self.C, self.N, self.cap
-        self._round_graphs = {}                           # captured round bodies point into the buffers below
+        self._graphs = {}                                 # captured round bodies point into the buffers below
         z = lambda *s, dt: torch.zeros(*s, dtype=dt, device=dev)
         e = lambda *s, dt: torch.empty(*s, dtype=dt, device=dev)
         with torch.cuda.device(dev):
@@ -510,8 +511,9 @@ class MergeEngine:
         L.check(L.dm_perimeter(_p(self.keys), _p(self.blen), _p(self.counts), self.cap, _p(self.border), _p(self.perim),
                                self.R, s), "dm_perimeter")
 
-    def _pool(self, labels, xs, ys, region_of_point, feats, with_mean=False):
-        """membership -> CSR -> per-region sums (-> means and norms in the same pass when with_mean and D <= 128)"""
+    def _pool(self, labels, xs, ys, region_of_point, feats):
+        """membership -> CSR -> per-region sums, and for a whole raster the means and norms (in the same pass when
+        D <= 128).  A row tile's engine leaves the means to the sharded loop: they need the other tiles' partial sums."""
         L, s = self.L, _stream()
         N = feats.shape[0]
         if N > self.N:
@@ -522,11 +524,10 @@ class MergeEngine:
             region_of_point = self.rop
         L.check(L.dm_csr_build(_p(region_of_point), N, self.R, _p(self.offsets), _p(self.pids), _p(self.ws_pool),
                                self.ws_pool_bytes, s), "dm_csr_build")
-        if with_mean and not self.pool_id_range and self.D <= 128 and os.environ.get("DM_POOL_MEAN", "1") != "0":
+        if not self.pool_id_range and self.D <= 128:
             L.check(L.dm_pool_points_csr_mean(_p(self.offsets), _p(self.pids), _p(feats), feats.stride(0), self.R, self.D,
                                               _p(self.sum), _p(self.cnt), _p(self.mean), _p(self.norm2), s),
                     "dm_pool_points_csr_mean")
-            self._means_fresh = True
             return
         rng = None
         if self.pool_id_range:          # a row tile's engine: only the id interval that holds the tile's points is visited
@@ -536,12 +537,13 @@ class MergeEngine:
             rng = self.id_range
         L.check(L.dm_pool_points_csr_tile(_p(self.offsets), _p(self.pids), _p(feats), feats.stride(0), self.R, self.D,
                                           _p(self.sum), _p(self.cnt), _p(rng), s), "dm_pool_points_csr_tile")
+        if not self.pool_id_range:
+            self._mean_all()
 
     def _mean_all(self):
         L = self.L
         L.check(L.dm_region_mean(_p(self.sum), _p(self.cnt), self.R, self.D, _p(self.mean), _p(self.norm2), None, _stream()),
                 "dm_region_mean")
-        self._means_fresh = True
 
     def _read_counts(self, after_enqueue=None):
         """The loop's host read-back; after_enqueue() is called between the enqueue of the copy and the wait for it."""
@@ -569,6 +571,8 @@ class MergeEngine:
 
     def merge_loaded_graph(self, tau, max_rounds=64, mlp=None):
         with torch.cuda.device(self.dev):
+            self._merge_init(mlp)
+            self._mean_all()
             rounds, merges = self._merge_loop(tau, max_rounds, mlp)
             E = int(self.host_counts[0])
         return MergeResult(None, self.parent, rounds, merges, self.keys[:E], self.blen[:E], self.scores[:E], self.area,
@@ -589,10 +593,8 @@ class MergeEngine:
                 cur = torch.cuda.current_stream(self.dev)
                 self.side.wait_stream(cur)
                 with torch.cuda.stream(self.side):
-                    self._merge_init()
-                    self._pool(labels, xs, ys, region_of_point, feats, with_mean=True)
-                    if not self._means_fresh:
-                        self._mean_all()
+                    self._merge_init(mlp)
+                    self._pool(labels, xs, ys, region_of_point, feats)
                 self._rag(labels, image, rows_own, top_border, bottom_border)
                 cur.wait_stream(self.side)
                 # The relabel is enqueued behind every selection, right AFTER the copy of the counters the host waits for and
@@ -604,11 +606,8 @@ class MergeEngine:
                     self.L.check(self.L.dm_relabel_gated(_p(labels), own, self.W, labels.stride(0), _p(self.parent), self.R,
                                                          _p(self.out), self.W, None if force else self.counts[4:5].data_ptr(),
                                                          _stream()), "dm_relabel_gated")
-                gated = relabel and os.environ.get("DM_GATED_RELABEL", "1") != "0"
                 try:
-                    rounds, merges = self._merge_loop(tau, max_rounds, mlp, after_read=gated_relabel if gated else None)
-                    if relabel and not gated:
-                        gated_relabel(True)
+                    rounds, merges = self._merge_loop(tau, max_rounds, mlp, after_read=gated_relabel if relabel else None)
                     break
                 except OverflowError as ov:            # raw edge list outgrew the capacity: resize, rerun
                     self.cap = int(ov.args[0]) + 1024
@@ -637,24 +636,15 @@ class MergeEngine:
     def mlp_status_shift(mlp):
         return mlp.status.to(_I64) << 1                            # counts[3]: 1 = bad label, >= 2 = internal error
 
-    def _merge_init(self):
-        """parent = identity, everything alive, round counters zero (run() does this beside the raster pass)."""
+    def _merge_init(self, mlp=None):
+        """A new merge loop: the pair-MLP (if any) must fit D; parent = identity, everything alive, round counters zero."""
+        _check_pair_mlp(mlp, self.D)
         self.parent.copy_(self.iota)
         self.alive.fill_(1)
         self.counts[5:8].zero_()
-        self._init_fresh = True
 
     def _merge_loop(self, tau, max_rounds, mlp=None, after_read=None):
-        L, s, R, D, cap = self.L, _stream(), self.R, self.D, self.cap
-        n_edges = self.counts[0:1]
-        if mlp is not None and mlp.in_features != 2 * D:
-            raise ValueError("the pair-MLP takes concat(mean[lo], mean[hi]): in_features must be 2 D")
-        if not self._init_fresh:
-            self._merge_init()
-        self._init_fresh = False
-        if not self._means_fresh:                         # run() computes them on the side stream right after the pooling
-            self._mean_all()
-        self._means_fresh = False
+        """The merge rounds; the caller has run _merge_init and computed the means of the initial graph."""
         self._score(mlp, None)
         self._select(tau, mlp)
         rounds = merges = 0
@@ -673,7 +663,7 @@ class MergeEngine:
             if c[4] == 0 or rounds == max_rounds:
                 break
             rounds += 1
-            self._round(tau, mlp)
+            self._graph_launch(lambda: self._round_body(tau, mlp), tau, mlp)
         return rounds, merges
 
     def _select(self, tau, mlp):
@@ -686,52 +676,60 @@ class MergeEngine:
             L.check(L.dm_merge_select_mlp(_p(self.logits), mlp.n_out, _p(n_edges), cap, _p(self.selected),
                                           self.counts[4:5].data_ptr(), s), "dm_merge_select_mlp")
 
-    def _round_body(self, tau, mlp):
-        """One merge round between two read-backs: unions of the selected edges, merged statistics, re-keyed edge list,
-        means and scores of what changed, the next selection."""
+    def _apply_and_rescore(self, mlp, root_mask=None):
+        """The part of a round after the unions: merged statistics, re-keyed edge list, means and scores of what changed.
+        root_mask (a row tile's engine): embedding sums are merged only for the components it flags."""
         L, s, R, D, cap = self.L, _stream(), self.R, self.D, self.cap
-        n_edges = self.counts[0:1]
-        L.check(L.dm_uf_union(_p(self.parent), _p(self.keys), _p(self.selected), _p(n_edges), cap, s), "dm_uf_union")
-        L.check(L.dm_uf_compress(_p(self.parent), R, s), "dm_uf_compress")
         # merged statistics (side stream) and edge re-keying (main stream) only share the parent array and integer
         # atomics on the perimeter: two chains of small kernels that fill the GPU better together
         cur = torch.cuda.current_stream(self.dev)
         self.side.wait_stream(cur)
         with torch.cuda.stream(self.side):
-            L.check(L.dm_merge_apply(_p(self.parent), _p(self.alive), _p(self.changed), _p(self.sum), _p(self.cnt),
-                                     _p(self.area), _p(self.perim), R, D, self.counts[5:6].data_ptr(), _p(self.ws_side),
-                                     self.ws_side_bytes, _stream()), "dm_merge_apply")
-        L.check(L.dm_edges_rekey(_p(self.parent), _p(self.keys), _p(self.blen), _p(self.scores), _p(n_edges), cap, R,
-                                 _p(self.perim), _p(self.ws), self.ws_bytes, s), "dm_edges_rekey")
+            L.check(L.dm_merge_apply_masked(_p(self.parent), _p(self.alive), _p(self.changed), _p(self.sum), _p(self.cnt),
+                                            _p(self.area), _p(self.perim), R, D, self.counts[5:6].data_ptr(), _p(root_mask),
+                                            _p(self.ws_side), self.ws_side_bytes, _stream()), "dm_merge_apply_masked")
+        L.check(L.dm_edges_rekey(_p(self.parent), _p(self.keys), _p(self.blen), _p(self.scores), _p(self.counts[0:1]), cap,
+                                 R, _p(self.perim), _p(self.ws), self.ws_bytes, s), "dm_edges_rekey")
         cur.wait_stream(self.side)
         L.check(L.dm_region_mean(_p(self.sum), _p(self.cnt), R, D, _p(self.mean), _p(self.norm2), _p(self.changed), s),
                 "dm_region_mean")
         self._score(mlp, self.changed)
+
+    def _round_body(self, tau, mlp):
+        """One merge round between two read-backs: unions of the selected edges, merged statistics, re-keyed edge list,
+        means and scores of what changed, the next selection."""
+        L, s = self.L, _stream()
+        L.check(L.dm_uf_union(_p(self.parent), _p(self.keys), _p(self.selected), _p(self.counts[0:1]), self.cap, s),
+                "dm_uf_union")
+        L.check(L.dm_uf_compress(_p(self.parent), self.R, s), "dm_uf_compress")
+        self._apply_and_rescore(mlp)
         self._select(tau, mlp)
 
-    def _round(self, tau, mlp):
-        """The round body as ONE CUDA graph launch (it only touches the engine's own buffers, so a captured body is valid
-        until they are re-allocated): a round is a dozen short kernels whose launch gaps otherwise show.  DM_GRAPHS=0:
-        plain launches."""
+    def _graph_launch(self, body, tau, mlp, *key):
+        """Runs a round body as ONE CUDA graph launch: a round is a dozen (sharded: ~35) short kernels whose launch gaps
+        otherwise show.  The body only touches the engine's own buffers, so it is captured once per (tau, mlp, capacity,
+        *key) and replayed until _alloc re-allocates them.  Returns what the captured body returned.  A refused capture
+        (driver / library in use) switches to plain launches from then on: the same kernels in the same order."""
         if not self.use_graphs:
-            return self._round_body(tau, mlp)
-        key = (float(tau), None if mlp is None else (id(mlp), mlp.blob.data_ptr()), self.cap)
-        ent = self._round_graphs.get(key)
+            return body()
+        key = (float(tau), None if mlp is None else (id(mlp), mlp.blob.data_ptr()), self.cap) + key
+        ent = self._graphs.get(key)
         if ent is None:
             g = torch.cuda.CUDAGraph()
             n0 = self.L.dm_launch_count()
             try:
                 with torch.cuda.graph(g, capture_error_mode="thread_local"):
-                    self._round_body(tau, mlp)
-            except Exception:                      # capture refused (driver / library in use): plain launches from now on
+                    out = body()
+            except Exception:
                 self.use_graphs = False
-                return self._round_body(tau, mlp)
-            ent = (g, self.L.dm_launch_count() - n0)
-            if len(self._round_graphs) >= 8:
-                self._round_graphs.clear()
-            self._round_graphs[key] = ent
+                return body()
+            ent = (g, self.L.dm_launch_count() - n0, out)
+            if len(self._graphs) >= 8:
+                self._graphs.clear()
+            self._graphs[key] = ent
         ent[0].replay()
         self.L.dm_launch_count_add(ent[1])          # the library's counter saw the capture only
+        return ent[2]
 
 
 class ScenePipeline:

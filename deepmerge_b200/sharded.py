@@ -10,24 +10,29 @@ in-process stand-in of the tests).
     selects, re-keys and uniques only those;
   * per-region small state is replicated: the parent array (int32 [R]), point counts, the alive /
     changed flags and a rank-visibility bit mask (bit g = rank g sees the region: it has pixels
-    or an edge of it).  Each round the local unions are merged with all_reduce(min) of the
-    parent array + re-union until nothing changes;
+    or an edge of it).  A component can span two tiles only through a region both ranks see, so
+    after its local unions a rank publishes (shared region, local root) pairs -- the frontier --
+    and every rank unites all ranks' pairs into its own forest; one all-reduce(MIN) of the parent
+    array then fills in the regions a rank does not see.  No iteration, no convergence test;
   * embedding sums [R, D] are NOT replicated: a rank holds the rows of the regions it sees.  Rows
     travel sparsely: once for the regions seen by two ranks (their per-tile partial sums are
     added in rank order), and per round for the members of components that grew across a tile
     border (shipped by the lowest rank that held the row), as fixed-capacity slots with
-    device-side counts (dm_rows_pack / all_gather_into_tensor / dm_rows_unpack);
+    device-side counts (dm_rows_pack / exchange / dm_rows_unpack);
   * area / border / perimeter / band sums stay per-tile partials through the loop (every update
     is linear) and are all-reduced once at the end together with the gathered final edge list.
 Integer outputs are bit-identical to the single-GPU result; the fp32 sums of regions whose points
 lie in two tiles are added in rank order instead of point order (last-bit differences).
 
-`ShardedMergeEngine.run_replicated` is the earlier scheme (global graph replicated on every rank).
+Transport: under torch.distributed over NCCL, when the symmetric-memory rendezvous succeeds, the
+slots are exchanged by peer stores of this library's kernels (PeerSlots) and the two replicated
+R-sized arrays are all-reduced by its peer kernels (PeerArray), so a step calls no collective and
+the round body is one CUDA graph launch.  Otherwise (gloo, the tests' in-process stand-in, a box
+without peer access) slots travel by all_gather_into_tensor and the arrays by all_reduce.
 """
 from __future__ import annotations
 
 import json
-import os
 import time
 from typing import Optional
 
@@ -147,11 +152,7 @@ class PeerArray:
 
 
 def _peer_exchange_possible(dist):
-    """Symmetric memory needs the real torch.distributed over NCCL (one process per GPU); DM_SHARD_PEER=0 forces the
-    collective path."""
-    import os
-    if os.environ.get("DM_SHARD_PEER", "1") == "0":
-        return False
+    """Symmetric memory needs the real torch.distributed over NCCL (one process per GPU)."""
     try:
         import torch.distributed as td
         return dist is td and td.is_initialized() and td.get_backend() == "nccl"
@@ -162,12 +163,12 @@ def _peer_exchange_possible(dist):
 class ShardedMergeEngine:
     """One rank's share of a scene sharded by rows.  Wraps a MergeEngine sized for the tile.
 
-    A step makes no host round trip before the merge loop's own read-back: the per-tile edge lists
+    A step makes no host round trip before the merge loop's own read-back: rows and frontier pairs
     travel as fixed-capacity slots together with their device-side counts, and overflow / bad-label
     flags of the tile pass are checked with that first read-back."""
 
-    def __init__(self, H, W, n_regions, D, C, n_points_local, dist, device, group=None, slot_capacity=None,
-                 row_capacity=None, edge_capacity=None, replicated=False):
+    def __init__(self, H, W, n_regions, D, C, n_points_local, dist, device, group=None, row_capacity=None,
+                 edge_capacity=None):
         from .raster import MergeEngine, default_edge_capacity
         self.dist, self.group = dist, group
         self.world, self.rank = dist.get_world_size(group), dist.get_rank(group)
@@ -180,16 +181,12 @@ class ShardedMergeEngine:
         self.has_halo = self.rank < self.world - 1
         # capacity: the raw per-tile entries of THIS tile must fit (an even share of the regions plus 50 %; a scene
         # whose regions crowd into one tile needs edge_capacity=...).  Kernel grids of the graph stages are sized by it.
-        from .raster import default_edge_capacity
-        glob_cap = default_edge_capacity(n_regions, H, W)
         cap = int(edge_capacity) if edge_capacity else min(
-            glob_cap, default_edge_capacity(int(1.5 * n_regions / self.world) + 1024, self.rows_own + 1, W))
-        self.slot_cap = int(slot_capacity) if slot_capacity else glob_cap // self.world + 4 * W + 4096   # run_replicated only
-        self.eng = MergeEngine(self.rows_own, W, n_regions, D, C=C, n_points=n_points_local,
-                               edge_capacity=glob_cap if replicated else cap, device=device)   # run_replicated holds the global list
-        dev = self.eng.dev
-        self.tile_counts = torch.zeros(4, dtype=torch.int64, device=dev)
-        self.cat_counts = torch.zeros(2, dtype=torch.int64, device=dev)
+            default_edge_capacity(n_regions, H, W),
+            default_edge_capacity(int(1.5 * n_regions / self.world) + 1024, self.rows_own + 1, W))
+        self.eng = MergeEngine(self.rows_own, W, n_regions, D, C=C, n_points=n_points_local, edge_capacity=cap,
+                               device=device)
+        self.cat_counts = torch.zeros(2, dtype=torch.int64, device=self.eng.dev)
 
     # ------------------------------------------------------------------------------------------------
     # distributed merge loop
@@ -224,22 +221,22 @@ class ShardedMergeEngine:
         self.fslot = z(self.fslot_bytes, dt=torch.uint8)
         self.fslot_flags = self.fslot[16:80].view(torch.int64)
         self.flags = z(8, dt=torch.int64)
+        # peer transport: both slot exchanges, and the two replicated R-sized arrays in symmetric memory so that their
+        # all-reduces are peer kernels -- all four or none
         self.peer_rows = self.peer_pairs = self.peer_mask_cnt = self.peer_parent = None
         if _peer_exchange_possible(self.dist):
             try:
-                self.peer_rows = PeerSlots(self.dist, self.group, self.slot_bytes, dev)
-                self.peer_pairs = PeerSlots(self.dist, self.group, self.fslot_bytes, dev)
-                if os.environ.get("DM_SHARD_PEER_REDUCE", "1") != "0":
-                    # the two replicated R-sized arrays live in symmetric memory: their all-reduces are peer kernels
-                    pm, pp = PeerArray(self.dist, self.group, 2 * R, dev), PeerArray(self.dist, self.group, R, dev)
-                    self.peer_mask_cnt, self.peer_parent = pm, pp
-                    self.mask_cnt, self.mask = pm.tensor, pm.tensor[:R]
-                    e.parent = pp.tensor
+                rows = PeerSlots(self.dist, self.group, self.slot_bytes, dev)
+                pairs = PeerSlots(self.dist, self.group, self.fslot_bytes, dev)
+                pm, pp = PeerArray(self.dist, self.group, 2 * R, dev), PeerArray(self.dist, self.group, R, dev)
             except Exception as ex:                                # no NVLink peer access / symmetric memory on this box
-                self.peer_rows = self.peer_pairs = self.peer_mask_cnt = self.peer_parent = None
                 self.peer_error = repr(ex)
+            else:
+                self.peer_rows, self.peer_pairs, self.peer_mask_cnt, self.peer_parent = rows, pairs, pm, pp
+                self.mask_cnt, self.mask = pm.tensor, pm.tensor[:R]
+                e.parent = pp.tensor
         e.sum.zero_()                                              # rows the pooling pass never writes start as zeros
-        self._dist_graphs, self._last_fg = {}, None
+        self._last_fg = None
         self.any_selected = z(1, dt=torch.int64)
         self.host_fflags = torch.zeros((self.world, 10), dtype=torch.int64).pin_memory()
         self.hdr_dev = z(self.world, 80, dt=torch.uint8)
@@ -318,7 +315,7 @@ class ShardedMergeEngine:
         round's selection + exchange."""
         from .raster import _p, _stream
         e, L, dist, grp, s = self.eng, self.eng.L, self.dist, self.group, _stream()
-        R, D, cap, n_edges = e.R, e.D, e.cap, e.counts[0:1]
+        R = e.R
         L.check(L.dm_uf_union_slots(_p(e.parent), _p(fg), self.world, self.fslot_bytes, self.row_cap, R, s),
                 "dm_uf_union_slots")
         L.check(L.dm_uf_compress(_p(e.parent), R, s), "dm_uf_compress")
@@ -332,49 +329,19 @@ class ShardedMergeEngine:
         L.check(L.dm_shard_plan(_p(e.parent), _p(e.alive), _p(self.mask_old), _p(self.mask), _p(self.grew), self.rank, R,
                                 _p(self.send), _p(self.seen_comp), s), "dm_shard_plan")
         self._exchange_rows(self.send, add=False, buf=1)
-        cur = torch.cuda.current_stream(e.dev)
-        e.side.wait_stream(cur)                            # merged statistics beside the edge re-keying (as on one GPU)
-        with torch.cuda.stream(e.side):
-            L.check(L.dm_merge_apply_masked(_p(e.parent), _p(e.alive), _p(e.changed), _p(e.sum), _p(e.cnt), _p(e.area),
-                                            _p(e.perim), R, D, e.counts[5:6].data_ptr(), _p(self.seen_comp),
-                                            _p(e.ws_side), e.ws_side_bytes, _stream()), "dm_merge_apply_masked")
-        L.check(L.dm_edges_rekey(_p(e.parent), _p(e.keys), _p(e.blen), _p(e.scores), _p(n_edges), cap, R, _p(e.perim),
-                                 _p(e.ws), e.ws_bytes, s), "dm_edges_rekey")
-        cur.wait_stream(e.side)
-        L.check(L.dm_region_mean(_p(e.sum), _p(e.cnt), R, D, _p(e.mean), _p(e.norm2), _p(e.changed), s), "dm_region_mean")
-        e._score(mlp, e.changed)
+        e._apply_and_rescore(mlp, self.seen_comp)          # embedding sums only of the components this rank sees
         return self._pre_exchange(tau, mlp, do_unions, False, 1)
 
     def _dist_round(self, tau, mlp, do_unions):
-        """The round body as one CUDA graph launch when every exchange in it is a kernel of this library (peer stores /
-        peer all-reduce over symmetric memory + signal-pad barriers): ~35 short launches issued from Python otherwise."""
-        e = self.eng
-        graphs_ok = (e.use_graphs and self.peer_pairs is not None and self.peer_rows is not None and
-                     self.peer_parent is not None and os.environ.get("DM_SHARD_GRAPHS", "1") != "0")
+        """The round body; one CUDA graph launch when every exchange in it is a kernel of this library (peer stores /
+        peer all-reduce over symmetric memory + signal-pad barriers): collective calls cannot be captured."""
         # the body reads the gathered pairs of the previous exchange: buffer 0 after the head, buffer 1 after a body
         src = self._last_fg
-        if not graphs_ok:
-            self._last_fg = self._dist_round_body(tau, mlp, do_unions, src)
-            return self._last_fg
-        key = (float(tau), None if mlp is None else (id(mlp), mlp.blob.data_ptr()), e.cap, bool(do_unions), src.data_ptr())
-        ent = self._dist_graphs.get(key)
-        if ent is None:
-            g = torch.cuda.CUDAGraph()
-            n0 = e.L.dm_launch_count()
-            try:
-                with torch.cuda.graph(g, capture_error_mode="thread_local"):
-                    out = self._dist_round_body(tau, mlp, do_unions, src)
-            except Exception:                      # capture refused: plain launches from now on (same kernels, same order)
-                e.use_graphs = False
-                self._last_fg = self._dist_round_body(tau, mlp, do_unions, src)
-                return self._last_fg
-            ent = (g, e.L.dm_launch_count() - n0, out)
-            if len(self._dist_graphs) >= 8:
-                self._dist_graphs.clear()
-            self._dist_graphs[key] = ent
-        ent[0].replay()
-        e.L.dm_launch_count_add(ent[1])
-        self._last_fg = ent[2]
+        body = lambda: self._dist_round_body(tau, mlp, do_unions, src)
+        if self.peer_rows is None:
+            self._last_fg = body()
+        else:
+            self._last_fg = self.eng._graph_launch(body, tau, mlp, bool(do_unions), src.data_ptr())
         return self._last_fg
 
     def run(self, labels_tile, feats_local, tau, *, image_tile=None, xs_local=None, ys_local_rel=None, max_rounds=64,
@@ -426,12 +393,8 @@ class ShardedMergeEngine:
             L.check(L.dm_shard_frontier(_p(self.mask_cnt), _p(self.cnt_local), R, _p(e.cnt), _p(self.send), s), "dm_shard_frontier")
             self._exchange_rows(self.send, add=True, buf=0)
             # (4) merge loop on the tile's edges with the replicated parent array
-            e.parent.copy_(e.iota)
-            e.alive.fill_(1)
-            e.counts[5:8].zero_()
+            e._merge_init(mlp)
             L.check(L.dm_region_mean(_p(e.sum), _p(e.cnt), R, D, _p(e.mean), _p(e.norm2), _p(self.seen), s), "dm_region_mean")
-            if mlp is not None and mlp.in_features != 2 * D:
-                raise ValueError("the pair-MLP takes concat(mean[lo], mean[hi]): in_features must be 2 D")
             e._score(mlp, None)
             rounds = merges = 0
             fg = self._last_fg = self._pre_exchange(tau, mlp, max_rounds > 0, True, 0)
@@ -480,51 +443,6 @@ class ShardedMergeEngine:
                 return MergeResult(e.out[: self.rows_own], e.parent, rounds, merges, out_k[:Ef], out_l[:Ef], None, e.area,
                                    e.perim, e.sum, e.cnt)
         return MergeResult(e.out[: self.rows_own], e.parent, rounds, merges, e.keys[:Ef], e.blen[:Ef], None, e.area,
-                           e.perim, e.sum, e.cnt)
-
-    def run_replicated(self, labels_tile, feats_local, tau, *, image_tile=None, xs_local=None, ys_local_rel=None, max_rounds=64):
-        if self.eng.cap < self.slot_cap:
-            raise ValueError("run_replicated needs the engine built with replicated=True (global edge capacity)")
-        """labels_tile: int32 [rows_own (+1 halo), W]; ys_local_rel are rows relative to the tile."""
-        from .raster import MergeResult, _p, _stream
-        e, L, dist = self.eng, self.eng.L, self.dist
-        e.pool_id_range = False                         # the partial sums are all-reduced as whole arrays here
-        with torch.cuda.device(e.dev):
-            s = _stream()
-            e._rag(labels_tile, image_tile, self.rows_own, self.rank == 0, self.rank == self.world - 1)
-            self.tile_counts.copy_(e.counts[:4])
-            # (1) edges: gather the per-tile lists (fixed slots + device counts), merge into the replicated global list
-            if self.slot_cap > e.cap:
-                raise ValueError("slot capacity exceeds the engine's edge capacity")
-            gk = all_gather_slots(e.keys[: self.slot_cap], dist, self.group)
-            gl = all_gather_slots(e.blen[: self.slot_cap], dist, self.group)
-            gc = all_gather_slots(e.counts[0:1], dist, self.group)
-            L.check(L.dm_edges_concat(_p(gk), _p(gl), _p(gc), self.world, self.slot_cap, _p(e.keys), _p(e.blen), e.cap,
-                                      _p(self.cat_counts), s), "dm_edges_concat")
-            e.counts[:4].zero_()
-            L.check(L.dm_edges_sort_unique(_p(e.keys), _p(e.blen), _p(self.cat_counts), e.cap, e.R, _p(e.counts), _p(e.ws),
-                                           e.ws_bytes, s), "dm_edges_sort_unique")
-            # tile-pass flags ride along with the merge loop's first read-back (counts[2] overflow, counts[3] bad label)
-            e.counts[2:3].copy_(torch.maximum(self.tile_counts[2:3], self.cat_counts[1:2]))
-            e.counts[3:4].copy_(self.tile_counts[3:4])
-            e.counts[1:2].copy_(self.tile_counts[1:2])
-            # (2) region statistics: one all-reduce over the fused int64 buffer, then the perimeter
-            allreduce_sum_(e.stats, dist, self.group)
-            L.check(L.dm_perimeter(_p(e.keys), _p(e.blen), _p(e.counts), e.cap, _p(e.border), _p(e.perim), e.R, s),
-                    "dm_perimeter")
-            # (3) embeddings of the tile's own points -> partial sums -> all-reduce
-            e._pool(labels_tile, xs_local, ys_local_rel, None, feats_local)
-            allreduce_sum_(e.sum, dist, self.group)
-            allreduce_sum_(e.cnt, dist, self.group)
-            # (4) replicated merge loop, (5) tile-local relabel
-            try:
-                rounds, merges = e._merge_loop(tau, max_rounds)
-            except OverflowError as ov:
-                raise RuntimeError("tile edge list overflow (capacity %d / slot %d, needed %s)" % (e.cap, self.slot_cap, ov.args[0]))
-            L.check(L.dm_relabel(_p(labels_tile), self.rows_own, self.W, labels_tile.stride(0), _p(e.parent), e.R, _p(e.out),
-                                 self.W, s), "dm_relabel")
-            Ef = int(e.host_counts[0])
-        return MergeResult(e.out[: self.rows_own], e.parent, rounds, merges, e.keys[:Ef], e.blen[:Ef], e.scores[:Ef], e.area,
                            e.perim, e.sum, e.cnt)
 
 

@@ -115,7 +115,7 @@ int dm_rag_finish(uint64_t* edge_keys, uint32_t* boundary_len, int64_t capacity,
                   int64_t* counts, void* ws, size_t ws_bytes, dm_stream_t stream);
 
 /* Which staging path the last dm_rag_scan on this thread took: 1 = TMA (cp.async.bulk.tensor),
- * 0 = ld.global (pitch / base not 16-byte aligned, or DM_RAG_NO_TMA=1), -1 = none yet; and the
+ * 0 = ld.global (pitch / base not 16-byte aligned), -1 = none yet; and the
  * CUresult of the last cuTensorMapEncodeTiled (-1: driver entry point missing). */
 int dm_rag_last_path(void);
 int dm_rag_last_encode_error(void);
@@ -318,12 +318,11 @@ int dm_shard_plan(const int32_t* parent, const uint8_t* alive, const int32_t* ma
                   dm_stream_t stream);
 /* fused per-region glue: dm_shard_seen: seen[r] |= area[r] > 0; mask_cnt[r] = seen ? 1 << rank : 0; mask_cnt[R + r] =
  * cnt_local[r] = cnt[r] (the buffer that is all-reduced).  dm_shard_frontier (after the all-reduce): cnt[r] = global count,
- * send[r] = region seen by two ranks and this rank has points of it.  dm_any_diff_i32: flag_dev[0] = any(a != b). */
+ * send[r] = region seen by two ranks and this rank has points of it. */
 int dm_shard_seen(const int64_t* area, uint8_t* seen, const int32_t* cnt, int rank, int64_t n_regions,
                   int32_t* mask_cnt, int32_t* cnt_local, dm_stream_t stream);
 int dm_shard_frontier(const int32_t* mask_cnt, const int32_t* cnt_local, int64_t n_regions, int32_t* cnt, uint8_t* send,
                       dm_stream_t stream);
-int dm_any_diff_i32(const int32_t* a, const int32_t* b, int64_t n, int64_t* flag_dev, dm_stream_t stream);
 /* Distributed union-find by FRONTIER EXCHANGE (one all-gather of a few hundred pairs per round, no iteration): a component
  * can span two row tiles only through a region both ranks see.  After its local unions (dm_uf_union + dm_uf_compress) a
  * rank writes, for every alive component x it shares with another rank (mask[x] has its bit and another one) and whose

@@ -140,9 +140,10 @@ def test_synth_matches_oracle(cuda, H, W, R, C):
 # ------------------------------------------------------------------------------------------
 # R1 RAG (+ fused band pooling)
 # ------------------------------------------------------------------------------------------
-def check_rag(cuda, L, R, image=None, **kw):
+def check_rag(cuda, L, R, image=None, labels_dev=None, **kw):
+    """build_rag on labels_dev (default: a contiguous device copy of L) against the oracle on L."""
     from deepmerge_b200 import build_rag
-    rag = build_rag(T(L, cuda), R, None if image is None else T(image, cuda), **kw)
+    rag = build_rag(T(L, cuda) if labels_dev is None else labels_dev, R, None if image is None else T(image, cuda), **kw)
     okw = {}
     if "rows_own" in kw:
         okw = dict(own_rows=kw["rows_own"], top_border=kw.get("top_border", True), bottom_border=kw.get("bottom_border", True))
@@ -237,17 +238,22 @@ def test_rag_strided_and_unaligned_rasters_take_fallback_path(cuda):
     assert np.array_equal(keys_np(rag.edge_keys), keys) and np.array_equal(rag.perimeter.cpu().numpy(), per)
 
 
-def test_rag_forced_fallback_equals_tma(cuda, monkeypatch):
+def test_rag_forced_fallback_equals_tma(cuda):
+    """One raster through both staging paths: TMA for the aligned copy, ld.global for a copy whose base is 4 bytes off
+    16-byte alignment (pitch still aligned)."""
+    from deepmerge_b200._lib import lib
     sc = o.synth_scene(130, 512, 400, C=4)
-    monkeypatch.setenv("DM_RAG_NO_TMA", "1")
     check_rag(cuda, sc["labels"], sc["n_regions"], sc["image"])
+    assert lib().dm_rag_last_path() == 1
+    wide = T(np.zeros((130, 516), np.int32), cuda)
+    view = wide[:, 1:513]
+    view.copy_(T(sc["labels"], cuda))
+    check_rag(cuda, sc["labels"], sc["n_regions"], sc["image"], labels_dev=view)
+    assert lib().dm_rag_last_path() == 0
 
 
-@pytest.mark.parametrize("env", [{}, {"DM_RAG_CFG": "1"}, {"DM_RAG_CFG": "2"}, {"DM_RAG_CFG": "3"}])
-def test_rag_alternative_kernel_shapes(cuda, monkeypatch, env):
-    """The measurement-only shapes of the raster kernel give the same answer; long strips wrap the item buffers."""
-    for k, v in env.items():
-        monkeypatch.setenv(k, v)
+def test_rag_alternative_kernel_shapes(cuda):
+    """4-band rasters of three shapes; long strips wrap the item buffers."""
     sc = o.synth_scene(300, 1024, 350, C=4)
     check_rag(cuda, sc["labels"], sc["n_regions"], sc["image"])
     rng = np.random.default_rng(3)

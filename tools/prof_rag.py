@@ -16,24 +16,16 @@ L = _lib.lib()
 dev = torch.device("cuda:0")
 sc = synth_scene(side, side, R, C=C, device=dev)
 eng = MergeEngine(side, side, sc.n_regions, 100, C=C, n_points=sc.feats.shape[0], device=dev)
-variants = [v for v in os.environ.get("DM_PROF_VARIANTS", "").split(",") if v]
-for var in variants or [""]:
-  if var:
-    for kk in ("DM_RAG_CFG", "DM_RAG_KERNEL"):
-        os.environ.pop(kk, None)
-    for kv in var.split("+"):
-        k, _, v = kv.partition("=")
-        os.environ[k] = v
-  ev = [(torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)) for _ in range(reps)]
-  for a, b in ev:
-      eng.stats.zero_()
-      a.record()
-      L.check(L.dm_rag_scan(_p(sc.labels), side, side, side, side, _p(sc.image), C, side * C, sc.n_regions, 1, 1, _p(eng.area),
-                            _p(eng.border), _p(eng.bsum), _p(eng.bsq), eng.cap, _p(eng.counts), _p(eng.ws), eng.ws_bytes,
-                            _stream()), "scan")
-      b.record()
-  torch.cuda.synchronize()
-  ms = [a.elapsed_time(b) for a, b in ev]
-  byts = (4 + C) * side * side
-  print(var or "default", "path", L.dm_rag_last_path(), "encode_err", L.dm_rag_last_encode_error(), "counts", eng.counts.tolist()[:4])
-  print("ms", ms, "GB/s", [byts / m / 1e6 for m in ms])
+ev = [(torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)) for _ in range(reps)]
+for a, b in ev:
+    eng.stats.zero_()
+    a.record()
+    L.check(L.dm_rag_scan(_p(sc.labels), side, side, side, side, _p(sc.image), C, side * C, sc.n_regions, 1, 1, _p(eng.area),
+                          _p(eng.border), _p(eng.bsum), _p(eng.bsq), eng.cap, _p(eng.counts), _p(eng.ws), eng.ws_bytes,
+                          _stream()), "scan")
+    b.record()
+torch.cuda.synchronize()
+ms = [a.elapsed_time(b) for a, b in ev]
+byts = (4 + C) * side * side
+print("path", L.dm_rag_last_path(), "encode_err", L.dm_rag_last_encode_error(), "counts", eng.counts.tolist()[:4])
+print("ms", ms, "GB/s", [byts / m / 1e6 for m in ms])
