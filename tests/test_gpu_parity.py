@@ -399,11 +399,12 @@ def random_graph(seed, R=300, E=900, D=16):
     return sum_, cnt, area, per, keys, blen
 
 
-@pytest.mark.parametrize("seed", range(5))
-@pytest.mark.parametrize("tau", [0.5, 1.5, 3.0])
-def test_merge_graph_matches_oracle(cuda, seed, tau):
+# D = 16 runs the vec L2 kernel in one trip, D = 7 the scalar kernel, D = 260 the vec kernel in three trips
+@pytest.mark.parametrize("seed,tau,D", [pytest.param(seed, tau, D, id="%s-%d%s" % (tau, seed, "" if D == 16 else "-D%d" % D))
+                                        for D in (16, 7, 260) for tau in (0.5, 1.5, 3.0) for seed in range(5)])
+def test_merge_graph_matches_oracle(cuda, seed, tau, D):
     from deepmerge_b200 import merge_graph
-    sum_, cnt, area, per, keys, blen = random_graph(seed)
+    sum_, cnt, area, per, keys, blen = random_graph(seed, D=D)
     want = o.merge_graph(sum_, cnt, area, per, keys, blen, tau=tau)
     got = merge_graph(T(sum_, cuda), T(cnt, cuda), T(area, cuda), T(per, cuda), T(keys.view(np.int64), cuda),
                       T(blen.view(np.int32), cuda), tau)
