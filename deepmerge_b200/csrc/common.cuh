@@ -7,8 +7,7 @@
 namespace dm {
 
 extern thread_local int g_last_cuda_error;
-extern long long g_launch_count;   // kernels launched by this library in this process
-#define DM_COUNT_LAUNCH() (__atomic_add_fetch(&dm::g_launch_count, 1, __ATOMIC_RELAXED))
+extern long long g_launch_count;   // kernels accepted by the runtime from this library in this process
 
 inline int cuda_fail(cudaError_t e) {
     g_last_cuda_error = (int)e;
@@ -20,8 +19,6 @@ inline int cuda_fail(cudaError_t e) {
         cudaError_t _e = (expr);                        \
         if (_e != cudaSuccess) return dm::cuda_fail(_e); \
     } while (0)
-
-#define DM_LAUNCH_CHECK() DM_CUDA(cudaPeekAtLastError())
 
 #define DM_TRY(expr)             \
     do {                         \
@@ -38,6 +35,43 @@ inline size_t align_up(size_t x, size_t a) { return (x + a - 1) / a * a; }
 inline int64_t ceil_div(int64_t a, int64_t b) { return (a + b - 1) / b; }
 
 int num_sms();
+
+// Grid of a grid-stride kernel: one thread per item, but at most per_sm blocks per SM.
+inline unsigned grid_for(int64_t items, int threads = 256, int per_sm = 8) {
+    return (unsigned)imax64(1, imin64(ceil_div(items, threads), (int64_t)num_sms() * per_sm));
+}
+
+// Outcome of a launch whose own result is e: the thread's CUDA error is read and cleared, so a refused launch is
+// reported once, as DM_ERR_CUDA, and is not seen again by the next check of this library or of the caller.  Only a
+// launch the runtime accepted is counted.
+inline int launched(cudaError_t e) {
+    const cudaError_t pending = cudaGetLastError();
+    if (e == cudaSuccess) e = pending;
+    if (e != cudaSuccess) return cuda_fail(e);
+    __atomic_add_fetch(&g_launch_count, 1, __ATOMIC_RELAXED);
+    return DM_OK;
+}
+
+// Keeps P out of template argument deduction: the kernel alone fixes the parameter types, and the arguments are
+// converted to them at the call, as in a triple-chevron launch.
+template <typename T> struct param { using type = T; };
+
+// Every kernel of the library is launched through here or launch_cooperative.  Dynamic shared memory above the 48 KB
+// a kernel gets by default is opted into first.
+template <typename... P>
+int launch(void (*k)(P...), dim3 grid, dim3 block, size_t smem, cudaStream_t s, typename param<P>::type... args) {
+    if (smem > 48 * 1024) DM_CUDA(cudaFuncSetAttribute((const void*)k, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    k<<<grid, block, smem, s>>>(args...);
+    return launched(cudaSuccess);
+}
+
+// A kernel whose blocks meet at grid-wide barriers: the runtime refuses the launch unless all of grid fits on the GPU
+// at once.
+template <typename... P>
+int launch_cooperative(void (*k)(P...), dim3 grid, dim3 block, cudaStream_t s, typename param<P>::type... args) {
+    void* argv[] = {(void*)&args...};
+    return launched(cudaLaunchCooperativeKernel((const void*)k, grid, block, argv, 0, s));
+}
 
 // Carves a caller-provided workspace into 256-byte aligned pieces.
 struct Carver {

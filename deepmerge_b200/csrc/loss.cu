@@ -66,17 +66,12 @@ using namespace dm;
 extern "C" int dm_contrastive_fwd_bwd(const float* a, const float* b, const int64_t* flag, int64_t B, int64_t D, float margin,
                                       float* loss, float* ga, float* gb, dm_stream_t stream) {
     if (B <= 0 || D <= 0 || !a || !b || !flag || !loss) return DM_ERR_BAD_ARG;
-    DM_COUNT_LAUNCH(); loss::contrastive_kernel<<<1, 1024, 0, S(stream)>>>(a, b, flag, B, (int)D, margin, loss, ga, gb);
-    DM_LAUNCH_CHECK();
-    return DM_OK;
+    return launch(loss::contrastive_kernel, 1, 1024, 0, S(stream), a, b, flag, B, (int)D, margin, loss, ga, gb);
 }
 
 extern "C" int dm_gather_rows(const float* table, int64_t D, const int64_t* idx, int64_t n, float* out, dm_stream_t stream) {
     if (n < 0 || D <= 0) return DM_ERR_BAD_ARG;
     if (n == 0) return DM_OK;
     if (!table || !idx || !out) return DM_ERR_BAD_ARG;
-    const int64_t g = imin64(ceil_div(n * 32, 256), (int64_t)num_sms() * 8);
-    DM_COUNT_LAUNCH(); loss::gather_rows_kernel<<<(unsigned)imax64(g, 1), 256, 0, S(stream)>>>(table, (int)D, idx, n, out);
-    DM_LAUNCH_CHECK();
-    return DM_OK;
+    return launch(loss::gather_rows_kernel, grid_for(n * 32), 256, 0, S(stream), table, (int)D, idx, n, out);
 }

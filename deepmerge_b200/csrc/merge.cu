@@ -8,12 +8,6 @@
 namespace dm {
 namespace merge {
 
-static unsigned grid_for(int64_t items, int threads = 256, int per_sm = 8) {
-    int64_t g = ceil_div(items, threads);
-    int64_t cap = (int64_t)num_sms() * per_sm;
-    return (unsigned)imax64(1, min(g, cap));
-}
-
 // ---- selection ------------------------------------------------------------------------
 template <bool MLP>
 __global__ void select_kernel(const float* __restrict__ v, float tau, int n_out, const int64_t* __restrict__ n_dev,
@@ -533,16 +527,14 @@ __global__ void slots_word_max_kernel(const unsigned char* __restrict__ slots, i
 }  // namespace dm
 
 using namespace dm;
-using merge::grid_for;
 
 extern "C" int dm_shard_seen(const int64_t* area, uint8_t* seen, const int32_t* cnt, int rank, int64_t n_regions,
                              int32_t* mask_cnt, int32_t* cnt_local, dm_stream_t stream) {
     if (n_regions < 0 || rank < 0 || rank > 30) return DM_ERR_BAD_ARG;
     if (n_regions == 0) return DM_OK;
     if (!area || !seen || !cnt || !mask_cnt || !cnt_local) return DM_ERR_BAD_ARG;
-    DM_COUNT_LAUNCH(); merge::shard_seen_kernel<<<grid_for(n_regions), 256, 0, S(stream)>>>(area, seen, cnt, 1 << rank, n_regions, mask_cnt, cnt_local);
-    DM_LAUNCH_CHECK();
-    return DM_OK;
+    return launch(merge::shard_seen_kernel, grid_for(n_regions), 256, 0, S(stream), area, seen, cnt, 1 << rank, n_regions,
+        mask_cnt, cnt_local);
 }
 
 extern "C" int dm_shard_frontier(const int32_t* mask_cnt, const int32_t* cnt_local, int64_t n_regions, int32_t* cnt,
@@ -550,22 +542,19 @@ extern "C" int dm_shard_frontier(const int32_t* mask_cnt, const int32_t* cnt_loc
     if (n_regions < 0) return DM_ERR_BAD_ARG;
     if (n_regions == 0) return DM_OK;
     if (!mask_cnt || !cnt_local || !cnt || !send) return DM_ERR_BAD_ARG;
-    DM_COUNT_LAUNCH(); merge::shard_frontier_kernel<<<grid_for(n_regions), 256, 0, S(stream)>>>(mask_cnt, cnt_local, n_regions, cnt, send);
-    DM_LAUNCH_CHECK();
-    return DM_OK;
+    return launch(merge::shard_frontier_kernel, grid_for(n_regions), 256, 0, S(stream), mask_cnt, cnt_local, n_regions, cnt,
+        send);
 }
 
 extern "C" int dm_shard_frontier_pairs(const int32_t* parent, const uint8_t* alive, const int32_t* mask, int rank,
                                        int64_t n_regions, void* slot, int64_t capacity, dm_stream_t stream) {
     if (n_regions < 0 || capacity < 0 || rank < 0 || rank > 30 || !slot || ((uintptr_t)slot & 15)) return DM_ERR_BAD_ARG;
+    if (n_regions > 0 && (!parent || !alive || !mask)) return DM_ERR_BAD_ARG;
     cudaStream_t s = S(stream);
     DM_CUDA(cudaMemsetAsync(slot, 0, 16, s));                       // count; the caller owns the 8 flag words behind it
     if (n_regions == 0) return DM_OK;
-    if (!parent || !alive || !mask) return DM_ERR_BAD_ARG;
-    DM_COUNT_LAUNCH(); merge::shard_frontier_pairs_kernel<<<grid_for(n_regions), 256, 0, s>>>(
-        parent, alive, mask, 1 << rank, n_regions, (uint64_t*)((unsigned char*)slot + 80), capacity, (unsigned long long*)slot);
-    DM_LAUNCH_CHECK();
-    return DM_OK;
+    return launch(merge::shard_frontier_pairs_kernel, grid_for(n_regions), 256, 0, s, parent, alive, mask, 1 << rank, n_regions,
+        (uint64_t*)((unsigned char*)slot + 80), capacity, (unsigned long long*)slot);
 }
 
 extern "C" int dm_uf_union_slots(int32_t* parent, const void* slots, int64_t n_slots, int64_t slot_bytes, int64_t capacity,
@@ -573,10 +562,8 @@ extern "C" int dm_uf_union_slots(int32_t* parent, const void* slots, int64_t n_s
     if (n_slots < 0 || capacity < 0 || n_regions < 0 || slot_bytes < 80 + 8 * capacity || (slot_bytes & 15)) return DM_ERR_BAD_ARG;
     if (n_slots == 0 || capacity == 0 || n_regions == 0) return DM_OK;
     if (!parent || !slots) return DM_ERR_BAD_ARG;
-    DM_COUNT_LAUNCH(); merge::uf_union_slots_kernel<<<grid_for(n_slots * capacity), 256, 0, S(stream)>>>(
-        parent, (const unsigned char*)slots, (int)n_slots, slot_bytes, capacity, n_regions);
-    DM_LAUNCH_CHECK();
-    return DM_OK;
+    return launch(merge::uf_union_slots_kernel, grid_for(n_slots * capacity), 256, 0, S(stream), parent,
+        (const unsigned char*)slots, (int)n_slots, slot_bytes, capacity, n_regions);
 }
 
 extern "C" int dm_peer_put_slot(const void* slot, const int64_t* peer_bases_dev, int64_t world, int64_t rank, int64_t slot_bytes,
@@ -588,11 +575,9 @@ extern "C" int dm_peer_put_slot(const void* slot, const int64_t* peer_bases_dev,
         return DM_ERR_BAD_ARG;
     if (!slot || !peer_bases_dev || ((uintptr_t)slot & 15)) return DM_ERR_BAD_ARG;
     const int64_t units = header_bytes / 16 + (capacity * seg0_elem_bytes + 15) / 16 + (capacity * seg1_elem_bytes + 15) / 16;
-    DM_COUNT_LAUNCH(); merge::peer_put_kernel<<<grid_for(units), 256, 0, S(stream)>>>(
-        (const unsigned char*)slot, (const long long*)peer_bases_dev, (int)world, (int)rank, slot_bytes, header_bytes / 16, seg0_offset,
-        seg0_elem_bytes, seg1_offset, seg1_elem_bytes, capacity);
-    DM_LAUNCH_CHECK();
-    return DM_OK;
+    return launch(merge::peer_put_kernel, grid_for(units), 256, 0, S(stream), (const unsigned char*)slot,
+        (const long long*)peer_bases_dev, (int)world, (int)rank, slot_bytes, header_bytes / 16, seg0_offset, seg0_elem_bytes,
+        seg1_offset, seg1_elem_bytes, capacity);
 }
 
 extern "C" int dm_peer_allreduce_i32(const void* peer_bases_dev, int64_t world, int64_t rank, int64_t offset_bytes, int64_t n,
@@ -603,18 +588,14 @@ extern "C" int dm_peer_allreduce_i32(const void* peer_bases_dev, int64_t world, 
     if (n == 0) return DM_OK;
     if (!peer_bases_dev) return DM_ERR_BAD_ARG;
     const int64_t n4 = n / 4, per = ceil_div(n4, world);
-    DM_COUNT_LAUNCH(); merge::peer_allreduce_i32_kernel<<<grid_for(per), 256, 0, S(stream)>>>(
-        (const long long*)peer_bases_dev, (int)world, (int)rank, offset_bytes, n4, op);
-    DM_LAUNCH_CHECK();
-    return DM_OK;
+    return launch(merge::peer_allreduce_i32_kernel, grid_for(per), 256, 0, S(stream), (const long long*)peer_bases_dev,
+        (int)world, (int)rank, offset_bytes, n4, op);
 }
 
 extern "C" int dm_shard_round_flags(const int64_t* counts, int64_t* flags, int first_round, int64_t* slot_flags,
                                     dm_stream_t stream) {
     if (!counts || !flags || !slot_flags) return DM_ERR_BAD_ARG;
-    DM_COUNT_LAUNCH(); merge::shard_round_flags_kernel<<<1, 32, 0, S(stream)>>>(counts, flags, first_round, slot_flags);
-    DM_LAUNCH_CHECK();
-    return DM_OK;
+    return launch(merge::shard_round_flags_kernel, 1, 32, 0, S(stream), counts, flags, first_round, slot_flags);
 }
 
 extern "C" int dm_slots_overflow(const void* slots, int64_t n_slots, int64_t slot_bytes, int64_t capacity, int64_t* flag_dev,
@@ -622,10 +603,8 @@ extern "C" int dm_slots_overflow(const void* slots, int64_t n_slots, int64_t slo
     if (n_slots < 0 || n_slots > 4096 || slot_bytes < 16 || capacity < 0 || !flag_dev) return DM_ERR_BAD_ARG;
     if (n_slots == 0) return DM_OK;
     if (!slots) return DM_ERR_BAD_ARG;
-    DM_COUNT_LAUNCH(); merge::slots_overflow_kernel<<<1, 64, 0, S(stream)>>>((const unsigned char*)slots, (int)n_slots, slot_bytes, capacity,
-                                                                       flag_dev);
-    DM_LAUNCH_CHECK();
-    return DM_OK;
+    return launch(merge::slots_overflow_kernel, 1, 64, 0, S(stream), (const unsigned char*)slots, (int)n_slots, slot_bytes,
+        capacity, flag_dev);
 }
 
 extern "C" int dm_slots_word_max(const void* slots, int64_t n_slots, int64_t slot_bytes, int64_t word_offset, int64_t* out_dev,
@@ -634,10 +613,8 @@ extern "C" int dm_slots_word_max(const void* slots, int64_t n_slots, int64_t slo
         !out_dev)
         return DM_ERR_BAD_ARG;
     if (n_slots > 0 && !slots) return DM_ERR_BAD_ARG;
-    DM_COUNT_LAUNCH(); merge::slots_word_max_kernel<<<1, 32, 0, S(stream)>>>((const unsigned char*)slots, (int)n_slots, slot_bytes, word_offset,
-                                                                       out_dev);
-    DM_LAUNCH_CHECK();
-    return DM_OK;
+    return launch(merge::slots_word_max_kernel, 1, 32, 0, S(stream), (const unsigned char*)slots, (int)n_slots, slot_bytes,
+        word_offset, out_dev);
 }
 
 extern "C" int dm_rows_unpack_slots(const void* slots, int64_t n_slots, int64_t slot_bytes, int64_t slot_capacity,
@@ -647,10 +624,8 @@ extern "C" int dm_rows_unpack_slots(const void* slots, int64_t n_slots, int64_t 
         return DM_ERR_BAD_ARG;
     if (n_slots == 0 || slot_capacity == 0 || n_regions == 0) return DM_OK;
     if (!slots || !rows) return DM_ERR_BAD_ARG;
-    DM_COUNT_LAUNCH(); merge::rows_unpack_slots_kernel<<<grid_for(n_slots * slot_capacity * 32), 256, 0, S(stream)>>>(
+    return launch(merge::rows_unpack_slots_kernel, grid_for(n_slots * slot_capacity * 32), 256, 0, S(stream),
         (const unsigned char*)slots, (int)n_slots, slot_bytes, slot_capacity, n_regions, (int)D, rows, zero);
-    DM_LAUNCH_CHECK();
-    return DM_OK;
 }
 
 extern "C" int dm_shard_propagate(const int32_t* parent, const uint8_t* alive, int32_t* mask, uint8_t* grew, int64_t n_regions,
@@ -660,9 +635,7 @@ extern "C" int dm_shard_propagate(const int32_t* parent, const uint8_t* alive, i
     if (!parent || !alive || !mask || !grew) return DM_ERR_BAD_ARG;
     cudaStream_t s = S(stream);
     DM_CUDA(cudaMemsetAsync(grew, 0, (size_t)n_regions, s));
-    DM_COUNT_LAUNCH(); merge::shard_propagate_kernel<<<grid_for(n_regions), 256, 0, s>>>(parent, alive, mask, grew, n_regions);
-    DM_LAUNCH_CHECK();
-    return DM_OK;
+    return launch(merge::shard_propagate_kernel, grid_for(n_regions), 256, 0, s, parent, alive, mask, grew, n_regions);
 }
 
 extern "C" int dm_shard_plan(const int32_t* parent, const uint8_t* alive, const int32_t* mask_old, const int32_t* mask_new,
@@ -671,10 +644,8 @@ extern "C" int dm_shard_plan(const int32_t* parent, const uint8_t* alive, const 
     if (n_regions < 0 || rank < 0 || rank > 30) return DM_ERR_BAD_ARG;
     if (n_regions == 0) return DM_OK;
     if (!parent || !alive || !mask_old || !mask_new || !grew || !send || !seen_comp) return DM_ERR_BAD_ARG;
-    DM_COUNT_LAUNCH(); merge::shard_plan_kernel<<<grid_for(n_regions), 256, 0, S(stream)>>>(parent, alive, mask_old, mask_new, grew, 1 << rank,
-                                                                         n_regions, send, seen_comp);
-    DM_LAUNCH_CHECK();
-    return DM_OK;
+    return launch(merge::shard_plan_kernel, grid_for(n_regions), 256, 0, S(stream), parent, alive, mask_old, mask_new, grew,
+        1 << rank, n_regions, send, seen_comp);
 }
 
 extern "C" int dm_mark_endpoints(const uint64_t* edge_keys, const int64_t* n_edges_dev, int64_t capacity, int64_t n_regions,
@@ -682,22 +653,18 @@ extern "C" int dm_mark_endpoints(const uint64_t* edge_keys, const int64_t* n_edg
     if (capacity < 0 || n_regions < 0) return DM_ERR_BAD_ARG;
     if (capacity == 0 || n_regions == 0) return DM_OK;
     if (!edge_keys || !n_edges_dev || !flags) return DM_ERR_BAD_ARG;
-    DM_COUNT_LAUNCH(); merge::mark_endpoints_kernel<<<grid_for(capacity), 256, 0, S(stream)>>>(edge_keys, n_edges_dev, n_regions, flags);
-    DM_LAUNCH_CHECK();
-    return DM_OK;
+    return launch(merge::mark_endpoints_kernel, grid_for(capacity), 256, 0, S(stream), edge_keys, n_edges_dev, n_regions, flags);
 }
 
 extern "C" int dm_rows_pack(const uint8_t* flag, const float* rows, int64_t n_regions, int64_t D, int32_t* out_ids,
                             float* out_rows, int64_t capacity, int64_t* n_out_dev, dm_stream_t stream) {
     if (n_regions < 0 || D <= 0 || capacity < 0 || !n_out_dev) return DM_ERR_BAD_ARG;
+    if (n_regions > 0 && (!flag || !rows || (capacity > 0 && (!out_ids || !out_rows)))) return DM_ERR_BAD_ARG;
     cudaStream_t s = S(stream);
     DM_CUDA(cudaMemsetAsync(n_out_dev, 0, sizeof(int64_t), s));
     if (n_regions == 0) return DM_OK;
-    if (!flag || !rows || (capacity > 0 && (!out_ids || !out_rows))) return DM_ERR_BAD_ARG;
-    DM_COUNT_LAUNCH(); merge::rows_pack_kernel<<<grid_for(n_regions), 256, 0, s>>>(flag, rows, n_regions, (int)D, out_ids, out_rows, capacity,
-                                                                (unsigned long long*)n_out_dev);
-    DM_LAUNCH_CHECK();
-    return DM_OK;
+    return launch(merge::rows_pack_kernel, grid_for(n_regions), 256, 0, s, flag, rows, n_regions, (int)D, out_ids, out_rows,
+        capacity, (unsigned long long*)n_out_dev);
 }
 
 extern "C" int dm_rows_unpack(const int32_t* ids, const float* in_rows, const int64_t* n_dev, int64_t capacity,
@@ -705,34 +672,28 @@ extern "C" int dm_rows_unpack(const int32_t* ids, const float* in_rows, const in
     if (n_regions < 0 || D <= 0 || capacity < 0) return DM_ERR_BAD_ARG;
     if (capacity == 0 || n_regions == 0) return DM_OK;
     if (!ids || !in_rows || !n_dev || !rows) return DM_ERR_BAD_ARG;
-    DM_COUNT_LAUNCH(); merge::rows_unpack_kernel<<<grid_for(capacity * 32), 256, 0, S(stream)>>>(ids, in_rows, n_dev, capacity, n_regions, (int)D,
-                                                                              rows, add);
-    DM_LAUNCH_CHECK();
-    return DM_OK;
+    return launch(merge::rows_unpack_kernel, grid_for(capacity * 32), 256, 0, S(stream), ids, in_rows, n_dev, capacity, n_regions,
+        (int)D, rows, add);
 }
 
 extern "C" int dm_merge_select_l2(const float* scores, float tau, const int64_t* n_dev, int64_t capacity, uint8_t* selected,
                                   int64_t* n_sel, dm_stream_t stream) {
     if (capacity < 0 || !n_sel) return DM_ERR_BAD_ARG;
+    if (capacity > 0 && (!scores || !n_dev || !selected)) return DM_ERR_BAD_ARG;
     DM_CUDA(cudaMemsetAsync(n_sel, 0, sizeof(int64_t), S(stream)));
     if (capacity == 0) return DM_OK;
-    if (!scores || !n_dev || !selected) return DM_ERR_BAD_ARG;
-    DM_COUNT_LAUNCH(); merge::select_kernel<false><<<grid_for(capacity), 256, 0, S(stream)>>>(scores, tau, 1, n_dev, selected,
-                                                                           (unsigned long long*)n_sel);
-    DM_LAUNCH_CHECK();
-    return DM_OK;
+    return launch(merge::select_kernel<false>, grid_for(capacity), 256, 0, S(stream), scores, tau, 1, n_dev, selected,
+        (unsigned long long*)n_sel);
 }
 
 extern "C" int dm_merge_select_mlp(const float* o, int64_t n_out, const int64_t* n_dev, int64_t capacity, uint8_t* selected,
                                    int64_t* n_sel, dm_stream_t stream) {
     if (capacity < 0 || !n_sel || n_out < 2) return DM_ERR_BAD_ARG;
+    if (capacity > 0 && (!o || !n_dev || !selected)) return DM_ERR_BAD_ARG;
     DM_CUDA(cudaMemsetAsync(n_sel, 0, sizeof(int64_t), S(stream)));
     if (capacity == 0) return DM_OK;
-    if (!o || !n_dev || !selected) return DM_ERR_BAD_ARG;
-    DM_COUNT_LAUNCH(); merge::select_kernel<true><<<grid_for(capacity), 256, 0, S(stream)>>>(o, 0.f, (int)n_out, n_dev, selected,
-                                                                          (unsigned long long*)n_sel);
-    DM_LAUNCH_CHECK();
-    return DM_OK;
+    return launch(merge::select_kernel<true>, grid_for(capacity), 256, 0, S(stream), o, 0.f, (int)n_out, n_dev, selected,
+        (unsigned long long*)n_sel);
 }
 
 extern "C" int dm_uf_union(int32_t* parent, const uint64_t* keys, const uint8_t* selected, const int64_t* n_dev,
@@ -740,18 +701,14 @@ extern "C" int dm_uf_union(int32_t* parent, const uint64_t* keys, const uint8_t*
     if (capacity < 0) return DM_ERR_BAD_ARG;
     if (capacity == 0) return DM_OK;
     if (!parent || !keys || !selected || !n_dev) return DM_ERR_BAD_ARG;
-    DM_COUNT_LAUNCH(); merge::uf_union_kernel<<<grid_for(capacity), 256, 0, S(stream)>>>(parent, keys, selected, n_dev);
-    DM_LAUNCH_CHECK();
-    return DM_OK;
+    return launch(merge::uf_union_kernel, grid_for(capacity), 256, 0, S(stream), parent, keys, selected, n_dev);
 }
 
 extern "C" int dm_uf_compress(int32_t* parent, int64_t R, dm_stream_t stream) {
     if (R < 0) return DM_ERR_BAD_ARG;
     if (R == 0) return DM_OK;
     if (!parent) return DM_ERR_BAD_ARG;
-    DM_COUNT_LAUNCH(); merge::uf_compress_kernel<<<grid_for(R), 256, 0, S(stream)>>>(parent, R);
-    DM_LAUNCH_CHECK();
-    return DM_OK;
+    return launch(merge::uf_compress_kernel, grid_for(R), 256, 0, S(stream), parent, R);
 }
 
 extern "C" size_t dm_merge_apply_workspace_bytes(int64_t R) {
@@ -763,26 +720,24 @@ extern "C" int dm_merge_apply_masked(const int32_t* parent, uint8_t* alive, uint
                                      int64_t* area, int64_t* perimeter, int64_t R, int64_t D, int64_t* n_merged,
                                      const uint8_t* root_mask, void* ws, size_t ws_bytes, dm_stream_t stream) {
     if (R < 0 || D <= 0 || !n_merged) return DM_ERR_BAD_ARG;
+    if (R > 0) {
+        if (!parent || !alive || !changed || !sum || !cnt || !area || !perimeter || !ws) return DM_ERR_BAD_ARG;
+        if (ws_bytes < dm_merge_apply_workspace_bytes(R)) return DM_ERR_WORKSPACE;
+    }
     cudaStream_t s = S(stream);
     DM_CUDA(cudaMemsetAsync(n_merged, 0, sizeof(int64_t), s));
     if (R == 0) return DM_OK;
-    if (!parent || !alive || !changed || !sum || !cnt || !area || !perimeter || !ws) return DM_ERR_BAD_ARG;
-    if (ws_bytes < dm_merge_apply_workspace_bytes(R)) return DM_ERR_WORKSPACE;
     Carver c(ws);
     uint64_t* list = c.take<uint64_t>(R);
     void* sws = c.take<char>(prims::ws_bytes(R, false));
     int64_t* n_list = c.take<int64_t>(1);
     DM_CUDA(cudaMemsetAsync(changed, 0, (size_t)R, s));
     DM_CUDA(cudaMemsetAsync(n_list, 0, sizeof(int64_t), s));
-    DM_COUNT_LAUNCH(); merge::collect_members_kernel<<<grid_for(R), 256, 0, s>>>(parent, alive, changed, cnt, (unsigned long long*)area,
-                                                              (unsigned long long*)perimeter, R, list,
-                                                              (unsigned long long*)n_list, (unsigned long long*)n_merged,
-                                                              root_mask);
+    DM_TRY(launch(merge::collect_members_kernel, grid_for(R), 256, 0, s, parent, alive, changed, cnt, (unsigned long long*)area,
+        (unsigned long long*)perimeter, R, list, (unsigned long long*)n_list, (unsigned long long*)n_merged, root_mask));
     const int b = bits_for(R);
     DM_TRY(prims::sort_pairs(list, nullptr, n_list, R, b, 2 * b, sws, s, R));
-    DM_COUNT_LAUNCH(); merge::merge_sums_kernel<<<grid_for(R * 32), 256, 0, s>>>(list, n_list, sum, (int)D);
-    DM_LAUNCH_CHECK();
-    return DM_OK;
+    return launch(merge::merge_sums_kernel, grid_for(R * 32), 256, 0, s, list, n_list, sum, (int)D);
 }
 
 extern "C" int dm_merge_apply(const int32_t* parent, uint8_t* alive, uint8_t* changed, float* sum, int32_t* cnt,
@@ -813,14 +768,12 @@ extern "C" int dm_edges_rekey(const int32_t* parent, uint64_t* keys, uint32_t* l
     float* os = c.take<float>(capacity);
     void* sws = c.take<char>(prims::ws_bytes(capacity, true));
     const uint64_t sentinel = ((uint64_t)R << 32) | (uint64_t)R;
-    DM_COUNT_LAUNCH(); merge::rekey_kernel<<<grid_for(capacity), 256, 0, s>>>(parent, keys, lens, n_dev, sentinel,
-                                                           (unsigned long long*)perimeter, nk, perm);
+    DM_TRY(launch(merge::rekey_kernel, grid_for(capacity), 256, 0, s, parent, keys, lens, n_dev, sentinel,
+        (unsigned long long*)perimeter, nk, perm));
     const int b = bits_for(R + 1);
     int64_t* n_new = c.take<int64_t>(1);
-    DM_TRY(prims::sort_unique(nk, perm, n_dev, capacity, b, 2 * b, sws, lens, scores, sentinel, ok, ol, scores ? os : nullptr,
-                              n_new, keys, lens, scores, n_dev, s, R));
-    DM_LAUNCH_CHECK();
-    return DM_OK;
+    return prims::sort_unique(nk, perm, n_dev, capacity, b, 2 * b, sws, lens, scores, sentinel, ok, ol, scores ? os : nullptr,
+                              n_new, keys, lens, scores, n_dev, s, R);
 }
 
 extern "C" int dm_relabel_gated(const int32_t* labels, int64_t H, int64_t W, int64_t ld_in, const int32_t* root, int64_t R,
@@ -833,14 +786,12 @@ extern "C" int dm_relabel_gated(const int32_t* labels, int64_t H, int64_t W, int
     const int64_t n = H * W;
     if (dense && n % 4 == 0 && (uintptr_t)labels % 16 == 0 && (uintptr_t)out % 16 == 0) {
         const int64_t n4 = n / 4;
-        // 4 x 16 B per thread per trip; grid sized to a whole number of waves of the SM count
-        const unsigned g = (unsigned)imax64(1, imin64(ceil_div(n4, 256 * 4), (int64_t)num_sms() * 8));
-        DM_COUNT_LAUNCH(); merge::relabel_vec_kernel<<<g, 256, 0, s>>>((const int4*)labels, n4, root, (int)R, (int4*)out, skip_if_nonzero);
-    } else {
-        DM_COUNT_LAUNCH(); merge::relabel_scalar_kernel<<<grid_for(n), 256, 0, s>>>(labels, H, W, ld_in, root, (int)R, out, ld_out, skip_if_nonzero);
+        // 4 x 16 B per thread per trip: a block covers 1024 int4
+        return launch(merge::relabel_vec_kernel, grid_for(n4, 1024), 256, 0, s, (const int4*)labels, n4, root, (int)R,
+            (int4*)out, skip_if_nonzero);
     }
-    DM_LAUNCH_CHECK();
-    return DM_OK;
+    return launch(merge::relabel_scalar_kernel, grid_for(n), 256, 0, s, labels, H, W, ld_in, root, (int)R, out, ld_out,
+        skip_if_nonzero);
 }
 
 extern "C" int dm_relabel(const int32_t* labels, int64_t H, int64_t W, int64_t ld_in, const int32_t* root, int64_t R,
@@ -868,24 +819,19 @@ extern "C" int dm_compact_roots(const int32_t* root, int64_t R, int32_t* compact
     uint32_t* excl = c.take<uint32_t>(R);
     void* sws = c.take<char>(prims::scan_ws_bytes(R));
     int64_t* n_dev = c.take<int64_t>(1);
-    DM_COUNT_LAUNCH(); merge::root_flags_kernel<<<grid_for(R), 256, 0, s>>>(root, R, flags, n_dev);
+    DM_TRY(launch(merge::root_flags_kernel, grid_for(R), 256, 0, s, root, R, flags, n_dev));
     DM_TRY(prims::scan_exclusive_u32(flags, excl, n_dev, R, n_roots, sws, s));
-    DM_COUNT_LAUNCH(); merge::compact_kernel<<<grid_for(R), 256, 0, s>>>(root, R, excl, compact);
-    DM_LAUNCH_CHECK();
-    return DM_OK;
+    return launch(merge::compact_kernel, grid_for(R), 256, 0, s, root, R, excl, compact);
 }
 
 extern "C" int dm_perimeter(const uint64_t* keys, const uint32_t* lens, const int64_t* n_dev, int64_t capacity,
                             const int64_t* border, int64_t* perimeter, int64_t R, dm_stream_t stream) {
     if (capacity < 0 || R < 0) return DM_ERR_BAD_ARG;
     if (R == 0) return DM_OK;
-    if (!border || !perimeter) return DM_ERR_BAD_ARG;
+    if (!border || !perimeter || (capacity > 0 && (!keys || !lens || !n_dev))) return DM_ERR_BAD_ARG;
     cudaStream_t s = S(stream);
-    DM_COUNT_LAUNCH(); merge::perimeter_init_kernel<<<grid_for(R), 256, 0, s>>>(border, perimeter, R);
-    if (capacity > 0) {
-        if (!keys || !lens || !n_dev) return DM_ERR_BAD_ARG;
-        DM_COUNT_LAUNCH(); merge::perimeter_edges_kernel<<<grid_for(capacity), 256, 0, s>>>(keys, lens, n_dev, (unsigned long long*)perimeter, R);
-    }
-    DM_LAUNCH_CHECK();
-    return DM_OK;
+    DM_TRY(launch(merge::perimeter_init_kernel, grid_for(R), 256, 0, s, border, perimeter, R));
+    if (capacity == 0) return DM_OK;
+    return launch(merge::perimeter_edges_kernel, grid_for(capacity), 256, 0, s, keys, lens, n_dev,
+        (unsigned long long*)perimeter, R);
 }

@@ -519,14 +519,10 @@ static int check_dims(int64_t in_features, int64_t hidden, int64_t n_out) {
     return DM_OK;
 }
 
-static int launch(const Params& P, int64_t rows_cap, cudaStream_t s) {
-    auto k = pair_mlp_kernel;
-    DM_CUDA(cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM_BYTES));
+static int run(const Params& P, int64_t rows_cap, cudaStream_t s) {
     const int64_t tiles = ceil_div(rows_cap, M_TILE);
     const int grid = (int)imax64(1, imin64(tiles, num_sms()));
-    DM_COUNT_LAUNCH(); k<<<grid, THREADS, SMEM_BYTES, s>>>(P);
-    DM_LAUNCH_CHECK();
-    return DM_OK;
+    return launch(pair_mlp_kernel, grid, THREADS, SMEM_BYTES, s, P);
 }
 
 }  // namespace mlp
@@ -552,10 +548,8 @@ extern "C" int dm_mlp_pack(const float* W1, const float* b1, const float* W2, co
     const int nk1 = (int)mlp::nk_for(in_features);
     cudaStream_t s = S(stream);
     DM_CUDA(cudaMemsetAsync((unsigned char*)packed + mlp::packed_bytes(nk1), 0, 16, s));
-    DM_COUNT_LAUNCH(); mlp::pack_kernel<<<num_sms() * 4, 256, 0, s>>>(W1, b1, W2, b2, W3, b3, (int)in_features, (int)hidden,
-                                                                    (int)n_out, nk1, (unsigned char*)packed);
-    DM_LAUNCH_CHECK();
-    return DM_OK;
+    return launch(mlp::pack_kernel, num_sms() * 4, 256, 0, s, W1, b1, W2, b2, W3, b3, (int)in_features, (int)hidden,
+                  (int)n_out, nk1, (unsigned char*)packed);
 }
 
 extern "C" int dm_score_mlp_bf16(const float* mean, int64_t D, const uint64_t* edge_keys, const int64_t* n_edges_dev,
@@ -580,7 +574,7 @@ extern "C" int dm_score_mlp_bf16(const float* mean, int64_t D, const uint64_t* e
     P.o = o;
     P.h2 = h2;
     P.status = (int*)((unsigned char*)packed + mlp::packed_bytes(P.nk1));
-    return mlp::launch(P, capacity, S(stream));
+    return mlp::run(P, capacity, S(stream));
 }
 
 extern "C" int dm_mlp_forward_bf16(const float* x, int64_t B, const void* packed, int64_t in_features, int64_t hidden,
@@ -604,5 +598,5 @@ extern "C" int dm_mlp_forward_bf16(const float* x, int64_t B, const void* packed
     P.o = o;
     P.h2 = h2;
     P.status = (int*)((unsigned char*)packed + mlp::packed_bytes(P.nk1));
-    return mlp::launch(P, B, S(stream));
+    return mlp::run(P, B, S(stream));
 }

@@ -244,10 +244,6 @@ __global__ void __launch_bounds__(NT) vertex_kernel(const int64_t* __restrict__ 
     }
 }
 
-unsigned grid_for(int64_t threads) {
-    return (unsigned)imax64(1, imin64(ceil_div(threads, NT), (int64_t)num_sms() * 16));
-}
-
 int ceil_log2(int64_t x) {
     int b = 0;
     while (((int64_t)1 << b) < x) ++b;
@@ -292,34 +288,30 @@ extern "C" int dm_polygonize(const int32_t* labels, int64_t H, int64_t W, int64_
     DM_CUDA(cudaMemsetAsync(counts, 0, 4 * sizeof(int64_t), s));
     DM_CUDA(cudaMemsetAsync(w.changed, 0, 2 * poly::MAX_PASSES * sizeof(int), s));
     if (ring_cap) DM_CUDA(cudaMemsetAsync(ring_area, 0, (size_t)ring_cap * sizeof(int64_t), s));
-    const unsigned g_words = poly::grid_for(n_words * 32), g_sides = poly::grid_for(capacity);
-    const unsigned g_rings = poly::grid_for(ring_cap + 1);
-    DM_COUNT_LAUNCH(); poly::mask_kernel<<<g_words, poly::NT, 0, s>>>(labels, H, W, ld, wpr, n_regions, w.masks, w.wcnt,
-                                                                      counts, w.n_words_dev);
+    const unsigned g_words = grid_for(n_words * 32, poly::NT, 16), g_sides = grid_for(capacity, poly::NT, 16);
+    const unsigned g_rings = grid_for(ring_cap + 1, poly::NT, 16);
+    DM_TRY(launch(poly::mask_kernel, g_words, poly::NT, 0, s, labels, H, W, ld, wpr, n_regions, w.masks, w.wcnt, counts,
+        w.n_words_dev));
     DM_TRY(prims::scan_exclusive_u32(w.wcnt, w.wbase, w.n_words_dev, n_words, nullptr, w.scan, s));
-    DM_COUNT_LAUNCH(); poly::emit_kernel<<<g_words, poly::NT, 0, s>>>(labels, H, W, ld, wpr, capacity, w.masks, w.wbase,
-                                                                      counts, w);
+    DM_TRY(launch(poly::emit_kernel, g_words, poly::NT, 0, s, labels, H, W, ld, wpr, capacity, w.masks, w.wbase, counts, w));
     const int passes = poly::ceil_log2(capacity) + 1;
     for (int phase = 0; phase < 2; ++phase) {
         for (int k = 0; k < passes; ++k) {
-            DM_COUNT_LAUNCH(); poly::jump_kernel<<<g_sides, poly::NT, 0, s>>>(w.jw, counts, w.changed, phase, k);
+            DM_TRY(launch(poly::jump_kernel, g_sides, poly::NT, 0, s, w.jw, counts, w.changed, phase, k));
         }
         if (phase == 0) {
-            DM_COUNT_LAUNCH(); poly::starts_kernel<<<g_sides, poly::NT, 0, s>>>(counts, ring_cap, w);
+            DM_TRY(launch(poly::starts_kernel, g_sides, poly::NT, 0, s, counts, ring_cap, w));
         }
     }
-    DM_LAUNCH_CHECK();
     // rings in raster order of their start vertex, then stably by region
     DM_TRY(prims::sort_pairs(w.rkeys, w.rvals, counts, ring_cap, bits_for((H + 1) * (W + 1)), bits_for((H + 1) * (W + 1)),
                              w.sort, s));
-    DM_COUNT_LAUNCH(); poly::region_keys_kernel<<<g_rings, poly::NT, 0, s>>>(counts, w);
+    DM_TRY(launch(poly::region_keys_kernel, g_rings, poly::NT, 0, s, counts, w));
     const int rb = bits_for(n_regions + 1);
     DM_TRY(prims::sort_pairs(w.rkeys, w.rvals, counts, ring_cap, rb, rb, w.sort, s, n_regions + 1, region_rings, nullptr));
     if (ring_cap == 0) DM_CUDA(cudaMemsetAsync(region_rings, 0, (size_t)(n_regions + 1) * sizeof(int64_t), s));
-    DM_COUNT_LAUNCH(); poly::ring_info_kernel<<<g_rings, poly::NT, 0, s>>>(counts, ring_region, w);
+    DM_TRY(launch(poly::ring_info_kernel, g_rings, poly::NT, 0, s, counts, ring_region, w));
     DM_TRY(prims::scan_exclusive_u32(w.ccount, w.offs, counts, ring_cap, counts + 1, w.scan, s));
-    DM_COUNT_LAUNCH(); poly::vertex_kernel<<<imax64(g_sides, g_rings), poly::NT, 0, s>>>(counts, W, w, vertices,
-                                                                                         ring_offsets, ring_area);
-    DM_LAUNCH_CHECK();
-    return DM_OK;
+    return launch(poly::vertex_kernel, imax64(g_sides, g_rings), poly::NT, 0, s, counts, W, w, vertices, ring_offsets,
+        ring_area);
 }

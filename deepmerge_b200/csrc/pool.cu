@@ -304,12 +304,6 @@ __global__ void __launch_bounds__(256) cut_windows_kernel(const uint8_t* __restr
     }
 }
 
-static unsigned grid_for(int64_t work_items, int threads, int per_sm) {
-    int64_t g = ceil_div(work_items, threads);
-    int64_t cap = (int64_t)num_sms() * per_sm;
-    return (unsigned)imax64(1, min(g, cap));
-}
-
 // N2: bounding boxes of the regions (for the designed attributes len / width / smooth / compact / border, MyUtils1.py:79-114).
 // A warp walks down a 32-pixel column strip; a lane keeps the vertical run of its column (label, first row) and publishes
 // it with four integer atomics when the label changes: min / max column, first / last row.
@@ -365,9 +359,7 @@ extern "C" int dm_points_region(const int32_t* labels, int64_t H, int64_t W, int
     if (n < 0 || H < 0 || W < 0 || ld < W) return DM_ERR_BAD_ARG;
     if (n == 0) return DM_OK;
     if (!labels || !xs || !ys || !out) return DM_ERR_BAD_ARG;
-    DM_COUNT_LAUNCH(); pool::points_region_kernel<<<pool::grid_for(n, 256, 8), 256, 0, S(stream)>>>(labels, H, W, ld, xs, ys, n, out);
-    DM_LAUNCH_CHECK();
-    return DM_OK;
+    return launch(pool::points_region_kernel, grid_for(n), 256, 0, S(stream), labels, H, W, ld, xs, ys, n, out);
 }
 
 extern "C" size_t dm_csr_workspace_bytes(int64_t n_points, int64_t n_regions) {
@@ -392,21 +384,30 @@ extern "C" int dm_csr_build(const int32_t* rop, int64_t n, int64_t R, int64_t* o
     uint32_t* vals = c.take<uint32_t>(n);
     int64_t* n_dev = c.take<int64_t>(1);
     void* sws = c.take<char>(prims::ws_bytes(n, false, R + 1));
-    const unsigned g = pool::grid_for(n, 256, 8);
-    DM_COUNT_LAUNCH(); pool::csr_keys_kernel<<<g, 256, 0, s>>>(rop, n, R, keys, vals, n_dev);
+    DM_TRY(launch(pool::csr_keys_kernel, grid_for(n), 256, 0, s, rop, n, R, keys, vals, n_dev));
     // stable sort by region only (input is in ascending point id): low bits_for(R+1) bits
     const int b = bits_for(R + 1);
     // bucket + rank in one cooperative launch, offsets and point ids included
-    DM_TRY(prims::sort_pairs(keys, vals, n_dev, n, b, b, sws, s, R + 1, offsets, point_ids));
-    DM_LAUNCH_CHECK();
-    return DM_OK;
+    return prims::sort_pairs(keys, vals, n_dev, n, b, b, sws, s, R + 1, offsets, point_ids);
 }
 
 template <int K>
-static void launch_pool_points(const int64_t* offsets, const int32_t* ids, const float* feats, int64_t ld, int64_t R,
-                               int D, int d_base, float* sum, int32_t* cnt, const int64_t* range, cudaStream_t s,
-                               float* mean = nullptr, float* norm2 = nullptr) {
-    DM_COUNT_LAUNCH(); pool::pool_points_kernel<K><<<pool::grid_for(R * 32, 256, 8), 256, 0, s>>>(offsets, ids, feats, ld, R, D, d_base, sum, cnt, range, mean, norm2);
+static int pool_points_groups(const int64_t* offsets, const int32_t* ids, const float* feats, int64_t ld, int64_t R, int D,
+                              int d0, float* sum, int32_t* cnt, const int64_t* range, float* mean, float* norm2,
+                              cudaStream_t s) {
+    return launch(pool::pool_points_kernel<K>, grid_for(R * 32), 256, 0, s, offsets, ids, feats, ld, R, D, d0, sum, cnt, range,
+                  mean, norm2);
+}
+
+// One pass of the pooling kernel over feature columns [d0, min(D, d0 + 128)): K = 1..4 groups of 32 columns.
+static int pool_points_pass(const int64_t* offsets, const int32_t* ids, const float* feats, int64_t ld, int64_t R, int D,
+                            int d0, float* sum, int32_t* cnt, const int64_t* range, float* mean, float* norm2,
+                            cudaStream_t s) {
+    const int rem = D - d0;
+    if (rem > 96) return pool_points_groups<4>(offsets, ids, feats, ld, R, D, d0, sum, cnt, range, mean, norm2, s);
+    if (rem > 64) return pool_points_groups<3>(offsets, ids, feats, ld, R, D, d0, sum, cnt, range, mean, norm2, s);
+    if (rem > 32) return pool_points_groups<2>(offsets, ids, feats, ld, R, D, d0, sum, cnt, range, mean, norm2, s);
+    return pool_points_groups<1>(offsets, ids, feats, ld, R, D, d0, sum, cnt, range, mean, norm2, s);
 }
 
 extern "C" int dm_pool_points_csr_tile(const int64_t* offsets, const int32_t* ids, const float* feats, int64_t ld, int64_t R,
@@ -416,14 +417,8 @@ extern "C" int dm_pool_points_csr_tile(const int64_t* offsets, const int32_t* id
     if (!offsets || !sum || !cnt) return DM_ERR_BAD_ARG;
     cudaStream_t s = S(stream);
     if (region_range) DM_CUDA(cudaMemsetAsync(cnt, 0, (size_t)R * sizeof(int32_t), s));   // no points outside the range
-    for (int d0 = 0; d0 < D; d0 += 128) {
-        const int rem = (int)D - d0;
-        if (rem > 96) launch_pool_points<4>(offsets, ids, feats, ld, R, (int)D, d0, sum, cnt, region_range, s);
-        else if (rem > 64) launch_pool_points<3>(offsets, ids, feats, ld, R, (int)D, d0, sum, cnt, region_range, s);
-        else if (rem > 32) launch_pool_points<2>(offsets, ids, feats, ld, R, (int)D, d0, sum, cnt, region_range, s);
-        else launch_pool_points<1>(offsets, ids, feats, ld, R, (int)D, d0, sum, cnt, region_range, s);
-    }
-    DM_LAUNCH_CHECK();
+    for (int d0 = 0; d0 < D; d0 += 128)
+        DM_TRY(pool_points_pass(offsets, ids, feats, ld, R, (int)D, d0, sum, cnt, region_range, nullptr, nullptr, s));
     return DM_OK;
 }
 
@@ -433,13 +428,7 @@ extern "C" int dm_pool_points_csr_mean(const int64_t* offsets, const int32_t* id
     if (D > 128) return DM_ERR_UNSUPPORTED;                 // the row must fit one pass of the pooling kernel
     if (R == 0) return DM_OK;
     if (!offsets || !sum || !cnt || !mean || !norm2) return DM_ERR_BAD_ARG;
-    cudaStream_t s = S(stream);
-    if (D > 96) launch_pool_points<4>(offsets, ids, feats, ld, R, (int)D, 0, sum, cnt, nullptr, s, mean, norm2);
-    else if (D > 64) launch_pool_points<3>(offsets, ids, feats, ld, R, (int)D, 0, sum, cnt, nullptr, s, mean, norm2);
-    else if (D > 32) launch_pool_points<2>(offsets, ids, feats, ld, R, (int)D, 0, sum, cnt, nullptr, s, mean, norm2);
-    else launch_pool_points<1>(offsets, ids, feats, ld, R, (int)D, 0, sum, cnt, nullptr, s, mean, norm2);
-    DM_LAUNCH_CHECK();
-    return DM_OK;
+    return pool_points_pass(offsets, ids, feats, ld, R, (int)D, 0, sum, cnt, nullptr, mean, norm2, S(stream));
 }
 
 extern "C" int dm_pool_points_csr(const int64_t* offsets, const int32_t* ids, const float* feats, int64_t ld, int64_t R,
@@ -477,15 +466,12 @@ __global__ void id_range_init_kernel(long long* range) {
 
 extern "C" int dm_points_id_range(const int32_t* region_of_point, int64_t n_points, int64_t n_regions, int64_t* range,
                                   dm_stream_t stream) {
-    if (n_points < 0 || n_regions < 0 || !range) return DM_ERR_BAD_ARG;
+    if (n_points < 0 || n_regions < 0 || !range || (n_points > 0 && !region_of_point)) return DM_ERR_BAD_ARG;
     cudaStream_t s = S(stream);
-    DM_COUNT_LAUNCH(); pool::id_range_init_kernel<<<1, 1, 0, s>>>((long long*)range);
-    if (n_points > 0) {
-        if (!region_of_point) return DM_ERR_BAD_ARG;
-        DM_COUNT_LAUNCH(); pool::id_range_kernel<<<pool::grid_for(n_points, 256, 4), 256, 0, s>>>(region_of_point, n_points, n_regions, (long long*)range);
-    }
-    DM_LAUNCH_CHECK();
-    return DM_OK;
+    DM_TRY(launch(pool::id_range_init_kernel, 1, 1, 0, s, (long long*)range));
+    if (n_points == 0) return DM_OK;
+    return launch(pool::id_range_kernel, grid_for(n_points, 256, 4), 256, 0, s, region_of_point, n_points, n_regions,
+        (long long*)range);
 }
 
 extern "C" int dm_region_mean(const float* sum, const int32_t* cnt, int64_t R, int64_t D, float* mean, float* norm2,
@@ -493,9 +479,8 @@ extern "C" int dm_region_mean(const float* sum, const int32_t* cnt, int64_t R, i
     if (R < 0 || D <= 0) return DM_ERR_BAD_ARG;
     if (R == 0) return DM_OK;
     if (!sum || !cnt || !mean || !norm2) return DM_ERR_BAD_ARG;
-    DM_COUNT_LAUNCH(); pool::region_mean_kernel<<<pool::grid_for(R * 32, 256, 8), 256, 0, S(stream)>>>(sum, cnt, R, (int)D, mean, norm2, only);
-    DM_LAUNCH_CHECK();
-    return DM_OK;
+    return launch(pool::region_mean_kernel, grid_for(R * 32), 256, 0, S(stream), sum, cnt, R, (int)D, mean, norm2,
+        only);
 }
 
 template <typename T>
@@ -503,20 +488,19 @@ static int pool_dense_t(const int32_t* labels, int64_t H, int64_t W, int64_t ld,
                         float* sum, int32_t* cnt, cudaStream_t s) {
     const int chunk = 64;
     const int64_t warps = H * ceil_div(W, chunk);
-    const unsigned g = pool::grid_for(warps * 32, 256, 8);
+    const unsigned g = grid_for(warps * 32);
     for (int d0 = 0; d0 < D; d0 += 128) {
         const int rem = (int)D - d0;
         if (rem > 96) {
-            DM_COUNT_LAUNCH(); pool::pool_dense_kernel<T, 4><<<g, 256, 0, s>>>(labels, H, W, ld, emb, (int)D, d0, R, sum, cnt, chunk);
+            DM_TRY(launch(pool::pool_dense_kernel<T, 4>, g, 256, 0, s, labels, H, W, ld, emb, (int)D, d0, R, sum, cnt, chunk));
         } else if (rem > 64) {
-            DM_COUNT_LAUNCH(); pool::pool_dense_kernel<T, 3><<<g, 256, 0, s>>>(labels, H, W, ld, emb, (int)D, d0, R, sum, cnt, chunk);
+            DM_TRY(launch(pool::pool_dense_kernel<T, 3>, g, 256, 0, s, labels, H, W, ld, emb, (int)D, d0, R, sum, cnt, chunk));
         } else if (rem > 32) {
-            DM_COUNT_LAUNCH(); pool::pool_dense_kernel<T, 2><<<g, 256, 0, s>>>(labels, H, W, ld, emb, (int)D, d0, R, sum, cnt, chunk);
+            DM_TRY(launch(pool::pool_dense_kernel<T, 2>, g, 256, 0, s, labels, H, W, ld, emb, (int)D, d0, R, sum, cnt, chunk));
         } else {
-            DM_COUNT_LAUNCH(); pool::pool_dense_kernel<T, 1><<<g, 256, 0, s>>>(labels, H, W, ld, emb, (int)D, d0, R, sum, cnt, chunk);
+            DM_TRY(launch(pool::pool_dense_kernel<T, 1>, g, 256, 0, s, labels, H, W, ld, emb, (int)D, d0, R, sum, cnt, chunk));
         }
     }
-    DM_LAUNCH_CHECK();
     return DM_OK;
 }
 
@@ -538,16 +522,12 @@ extern "C" int dm_pool_boundary(const int32_t* labels, int64_t rows_own, int64_t
     if (rows_own == 0 || W == 0 || capacity == 0) return DM_OK;
     if (!labels || !emb || !edge_keys || !n_edges_dev || !bsum || !bcnt) return DM_ERR_BAD_ARG;
     cudaStream_t s = S(stream);
-    const unsigned g = pool::grid_for(rows_own * ceil_div(W, 32) * 32, 256, 8);
-    if (dtype_bf16) {
-        DM_COUNT_LAUNCH(); pool::pool_boundary_kernel<__nv_bfloat16><<<g, 256, 0, s>>>(labels, rows_own, W, ld, rows_avail, (const __nv_bfloat16*)emb,
-                                                                        (int)D, edge_keys, n_edges_dev, bsum, bcnt);
-    } else {
-        DM_COUNT_LAUNCH(); pool::pool_boundary_kernel<float><<<g, 256, 0, s>>>(labels, rows_own, W, ld, rows_avail, (const float*)emb, (int)D,
-                                                                edge_keys, n_edges_dev, bsum, bcnt);
-    }
-    DM_LAUNCH_CHECK();
-    return DM_OK;
+    const unsigned g = grid_for(rows_own * ceil_div(W, 32) * 32);
+    if (dtype_bf16)
+        return launch(pool::pool_boundary_kernel<__nv_bfloat16>, g, 256, 0, s, labels, rows_own, W, ld, rows_avail,
+            (const __nv_bfloat16*)emb, (int)D, edge_keys, n_edges_dev, bsum, bcnt);
+    return launch(pool::pool_boundary_kernel<float>, g, 256, 0, s, labels, rows_own, W, ld, rows_avail, (const float*)emb,
+        (int)D, edge_keys, n_edges_dev, bsum, bcnt);
 }
 
 extern "C" int dm_cut_windows(const uint8_t* image, int64_t C, int64_t H, int64_t W, const int32_t* x0, const int32_t* y0,
@@ -555,27 +535,22 @@ extern "C" int dm_cut_windows(const uint8_t* image, int64_t C, int64_t H, int64_
     if (C < 1 || H < 0 || W < 0 || n < 0 || size < 1 || size > (1 << 14)) return DM_ERR_BAD_ARG;
     if (n == 0) return DM_OK;
     if (!image || !x0 || !y0 || !out) return DM_ERR_BAD_ARG;
-    DM_COUNT_LAUNCH(); pool::cut_windows_kernel<<<pool::grid_for(n * C * size * 32, 256, 8), 256, 0, S(stream)>>>(image, (int)C, H, W, x0, y0, n,
-                                                                                           (int)size, out);
-    DM_LAUNCH_CHECK();
-    return DM_OK;
+    return launch(pool::cut_windows_kernel, grid_for(n * C * size * 32), 256, 0, S(stream), image, (int)C, H, W, x0,
+        y0, n, (int)size, out);
 }
 
 extern "C" int dm_region_bbox(const int32_t* labels, int64_t H, int64_t W, int64_t ld, int64_t n_regions, int32_t* bbox,
                               int64_t* bad_label, dm_stream_t stream) {
     if (H < 0 || W < 0 || ld < W || n_regions < 0 || H > 0x7ffffff0 || W > 0x7ffffff0) return DM_ERR_BAD_ARG;
+    const bool pixels = H > 0 && W > 0;
+    if (n_regions > 0 && (!bbox || !bad_label || (pixels && !labels))) return DM_ERR_BAD_ARG;
     cudaStream_t s = S(stream);
     if (bad_label) DM_CUDA(cudaMemsetAsync(bad_label, 0, sizeof(int64_t), s));
     if (n_regions == 0) return DM_OK;
-    if (!bbox || !bad_label) return DM_ERR_BAD_ARG;
-    DM_COUNT_LAUNCH(); pool::region_bbox_init_kernel<<<pool::grid_for(n_regions, 256, 8), 256, 0, s>>>(bbox, n_regions);
-    if (H > 0 && W > 0) {
-        if (!labels) return DM_ERR_BAD_ARG;
-        const int rows_per_warp = 128;
-        const int64_t warps = ceil_div(W, 32) * ceil_div(H, rows_per_warp);
-        DM_COUNT_LAUNCH(); pool::region_bbox_kernel<<<pool::grid_for(warps * 32, 256, 8), 256, 0, s>>>(
-            labels, H, W, ld, n_regions, bbox, rows_per_warp, (unsigned long long*)bad_label);
-    }
-    DM_LAUNCH_CHECK();
-    return DM_OK;
+    DM_TRY(launch(pool::region_bbox_init_kernel, grid_for(n_regions), 256, 0, s, bbox, n_regions));
+    if (!pixels) return DM_OK;
+    const int rows_per_warp = 128;
+    const int64_t warps = ceil_div(W, 32) * ceil_div(H, rows_per_warp);
+    return launch(pool::region_bbox_kernel, grid_for(warps * 32), 256, 0, s, labels, H, W, ld, n_regions, bbox, rows_per_warp,
+        (unsigned long long*)bad_label);
 }

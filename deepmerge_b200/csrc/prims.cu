@@ -85,11 +85,9 @@ int scan_exclusive_u32(const uint32_t* in, uint32_t* out, const int64_t* n_dev, 
     }
     uint32_t* tile_sum = (uint32_t*)ws;
     const unsigned tiles = (unsigned)ceil_div(cap, SCAN_TILE);
-    DM_COUNT_LAUNCH(); scan_tile_sums<<<tiles, SCAN_THREADS, 0, s>>>(in, n_dev, tile_sum);
-    DM_COUNT_LAUNCH(); scan_tile_offsets<<<1, 1024, 0, s>>>(tile_sum, n_dev, total_dev);
-    DM_COUNT_LAUNCH(); scan_apply<<<tiles, SCAN_THREADS, 0, s>>>(in, out, n_dev, tile_sum);
-    DM_LAUNCH_CHECK();
-    return DM_OK;
+    DM_TRY(launch(scan_tile_sums, tiles, SCAN_THREADS, 0, s, in, n_dev, tile_sum));
+    DM_TRY(launch(scan_tile_offsets, 1, 1024, 0, s, tile_sum, n_dev, total_dev));
+    return launch(scan_apply, tiles, SCAN_THREADS, 0, s, in, out, n_dev, tile_sum);
 }
 
 // ------------------------------------------------------------------------------------ //
@@ -926,20 +924,18 @@ int coop_grid_limit(const void* kernel, int per_sm_cap) {
 // Zeroes the grid barrier words (and, when given, the hub count and fall-back flag of misc) and launches `kernel`
 // cooperatively on `grid` blocks.  grid < 1 means the device has no cooperative launch: DM_ERR_UNSUPPORTED.  A refused
 // launch is DM_ERR_CUDA with the CUDA error recorded; there is no other path to fall back to.
-int launch_coop(const void* kernel, int64_t grid, void** args, unsigned* bar, unsigned* misc, cudaStream_t s) {
+template <typename... P>
+int launch_coop(void (*kernel)(P...), int64_t grid, unsigned* bar, unsigned* misc, cudaStream_t s, const P&... args) {
     if (grid < 1) return DM_ERR_UNSUPPORTED;
     DM_CUDA(cudaMemsetAsync(bar, 0, 2 * sizeof(unsigned), s));
     if (misc) DM_CUDA(cudaMemsetAsync(misc, 0, 4 * sizeof(unsigned), s));
-    DM_COUNT_LAUNCH();
-    DM_CUDA(cudaLaunchCooperativeKernel(kernel, dim3((unsigned)grid), dim3(SORT_THREADS), args, 0, s));
-    return DM_OK;
+    return launch_cooperative(kernel, (unsigned)grid, SORT_THREADS, s, args...);
 }
 
 int launch_radix(FusedArgs& A, int64_t cap, cudaStream_t s) {
     // measured: a third block per SM costs more in the barriers than it saves in the phases
     const int64_t grid = imin64(ceil_div(cap, SORT_TILE), coop_grid_limit((const void*)radix_sort_fused, 2));
-    void* args[] = {(void*)&A};
-    return launch_coop((const void*)radix_sort_fused, grid, args, A.bar, nullptr, s);
+    return launch_coop(radix_sort_fused, grid, A.bar, nullptr, s, A);
 }
 }  // namespace
 
@@ -963,8 +959,7 @@ int sort_pairs(uint64_t* keys, uint32_t* vals, const int64_t* n_dev, int64_t cap
     // blocks, 26.4 at 592)
     const int64_t limit = imin64(coop_grid_limit((const void*)bucket_sort_fused, HASH_BLOCKS_PER_SM), HASH_MAX_GRID);
     const int64_t grid = imin64(imin64(ceil_div(imax64(cap, n_ids), SORT_THREADS), limit), 5 * num_sms() / 2);
-    void* args[] = {(void*)&H, (void*)&X};
-    return launch_coop((const void*)bucket_sort_fused, grid, args, H.F.bar, H.misc, s);
+    return launch_coop(bucket_sort_fused, grid, H.F.bar, H.misc, s, H, X);
 }
 
 int sort_unique(uint64_t* keys, uint32_t* vals, const int64_t* n_dev, int64_t cap, int id_bits, int key_bits, void* ws,
@@ -988,8 +983,7 @@ int sort_unique(uint64_t* keys, uint32_t* vals, const int64_t* n_dev, int64_t ca
         return launch_radix(A, cap, s);
     const int64_t limit = imin64(coop_grid_limit((const void*)edge_unique_hashed, HASH_BLOCKS_PER_SM), HASH_MAX_GRID);
     const int64_t grid = imin64(ceil_div(imax64(cap, n_ids), SORT_THREADS * 4), limit);
-    void* args[] = {(void*)&H};
-    DM_TRY(launch_coop((const void*)edge_unique_hashed, grid, args, A.bar, H.misc, s));
+    DM_TRY(launch_coop(edge_unique_hashed, grid, A.bar, H.misc, s, H));
     static const bool print_ts = getenv("DM_HASH_TS") != nullptr;
     if (print_ts) {                                        // profiling aid: phase boundaries seen by block 0 (ns)
         unsigned long long t[6];

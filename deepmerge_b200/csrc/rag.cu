@@ -94,11 +94,14 @@ extern "C" int dm_rag_scan(const int32_t* labels, int64_t rows_own, int64_t rows
     if (!image) C = 0;
     if (C < 0 || C > 4) return DM_ERR_BAD_ARG;
     if (C > 0 && (!band_sum || !band_sumsq || image_pitch < W * C)) return DM_ERR_BAD_ARG;
+    const bool empty = rows_own == 0 || W == 0;
+    if (!empty) {
+        if (!labels || !area || !border || !ws) return DM_ERR_BAD_ARG;
+        if (ws_bytes < dm_rag_workspace_bytes(capacity)) return DM_ERR_WORKSPACE;
+    }
     cudaStream_t s = S(stream);
     DM_CUDA(cudaMemsetAsync(counts, 0, 4 * sizeof(int64_t), s));
-    if (rows_own == 0 || W == 0) return DM_OK;
-    if (!labels || !area || !border || !ws) return DM_ERR_BAD_ARG;
-    if (ws_bytes < dm_rag_workspace_bytes(capacity)) return DM_ERR_WORKSPACE;
+    if (empty) return DM_OK;
     RagWs w = carve_rag_ws(ws, capacity);
     rag::Params P;
     P.labels = labels;
@@ -133,10 +136,8 @@ extern "C" int dm_rag_finish(uint64_t* edge_keys, uint32_t* boundary_len, int64_
     RagWs w = carve_rag_ws(ws, capacity);
     const int b = bits_for(n_regions);
     // counts[1] may exceed capacity (an overflowed raw list): sort_unique reads min(counts[1], capacity) entries
-    DM_TRY(prims::sort_unique(w.raw_keys, w.raw_cnt, counts + 1, capacity, b, 2 * b, w.sws, nullptr, nullptr, ~0ull,
-                              edge_keys, boundary_len, nullptr, counts, nullptr, nullptr, nullptr, nullptr, s, n_regions));
-    DM_LAUNCH_CHECK();
-    return DM_OK;
+    return prims::sort_unique(w.raw_keys, w.raw_cnt, counts + 1, capacity, b, 2 * b, w.sws, nullptr, nullptr, ~0ull,
+                              edge_keys, boundary_len, nullptr, counts, nullptr, nullptr, nullptr, nullptr, s, n_regions);
 }
 
 extern "C" int dm_rag_build(const int32_t* labels, int64_t rows_own, int64_t rows_avail, int64_t W, int64_t ld,
@@ -194,11 +195,8 @@ extern "C" int dm_edges_concat(const uint64_t* src_keys, const uint32_t* src_len
         return DM_OK;
     }
     if (!src_keys || !src_lens || !counts || !dst_keys || !dst_lens) return DM_ERR_BAD_ARG;
-    const unsigned g = (unsigned)imax64(1, imin64(ceil_div(n_lists * slot_capacity, 256), (int64_t)num_sms() * 8));
-    DM_COUNT_LAUNCH(); rag::concat_kernel<<<g, 256, 0, s>>>(src_keys, src_lens, counts, (int)n_lists, slot_capacity, dst_keys,
-                                                         dst_lens, dst_capacity, n_out_dev);
-    DM_LAUNCH_CHECK();
-    return DM_OK;
+    return launch(rag::concat_kernel, grid_for(n_lists * slot_capacity), 256, 0, s, src_keys, src_lens, counts, (int)n_lists,
+        slot_capacity, dst_keys, dst_lens, dst_capacity, n_out_dev);
 }
 
 extern "C" size_t dm_edges_unique_workspace_bytes(int64_t capacity) {
@@ -222,8 +220,6 @@ extern "C" int dm_edges_sort_unique(uint64_t* keys, uint32_t* lens, const int64_
     int64_t* n_new = c.take<int64_t>(1);
     void* sws = c.take<char>(prims::ws_bytes(capacity, true));
     const int b = bits_for(n_regions);
-    DM_TRY(prims::sort_unique(keys, lens, n_in, capacity, b, 2 * b, sws, nullptr, nullptr, ~0ull, ok, ol, nullptr, n_new,
-                              keys, lens, nullptr, n_out, s, n_regions));
-    DM_LAUNCH_CHECK();
-    return DM_OK;
+    return prims::sort_unique(keys, lens, n_in, capacity, b, 2 * b, sws, nullptr, nullptr, ~0ull, ok, ol, nullptr, n_new,
+                              keys, lens, nullptr, n_out, s, n_regions);
 }

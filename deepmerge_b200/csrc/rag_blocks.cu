@@ -335,7 +335,7 @@ rag_blocks_kernel(const __grid_constant__ CUtensorMap mapL, const __grid_constan
 }
 
 template <typename CF>
-static int launch(const Params& Pin, cudaStream_t s) {
+static int run(const Params& Pin, cudaStream_t s) {
     Params P = Pin;
     P.tiles_x = (int)ceil_div(P.W, STRIP_W);            // strips
     P.tiles_y = (int)ceil_div(P.rows_avail, CF::TH);    // units per strip (a halo row below counts)
@@ -361,17 +361,8 @@ static int launch(const Params& Pin, cudaStream_t s) {
         tma = make_map_2d(&mapI, P.image, (uint64_t)P.W * CF::C / 4, (uint64_t)P.rows_own, (uint64_t)P.image_pitch,
                           CF::IMG_ROW_WORDS, CF::TH);
     set_last_path(tma ? 1 : 0);
-    if (tma) {
-        auto k = rag_blocks_kernel<CF, true>;
-        DM_CUDA(cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, CF::SMEM_BYTES));
-        DM_COUNT_LAUNCH(); k<<<grid, CF::THREADS, CF::SMEM_BYTES, s>>>(mapL, mapI, P);
-    } else {
-        auto k = rag_blocks_kernel<CF, false>;
-        DM_CUDA(cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, CF::SMEM_BYTES));
-        DM_COUNT_LAUNCH(); k<<<grid, CF::THREADS, CF::SMEM_BYTES, s>>>(mapL, mapI, P);
-    }
-    DM_LAUNCH_CHECK();
-    return DM_OK;
+    return launch(tma ? rag_blocks_kernel<CF, true> : rag_blocks_kernel<CF, false>, grid, CF::THREADS, CF::SMEM_BYTES, s,
+                  mapL, mapI, P);
 }
 
 }  // namespace blk
@@ -380,11 +371,11 @@ static int launch(const Params& Pin, cudaStream_t s) {
 int run_blocks(const Params& P, int C, cudaStream_t s) {
     using namespace blk;
     switch (C) {
-        case 0: return launch<Cfg<0, 8, 2, 14, 48>>(P, s);
-        case 1: return launch<Cfg<1, 4, 2, 16, 48>>(P, s);
-        case 2: return launch<Cfg<2, 4, 2, 14, 48>>(P, s);
-        case 3: return launch<Cfg<3, 4, 2, 12, 48>>(P, s);
-        case 4: return launch<Cfg<4, 4, 2, 12, 48>>(P, s);
+        case 0: return run<Cfg<0, 8, 2, 14, 48>>(P, s);
+        case 1: return run<Cfg<1, 4, 2, 16, 48>>(P, s);
+        case 2: return run<Cfg<2, 4, 2, 14, 48>>(P, s);
+        case 3: return run<Cfg<3, 4, 2, 12, 48>>(P, s);
+        case 4: return run<Cfg<4, 4, 2, 12, 48>>(P, s);
         default: return DM_ERR_BAD_ARG;
     }
 }

@@ -53,10 +53,7 @@ extern "C" int dm_resize_area(const uint8_t* patches, int64_t n_planes, int64_t 
     if (mode == 1) {
         smem = (size_t)s * t * sizeof(float);
         if (smem > 200 * 1024) return DM_ERR_UNSUPPORTED;     // rows of one plane must fit in shared memory
-        if (smem > 48 * 1024)
-            DM_CUDA(cudaFuncSetAttribute(resize::resize_area_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
     }
-    DM_COUNT_LAUNCH(); resize::resize_area_kernel<<<(unsigned)n_planes, 256, smem, S(stream)>>>(patches, (int)s, (int)t, mode, ti, tf, out);
-    DM_LAUNCH_CHECK();
-    return DM_OK;
+    return launch(resize::resize_area_kernel, (unsigned)n_planes, 256, smem, S(stream), patches, (int)s, (int)t, mode, ti, tf,
+                  out);
 }

@@ -125,16 +125,11 @@ extern "C" int dm_score_l2(const float* mean, const float* norm2, int64_t D, con
     if (D <= 0 || capacity < 0) return DM_ERR_BAD_ARG;
     if (capacity == 0) return DM_OK;
     if (!mean || !norm2 || !keys || !n_dev || !scores) return DM_ERR_BAD_ARG;
-    if (D % 4 == 0 && (uintptr_t)mean % 16 == 0) {
-        const int64_t g = imin64(ceil_div(capacity * 8, 256), (int64_t)num_sms() * 8);
-        DM_COUNT_LAUNCH(); score::score_l2_vec_kernel<<<(unsigned)imax64(g, 1), 256, 0, S(stream)>>>(mean, norm2, (int)(D / 4), keys, n_dev,
-                                                                                  rescore, scores);
-    } else {
-        const int64_t g = imin64(ceil_div(capacity * 32, 256), (int64_t)num_sms() * 8);
-        DM_COUNT_LAUNCH(); score::score_l2_kernel<<<(unsigned)imax64(g, 1), 256, 0, S(stream)>>>(mean, norm2, (int)D, keys, n_dev, rescore, scores);
-    }
-    DM_LAUNCH_CHECK();
-    return DM_OK;
+    if (D % 4 == 0 && (uintptr_t)mean % 16 == 0)
+        return launch(score::score_l2_vec_kernel, grid_for(capacity * 8), 256, 0, S(stream), mean, norm2, (int)(D / 4), keys,
+            n_dev, rescore, scores);
+    return launch(score::score_l2_kernel, grid_for(capacity * 32), 256, 0, S(stream), mean, norm2, (int)D, keys, n_dev, rescore,
+        scores);
 }
 
 extern "C" int dm_euclidean_matrix(const float* X, const float* Y, int64_t n, int64_t m, int64_t p, float* Dm,
@@ -142,8 +137,5 @@ extern "C" int dm_euclidean_matrix(const float* X, const float* Y, int64_t n, in
     if (n < 0 || m < 0 || p < 0) return DM_ERR_BAD_ARG;
     if (n == 0 || m == 0) return DM_OK;
     if (!X || !Y || !Dm) return DM_ERR_BAD_ARG;
-    const int64_t g = imin64(ceil_div(n * m * 32, 256), (int64_t)num_sms() * 8);
-    DM_COUNT_LAUNCH(); score::euclid_matrix_kernel<<<(unsigned)imax64(g, 1), 256, 0, S(stream)>>>(X, Y, n, m, p, Dm);
-    DM_LAUNCH_CHECK();
-    return DM_OK;
+    return launch(score::euclid_matrix_kernel, grid_for(n * m * 32), 256, 0, S(stream), X, Y, n, m, p, Dm);
 }

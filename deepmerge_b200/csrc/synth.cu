@@ -138,10 +138,6 @@ __global__ void feats_kernel(float* __restrict__ feats, const int32_t* __restric
     }
 }
 
-static unsigned grid_for(int64_t items) {
-    return (unsigned)imax64(1, imin64(ceil_div(items, 256), (int64_t)num_sms() * 16));
-}
-
 }  // namespace synth
 }  // namespace dm
 
@@ -151,35 +147,30 @@ extern "C" int dm_synth_labels(int32_t* labels, int64_t y0, int64_t rows, int64_
                                uint32_t seed, dm_stream_t stream) {
     if (!labels || rows < 0 || W <= 0 || H <= 0 || g <= 0 || ld < W) return DM_ERR_BAD_ARG;
     if (rows == 0) return DM_OK;
-    DM_COUNT_LAUNCH(); synth::labels_kernel<<<synth::grid_for(rows * W), 256, 0, S(stream)>>>(labels, y0, rows, W, ld, synth::make_grid(H, W, g, seed));
-    DM_LAUNCH_CHECK();
-    return DM_OK;
+    return launch(synth::labels_kernel, grid_for(rows * W, 256, 16), 256, 0, S(stream), labels, y0, rows, W, ld,
+        synth::make_grid(H, W, g, seed));
 }
 
 extern "C" int dm_synth_region_objects(int32_t* region_obj, int64_t H, int64_t W, int64_t g, uint32_t seed, dm_stream_t stream) {
     if (!region_obj || W <= 0 || H <= 0 || g <= 0) return DM_ERR_BAD_ARG;
     synth::Grid G = synth::make_grid(H, W, g, seed), O = synth::make_grid(H, W, 4 * g, seed + 1);
-    DM_COUNT_LAUNCH(); synth::region_objects_kernel<<<synth::grid_for((int64_t)G.ncx * G.ncy), 256, 0, S(stream)>>>(region_obj, G, O);
-    DM_LAUNCH_CHECK();
-    return DM_OK;
+    return launch(synth::region_objects_kernel, grid_for((int64_t)G.ncx * G.ncy, 256, 16), 256, 0, S(stream), region_obj, G, O);
 }
 
 extern "C" int dm_synth_image(uint8_t* image, const int32_t* labels, int64_t y0, int64_t rows, int64_t W, int64_t ld,
                               int64_t C, const int32_t* region_obj, uint32_t seed, dm_stream_t stream) {
     if (!image || !labels || !region_obj || rows < 0 || W <= 0 || C <= 0 || ld < W) return DM_ERR_BAD_ARG;
     if (rows == 0) return DM_OK;
-    DM_COUNT_LAUNCH(); synth::image_kernel<<<synth::grid_for(rows * W), 256, 0, S(stream)>>>(image, labels, y0, rows, W, ld, (int)C, region_obj, seed);
-    DM_LAUNCH_CHECK();
-    return DM_OK;
+    return launch(synth::image_kernel, grid_for(rows * W, 256, 16), 256, 0, S(stream), image, labels, y0, rows, W, ld, (int)C,
+        region_obj, seed);
 }
 
 extern "C" int dm_synth_points(int32_t* xs, int32_t* ys, int64_t H, int64_t W, int64_t g, int64_t P, uint32_t seed,
                                dm_stream_t stream) {
     if (!xs || !ys || W <= 0 || H <= 0 || g <= 0 || P <= 0) return DM_ERR_BAD_ARG;
     synth::Grid G = synth::make_grid(H, W, g, seed);
-    DM_COUNT_LAUNCH(); synth::points_kernel<<<synth::grid_for((int64_t)G.ncx * G.ncy * P), 256, 0, S(stream)>>>(xs, ys, H, W, G, (int)P, seed);
-    DM_LAUNCH_CHECK();
-    return DM_OK;
+    return launch(synth::points_kernel, grid_for((int64_t)G.ncx * G.ncy * P, 256, 16), 256, 0, S(stream), xs, ys, H, W, G, (int)P,
+        seed);
 }
 
 extern "C" int dm_synth_feats(float* feats, const int32_t* rop, const int32_t* region_obj, const int64_t* point_ids,
@@ -187,7 +178,6 @@ extern "C" int dm_synth_feats(float* feats, const int32_t* rop, const int32_t* r
     if (n < 0 || D <= 0) return DM_ERR_BAD_ARG;
     if (n == 0) return DM_OK;
     if (!feats || !rop || !region_obj) return DM_ERR_BAD_ARG;
-    DM_COUNT_LAUNCH(); synth::feats_kernel<<<synth::grid_for(n * D), 256, 0, S(stream)>>>(feats, rop, region_obj, point_ids, n, (int)D, seed);
-    DM_LAUNCH_CHECK();
-    return DM_OK;
+    return launch(synth::feats_kernel, grid_for(n * D, 256, 16), 256, 0, S(stream), feats, rop, region_obj, point_ids, n, (int)D,
+        seed);
 }

@@ -49,7 +49,7 @@ int dm_version(void);
 const char* dm_error_string(int code);
 int dm_last_cuda_error(void);   /* cudaError_t of the last DM_ERR_CUDA on this thread */
 int dm_num_sms(void);           /* SM count of the current device (148 on B200), <0 on error */
-int64_t dm_launch_count(void);  /* kernels this library has launched in this process (all threads) */
+int64_t dm_launch_count(void);  /* kernels of this library accepted by the runtime in this process (all threads) */
 void dm_launch_count_add(int64_t n);  /* a host layer that replays a CUDA graph captured from n of this library's launches
                                          reports them here (the counter itself only sees the capture) */
 

@@ -112,3 +112,80 @@ def test_product_never_imports_the_oracle():
                     src = f.read()
                 assert not re.search(r"^\s*(from|import)\s+oracle\b", src, flags=re.M), fn
                 assert "/root/reference" not in src, fn
+
+
+def test_no_work_is_enqueued_before_an_argument_error(L):
+    """An entry point checks every argument, the workspace size included, before it enqueues anything: a call that
+    returns DM_ERR_BAD_ARG or DM_ERR_WORKSPACE has launched no kernel and written no output."""
+    import torch
+    cuda = torch.cuda.is_available()
+    probes = []
+
+    def buf(nbytes):
+        # With CUDA: device memory holding a sentinel of its own, which must survive the call.  Without: an address
+        # that nothing may dereference -- every CUDA call fails there first (DM_ERR_CUDA), so a bad-argument result
+        # shows that no CUDA call was made.
+        if not cuda:
+            return 16
+        t = torch.full((nbytes,), 0x41 + len(probes), dtype=torch.uint8, device="cuda")
+        probes.append((t, t.clone()))
+        return t.data_ptr()
+
+    bad, short = _lib.DM_ERR_BAD_ARG, _lib.DM_ERR_WORKSPACE
+    R, D, cap, H, W = 10, 4, 10, 4, 4
+    merge_ws, rag_ws = L.dm_merge_apply_workspace_bytes(R), L.dm_rag_workspace_bytes(cap)
+
+    def merge_stats():      # alive, changed, sum, cnt, area, perimeter, R, D, n_merged
+        return buf(R), buf(R), buf(4 * R * D), buf(4 * R), buf(8 * R), buf(8 * R), R, D, buf(8)
+
+    def rag_head(labels):   # labels, rows_own, rows_avail, W, ld, image, C, pitch, n_regions, borders, area, border, bands
+        return labels, H, H, W, W, None, 0, 0, R, 1, 1, buf(8 * R), buf(8 * R), None, None
+
+    cases = [
+        ("dm_merge_select_l2", bad, lambda: L.dm_merge_select_l2(None, 0.5, buf(8), cap, buf(cap), buf(8), None)),
+        ("dm_merge_select_mlp", bad, lambda: L.dm_merge_select_mlp(None, 2, buf(8), cap, buf(cap), buf(8), None)),
+        ("dm_merge_apply_masked", bad,
+         lambda: L.dm_merge_apply_masked(None, *merge_stats(), None, buf(merge_ws), merge_ws, None)),
+        ("dm_merge_apply", bad, lambda: L.dm_merge_apply(None, *merge_stats(), buf(merge_ws), merge_ws, None)),
+        ("dm_merge_apply_masked workspace", short,
+         lambda: L.dm_merge_apply_masked(buf(4 * R), *merge_stats(), None, buf(merge_ws), merge_ws - 1, None)),
+        ("dm_rows_pack", bad, lambda: L.dm_rows_pack(None, buf(4 * R * D), R, D, buf(4 * cap), buf(4 * cap * D), cap,
+                                                      buf(8), None)),
+        ("dm_shard_frontier_pairs", bad,
+         lambda: L.dm_shard_frontier_pairs(None, buf(R), buf(4 * R), 0, R, buf(80 + 8 * cap), cap, None)),
+        ("dm_perimeter", bad, lambda: L.dm_perimeter(None, buf(4 * cap), buf(8), cap, buf(8 * R), buf(8 * R), R, None)),
+        ("dm_points_id_range", bad, lambda: L.dm_points_id_range(None, 10, R, buf(16), None)),
+        ("dm_region_bbox", bad, lambda: L.dm_region_bbox(None, H, W, W, R, buf(16 * R), buf(8), None)),
+        ("dm_rag_scan", bad, lambda: L.dm_rag_scan(*rag_head(None), cap, buf(32), buf(rag_ws), rag_ws, None)),
+        ("dm_rag_build", bad, lambda: L.dm_rag_build(*rag_head(None), buf(8 * cap), buf(4 * cap), cap, buf(32),
+                                                      buf(rag_ws), rag_ws, None)),
+        ("dm_rag_scan workspace", short,
+         lambda: L.dm_rag_scan(*rag_head(buf(4 * H * W)), cap, buf(32), buf(rag_ws), rag_ws - 1, None)),
+    ]
+    for name, want, call in cases:
+        del probes[:]
+        n0 = L.dm_launch_count()
+        assert call() == want, name
+        assert L.dm_launch_count() == n0, name
+        if cuda:
+            torch.cuda.synchronize()
+            assert all(torch.equal(t, t0) for t, t0 in probes), name
+
+
+def test_every_launch_goes_through_the_launch_helper():
+    """Kernels are launched only by launch() and launch_cooperative() of common.cuh, which count a launch once the
+    runtime accepted it and read and clear its error; the grid rule of the grid-stride kernels is defined there once."""
+    csrc = os.path.join(ROOT, "deepmerge_b200", "csrc")
+    srcs = {}
+    for fn in sorted(os.listdir(csrc)):
+        if fn.endswith((".cu", ".cuh")):
+            with open(os.path.join(csrc, fn)) as f:
+                srcs[fn] = f.read()
+    for fn, src in srcs.items():
+        for token in ("<<<", "cudaLaunch"):
+            assert src.count(token) == (1 if fn == "common.cuh" else 0), (fn, token)
+        assert "DM_COUNT_LAUNCH" not in src and "DM_LAUNCH_CHECK" not in src, fn
+    body = lambda name: re.search(r"\bint %s\(.*?\n\}" % name, srcs["common.cuh"], flags=re.S).group(0)
+    assert "<<<" in body("launch") and "cudaLaunch" in body("launch_cooperative")
+    defs = [fn for fn, src in srcs.items() for _ in re.finditer(r"\bgrid_for\s*\(\s*(const\s+)?(int64_t|long long|int)\s", src)]
+    assert defs == ["common.cuh"], defs
