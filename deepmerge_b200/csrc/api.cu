@@ -60,12 +60,12 @@ extern "C" int dm_sort_edges(uint64_t* keys, uint32_t* vals, const int64_t* n_de
     return prims::sort_pairs(keys, vals, n_dev, capacity, b, 2 * b, ws, S(stream));
 }
 
-extern "C" size_t dm_scan_workspace_bytes(int64_t capacity) { return prims::scan_ws_bytes(capacity < 1 ? 1 : capacity); }
+extern "C" size_t dm_scan_workspace_bytes(int64_t capacity) { return prims::scan_ws_bytes(capacity); }
 
 extern "C" int dm_scan_exclusive_u32(const uint32_t* in, uint32_t* out, const int64_t* n_dev, int64_t capacity,
                                      int64_t* total_dev, void* ws, size_t ws_bytes, dm_stream_t stream) {
     if (capacity < 0) return DM_ERR_BAD_ARG;
     if (capacity > 0 && (!in || !out || !n_dev || !ws)) return DM_ERR_BAD_ARG;
-    if (ws_bytes < prims::scan_ws_bytes(capacity < 1 ? 1 : capacity)) return DM_ERR_WORKSPACE;
+    if (ws_bytes < prims::scan_ws_bytes(capacity)) return DM_ERR_WORKSPACE;
     return prims::scan_exclusive_u32(in, out, n_dev, capacity, total_dev, ws, S(stream));
 }

@@ -73,7 +73,9 @@ int launch_cooperative(void (*k)(P...), dim3 grid, dim3 block, cudaStream_t s, t
     return launched(cudaLaunchCooperativeKernel((const void*)k, grid, block, argv, 0, s));
 }
 
-// Carves a caller-provided workspace into 256-byte aligned pieces.
+// Carves a caller-provided workspace into 256-byte aligned pieces.  Each workspace has one layout function that takes
+// its pieces in order and returns them with used(): from the caller's base it gives the pieces, from a null base the
+// bytes they span, which is what the workspace query returns.
 struct Carver {
     char* base;
     size_t off = 0;

@@ -711,33 +711,41 @@ extern "C" int dm_uf_compress(int32_t* parent, int64_t R, dm_stream_t stream) {
     return launch(merge::uf_compress_kernel, grid_for(R), 256, 0, S(stream), parent, R);
 }
 
-extern "C" size_t dm_merge_apply_workspace_bytes(int64_t R) {
-    const int64_t cap = R < 1 ? 1 : R;
-    return align_up((size_t)cap * 8, 256) + prims::ws_bytes(cap, false) + 512;
+namespace {
+struct ApplyWs {
+    uint64_t* list;
+    void* sort;
+    int64_t* n_list;
+    size_t bytes;
+};
+ApplyWs merge_apply_ws(void* base, int64_t R) {
+    const int64_t cap = imax64(R, 1);
+    Carver c(base);
+    return {c.take<uint64_t>(cap), c.take<char>(prims::ws_bytes(cap, false)), c.take<int64_t>(1), c.used()};
 }
+}  // namespace
+
+extern "C" size_t dm_merge_apply_workspace_bytes(int64_t R) { return merge_apply_ws(nullptr, R).bytes; }
 
 extern "C" int dm_merge_apply_masked(const int32_t* parent, uint8_t* alive, uint8_t* changed, float* sum, int32_t* cnt,
                                      int64_t* area, int64_t* perimeter, int64_t R, int64_t D, int64_t* n_merged,
                                      const uint8_t* root_mask, void* ws, size_t ws_bytes, dm_stream_t stream) {
     if (R < 0 || D <= 0 || !n_merged) return DM_ERR_BAD_ARG;
+    const ApplyWs w = merge_apply_ws(ws, R);
     if (R > 0) {
         if (!parent || !alive || !changed || !sum || !cnt || !area || !perimeter || !ws) return DM_ERR_BAD_ARG;
-        if (ws_bytes < dm_merge_apply_workspace_bytes(R)) return DM_ERR_WORKSPACE;
+        if (ws_bytes < w.bytes) return DM_ERR_WORKSPACE;
     }
     cudaStream_t s = S(stream);
     DM_CUDA(cudaMemsetAsync(n_merged, 0, sizeof(int64_t), s));
     if (R == 0) return DM_OK;
-    Carver c(ws);
-    uint64_t* list = c.take<uint64_t>(R);
-    void* sws = c.take<char>(prims::ws_bytes(R, false));
-    int64_t* n_list = c.take<int64_t>(1);
     DM_CUDA(cudaMemsetAsync(changed, 0, (size_t)R, s));
-    DM_CUDA(cudaMemsetAsync(n_list, 0, sizeof(int64_t), s));
+    DM_CUDA(cudaMemsetAsync(w.n_list, 0, sizeof(int64_t), s));
     DM_TRY(launch(merge::collect_members_kernel, grid_for(R), 256, 0, s, parent, alive, changed, cnt, (unsigned long long*)area,
-        (unsigned long long*)perimeter, R, list, (unsigned long long*)n_list, (unsigned long long*)n_merged, root_mask));
+        (unsigned long long*)perimeter, R, w.list, (unsigned long long*)w.n_list, (unsigned long long*)n_merged, root_mask));
     const int b = bits_for(R);
-    DM_TRY(prims::sort_pairs(list, nullptr, n_list, R, b, 2 * b, sws, s, R));
-    return launch(merge::merge_sums_kernel, grid_for(R * 32), 256, 0, s, list, n_list, sum, (int)D);
+    DM_TRY(prims::sort_pairs(w.list, nullptr, w.n_list, R, b, 2 * b, w.sort, s, R));
+    return launch(merge::merge_sums_kernel, grid_for(R * 32), 256, 0, s, w.list, w.n_list, sum, (int)D);
 }
 
 extern "C" int dm_merge_apply(const int32_t* parent, uint8_t* alive, uint8_t* changed, float* sum, int32_t* cnt,
@@ -747,10 +755,24 @@ extern "C" int dm_merge_apply(const int32_t* parent, uint8_t* alive, uint8_t* ch
                                  stream);
 }
 
-extern "C" size_t dm_edges_rekey_workspace_bytes(int64_t capacity) {
-    const int64_t cap = capacity < 1 ? 1 : capacity;
-    return 2 * align_up((size_t)cap * 8, 256) + 3 * align_up((size_t)cap * 4, 256) + prims::ws_bytes(cap, true) + 256;
+namespace {
+struct RekeyWs {
+    uint64_t *new_keys, *out_keys;
+    uint32_t *perm, *out_lens;
+    float* out_scores;
+    void* sort;
+    int64_t* n_new;
+    size_t bytes;
+};
+RekeyWs edges_rekey_ws(void* base, int64_t capacity) {
+    const int64_t cap = imax64(capacity, 1);
+    Carver c(base);
+    return {c.take<uint64_t>(cap), c.take<uint64_t>(cap), c.take<uint32_t>(cap), c.take<uint32_t>(cap), c.take<float>(cap),
+            c.take<char>(prims::ws_bytes(cap, true)), c.take<int64_t>(1), c.used()};
 }
+}  // namespace
+
+extern "C" size_t dm_edges_rekey_workspace_bytes(int64_t capacity) { return edges_rekey_ws(nullptr, capacity).bytes; }
 
 extern "C" int dm_edges_rekey(const int32_t* parent, uint64_t* keys, uint32_t* lens, float* scores, int64_t* n_dev,
                               int64_t capacity, int64_t R, int64_t* perimeter, void* ws, size_t ws_bytes,
@@ -758,22 +780,19 @@ extern "C" int dm_edges_rekey(const int32_t* parent, uint64_t* keys, uint32_t* l
     if (capacity < 0 || R < 0) return DM_ERR_BAD_ARG;
     if (capacity == 0) return DM_OK;
     if (!parent || !keys || !lens || !n_dev || !perimeter || !ws) return DM_ERR_BAD_ARG;
-    if (ws_bytes < dm_edges_rekey_workspace_bytes(capacity)) return DM_ERR_WORKSPACE;
+    const RekeyWs w = edges_rekey_ws(ws, capacity);
+    if (ws_bytes < w.bytes) return DM_ERR_WORKSPACE;
     cudaStream_t s = S(stream);
-    Carver c(ws);
-    uint64_t* nk = c.take<uint64_t>(capacity);
-    uint64_t* ok = c.take<uint64_t>(capacity);
-    uint32_t* perm = c.take<uint32_t>(capacity);
-    uint32_t* ol = c.take<uint32_t>(capacity);
-    float* os = c.take<float>(capacity);
-    void* sws = c.take<char>(prims::ws_bytes(capacity, true));
-    const uint64_t sentinel = ((uint64_t)R << 32) | (uint64_t)R;
-    DM_TRY(launch(merge::rekey_kernel, grid_for(capacity), 256, 0, s, parent, keys, lens, n_dev, sentinel,
-        (unsigned long long*)perimeter, nk, perm));
+    prims::Reduce r;
+    r.sentinel = ((uint64_t)R << 32) | (uint64_t)R;
+    r.gather_lens = lens;
+    r.gather_scores = scores;
+    r.out = {w.out_keys, w.out_lens, scores ? w.out_scores : nullptr, w.n_new};
+    r.back = {keys, lens, scores, n_dev};
+    DM_TRY(launch(merge::rekey_kernel, grid_for(capacity), 256, 0, s, parent, keys, lens, n_dev, r.sentinel,
+        (unsigned long long*)perimeter, w.new_keys, w.perm));
     const int b = bits_for(R + 1);
-    int64_t* n_new = c.take<int64_t>(1);
-    return prims::sort_unique(nk, perm, n_dev, capacity, b, 2 * b, sws, lens, scores, sentinel, ok, ol, scores ? os : nullptr,
-                              n_new, keys, lens, scores, n_dev, s, R);
+    return prims::sort_unique(w.new_keys, w.perm, n_dev, capacity, b, 2 * b, w.sort, r, s, R);
 }
 
 extern "C" int dm_relabel_gated(const int32_t* labels, int64_t H, int64_t W, int64_t ld_in, const int32_t* root, int64_t R,
@@ -799,10 +818,22 @@ extern "C" int dm_relabel(const int32_t* labels, int64_t H, int64_t W, int64_t l
     return dm_relabel_gated(labels, H, W, ld_in, root, R, out, ld_out, nullptr, stream);
 }
 
-extern "C" size_t dm_compact_roots_workspace_bytes(int64_t R) {
-    const int64_t cap = R < 1 ? 1 : R;
-    return 2 * align_up((size_t)cap * 4, 256) + prims::scan_ws_bytes(cap) + 256;
+namespace {
+struct RootsWs {
+    uint32_t *flags, *excl;
+    void* scan;
+    int64_t* n_dev;
+    size_t bytes;
+};
+RootsWs compact_roots_ws(void* base, int64_t R) {
+    const int64_t cap = imax64(R, 1);
+    Carver c(base);
+    return {c.take<uint32_t>(cap), c.take<uint32_t>(cap), c.take<char>(prims::scan_ws_bytes(cap)), c.take<int64_t>(1),
+            c.used()};
 }
+}  // namespace
+
+extern "C" size_t dm_compact_roots_workspace_bytes(int64_t R) { return compact_roots_ws(nullptr, R).bytes; }
 
 extern "C" int dm_compact_roots(const int32_t* root, int64_t R, int32_t* compact, int64_t* n_roots, void* ws,
                                 size_t ws_bytes, dm_stream_t stream) {
@@ -813,15 +844,11 @@ extern "C" int dm_compact_roots(const int32_t* root, int64_t R, int32_t* compact
         return DM_OK;
     }
     if (!root || !compact || !ws) return DM_ERR_BAD_ARG;
-    if (ws_bytes < dm_compact_roots_workspace_bytes(R)) return DM_ERR_WORKSPACE;
-    Carver c(ws);
-    uint32_t* flags = c.take<uint32_t>(R);
-    uint32_t* excl = c.take<uint32_t>(R);
-    void* sws = c.take<char>(prims::scan_ws_bytes(R));
-    int64_t* n_dev = c.take<int64_t>(1);
-    DM_TRY(launch(merge::root_flags_kernel, grid_for(R), 256, 0, s, root, R, flags, n_dev));
-    DM_TRY(prims::scan_exclusive_u32(flags, excl, n_dev, R, n_roots, sws, s));
-    return launch(merge::compact_kernel, grid_for(R), 256, 0, s, root, R, excl, compact);
+    const RootsWs w = compact_roots_ws(ws, R);
+    if (ws_bytes < w.bytes) return DM_ERR_WORKSPACE;
+    DM_TRY(launch(merge::root_flags_kernel, grid_for(R), 256, 0, s, root, R, w.flags, w.n_dev));
+    DM_TRY(prims::scan_exclusive_u32(w.flags, w.excl, w.n_dev, R, n_roots, w.scan, s));
+    return launch(merge::compact_kernel, grid_for(R), 256, 0, s, root, R, w.excl, compact);
 }
 
 extern "C" int dm_perimeter(const uint64_t* keys, const uint32_t* lens, const int64_t* n_dev, int64_t capacity,

@@ -36,7 +36,8 @@ __device__ __forceinline__ void st_relaxed(uint64_t* p, uint64_t v) {
 }
 
 struct Ws {
-    uint32_t *masks, *wcnt, *wbase, *scan;
+    uint32_t *masks, *wcnt, *wbase;
+    void* scan;
     int64_t* n_words_dev;
     int* changed;                       // [2][MAX_PASSES]: pass k of phase f changed a word
     uint32_t *hv, *nxt, *ring_of;       // per side: head vertex index y (W+1) + x, successor, ring of a start side
@@ -54,7 +55,7 @@ size_t carve(Ws& w, void* base, int64_t H, int64_t W, int64_t n_regions, int64_t
     w.masks = c.take<uint32_t>((size_t)n_words * 4);
     w.wcnt = c.take<uint32_t>((size_t)n_words);
     w.wbase = c.take<uint32_t>((size_t)n_words);
-    w.scan = c.take<uint32_t>(prims::scan_ws_bytes(imax64(imax64(n_words, ring_cap), 1)) / sizeof(uint32_t));
+    w.scan = c.take<char>(prims::scan_ws_bytes(imax64(n_words, ring_cap)));
     w.n_words_dev = c.take<int64_t>(1);
     w.changed = c.take<int>(2 * MAX_PASSES);
     w.hv = c.take<uint32_t>((size_t)cap);
@@ -67,7 +68,7 @@ size_t carve(Ws& w, void* base, int64_t H, int64_t W, int64_t n_regions, int64_t
     w.rvals = c.take<uint32_t>((size_t)ring_cap);
     w.ccount = c.take<uint32_t>((size_t)ring_cap);
     w.offs = c.take<uint32_t>((size_t)ring_cap);
-    w.sort = c.take<char>(prims::ws_bytes(imax64(ring_cap, 1), false, n_regions + 1));
+    w.sort = c.take<char>(prims::ws_bytes(ring_cap, false, n_regions + 1));
     return c.used();
 }
 

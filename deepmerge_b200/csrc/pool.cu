@@ -362,11 +362,25 @@ extern "C" int dm_points_region(const int32_t* labels, int64_t H, int64_t W, int
     return launch(pool::points_region_kernel, grid_for(n), 256, 0, S(stream), labels, H, W, ld, xs, ys, n, out);
 }
 
-extern "C" size_t dm_csr_workspace_bytes(int64_t n_points, int64_t n_regions) {
-    const int64_t cap = n_points < 1 ? 1 : n_points;
+namespace {
+struct CsrWs {
+    uint64_t* keys;
+    uint32_t* vals;
+    int64_t* n_dev;
+    void* sort;
+    size_t bytes;
+};
+CsrWs csr_ws(void* base, int64_t n_points, int64_t n_regions) {
+    const int64_t cap = imax64(n_points, 1);
+    Carver c(base);
     // the bucket sort keeps per-id arrays for the n_regions + 1 keys (region ids and the "no region" key)
-    return align_up((size_t)cap * 8, 256) + align_up((size_t)cap * 4, 256) + 256 +
-           prims::ws_bytes(cap, false, n_regions + 1);
+    return {c.take<uint64_t>(cap), c.take<uint32_t>(cap), c.take<int64_t>(1),
+            c.take<char>(prims::ws_bytes(cap, false, n_regions + 1)), c.used()};
+}
+}  // namespace
+
+extern "C" size_t dm_csr_workspace_bytes(int64_t n_points, int64_t n_regions) {
+    return csr_ws(nullptr, n_points, n_regions).bytes;
 }
 
 extern "C" int dm_csr_build(const int32_t* rop, int64_t n, int64_t R, int64_t* offsets, int32_t* point_ids, void* ws,
@@ -378,17 +392,13 @@ extern "C" int dm_csr_build(const int32_t* rop, int64_t n, int64_t R, int64_t* o
         return DM_OK;
     }
     if (!rop || !point_ids || !ws) return DM_ERR_BAD_ARG;
-    if (ws_bytes < dm_csr_workspace_bytes(n, R)) return DM_ERR_WORKSPACE;
-    Carver c(ws);
-    uint64_t* keys = c.take<uint64_t>(n);
-    uint32_t* vals = c.take<uint32_t>(n);
-    int64_t* n_dev = c.take<int64_t>(1);
-    void* sws = c.take<char>(prims::ws_bytes(n, false, R + 1));
-    DM_TRY(launch(pool::csr_keys_kernel, grid_for(n), 256, 0, s, rop, n, R, keys, vals, n_dev));
+    const CsrWs w = csr_ws(ws, n, R);
+    if (ws_bytes < w.bytes) return DM_ERR_WORKSPACE;
+    DM_TRY(launch(pool::csr_keys_kernel, grid_for(n), 256, 0, s, rop, n, R, w.keys, w.vals, w.n_dev));
     // stable sort by region only (input is in ascending point id): low bits_for(R+1) bits
     const int b = bits_for(R + 1);
     // bucket + rank in one cooperative launch, offsets and point ids included
-    return prims::sort_pairs(keys, vals, n_dev, n, b, b, sws, s, R + 1, offsets, point_ids);
+    return prims::sort_pairs(w.keys, w.vals, w.n_dev, n, b, b, w.sort, s, R + 1, offsets, point_ids);
 }
 
 template <int K>

@@ -75,7 +75,11 @@ __global__ void __launch_bounds__(SCAN_THREADS) scan_apply(const uint32_t* __res
     }
 }
 
-size_t scan_ws_bytes(int64_t cap) { return align_up((size_t)(ceil_div(cap, SCAN_TILE) + 1) * sizeof(uint32_t), 256); }
+size_t scan_ws_bytes(int64_t cap) {
+    Carver c(nullptr);
+    c.take<uint32_t>(ceil_div(imax64(cap, 1), SCAN_TILE) + 1);   // tile sums
+    return c.used();
+}
 
 int scan_exclusive_u32(const uint32_t* in, uint32_t* out, const int64_t* n_dev, int64_t cap, int64_t* total_dev,
                        void* ws, cudaStream_t s) {
@@ -941,7 +945,7 @@ int launch_radix(FusedArgs& A, int64_t cap, cudaStream_t s) {
 
 size_t ws_bytes(int64_t cap, bool unique, int64_t n_ids) {
     HashArgs H;
-    return carve_ws(H, nullptr, cap < 1 ? 1 : cap, unique, n_ids);
+    return carve_ws(H, nullptr, imax64(cap, 1), unique, n_ids);
 }
 
 int sort_pairs(uint64_t* keys, uint32_t* vals, const int64_t* n_dev, int64_t cap, int id_bits, int key_bits, void* ws,
@@ -963,22 +967,20 @@ int sort_pairs(uint64_t* keys, uint32_t* vals, const int64_t* n_dev, int64_t cap
 }
 
 int sort_unique(uint64_t* keys, uint32_t* vals, const int64_t* n_dev, int64_t cap, int id_bits, int key_bits, void* ws,
-                const uint32_t* gather_lens, const float* gather_scores, uint64_t sentinel, uint64_t* out_keys,
-                uint32_t* out_lens, float* out_scores, int64_t* n_out_dev, uint64_t* back_keys, uint32_t* back_lens,
-                float* back_scores, int64_t* back_n, cudaStream_t s, int64_t n_ids) {
+                const Reduce& r, cudaStream_t s, int64_t n_ids) {
     if (cap <= 0) {
-        DM_CUDA(cudaMemsetAsync(n_out_dev, 0, sizeof(int64_t), s));
-        if (back_n) DM_CUDA(cudaMemsetAsync(back_n, 0, sizeof(int64_t), s));
+        DM_CUDA(cudaMemsetAsync(r.out.n, 0, sizeof(int64_t), s));
+        if (r.back.n) DM_CUDA(cudaMemsetAsync(r.back.n, 0, sizeof(int64_t), s));
         return DM_OK;
     }
     if (!vals || id_bits < 1 || id_bits > 32 || key_bits < 1 || key_bits > 2 * id_bits) return DM_ERR_BAD_ARG;
     HashArgs H = make_args(ws, cap, true, 0, keys, vals, n_dev, id_bits, key_bits, n_ids);
     FusedArgs& A = H.F;
     A.do_unique = 1;
-    A.gather_lens = gather_lens; A.gather_scores = gather_lens ? gather_scores : nullptr;
-    A.sentinel = sentinel;
-    A.out_keys = out_keys; A.out_lens = out_lens; A.out_scores = out_scores; A.n_out = n_out_dev;
-    A.back_keys = back_keys; A.back_lens = back_lens; A.back_scores = back_scores; A.back_n = back_n;
+    A.gather_lens = r.gather_lens; A.gather_scores = r.gather_lens ? r.gather_scores : nullptr;
+    A.sentinel = r.sentinel;
+    A.out_keys = r.out.keys; A.out_lens = r.out.lens; A.out_scores = r.out.scores; A.n_out = r.out.n;
+    A.back_keys = r.back.keys; A.back_lens = r.back.lens; A.back_scores = r.back.scores; A.back_n = r.back.n;
     if (!(n_ids > 0 && n_ids <= hash_ids_cap(cap) && key_bits == 2 * id_bits && cap < (1ll << 31)))
         return launch_radix(A, cap, s);
     const int64_t limit = imin64(coop_grid_limit((const void*)edge_unique_hashed, HASH_BLOCKS_PER_SM), HASH_MAX_GRID);

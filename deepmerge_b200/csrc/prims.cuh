@@ -15,6 +15,7 @@ constexpr int SORT_THREADS = 256;
 constexpr int SORT_ITEMS = 8;
 constexpr int SORT_TILE = SORT_THREADS * SORT_ITEMS;
 
+// Workspace of scan_exclusive_u32 over `cap` items (at least one).
 size_t scan_ws_bytes(int64_t cap);
 int scan_exclusive_u32(const uint32_t* in, uint32_t* out, const int64_t* n_dev, int64_t cap,
                        int64_t* total_dev, void* ws, cudaStream_t s);
@@ -38,21 +39,38 @@ size_t ws_bytes(int64_t cap, bool unique, int64_t n_ids = 0);
 int sort_pairs(uint64_t* keys, uint32_t* vals, const int64_t* n_dev, int64_t cap, int id_bits, int key_bits,
                void* ws, cudaStream_t s, int64_t n_ids = 0, int64_t* csr_offsets = nullptr, int32_t* csr_ids = nullptr);
 
+// A list of runs: keys[r], lens[r], scores[r] for r < *n.
+struct RunList {
+    uint64_t* keys = nullptr;
+    uint32_t* lens = nullptr;
+    float* scores = nullptr;
+    int64_t* n = nullptr;
+};
+
+// What sort_unique gathers and drops, and where it writes the runs.  The defaults gather nothing and drop nothing
+// (~0 is not the key of two ids below 2^31).
+struct Reduce {
+    RunList out;                              // keys, lens and n are required; scores is written when set
+    RunList back;                             // a copy of out, e.g. over the input arrays: see sort_unique
+    const uint32_t* gather_lens = nullptr;
+    const float* gather_scores = nullptr;
+    uint64_t sentinel = ~0ull;
+};
+
 // Sort + run reduction of n = min(*n_dev, cap) pairs; ws holds ws_bytes(cap, true) bytes.  For every run of equal keys
-// (runs of `sentinel` are dropped), in ascending key order:
-//   out_keys[r] = key, out_lens[r] = sum of the run's lengths, out_scores[r] = score of the run's first pair;
-// *n_out_dev = number of runs.  gather_lens == null: the values are the lengths.  Otherwise the values are a
-// permutation and lengths / scores are gathered through it (gather_lens[vals[i]], gather_scores[vals[i]]; out_scores
-// is written when gather_scores is set).  back_keys / back_lens / back_scores / back_n (nullable): a copy of the
-// reduced list and its length, e.g. over the input arrays.  keys / vals are left sorted or untouched.
+// (runs of r.sentinel are dropped), in ascending key order:
+//   out.keys[i] = key, out.lens[i] = sum of the run's lengths, out.scores[i] = score of the run's first pair;
+// *out.n = number of runs.  r.gather_lens == null: the values are the lengths.  Otherwise the values are a permutation
+// and lengths / scores are gathered through it (gather_lens[vals[i]], gather_scores[vals[i]]; out.scores needs
+// gather_scores).  r.back.keys set: the keys and lens of the list are copied there, and the scores when both out.scores
+// and back.scores are set; r.back.n set: the number of runs is written there too.  keys / vals are left sorted or
+// untouched.
 // n_ids in (0, 4 cap + 65536] with key_bits = 2 id_bits and cap < 2^31: both halves of every key that is not the
 // sentinel are ids < n_ids, and the run reduction goes through a hash table + per-id buckets without sorting the raw
 // pairs (edge_unique_hashed in prims.cu), which takes the radix path inside the same launch when a bucket is too large
 // or an id is out of range.  Otherwise: the LSD radix sort of the pairs, then the reduction (radix_sort_fused).
 int sort_unique(uint64_t* keys, uint32_t* vals, const int64_t* n_dev, int64_t cap, int id_bits, int key_bits, void* ws,
-                const uint32_t* gather_lens, const float* gather_scores, uint64_t sentinel, uint64_t* out_keys,
-                uint32_t* out_lens, float* out_scores, int64_t* n_out_dev, uint64_t* back_keys, uint32_t* back_lens,
-                float* back_scores, int64_t* back_n, cudaStream_t s, int64_t n_ids = 0);
+                const Reduce& r, cudaStream_t s, int64_t n_ids = 0);
 
 // ---- device helpers -------------------------------------------------------------------
 

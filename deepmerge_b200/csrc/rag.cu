@@ -61,27 +61,21 @@ using namespace dm;
 extern "C" int dm_rag_last_path(void) { return rag::last_path(); }
 extern "C" int dm_rag_last_encode_error(void) { return rag::last_encode_error(); }
 
-extern "C" size_t dm_rag_workspace_bytes(int64_t capacity) {
-    const int64_t cap = capacity < 1 ? 1 : capacity;
-    return align_up((size_t)cap * 8, 256) + align_up((size_t)cap * 4, 256) + prims::ws_bytes(cap, true);
-}
-
 namespace {
 struct RagWs {
     uint64_t* raw_keys;
     uint32_t* raw_cnt;
-    void* sws;
+    void* sort;
+    size_t bytes;
 };
-RagWs carve_rag_ws(void* ws, int64_t capacity) {
-    const int64_t cap = capacity < 1 ? 1 : capacity;
-    Carver c(ws);
-    RagWs w;
-    w.raw_keys = c.take<uint64_t>(cap);
-    w.raw_cnt = c.take<uint32_t>(cap);
-    w.sws = c.take<char>(prims::ws_bytes(cap, true));
-    return w;
+RagWs rag_ws(void* base, int64_t capacity) {
+    const int64_t cap = imax64(capacity, 1);
+    Carver c(base);
+    return {c.take<uint64_t>(cap), c.take<uint32_t>(cap), c.take<char>(prims::ws_bytes(cap, true)), c.used()};
 }
 }  // namespace
+
+extern "C" size_t dm_rag_workspace_bytes(int64_t capacity) { return rag_ws(nullptr, capacity).bytes; }
 
 extern "C" int dm_rag_scan(const int32_t* labels, int64_t rows_own, int64_t rows_avail, int64_t W, int64_t ld,
                            const uint8_t* image, int64_t C, int64_t image_pitch, int64_t n_regions, int top_border,
@@ -95,14 +89,14 @@ extern "C" int dm_rag_scan(const int32_t* labels, int64_t rows_own, int64_t rows
     if (C < 0 || C > 4) return DM_ERR_BAD_ARG;
     if (C > 0 && (!band_sum || !band_sumsq || image_pitch < W * C)) return DM_ERR_BAD_ARG;
     const bool empty = rows_own == 0 || W == 0;
+    const RagWs w = rag_ws(ws, capacity);
     if (!empty) {
         if (!labels || !area || !border || !ws) return DM_ERR_BAD_ARG;
-        if (ws_bytes < dm_rag_workspace_bytes(capacity)) return DM_ERR_WORKSPACE;
+        if (ws_bytes < w.bytes) return DM_ERR_WORKSPACE;
     }
     cudaStream_t s = S(stream);
     DM_CUDA(cudaMemsetAsync(counts, 0, 4 * sizeof(int64_t), s));
     if (empty) return DM_OK;
-    RagWs w = carve_rag_ws(ws, capacity);
     rag::Params P;
     P.labels = labels;
     P.ld = ld;
@@ -131,13 +125,13 @@ extern "C" int dm_rag_finish(uint64_t* edge_keys, uint32_t* boundary_len, int64_
     if (capacity < 0 || n_regions < 0 || !counts) return DM_ERR_BAD_ARG;
     if (capacity == 0) return DM_OK;
     if (!edge_keys || !boundary_len || !ws) return DM_ERR_BAD_ARG;
-    if (ws_bytes < dm_rag_workspace_bytes(capacity)) return DM_ERR_WORKSPACE;
-    cudaStream_t s = S(stream);
-    RagWs w = carve_rag_ws(ws, capacity);
+    const RagWs w = rag_ws(ws, capacity);
+    if (ws_bytes < w.bytes) return DM_ERR_WORKSPACE;
+    prims::Reduce r;
+    r.out = {edge_keys, boundary_len, nullptr, counts};
     const int b = bits_for(n_regions);
     // counts[1] may exceed capacity (an overflowed raw list): sort_unique reads min(counts[1], capacity) entries
-    return prims::sort_unique(w.raw_keys, w.raw_cnt, counts + 1, capacity, b, 2 * b, w.sws, nullptr, nullptr, ~0ull,
-                              edge_keys, boundary_len, nullptr, counts, nullptr, nullptr, nullptr, nullptr, s, n_regions);
+    return prims::sort_unique(w.raw_keys, w.raw_cnt, counts + 1, capacity, b, 2 * b, w.sort, r, S(stream), n_regions);
 }
 
 extern "C" int dm_rag_build(const int32_t* labels, int64_t rows_own, int64_t rows_avail, int64_t W, int64_t ld,
@@ -199,10 +193,23 @@ extern "C" int dm_edges_concat(const uint64_t* src_keys, const uint32_t* src_len
         slot_capacity, dst_keys, dst_lens, dst_capacity, n_out_dev);
 }
 
-extern "C" size_t dm_edges_unique_workspace_bytes(int64_t capacity) {
-    const int64_t cap = capacity < 1 ? 1 : capacity;
-    return align_up((size_t)cap * 8, 256) + align_up((size_t)cap * 4, 256) + 256 + prims::ws_bytes(cap, true);
+namespace {
+struct UniqueWs {
+    uint64_t* out_keys;
+    uint32_t* out_lens;
+    int64_t* n_new;
+    void* sort;
+    size_t bytes;
+};
+UniqueWs edges_unique_ws(void* base, int64_t capacity) {
+    const int64_t cap = imax64(capacity, 1);
+    Carver c(base);
+    return {c.take<uint64_t>(cap), c.take<uint32_t>(cap), c.take<int64_t>(1), c.take<char>(prims::ws_bytes(cap, true)),
+            c.used()};
 }
+}  // namespace
+
+extern "C" size_t dm_edges_unique_workspace_bytes(int64_t capacity) { return edges_unique_ws(nullptr, capacity).bytes; }
 
 extern "C" int dm_edges_sort_unique(uint64_t* keys, uint32_t* lens, const int64_t* n_in, int64_t capacity, int64_t n_regions,
                                     int64_t* n_out, void* ws, size_t ws_bytes, dm_stream_t stream) {
@@ -213,13 +220,11 @@ extern "C" int dm_edges_sort_unique(uint64_t* keys, uint32_t* lens, const int64_
         return DM_OK;
     }
     if (!keys || !lens || !n_in || !ws) return DM_ERR_BAD_ARG;
-    if (ws_bytes < dm_edges_unique_workspace_bytes(capacity)) return DM_ERR_WORKSPACE;
-    Carver c(ws);
-    uint64_t* ok = c.take<uint64_t>(capacity);
-    uint32_t* ol = c.take<uint32_t>(capacity);
-    int64_t* n_new = c.take<int64_t>(1);
-    void* sws = c.take<char>(prims::ws_bytes(capacity, true));
+    const UniqueWs w = edges_unique_ws(ws, capacity);
+    if (ws_bytes < w.bytes) return DM_ERR_WORKSPACE;
+    prims::Reduce r;
+    r.out = {w.out_keys, w.out_lens, nullptr, w.n_new};
+    r.back = {keys, lens, nullptr, n_out};
     const int b = bits_for(n_regions);
-    return prims::sort_unique(keys, lens, n_in, capacity, b, 2 * b, sws, nullptr, nullptr, ~0ull, ok, ol, nullptr, n_new,
-                              keys, lens, nullptr, n_out, s, n_regions);
+    return prims::sort_unique(keys, lens, n_in, capacity, b, 2 * b, w.sort, r, s, n_regions);
 }

@@ -486,9 +486,8 @@ class MergeEngine:
             self.iota = torch.arange(R, dtype=_I32, device=dev)
             self.alive, self.changed = e(R, dt=_U8), e(R, dt=_U8)
             self.out = e((self.H, self.W), dt=_I32)
-            sizes = [L.dm_rag_workspace_bytes(cap), L.dm_csr_workspace_bytes(N, R), L.dm_merge_apply_workspace_bytes(R),
-                     L.dm_edges_rekey_workspace_bytes(cap)]
-            self.ws_bytes = max(sizes)
+            # the raster pass (dm_rag_build / dm_rag_scan) and the edge re-keying are the calls that use ws
+            self.ws_bytes = max(L.dm_rag_workspace_bytes(cap), L.dm_edges_rekey_workspace_bytes(cap))
             self.ws = e(self.ws_bytes, dt=_U8)
             # pooling runs on its own stream beside the raster pass (independent until the merge loop): own workspace
             self.ws_pool_bytes = L.dm_csr_workspace_bytes(N, R)

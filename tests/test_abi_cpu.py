@@ -172,15 +172,21 @@ def test_no_work_is_enqueued_before_an_argument_error(L):
             assert all(torch.equal(t, t0) for t, t0 in probes), name
 
 
-def test_every_launch_goes_through_the_launch_helper():
-    """Kernels are launched only by launch() and launch_cooperative() of common.cuh, which count a launch once the
-    runtime accepted it and read and clear its error; the grid rule of the grid-stride kernels is defined there once."""
+def _csrc():
+    """file name -> text of every CUDA source of the library"""
     csrc = os.path.join(ROOT, "deepmerge_b200", "csrc")
     srcs = {}
     for fn in sorted(os.listdir(csrc)):
         if fn.endswith((".cu", ".cuh")):
             with open(os.path.join(csrc, fn)) as f:
                 srcs[fn] = f.read()
+    return srcs
+
+
+def test_every_launch_goes_through_the_launch_helper():
+    """Kernels are launched only by launch() and launch_cooperative() of common.cuh, which count a launch once the
+    runtime accepted it and read and clear its error; the grid rule of the grid-stride kernels is defined there once."""
+    srcs = _csrc()
     for fn, src in srcs.items():
         for token in ("<<<", "cudaLaunch"):
             assert src.count(token) == (1 if fn == "common.cuh" else 0), (fn, token)
@@ -189,3 +195,22 @@ def test_every_launch_goes_through_the_launch_helper():
     assert "<<<" in body("launch") and "cudaLaunch" in body("launch_cooperative")
     defs = [fn for fn, src in srcs.items() for _ in re.finditer(r"\bgrid_for\s*\(\s*(const\s+)?(int64_t|long long|int)\s", src)]
     assert defs == ["common.cuh"], defs
+
+
+def test_workspace_queries_measure_the_carve():
+    """A workspace query returns the extent of the carve that lays the workspace out, so the bytes a caller allocates
+    and the pieces an entry point takes cannot disagree: no query sums piece sizes by hand, and only Carver rounds."""
+    srcs = _csrc()
+    assert [fn for fn, src in srcs.items() if re.search(r"\balign_up\b", src)] == ["common.cuh"]
+    queries = {}
+    for fn, src in srcs.items():
+        for m in re.finditer(r'extern "C" size_t (dm_\w+_workspace_bytes)\(([^)]*)\)\s*\{(.*?)\n?\}\n', src, flags=re.S):
+            queries[m.group(1)] = m.group(3)
+    with open(os.path.join(ROOT, "include", "deepmerge_b200.h")) as f:
+        assert set(queries) == set(re.findall(r"\b(dm_\w+_workspace_bytes)\s*\(", f.read()))
+    for name, body in queries.items():
+        assert not re.search(r"[+*]", body), name
+        returns = re.findall(r"\breturn\b([^;]*);", body)
+        # the last return measures a carve; an earlier one may only answer 0 for extents the entry point rejects
+        assert returns and all(r.strip() == "0" for r in returns[:-1]), (name, returns)
+        assert re.fullmatch(r"\s*[\w:]+\(.*\)(\.bytes)?\s*", returns[-1], flags=re.S), (name, returns[-1])
