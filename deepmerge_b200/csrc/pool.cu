@@ -40,7 +40,10 @@ __global__ void __launch_bounds__(256) pool_points_kernel(const int64_t* __restr
     const int lane = threadIdx.x & 31;
     // range (row tiles of a sharded scene: ids are global, the tile's points fall into a small id interval): only
     // regions [range[0], range[1]] are visited; rows and counts outside are the caller's
-    const int64_t r_first = range ? imax64(range[0], 0) : 0, R = range ? imin64(range[1] + 1, R_all) : R_all;
+    const int64_t r_first = range ? imax64(range[0], 0) : 0, R = range ? imin64(range[1], R_all - 1) + 1 : R_all;
+    // An empty interval -- (INT64_MAX, -1) from dm_points_id_range for a tile without points -- visits nothing: return
+    // before r_first + warp index can overflow (the same decision in every thread, before any shuffle).
+    if (r_first >= R) return;
     const int64_t warp0 = r_first + (((int64_t)blockIdx.x * blockDim.x + threadIdx.x) >> 5);
     const int64_t nwarps = ((int64_t)gridDim.x * blockDim.x) >> 5;
     // A region costs three dependent round trips (offsets -> point ids -> rows).  The warp therefore looks one region

@@ -517,6 +517,7 @@ class MergeEngine:
         N = feats.shape[0]
         if N > self.N:
             raise ValueError("more points than the engine was sized for")
+        ld = feats.stride(0) if N else self.D        # a [0, D] tensor may report any strides (0 from numpy); no row is read
         if region_of_point is None:
             L.check(L.dm_points_region(_p(labels), labels.shape[0], self.W, labels.stride(0), _p(xs), _p(ys), N,
                                        _p(self.rop), s), "dm_points_region")
@@ -524,7 +525,7 @@ class MergeEngine:
         L.check(L.dm_csr_build(_p(region_of_point), N, self.R, _p(self.offsets), _p(self.pids), _p(self.ws_pool),
                                self.ws_pool_bytes, s), "dm_csr_build")
         if not self.pool_id_range and self.D <= 128:
-            L.check(L.dm_pool_points_csr_mean(_p(self.offsets), _p(self.pids), _p(feats), feats.stride(0), self.R, self.D,
+            L.check(L.dm_pool_points_csr_mean(_p(self.offsets), _p(self.pids), _p(feats), ld, self.R, self.D,
                                               _p(self.sum), _p(self.cnt), _p(self.mean), _p(self.norm2), s),
                     "dm_pool_points_csr_mean")
             return
@@ -534,7 +535,7 @@ class MergeEngine:
                 self.id_range = torch.zeros(2, dtype=_I64, device=self.dev)
             L.check(L.dm_points_id_range(_p(region_of_point), N, self.R, _p(self.id_range), s), "dm_points_id_range")
             rng = self.id_range
-        L.check(L.dm_pool_points_csr_tile(_p(self.offsets), _p(self.pids), _p(feats), feats.stride(0), self.R, self.D,
+        L.check(L.dm_pool_points_csr_tile(_p(self.offsets), _p(self.pids), _p(feats), ld, self.R, self.D,
                                           _p(self.sum), _p(self.cnt), _p(rng), s), "dm_pool_points_csr_tile")
         if not self.pool_id_range:
             self._mean_all()
