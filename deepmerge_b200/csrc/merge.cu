@@ -293,7 +293,7 @@ __global__ void perimeter_edges_kernel(const uint64_t* __restrict__ keys, const 
     const int64_t n = *n_dev;
     for (int64_t e = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; e < n; e += (int64_t)gridDim.x * blockDim.x) {
         const uint64_t k = keys[e];
-        if (key_hi(k) >= R) continue;
+        if ((k >> 32) >= (uint64_t)R || (k & 0xffffffffu) >= (uint64_t)R) continue;   // sentinels and foreign keys
         atomicAdd(&perimeter[key_lo(k)], (unsigned long long)lens[e]);
         atomicAdd(&perimeter[key_hi(k)], (unsigned long long)lens[e]);
     }
@@ -305,7 +305,7 @@ __global__ void mark_endpoints_kernel(const uint64_t* __restrict__ keys, const i
     const int64_t n = *n_dev;
     for (int64_t e = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; e < n; e += (int64_t)gridDim.x * blockDim.x) {
         const uint64_t k = keys[e];
-        if (key_hi(k) < R) {
+        if ((k >> 32) < (uint64_t)R && (k & 0xffffffffu) < (uint64_t)R) {   // both ids in [0, R), compared unsigned
             flags[key_lo(k)] = 1;
             flags[key_hi(k)] = 1;
         }

@@ -135,7 +135,8 @@ int dm_edges_concat(const uint64_t* src_keys, const uint32_t* src_lens, const in
                     int64_t slot_capacity, uint64_t* dst_keys, uint32_t* dst_lens, int64_t dst_capacity,
                     int64_t* n_out_dev, dm_stream_t stream);
 
-/* perimeter[r] = border[r] + sum of boundary_len over edges incident to r. */
+/* perimeter[r] = border[r] + sum of boundary_len over edges incident to r; a key whose two ids are not both in
+ * [0, n_regions) (the (R, R) sentinel, ~0) adds nothing. */
 int dm_perimeter(const uint64_t* edge_keys, const uint32_t* boundary_len, const int64_t* n_edges_dev,
                  int64_t capacity, const int64_t* border, int64_t* perimeter, int64_t n_regions,
                  dm_stream_t stream);
@@ -303,7 +304,8 @@ int dm_compact_roots(const int32_t* root, int64_t n_regions, int32_t* compact, i
 /* ----------------------------------------------------------------------------------- *
  * Row-tile sharding helpers (SURVEY.md section 8(e)): the sparse exchanges of the owner-free
  * distributed merge loop (deepmerge_b200/sharded.py).
- * dm_mark_endpoints: flags[lo] = flags[hi] = 1 for every edge of the list (regions this tile sees).
+ * dm_mark_endpoints: flags[lo] = flags[hi] = 1 for every edge of the list (regions this tile sees); a key whose two ids
+ *                    are not both in [0, n_regions) (the (R, R) sentinel, ~0) is skipped.
  * dm_rows_pack:  rows of the regions with flag[r] != 0 -> (out_ids, out_rows) in arbitrary order;
  *                n_out_dev[0] = number of flagged regions (> capacity: the slot overflowed).
  * dm_rows_unpack: rows[ids[i]] = in_rows[i] (add == 0) or += (add != 0); ids distinct within a call.
@@ -340,7 +342,8 @@ int dm_uf_union_slots(int32_t* parent, const void* slots, int64_t n_slots, int64
  * this rank -- a header (header_bytes, its first int64 the entry count) and up to two segments holding count entries of
  * segK_elem_bytes each at segK_offset -- is stored into slot `rank` of every rank's gathered buffer [world x slot_bytes];
  * peer_bases_dev[p] is the device address of rank p's buffer as mapped into this process (CUDA IPC / symmetric memory;
- * the caller's communicator stays opaque to the library).  Only the used part travels.  The caller runs a barrier over
+ * the caller's communicator stays opaque to the library).  Only the used part travels: the header, and of each segment
+ * min(count, capacity) * segK_elem_bytes rounded up to a multiple of 16 bytes.  The caller runs a barrier over
  * the ranks after it (and alternates two buffers, so that a buffer is rewritten only after every rank has passed the
  * barrier that follows its last read).  All offsets / sizes in bytes, multiples of 16 where they are addresses. */
 /* Two-shot all-reduce of an int32 array over NVLink peer memory (the replicated per-region state of the sharded merge
