@@ -325,6 +325,56 @@ def score_l2(mean, edge_keys, norm2=None):
     return scores
 
 
+def _spectral_params(C, shape, compactness, band_weights, scale=None):
+    """Checks the parameters of the spectral criterion -> (w_shape, w_cmpct, band weights float32 [C] on the CPU or None,
+    threshold = float32(scale^2) or None)."""
+    import math
+
+    def real(v, name, ok):
+        try:
+            f = float(v)
+        except (TypeError, ValueError):
+            f = math.nan
+        if not ok(f):
+            raise ValueError(name)
+        return f
+    thr = None
+    if scale is not None:
+        scale = real(scale, "scale must be a finite number > 0", lambda f: math.isfinite(f) and f > 0)
+        thr = float(torch.tensor(scale * scale, dtype=torch.float64).to(_F32))
+    w_shape = real(shape, "shape must be in [0, 1]", lambda f: 0.0 <= f <= 1.0)
+    w_cmpct = real(compactness, "compactness must be in [0, 1]", lambda f: 0.0 <= f <= 1.0)
+    bw = None
+    if band_weights is not None:
+        bw = torch.as_tensor(band_weights).detach().cpu().to(_F32).reshape(-1)
+        if bw.numel() != C or not bool(torch.isfinite(bw).all()) or bool((bw < 0).any()):
+            raise ValueError("band_weights must be %d finite values >= 0" % C)
+    return w_shape, w_cmpct, bw, thr
+
+
+def score_spectral(rag: RAG, shape=0.1, compactness=0.5, band_weights=None):
+    """Fusion values (Baatz & Schaepe 2000, multiresolution segmentation) of every edge of a RAG built with an image and
+    bbox=True: (1 - shape) h_color + shape (compactness h_cmpct + (1 - compactness) h_smooth) of the merged candidate,
+    fp64 from the integer statistics, rounded to fp32 (include/deepmerge_b200.h, dm_score_spectral) -> fp32 [E]."""
+    L = lib()
+    if rag.band_sum is None or rag.bbox is None:
+        raise ValueError("score_spectral needs a RAG built with an image and bbox=True")
+    _need_cuda(rag.edge_keys, rag.band_sum, rag.bbox)
+    C = rag.band_sum.shape[1]
+    w_shape, w_cmpct, bw, _ = _spectral_params(C, shape, compactness, band_weights)
+    dev = rag.edge_keys.device
+    E = rag.n_edges
+    scores = torch.empty(E, dtype=_F32, device=dev)
+    with torch.cuda.device(dev):
+        n = torch.tensor([E], dtype=_I64, device=dev)
+        bw_d = None if bw is None else bw.to(dev)
+        L.check(L.dm_score_spectral(_p(rag.edge_keys.contiguous()), _p(rag.boundary_len.contiguous()), _p(n), E,
+                                    _p(rag.area), _p(rag.perimeter), _p(rag.band_sum.contiguous()),
+                                    _p(rag.band_sumsq.contiguous()), C, _p(rag.bbox.contiguous()), _p(bw_d), w_shape, w_cmpct,
+                                    None, _p(scores), _stream()), "dm_score_spectral")
+    return scores
+
+
 class PackedMLP:
     """bf16 weights of a Nets.MLP-structured network (Nets.py:11-35) in the padded tensor-core
     layout dm_score_mlp_bf16 / dm_mlp_forward_bf16 read (dm_mlp_pack).  hidden <= 256, n_out <= 16."""
@@ -445,6 +495,9 @@ class MergeResult:
     sum: torch.Tensor
     cnt: torch.Tensor
     rag: Optional[RAG] = None       # the initial graph
+    band_sum: Optional[torch.Tensor] = None     # int64 [R, C] merged band sums (run_spectral)
+    band_sumsq: Optional[torch.Tensor] = None   # int64 [R, C]
+    bbox: Optional[torch.Tensor] = None         # int32 [R, 4] merged bounding boxes
 
 
 class MergeEngine:
@@ -461,6 +514,7 @@ class MergeEngine:
         self.logits = None
         self.use_graphs = True                           # False once a capture was refused: plain launches from then on
         self.pool_id_range, self.id_range = False, None  # a row tile's engine (sharded.py) pools only the id interval of its points
+        self.sbox = None                                  # buffers of run_spectral, allocated by its first call
         self._alloc()
 
     def _alloc(self):
@@ -617,6 +671,68 @@ class MergeEngine:
                            self.parent, rounds, merges, self.keys[:E], self.blen[:E], self.scores[:E], self.area,
                            self.perim, self.sum, self.cnt)
 
+    def run_spectral(self, labels, image, scale, *, shape=0.1, compactness=0.5, band_weights=None, max_rounds=None,
+                     relabel=True) -> MergeResult:
+        """Merge by spectral and shape heterogeneity, without embeddings (the engine may be built with D = 0 and
+        n_points = 0): RAG, band sums and boxes of the label raster, then rounds of local mutual best fitting on the
+        fusion values of Baatz & Schaepe until no adjacent pair fuses below scale^2 (or max_rounds rounds; None = no
+        limit).  shape / compactness are MRS's weights, band_weights one weight per band (None = ones).  `scores` of
+        the result are the final fusion values; band_sum / band_sumsq / bbox the merged statistics."""
+        labels = _labels_2d(labels)
+        _need_cuda(labels, image)
+        if image is None or image.dtype != _U8 or image.dim() != 3 or image.shape[2] < 1:
+            raise ValueError("image must be a uint8 [H, W, C >= 1] tensor")
+        if tuple(labels.shape) != (self.H, self.W) or tuple(image.shape) != (self.H, self.W, self.C):
+            raise ValueError("engine was sized for [%d, %d] labels and a [%d, %d, %d] image" % (self.H, self.W, self.H,
+                                                                                                self.W, self.C))
+        w_shape, w_cmpct, bw, thr = _spectral_params(self.C, shape, compactness, band_weights, scale)
+        image = image.contiguous()
+        with torch.cuda.device(self.dev):
+            if self.sbox is None:                 # first spectral run: its buffers (existing engines do not pay for them)
+                self.sbox = torch.empty((self.R, 4), dtype=_I32, device=self.dev)
+                self.sbox_bad = torch.zeros(1, dtype=_I64, device=self.dev)
+                self.band_w = torch.empty(self.C, dtype=_F32, device=self.dev)
+                self.ws_mutual_bytes = self.L.dm_merge_select_mutual_workspace_bytes(self.R)
+                self.ws_mutual = torch.empty(self.ws_mutual_bytes, dtype=_U8, device=self.dev)
+            if bw is not None:
+                self.band_w.copy_(bw)
+            crit = ("spectral", w_shape, w_cmpct, None if bw is None else tuple(bw.tolist()))
+            while True:
+                self._merge_init()
+                self._rag(labels, image, None, True, True)
+                self.L.check(self.L.dm_region_bbox(_p(labels), self.H, self.W, labels.stride(0), self.R, _p(self.sbox),
+                                                   _p(self.sbox_bad), _stream()), "dm_region_bbox")
+
+                def gated_relabel(force):
+                    self.L.check(self.L.dm_relabel_gated(_p(labels), self.H, self.W, labels.stride(0), _p(self.parent),
+                                                         self.R, _p(self.out), self.W,
+                                                         None if force else self.counts[4:5].data_ptr(), _stream()),
+                                 "dm_relabel_gated")
+                try:
+                    rounds, merges = self._merge_loop(thr, max_rounds, after_read=gated_relabel if relabel else None,
+                                                      spectral=crit)
+                    break
+                except OverflowError as ov:
+                    self.cap = int(ov.args[0]) + 1024
+                    self._alloc()
+            E = int(self.host_counts[0])
+        return MergeResult(self.out if relabel else None, self.parent, rounds, merges, self.keys[:E], self.blen[:E],
+                           self.scores[:E], self.area, self.perim, None, None, band_sum=self.bsum, band_sumsq=self.bsq,
+                           bbox=self.sbox)
+
+    def _score_spectral(self, crit, only):
+        L = self.L
+        L.check(L.dm_score_spectral(_p(self.keys), _p(self.blen), _p(self.counts[0:1]), self.cap, _p(self.area),
+                                    _p(self.perim), _p(self.bsum), _p(self.bsq), self.C, _p(self.sbox),
+                                    None if crit[3] is None else _p(self.band_w), crit[1], crit[2], _p(only),
+                                    _p(self.scores), _stream()), "dm_score_spectral")
+
+    def _select_mutual(self, thr):
+        L = self.L
+        L.check(L.dm_merge_select_mutual(_p(self.scores), float(thr), _p(self.keys), _p(self.counts[0:1]), self.cap, self.R,
+                                         _p(self.selected), self.counts[4:5].data_ptr(), _p(self.ws_mutual),
+                                         self.ws_mutual_bytes, _stream()), "dm_merge_select_mutual")
+
     def _score(self, mlp, only):
         """scores of the live edges: L2 distance (R6), or the pair-MLP logits (R8) when mlp is given.
         The MLP re-scores every live edge each round (one tensor-core pass; `only` is ignored)."""
@@ -643,10 +759,16 @@ class MergeEngine:
         self.alive.fill_(1)
         self.counts[5:8].zero_()
 
-    def _merge_loop(self, tau, max_rounds, mlp=None, after_read=None):
-        """The merge rounds; the caller has run _merge_init and computed the means of the initial graph."""
-        self._score(mlp, None)
-        self._select(tau, mlp)
+    def _merge_loop(self, tau, max_rounds, mlp=None, after_read=None, spectral=None):
+        """The merge rounds; the caller has run _merge_init and computed the means of the initial graph.  spectral (the
+        criterion of run_spectral: ("spectral", w_shape, w_cmpct, band weights)) replaces the embedding scorer: fusion
+        values, mutual best selection below tau = scale^2, integer statistics merged."""
+        if spectral is None:
+            self._score(mlp, None)
+            self._select(tau, mlp)
+        else:
+            self._score_spectral(spectral, None)
+            self._select_mutual(tau)
         rounds = merges = 0
         while True:
             c = self._read_counts(None if after_read is None else (lambda: after_read(rounds == max_rounds)))
@@ -663,7 +785,7 @@ class MergeEngine:
             if c[4] == 0 or rounds == max_rounds:
                 break
             rounds += 1
-            self._graph_launch(lambda: self._round_body(tau, mlp), tau, mlp)
+            self._graph_launch(lambda: self._round_body(tau, mlp, spectral), tau, mlp, *(() if spectral is None else spectral))
         return rounds, merges
 
     def _select(self, tau, mlp):
@@ -695,15 +817,24 @@ class MergeEngine:
                 "dm_region_mean")
         self._score(mlp, self.changed)
 
-    def _round_body(self, tau, mlp):
+    def _round_body(self, tau, mlp, spectral=None):
         """One merge round between two read-backs: unions of the selected edges, merged statistics, re-keyed edge list,
         means and scores of what changed, the next selection."""
         L, s = self.L, _stream()
         L.check(L.dm_uf_union(_p(self.parent), _p(self.keys), _p(self.selected), _p(self.counts[0:1]), self.cap, s),
                 "dm_uf_union")
         L.check(L.dm_uf_compress(_p(self.parent), self.R, s), "dm_uf_compress")
-        self._apply_and_rescore(mlp)
-        self._select(tau, mlp)
+        if spectral is None:
+            self._apply_and_rescore(mlp)
+            self._select(tau, mlp)
+            return
+        L.check(L.dm_merge_apply_regions(_p(self.parent), _p(self.alive), _p(self.changed), _p(self.area), _p(self.perim),
+                                         _p(self.bsum), _p(self.bsq), self.C, _p(self.sbox), self.R,
+                                         self.counts[5:6].data_ptr(), s), "dm_merge_apply_regions")
+        L.check(L.dm_edges_rekey(_p(self.parent), _p(self.keys), _p(self.blen), _p(self.scores), _p(self.counts[0:1]),
+                                 self.cap, self.R, _p(self.perim), _p(self.ws), self.ws_bytes, s), "dm_edges_rekey")
+        self._score_spectral(spectral, self.changed)
+        self._select_mutual(tau)
 
     def _graph_launch(self, body, tau, mlp, *key):
         """Runs a round body as ONE CUDA graph launch: a round is a dozen (sharded: ~35) short kernels whose launch gaps
@@ -860,6 +991,38 @@ def merge_scene(labels, feats, tau, *, n_regions, image=None, xs=None, ys=None, 
                              n_points=feats_d.shape[0], device=labels_d.device)
     res = engine.run(labels_d, feats_d, tau, image=image_d, xs=xs_d, ys=ys_d, region_of_point=rop_d, max_rounds=max_rounds,
                      mlp=mlp)
+    if host:
+        res.labels = res.labels.cpu()
+        res.root = res.root.cpu()
+    return res
+
+
+def merge_scene_spectral(labels, image, *, n_regions, scale, shape=0.1, compactness=0.5, band_weights=None,
+                         max_rounds=None, engine: Optional[MergeEngine] = None) -> MergeResult:
+    """Merge by spectral and shape heterogeneity end to end on one GPU (MergeEngine.run_spectral): label raster and
+    uint8 [H, W, C] image -> merged label map, no embeddings.  Host (CPU / numpy) inputs are staged through pinned
+    memory and the label map and roots come back on the host, as with merge_scene; CUDA inputs stay on the device."""
+    import numpy as np
+
+    if image is None or str(image.dtype) not in ("uint8", "torch.uint8") or len(image.shape) != 3 or image.shape[2] < 1 \
+            or len(labels.shape) != 2 or tuple(image.shape[:2]) != tuple(labels.shape):
+        raise ValueError("merge_scene_spectral needs labels [H, W] and the image as uint8 [H, W, C >= 1]")
+    _spectral_params(image.shape[2], shape, compactness, band_weights, scale)
+    host = not (isinstance(labels, torch.Tensor) and labels.is_cuda)
+    dev = torch.device("cuda", torch.cuda.current_device())
+
+    def up(x, dt):
+        t = torch.from_numpy(np.ascontiguousarray(x)) if isinstance(x, np.ndarray) else x
+        if t.dtype != dt:
+            t = t.to(dt)
+        return t if t.is_cuda else t.pin_memory().to(dev, non_blocking=True)
+
+    labels_d, image_d = up(labels, _I32), up(image, _U8)
+    H, W = labels_d.shape
+    if engine is None:
+        engine = MergeEngine(H, W, n_regions, 0, C=image_d.shape[2], n_points=0, device=labels_d.device)
+    res = engine.run_spectral(labels_d, image_d, scale, shape=shape, compactness=compactness, band_weights=band_weights,
+                              max_rounds=max_rounds)
     if host:
         res.labels = res.labels.cpu()
         res.root = res.root.cpu()

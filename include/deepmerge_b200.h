@@ -302,6 +302,48 @@ int dm_compact_roots(const int32_t* root, int64_t n_regions, int32_t* compact, i
                      void* ws, size_t ws_bytes, dm_stream_t stream);
 
 /* ----------------------------------------------------------------------------------- *
+ * Merge by spectral and shape heterogeneity: the fusion criterion of multiresolution segmentation (Baatz, M. and
+ * Schaepe, A., 2000, "Multiresolution Segmentation: an optimization approach for high quality multi-scale image
+ * segmentation"), computed from the statistics of the raster pass alone, so that no embedding is needed.  It
+ * reproduces, for merged candidates, the area / peri / mean<c> / std<c> / smooth / compact columns of the reference's
+ * polygon tables (MyUtils1.py:79-114), which the multiresolution segmentation behind its initial segments wrote.
+ *
+ * Region i: n = area, l = perimeter, b = 2 (w + h) of its bounding box (bbox int32 [R, 4] as dm_region_bbox), per band
+ * c the exact sums S_ic, Q_ic (band_sum / band_sumsq [R, C]) and sigma_ic = sqrt(max(Q/n - (S/n)^2, 0)).  The merged
+ * candidate m of an edge (a, b) with boundary length L has n_a + n_b pixels, the summed band sums, l_a + l_b - 2 L and
+ * the union of the two boxes; then, all in fp64 from the integers (every operation rounded once, no fused multiply-add):
+ *     h_color  = sum_c w_c (n_m sigma_mc - (n_a sigma_ac + n_b sigma_bc))          (c ascending, from 0.0)
+ *     h_cmpct  = n_m l_m / sqrt(n_m) - (n_a l_a / sqrt(n_a) + n_b l_b / sqrt(n_b))
+ *     h_smooth = n_m l_m / b_m - (n_a l_a / b_a + n_b l_b / b_b)
+ *     f = (1 - w_shape) h_color + w_shape (w_cmpct h_cmpct + (1 - w_cmpct) h_smooth)
+ * dm_score_spectral: scores[e] = (float) f(e); w_shape, w_cmpct in [0, 1], band_weights float [C] (NULL = ones) are
+ *     widened exactly.  `rescore` (nullable, uint8 [R]) as for dm_score_l2.
+ * dm_merge_select_mutual: local mutual best fitting.  Edge e is selected iff scores[e] < threshold and e holds the
+ *     minimum of (score, edge index) over the edges of both of its endpoints (edges not below the threshold, NaN
+ *     included, take no part; -0 and +0 are equal).  Every region takes part in at most one merge per round, and
+ *     the global minimum edge is always selected while any edge is below the threshold.  One atomicMin pass on
+ *     (ordered score bits << 32 | edge index) keys into the workspace (8 bytes a region), one decision pass;
+ *     n_selected_dev[0] = number selected.  capacity < 2^32.
+ * dm_merge_apply_regions: the integer-only counterpart of dm_merge_apply for a loop without embeddings: every region
+ *     that stopped being a root this round adds its area, perimeter, band sums and sums of squares into the root
+ *     (integer atomics) and widens the root's box (atomicMin / atomicMax); alive[x] cleared, changed[root] = 1 (changed
+ *     is cleared first), n_merged_dev[0] = regions absorbed.  No workspace.
+ * A round: select -> dm_uf_union + dm_uf_compress -> dm_merge_apply_regions -> dm_edges_rekey -> dm_score_spectral
+ * (rescore = changed) -> select.
+ * ----------------------------------------------------------------------------------- */
+int dm_score_spectral(const uint64_t* edge_keys, const uint32_t* boundary_len, const int64_t* n_edges_dev,
+                      int64_t capacity, const int64_t* area, const int64_t* perimeter, const uint64_t* band_sum,
+                      const uint64_t* band_sumsq, int64_t C, const int32_t* bbox, const float* band_weights,
+                      float w_shape, float w_cmpct, const uint8_t* rescore, float* scores, dm_stream_t stream);
+size_t dm_merge_select_mutual_workspace_bytes(int64_t n_regions);
+int dm_merge_select_mutual(const float* scores, float threshold, const uint64_t* edge_keys, const int64_t* n_edges_dev,
+                           int64_t capacity, int64_t n_regions, uint8_t* selected, int64_t* n_selected_dev, void* ws,
+                           size_t ws_bytes, dm_stream_t stream);
+int dm_merge_apply_regions(const int32_t* parent, uint8_t* alive, uint8_t* changed, int64_t* area, int64_t* perimeter,
+                           uint64_t* band_sum, uint64_t* band_sumsq, int64_t C, int32_t* bbox, int64_t n_regions,
+                           int64_t* n_merged_dev, dm_stream_t stream);
+
+/* ----------------------------------------------------------------------------------- *
  * Row-tile sharding helpers (SURVEY.md section 8(e)): the sparse exchanges of the owner-free
  * distributed merge loop (deepmerge_b200/sharded.py).
  * dm_mark_endpoints: flags[lo] = flags[hi] = 1 for every edge of the list (regions this tile sees); a key whose two ids
