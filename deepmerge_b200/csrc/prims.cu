@@ -10,13 +10,13 @@ namespace dm {
 namespace prims {
 
 // ------------------------------------------------------------------------------------ //
-// exclusive scan: tile sums -> single-block scan of tile sums -> tile scan + offset
+// exclusive scan: tile sums -> single-block scan of tile sums -> tile scan + offset; n = min(*n_dev, cap) as in the sorts
 // ------------------------------------------------------------------------------------ //
 
 __global__ void __launch_bounds__(SCAN_THREADS) scan_tile_sums(const uint32_t* __restrict__ in,
-                                                               const int64_t* __restrict__ n_dev,
+                                                               const int64_t* __restrict__ n_dev, int64_t cap,
                                                                uint32_t* __restrict__ tile_sum) {
-    const int64_t n = *n_dev;
+    const int64_t n = imin64(*n_dev, cap);
     const int64_t base = (int64_t)blockIdx.x * SCAN_TILE;
     if (base >= n) return;
     uint32_t s = 0;
@@ -32,9 +32,9 @@ __global__ void __launch_bounds__(SCAN_THREADS) scan_tile_sums(const uint32_t* _
 }
 
 __global__ void __launch_bounds__(1024) scan_tile_offsets(uint32_t* __restrict__ tile_sum,
-                                                          const int64_t* __restrict__ n_dev,
+                                                          const int64_t* __restrict__ n_dev, int64_t cap,
                                                           int64_t* __restrict__ total_dev) {
-    const int64_t n = *n_dev;
+    const int64_t n = imin64(*n_dev, cap);
     const int64_t tiles = (n + SCAN_TILE - 1) / SCAN_TILE;
     __shared__ uint32_t sm[1024 / 32 + 1];
     uint32_t carry = 0;
@@ -50,9 +50,9 @@ __global__ void __launch_bounds__(1024) scan_tile_offsets(uint32_t* __restrict__
 }
 
 __global__ void __launch_bounds__(SCAN_THREADS) scan_apply(const uint32_t* __restrict__ in, uint32_t* __restrict__ out,
-                                                           const int64_t* __restrict__ n_dev,
+                                                           const int64_t* __restrict__ n_dev, int64_t cap,
                                                            const uint32_t* __restrict__ tile_off) {
-    const int64_t n = *n_dev;
+    const int64_t n = imin64(*n_dev, cap);
     const int64_t base = (int64_t)blockIdx.x * SCAN_TILE;
     if (base >= n) return;
     // blocked arrangement: thread t owns items [t*ITEMS, (t+1)*ITEMS)
@@ -89,9 +89,9 @@ int scan_exclusive_u32(const uint32_t* in, uint32_t* out, const int64_t* n_dev, 
     }
     uint32_t* tile_sum = (uint32_t*)ws;
     const unsigned tiles = (unsigned)ceil_div(cap, SCAN_TILE);
-    DM_TRY(launch(scan_tile_sums, tiles, SCAN_THREADS, 0, s, in, n_dev, tile_sum));
-    DM_TRY(launch(scan_tile_offsets, 1, 1024, 0, s, tile_sum, n_dev, total_dev));
-    return launch(scan_apply, tiles, SCAN_THREADS, 0, s, in, out, n_dev, tile_sum);
+    DM_TRY(launch(scan_tile_sums, tiles, SCAN_THREADS, 0, s, in, n_dev, cap, tile_sum));
+    DM_TRY(launch(scan_tile_offsets, 1, 1024, 0, s, tile_sum, n_dev, cap, total_dev));
+    return launch(scan_apply, tiles, SCAN_THREADS, 0, s, in, out, n_dev, cap, tile_sum);
 }
 
 // ------------------------------------------------------------------------------------ //

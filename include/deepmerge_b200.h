@@ -65,7 +65,9 @@ size_t dm_sort_edges_workspace_bytes(int64_t capacity);
 int dm_sort_edges(uint64_t* keys, uint32_t* vals, const int64_t* n_dev, int64_t capacity,
                   int64_t n_regions, void* ws, size_t ws_bytes, dm_stream_t stream);
 
-/* Exclusive prefix sum of uint32 -> uint32; total written to total_dev[0] (int64). */
+/* Exclusive prefix sum of uint32 -> uint32 over n = min(n_dev[0], capacity) items: out[i] = in[0] + ... + in[i-1]
+ * mod 2^32 for i < n; nothing at or past n is read or written.  total_dev (nullable) receives the sum of all n items
+ * mod 2^32, stored as an int64 in [0, 2^32). */
 size_t dm_scan_workspace_bytes(int64_t capacity);
 int dm_scan_exclusive_u32(const uint32_t* in, uint32_t* out, const int64_t* n_dev, int64_t capacity,
                           int64_t* total_dev, void* ws, size_t ws_bytes, dm_stream_t stream);
@@ -105,7 +107,10 @@ int dm_rag_build(const int32_t* labels, int64_t rows_own, int64_t rows_avail, in
  *                 per-CTA (key,count) entries appended inside the workspace, counts[1..3] set;
  *   dm_rag_finish run reduction of the raw entries (one cooperative launch, normally through a
  *                 hash table and per-region buckets instead of a sort) -> ascending unique
- *                 edge_keys, summed boundary_len, counts[0].  Same ws / capacity as the scan call. */
+ *                 edge_keys, summed boundary_len, counts[0].  Same ws / capacity as the scan call.
+ *                 It reduces min(counts[1], capacity) entries.  Both 32-bit halves of every key
+ *                 must be < n_regions; a first id at or above n_regions (below 2^bits,
+ *                 2^bits >= n_regions) is still reduced correctly, through the radix sort. */
 int dm_rag_scan(const int32_t* labels, int64_t rows_own, int64_t rows_avail, int64_t W, int64_t ld,
                 const uint8_t* image, int64_t C, int64_t image_pitch, int64_t n_regions,
                 int top_border, int bottom_border,
@@ -121,7 +126,11 @@ int dm_rag_last_path(void);
 int dm_rag_last_encode_error(void);
 
 /* Sort + unique (summing lengths) an arbitrary concatenation of (key,len) lists: used to
- * merge the per-tile lists of a sharded scene and inside the merge loop.  In place. */
+ * merge the per-tile lists of a sharded scene and inside the merge loop.  In place: the n = min(n_in_dev[0], capacity)
+ * pairs are read, keys[0, E) / lens[0, E) receive the unique keys ascending with their lengths summed mod 2^32, and
+ * n_out_dev[0] = E (n_out_dev may be n_in_dev).  Keys equal to ~0 are dropped.  Both 32-bit halves of every other key
+ * must be < n_regions; a first id at or above n_regions (below 2^bits, 2^bits >= n_regions) is still reduced correctly,
+ * through the radix sort instead of the hash table. */
 size_t dm_edges_unique_workspace_bytes(int64_t capacity);
 int dm_edges_sort_unique(uint64_t* keys, uint32_t* lens, const int64_t* n_in_dev, int64_t capacity,
                          int64_t n_regions, int64_t* n_out_dev, void* ws, size_t ws_bytes, dm_stream_t stream);

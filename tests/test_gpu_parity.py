@@ -54,7 +54,9 @@ def test_sort_edges(cuda, n, R):
 def test_edges_sort_unique(cuda, n, R):
     """Run reduction of an edge list (one cooperative launch when available): unique keys ascending, lengths summed.
     The cases cover the hashed path with small buckets, with hub buckets (R = 100, 700), and its fall-back to the radix
-    sort (more hubs than the hub list holds: R = 2500; a bucket above the hub limit: R = 6000)."""
+    sort because more buckets are hubs than the hub list holds (R = 2500 and R = 6000; the largest bucket of R = 6000
+    holds 544 unique keys, far below the hub limit).  tests/test_gpu_prims_exact.py covers every path at its
+    thresholds."""
     import torch
     from deepmerge_b200._lib import lib
     L = lib()

@@ -39,7 +39,9 @@ def test_bad_arguments_are_rejected_before_anything_is_enqueued(L):
     def buf(nbytes):
         if not cuda:
             return 16
-        t = torch.full((nbytes,), 0x41 + len(probes), dtype=torch.uint8, device="cuda")
+        # at least one byte and at most 1 MiB: the bad-extent cases (capacity -1 or 2^32) need an address to pass, not
+        # the bytes their extent implies
+        t = torch.full((min(max(nbytes, 1), 1 << 20),), 0x41 + len(probes), dtype=torch.uint8, device="cuda")
         probes.append((t, t.clone()))
         return t.data_ptr()
 
