@@ -9,7 +9,7 @@ signed view orders like the unsigned key).
 """
 from __future__ import annotations
 
-from dataclasses import dataclass
+from dataclasses import dataclass, replace
 from typing import Optional, Sequence
 
 import torch
@@ -17,6 +17,20 @@ import torch
 from ._lib import lib
 
 _I64, _I32, _U8, _F32 = torch.int64, torch.int32, torch.uint8, torch.float32
+
+# Slots of the int64 counter array the raster pass and the merge kernels write (dm_shard_round_flags reads this layout):
+# edges, raw entries needed, overflow flag, status (1 = bad label, >= 2 = internal error / pair-MLP status), selected, merged
+_EDGES, _RAW_NEEDED, _OVERFLOW, _STATUS, _SELECTED, _MERGED = range(6)
+
+
+def _check_raster_flags(c):
+    """Raises on the raster pass's flags in read-back counters; OverflowError(raw entries needed) when the edges overflowed."""
+    if c[_STATUS] == 1:
+        raise ValueError("labels contain ids >= n_regions")
+    if c[_STATUS] != 0:
+        raise RuntimeError("dm_rag_build: internal pipeline error")
+    if c[_OVERFLOW] != 0:
+        raise OverflowError(int(c[_RAW_NEEDED]))
 
 
 def _stream():
@@ -138,14 +152,12 @@ def build_rag(labels: torch.Tensor, n_regions: int, image: Optional[torch.Tensor
                                    int(top_border), int(bottom_border), _p(area), _p(border), _p(bsum), _p(bsq),
                                    _p(keys), _p(blen), cap, _p(counts), _p(ws), ws_bytes, _stream()), "dm_rag_build")
             c = counts.tolist()
-            if c[3] == 1:
-                raise ValueError("labels contain ids >= n_regions")
-            if c[3] != 0:
-                raise RuntimeError("dm_rag_build: internal pipeline error")
-            if c[2] == 0:
+            try:
+                _check_raster_flags(c)
                 break
-            cap = int(c[1]) + 1024          # overflow: counts[1] is the exact raw size needed
-        E = int(c[0])
+            except OverflowError as ov:
+                cap = int(ov.args[0]) + 1024    # the exact raw size needed
+        E = int(c[_EDGES])
         perim = torch.empty(n_regions, dtype=_I64, device=dev)
         L.check(L.dm_perimeter(_p(keys), _p(blen), _p(counts), cap, _p(border), _p(perim), n_regions, _stream()),
                 "dm_perimeter")
@@ -153,7 +165,7 @@ def build_rag(labels: torch.Tensor, n_regions: int, image: Optional[torch.Tensor
     if bbox:
         rag.bbox = region_bbox(labels[:own], n_regions)
     if return_raw:
-        return rag, int(c[1])
+        return rag, int(c[_RAW_NEEDED])
     return rag
 
 
@@ -530,7 +542,8 @@ class MergeEngine:
             self.perim = self.stats[2 * R + 2 * R * max(C, 1):]          # (one buffer -> one all-reduce when sharded)
             self.keys, self.blen, self.scores = e(cap, dt=_I64), e(cap, dt=_I32), e(cap, dt=_F32)
             self.selected = e(cap, dt=_U8)
-            self.counts = z(8, dt=_I64)       # [0..3] rag counts, [4] n_selected, [5] n_merged
+            self.counts = z(8, dt=_I64)       # slots _EDGES .. _MERGED
+            self.n_edges, self.n_selected, self.n_merged = (self.counts[i:i + 1] for i in (_EDGES, _SELECTED, _MERGED))
             self.host_counts = torch.zeros(8, dtype=_I64).pin_memory()
             self.rop = e(max(N, 1), dt=_I32)
             self.offsets, self.pids = e(R + 1, dt=_I64), e(max(N, 1), dt=_I32)
@@ -621,16 +634,16 @@ class MergeEngine:
         self.keys[:E].copy_(edge_keys)
         self.blen[:E].copy_(boundary_len)
         self.counts.zero_()
-        self.counts[0] = E
+        self.counts[_EDGES] = E
 
     def merge_loaded_graph(self, tau, max_rounds=64, mlp=None):
+        rule = _EmbeddingRule(tau, mlp)
         with torch.cuda.device(self.dev):
-            self._merge_init(mlp)
+            rule.prepare(self)
+            self._merge_init()
             self._mean_all()
-            rounds, merges = self._merge_loop(tau, max_rounds, mlp)
-            E = int(self.host_counts[0])
-        return MergeResult(None, self.parent, rounds, merges, self.keys[:E], self.blen[:E], self.scores[:E], self.area,
-                           self.perim, self.sum, self.cnt)
+            rounds, merges = self._merge_loop(rule, max_rounds)
+        return self._result(None, rounds, merges)
 
     def run(self, labels, feats, tau, *, image=None, xs=None, ys=None, region_of_point=None, max_rounds=64,
             rows_own=None, top_border=True, bottom_border=True, relabel=True, mlp=None):
@@ -640,36 +653,8 @@ class MergeEngine:
             raise ValueError("feats must be float32 [N, D]")
         if (image is None) != (self.C == 0):
             raise ValueError("engine was sized for C=%d bands" % self.C)
-        with torch.cuda.device(self.dev):
-            while True:
-                # point pooling (membership, CSR, segment sums) only needs the labels: it runs on a side stream while
-                # the raster pass -- instruction-issue bound, light on memory -- and its edge sort occupy the main one
-                cur = torch.cuda.current_stream(self.dev)
-                self.side.wait_stream(cur)
-                with torch.cuda.stream(self.side):
-                    self._merge_init(mlp)
-                    self._pool(labels, xs, ys, region_of_point, feats)
-                self._rag(labels, image, rows_own, top_border, bottom_border)
-                cur.wait_stream(self.side)
-                # The relabel is enqueued behind every selection, right AFTER the copy of the counters the host waits for and
-                # gated on the device by the selection's count: when the loop ends it is already running (no idle device
-                # during the last read-back), when it goes on the kernel returns at once.  The host never waits for it.
-                own = labels.shape[0] if rows_own is None else rows_own
-
-                def gated_relabel(force):
-                    self.L.check(self.L.dm_relabel_gated(_p(labels), own, self.W, labels.stride(0), _p(self.parent), self.R,
-                                                         _p(self.out), self.W, None if force else self.counts[4:5].data_ptr(),
-                                                         _stream()), "dm_relabel_gated")
-                try:
-                    rounds, merges = self._merge_loop(tau, max_rounds, mlp, after_read=gated_relabel if relabel else None)
-                    break
-                except OverflowError as ov:            # raw edge list outgrew the capacity: resize, rerun
-                    self.cap = int(ov.args[0]) + 1024
-                    self._alloc()
-            E = int(self.host_counts[0])
-        return MergeResult(self.out[:labels.shape[0] if rows_own is None else rows_own] if relabel else None,
-                           self.parent, rounds, merges, self.keys[:E], self.blen[:E], self.scores[:E], self.area,
-                           self.perim, self.sum, self.cnt)
+        return self._run(_EmbeddingRule(tau, mlp), labels, image, max_rounds, relabel, rows_own, top_border, bottom_border,
+                         points=(xs, ys, region_of_point, feats))
 
     def run_spectral(self, labels, image, scale, *, shape=0.1, compactness=0.5, band_weights=None, max_rounds=None,
                      relabel=True) -> MergeResult:
@@ -686,164 +671,98 @@ class MergeEngine:
             raise ValueError("engine was sized for [%d, %d] labels and a [%d, %d, %d] image" % (self.H, self.W, self.H,
                                                                                                 self.W, self.C))
         w_shape, w_cmpct, bw, thr = _spectral_params(self.C, shape, compactness, band_weights, scale)
-        image = image.contiguous()
-        with torch.cuda.device(self.dev):
-            if self.sbox is None:                 # first spectral run: its buffers (existing engines do not pay for them)
-                self.sbox = torch.empty((self.R, 4), dtype=_I32, device=self.dev)
-                self.sbox_bad = torch.zeros(1, dtype=_I64, device=self.dev)
-                self.band_w = torch.empty(self.C, dtype=_F32, device=self.dev)
-                self.ws_mutual_bytes = self.L.dm_merge_select_mutual_workspace_bytes(self.R)
-                self.ws_mutual = torch.empty(self.ws_mutual_bytes, dtype=_U8, device=self.dev)
-            if bw is not None:
-                self.band_w.copy_(bw)
-            crit = ("spectral", w_shape, w_cmpct, None if bw is None else tuple(bw.tolist()))
-            while True:
-                self._merge_init()
-                self._rag(labels, image, None, True, True)
-                self.L.check(self.L.dm_region_bbox(_p(labels), self.H, self.W, labels.stride(0), self.R, _p(self.sbox),
-                                                   _p(self.sbox_bad), _stream()), "dm_region_bbox")
+        res = self._run(_SpectralRule(thr, w_shape, w_cmpct, bw), labels, image.contiguous(), max_rounds, relabel)
+        return replace(res, sum=None, cnt=None, band_sum=self.bsum, band_sumsq=self.bsq, bbox=self.sbox)
 
-                def gated_relabel(force):
-                    self.L.check(self.L.dm_relabel_gated(_p(labels), self.H, self.W, labels.stride(0), _p(self.parent),
-                                                         self.R, _p(self.out), self.W,
-                                                         None if force else self.counts[4:5].data_ptr(), _stream()),
-                                 "dm_relabel_gated")
+    def _run(self, rule, labels, image, max_rounds, relabel, rows_own=None, top_border=True, bottom_border=True,
+             points=None):
+        """Raster pass (and point pooling beside it), merge loop of `rule`, relabel; reruns when the edges outgrew `cap`."""
+        own = labels.shape[0] if rows_own is None else rows_own
+        # The relabel is enqueued behind every selection, right AFTER the copy of the counters the host waits for and
+        # gated on the device by the selection's count: when the loop ends it is already running (no idle device
+        # during the last read-back), when it goes on the kernel returns at once.  The host never waits for it.
+        after_read = (lambda last: self._relabel_gated(labels, own, None if last else self.n_selected)) if relabel else None
+        with torch.cuda.device(self.dev):
+            while True:
+                rule.prepare(self)
+                if points is None:
+                    self._merge_init()
+                    self._rag(labels, image, rows_own, top_border, bottom_border)
+                else:
+                    # point pooling (membership, CSR, segment sums) only needs the labels: it runs on a side stream while
+                    # the raster pass -- instruction-issue bound, light on memory -- and its edge sort occupy the main one
+                    cur = torch.cuda.current_stream(self.dev)
+                    self.side.wait_stream(cur)
+                    with torch.cuda.stream(self.side):
+                        self._merge_init()
+                        self._pool(labels, *points)
+                    self._rag(labels, image, rows_own, top_border, bottom_border)
+                    cur.wait_stream(self.side)
+                rule.after_raster(self, labels)
                 try:
-                    rounds, merges = self._merge_loop(thr, max_rounds, after_read=gated_relabel if relabel else None,
-                                                      spectral=crit)
+                    rounds, merges = self._merge_loop(rule, max_rounds, after_read)
                     break
-                except OverflowError as ov:
+                except OverflowError as ov:            # raw edge list outgrew the capacity: resize, rerun
                     self.cap = int(ov.args[0]) + 1024
                     self._alloc()
-            E = int(self.host_counts[0])
-        return MergeResult(self.out if relabel else None, self.parent, rounds, merges, self.keys[:E], self.blen[:E],
-                           self.scores[:E], self.area, self.perim, None, None, band_sum=self.bsum, band_sumsq=self.bsq,
-                           bbox=self.sbox)
+        return self._result(self.out[:own] if relabel else None, rounds, merges)
 
-    def _score_spectral(self, crit, only):
-        L = self.L
-        L.check(L.dm_score_spectral(_p(self.keys), _p(self.blen), _p(self.counts[0:1]), self.cap, _p(self.area),
-                                    _p(self.perim), _p(self.bsum), _p(self.bsq), self.C, _p(self.sbox),
-                                    None if crit[3] is None else _p(self.band_w), crit[1], crit[2], _p(only),
-                                    _p(self.scores), _stream()), "dm_score_spectral")
+    def _result(self, labels, rounds, merges):
+        E = int(self.host_counts[_EDGES])
+        return MergeResult(labels, self.parent, rounds, merges, self.keys[:E], self.blen[:E], self.scores[:E], self.area,
+                           self.perim, self.sum, self.cnt)
 
-    def _select_mutual(self, thr):
-        L = self.L
-        L.check(L.dm_merge_select_mutual(_p(self.scores), float(thr), _p(self.keys), _p(self.counts[0:1]), self.cap, self.R,
-                                         _p(self.selected), self.counts[4:5].data_ptr(), _p(self.ws_mutual),
-                                         self.ws_mutual_bytes, _stream()), "dm_merge_select_mutual")
+    def _relabel_gated(self, labels, rows, gate):
+        """out = parent[labels] over `rows` rows; the kernel returns at once when the int64 `gate` is nonzero (None: never)."""
+        self.L.check(self.L.dm_relabel_gated(_p(labels), rows, self.W, labels.stride(0), _p(self.parent), self.R,
+                                             _p(self.out), self.W, _p(gate), _stream()), "dm_relabel_gated")
 
-    def _score(self, mlp, only):
-        """scores of the live edges: L2 distance (R6), or the pair-MLP logits (R8) when mlp is given.
-        The MLP re-scores every live edge each round (one tensor-core pass; `only` is ignored)."""
-        L, s, D, cap = self.L, _stream(), self.D, self.cap
-        n_edges = self.counts[0:1]
-        if mlp is None:
-            L.check(L.dm_score_l2(_p(self.mean), _p(self.norm2), D, _p(self.keys), _p(n_edges), cap, _p(only),
-                                  _p(self.scores), s), "dm_score_l2")
-        else:
-            if self.logits is None or self.logits.shape != (cap, mlp.n_out):
-                self.logits = torch.empty((cap, mlp.n_out), dtype=_F32, device=self.dev)
-            L.check(L.dm_score_mlp_bf16(_p(self.mean), D, _p(self.keys), _p(n_edges), cap, _p(mlp.blob), mlp.in_features,
-                                        mlp.hidden, mlp.n_out, _p(self.logits), None, s), "dm_score_mlp_bf16")
-            self.counts[3:4].add_(self.mlp_status_shift(mlp))       # the kernel's status word travels with the round's read-back
-
-    @staticmethod
-    def mlp_status_shift(mlp):
-        return mlp.status.to(_I64) << 1                            # counts[3]: 1 = bad label, >= 2 = internal error
-
-    def _merge_init(self, mlp=None):
-        """A new merge loop: the pair-MLP (if any) must fit D; parent = identity, everything alive, round counters zero."""
-        _check_pair_mlp(mlp, self.D)
+    def _merge_init(self):
+        """A new merge loop: parent = identity, everything alive, round counters zero."""
         self.parent.copy_(self.iota)
         self.alive.fill_(1)
-        self.counts[5:8].zero_()
+        self.counts[_MERGED:].zero_()
 
-    def _merge_loop(self, tau, max_rounds, mlp=None, after_read=None, spectral=None):
-        """The merge rounds; the caller has run _merge_init and computed the means of the initial graph.  spectral (the
-        criterion of run_spectral: ("spectral", w_shape, w_cmpct, band weights)) replaces the embedding scorer: fusion
-        values, mutual best selection below tau = scale^2, integer statistics merged."""
-        if spectral is None:
-            self._score(mlp, None)
-            self._select(tau, mlp)
-        else:
-            self._score_spectral(spectral, None)
-            self._select_mutual(tau)
+    def _merge_loop(self, rule, max_rounds, after_read=None):
+        """The merge rounds of `rule` on the engine's graph; after_read(last) is enqueued behind each read-back's copy."""
+        rule.score(self, None)
+        rule.select(self)
         rounds = merges = 0
         while True:
             c = self._read_counts(None if after_read is None else (lambda: after_read(rounds == max_rounds)))
             if rounds == 0:
-                if c[3] == 1:
-                    raise ValueError("labels contain ids >= n_regions")
-                if c[3] != 0:
-                    raise RuntimeError("dm_rag_build: internal pipeline error")
-                if c[2] != 0:
-                    raise OverflowError(int(c[1]))
-            if c[3] > 1:
+                _check_raster_flags(c)
+            if c[_STATUS] > 1:
                 raise RuntimeError("pair-MLP kernel: a bounded wait expired (lost TMA / tensor-core signal)")
-            merges += int(c[5])                       # members absorbed by the previous round
-            if c[4] == 0 or rounds == max_rounds:
+            merges += int(c[_MERGED])                 # members absorbed by the previous round
+            if c[_SELECTED] == 0 or rounds == max_rounds:
                 break
             rounds += 1
-            self._graph_launch(lambda: self._round_body(tau, mlp, spectral), tau, mlp, *(() if spectral is None else spectral))
+            self._graph_launch(lambda: self._round_body(rule), rule)
         return rounds, merges
 
-    def _select(self, tau, mlp):
-        L, s, cap = self.L, _stream(), self.cap
-        n_edges = self.counts[0:1]
-        if mlp is None:
-            L.check(L.dm_merge_select_l2(_p(self.scores), float(tau), _p(n_edges), cap, _p(self.selected),
-                                         self.counts[4:5].data_ptr(), s), "dm_merge_select_l2")
-        else:
-            L.check(L.dm_merge_select_mlp(_p(self.logits), mlp.n_out, _p(n_edges), cap, _p(self.selected),
-                                          self.counts[4:5].data_ptr(), s), "dm_merge_select_mlp")
+    def _rekey(self):
+        L = self.L
+        L.check(L.dm_edges_rekey(_p(self.parent), _p(self.keys), _p(self.blen), _p(self.scores), _p(self.n_edges), self.cap,
+                                 self.R, _p(self.perim), _p(self.ws), self.ws_bytes, _stream()), "dm_edges_rekey")
 
-    def _apply_and_rescore(self, mlp, root_mask=None):
-        """The part of a round after the unions: merged statistics, re-keyed edge list, means and scores of what changed.
-        root_mask (a row tile's engine): embedding sums are merged only for the components it flags."""
-        L, s, R, D, cap = self.L, _stream(), self.R, self.D, self.cap
-        # merged statistics (side stream) and edge re-keying (main stream) only share the parent array and integer
-        # atomics on the perimeter: two chains of small kernels that fill the GPU better together
-        cur = torch.cuda.current_stream(self.dev)
-        self.side.wait_stream(cur)
-        with torch.cuda.stream(self.side):
-            L.check(L.dm_merge_apply_masked(_p(self.parent), _p(self.alive), _p(self.changed), _p(self.sum), _p(self.cnt),
-                                            _p(self.area), _p(self.perim), R, D, self.counts[5:6].data_ptr(), _p(root_mask),
-                                            _p(self.ws_side), self.ws_side_bytes, _stream()), "dm_merge_apply_masked")
-        L.check(L.dm_edges_rekey(_p(self.parent), _p(self.keys), _p(self.blen), _p(self.scores), _p(self.counts[0:1]), cap,
-                                 R, _p(self.perim), _p(self.ws), self.ws_bytes, s), "dm_edges_rekey")
-        cur.wait_stream(self.side)
-        L.check(L.dm_region_mean(_p(self.sum), _p(self.cnt), R, D, _p(self.mean), _p(self.norm2), _p(self.changed), s),
-                "dm_region_mean")
-        self._score(mlp, self.changed)
-
-    def _round_body(self, tau, mlp, spectral=None):
+    def _round_body(self, rule):
         """One merge round between two read-backs: unions of the selected edges, merged statistics, re-keyed edge list,
-        means and scores of what changed, the next selection."""
+        scores of what changed, the next selection."""
         L, s = self.L, _stream()
-        L.check(L.dm_uf_union(_p(self.parent), _p(self.keys), _p(self.selected), _p(self.counts[0:1]), self.cap, s),
-                "dm_uf_union")
+        L.check(L.dm_uf_union(_p(self.parent), _p(self.keys), _p(self.selected), _p(self.n_edges), self.cap, s), "dm_uf_union")
         L.check(L.dm_uf_compress(_p(self.parent), self.R, s), "dm_uf_compress")
-        if spectral is None:
-            self._apply_and_rescore(mlp)
-            self._select(tau, mlp)
-            return
-        L.check(L.dm_merge_apply_regions(_p(self.parent), _p(self.alive), _p(self.changed), _p(self.area), _p(self.perim),
-                                         _p(self.bsum), _p(self.bsq), self.C, _p(self.sbox), self.R,
-                                         self.counts[5:6].data_ptr(), s), "dm_merge_apply_regions")
-        L.check(L.dm_edges_rekey(_p(self.parent), _p(self.keys), _p(self.blen), _p(self.scores), _p(self.counts[0:1]),
-                                 self.cap, self.R, _p(self.perim), _p(self.ws), self.ws_bytes, s), "dm_edges_rekey")
-        self._score_spectral(spectral, self.changed)
-        self._select_mutual(tau)
+        rule.merge_and_rescore(self, None)
+        rule.select(self)
 
-    def _graph_launch(self, body, tau, mlp, *key):
+    def _graph_launch(self, body, rule, *extra):
         """Runs a round body as ONE CUDA graph launch: a round is a dozen (sharded: ~35) short kernels whose launch gaps
-        otherwise show.  The body only touches the engine's own buffers, so it is captured once per (tau, mlp, capacity,
-        *key) and replayed until _alloc re-allocates them.  Returns what the captured body returned.  A refused capture
+        otherwise show.  The body only touches the engine's own buffers, so it is captured once per (rule.key, capacity,
+        *extra) and replayed until _alloc re-allocates them.  Returns what the captured body returned.  A refused capture
         (driver / library in use) switches to plain launches from then on: the same kernels in the same order."""
         if not self.use_graphs:
             return body()
-        key = (float(tau), None if mlp is None else (id(mlp), mlp.blob.data_ptr()), self.cap) + key
+        key = rule.key + (self.cap,) + extra
         ent = self._graphs.get(key)
         if ent is None:
             g = torch.cuda.CUDAGraph()
@@ -862,6 +781,103 @@ class MergeEngine:
         self.L.dm_launch_count_add(ent[1])          # the library's counter saw the capture only
         return ent[2]
 
+
+class _EmbeddingRule:
+    """Merge criterion of run, merge_graph and the sharded loop: L2 distance of the pooled means below tau, or -- when a
+    PackedMLP is given -- its pair decision (logit 1 > logit 0).  Embedding sums and counts, area and perimeter are merged."""
+
+    def __init__(self, tau, mlp):
+        self.tau, self.mlp = float(tau), mlp
+        self.key = (self.tau, None if mlp is None else (id(mlp), mlp.blob.data_ptr()))
+
+    def prepare(self, eng):
+        mlp = self.mlp
+        _check_pair_mlp(mlp, eng.D)
+        if mlp is not None and (eng.logits is None or eng.logits.shape != (eng.cap, mlp.n_out)):
+            eng.logits = torch.empty((eng.cap, mlp.n_out), dtype=_F32, device=eng.dev)
+
+    def after_raster(self, eng, labels):
+        pass                                       # the means come from the pooling pass
+
+    def score(self, eng, only):
+        """L2 distance (R6) of the live edges with an endpoint in `only` (None: all), or the pair-MLP logits (R8), which
+        re-score every live edge each round (one tensor-core pass)."""
+        L, s, mlp = eng.L, _stream(), self.mlp
+        if mlp is None:
+            L.check(L.dm_score_l2(_p(eng.mean), _p(eng.norm2), eng.D, _p(eng.keys), _p(eng.n_edges), eng.cap, _p(only),
+                                  _p(eng.scores), s), "dm_score_l2")
+            return
+        L.check(L.dm_score_mlp_bf16(_p(eng.mean), eng.D, _p(eng.keys), _p(eng.n_edges), eng.cap, _p(mlp.blob),
+                                    mlp.in_features, mlp.hidden, mlp.n_out, _p(eng.logits), None, s), "dm_score_mlp_bf16")
+        eng.counts[_STATUS:_STATUS + 1].add_(mlp.status.to(_I64) << 1)     # the kernel's status word travels with the read-back
+
+    def select(self, eng):
+        L, s = eng.L, _stream()
+        if self.mlp is None:
+            L.check(L.dm_merge_select_l2(_p(eng.scores), self.tau, _p(eng.n_edges), eng.cap, _p(eng.selected),
+                                         _p(eng.n_selected), s), "dm_merge_select_l2")
+        else:
+            L.check(L.dm_merge_select_mlp(_p(eng.logits), self.mlp.n_out, _p(eng.n_edges), eng.cap, _p(eng.selected),
+                                          _p(eng.n_selected), s), "dm_merge_select_mlp")
+
+    def merge_and_rescore(self, eng, root_mask):
+        """Merged statistics, re-keyed edge list, means and scores of what changed.  root_mask (a row tile's engine):
+        embedding sums are merged only for the components it flags."""
+        L, R, D = eng.L, eng.R, eng.D
+        # merged statistics (side stream) and edge re-keying (main stream) only share the parent array and integer
+        # atomics on the perimeter: two chains of small kernels that fill the GPU better together
+        cur = torch.cuda.current_stream(eng.dev)
+        eng.side.wait_stream(cur)
+        with torch.cuda.stream(eng.side):
+            L.check(L.dm_merge_apply_masked(_p(eng.parent), _p(eng.alive), _p(eng.changed), _p(eng.sum), _p(eng.cnt),
+                                            _p(eng.area), _p(eng.perim), R, D, _p(eng.n_merged), _p(root_mask),
+                                            _p(eng.ws_side), eng.ws_side_bytes, _stream()), "dm_merge_apply_masked")
+        eng._rekey()
+        cur.wait_stream(eng.side)
+        L.check(L.dm_region_mean(_p(eng.sum), _p(eng.cnt), R, D, _p(eng.mean), _p(eng.norm2), _p(eng.changed), _stream()),
+                "dm_region_mean")
+        self.score(eng, eng.changed)
+
+
+class _SpectralRule:
+    """Merge criterion of run_spectral: fusion values of Baatz & Schaepe, local mutual best pairs below thr = scale^2;
+    area, perimeter, band sums and boxes are merged (integers)."""
+
+    def __init__(self, thr, w_shape, w_cmpct, bw):
+        self.thr, self.w_shape, self.w_cmpct, self.bw = thr, w_shape, w_cmpct, bw
+        self.key = (thr, w_shape, w_cmpct, None if bw is None else tuple(bw.tolist()))
+
+    def prepare(self, eng):
+        if eng.sbox is None:                 # first spectral run: its buffers (existing engines do not pay for them)
+            eng.sbox = torch.empty((eng.R, 4), dtype=_I32, device=eng.dev)
+            eng.sbox_bad = torch.zeros(1, dtype=_I64, device=eng.dev)
+            eng.band_w = torch.empty(eng.C, dtype=_F32, device=eng.dev)
+            eng.ws_mutual_bytes = eng.L.dm_merge_select_mutual_workspace_bytes(eng.R)
+            eng.ws_mutual = torch.empty(eng.ws_mutual_bytes, dtype=_U8, device=eng.dev)
+        if self.bw is not None:
+            eng.band_w.copy_(self.bw)
+
+    def after_raster(self, eng, labels):
+        eng.L.check(eng.L.dm_region_bbox(_p(labels), eng.H, eng.W, labels.stride(0), eng.R, _p(eng.sbox), _p(eng.sbox_bad),
+                                         _stream()), "dm_region_bbox")
+
+    def score(self, eng, only):
+        eng.L.check(eng.L.dm_score_spectral(_p(eng.keys), _p(eng.blen), _p(eng.n_edges), eng.cap, _p(eng.area), _p(eng.perim),
+                                            _p(eng.bsum), _p(eng.bsq), eng.C, _p(eng.sbox),
+                                            None if self.bw is None else _p(eng.band_w), self.w_shape, self.w_cmpct, _p(only),
+                                            _p(eng.scores), _stream()), "dm_score_spectral")
+
+    def select(self, eng):
+        eng.L.check(eng.L.dm_merge_select_mutual(_p(eng.scores), self.thr, _p(eng.keys), _p(eng.n_edges), eng.cap, eng.R,
+                                                 _p(eng.selected), _p(eng.n_selected), _p(eng.ws_mutual),
+                                                 eng.ws_mutual_bytes, _stream()), "dm_merge_select_mutual")
+
+    def merge_and_rescore(self, eng, root_mask):
+        eng.L.check(eng.L.dm_merge_apply_regions(_p(eng.parent), _p(eng.alive), _p(eng.changed), _p(eng.area), _p(eng.perim),
+                                                 _p(eng.bsum), _p(eng.bsq), eng.C, _p(eng.sbox), eng.R, _p(eng.n_merged),
+                                                 _stream()), "dm_merge_apply_regions")
+        eng._rekey()
+        self.score(eng, eng.changed)
 
 class ScenePipeline:
     """Throughput mode for a stream of same-sized HOST scenes (the public API behind bench.py's `e2e`):
@@ -962,39 +978,40 @@ def merge_graph(sum_, cnt, area, perimeter, edge_keys, boundary_len, tau, max_ro
     return eng.merge_loaded_graph(tau, max_rounds, mlp)
 
 
+def _stage(x, dt):
+    """A host input (numpy array or CPU tensor) -> dtype dt on the current device, staged through pinned memory; CUDA
+    tensors stay on the device, None stays None."""
+    import numpy as np
+    if x is None:
+        return None
+    t = torch.from_numpy(np.ascontiguousarray(x)) if isinstance(x, np.ndarray) else x
+    if t.dtype != dt:
+        t = t.to(dt)
+    return t if t.is_cuda else t.pin_memory().to(torch.device("cuda", torch.cuda.current_device()), non_blocking=True)
+
+
+def _to_host_like(res, labels):
+    """The label map and roots of `res` go back to the host when the input `labels` came from there."""
+    if not (isinstance(labels, torch.Tensor) and labels.is_cuda):
+        res.labels, res.root = res.labels.cpu(), res.root.cpu()
+    return res
+
+
 def merge_scene(labels, feats, tau, *, n_regions, image=None, xs=None, ys=None, region_of_point=None, max_rounds=64,
                 engine: Optional[MergeEngine] = None, mlp=None) -> MergeResult:
     """End to end on one GPU: label raster (+ optional image bands) and sample-point
     embeddings -> merged label map.  Host (CPU / numpy) inputs are staged through pinned
     memory and the label map comes back on the host, so the call is a drop-in for a CPU
     pipeline; CUDA inputs stay on the device."""
-    import numpy as np
-
-    host = not (isinstance(labels, torch.Tensor) and labels.is_cuda)
-    dev = torch.device("cuda", torch.cuda.current_device())
-
-    def up(x, dt):
-        if x is None:
-            return None
-        t = torch.from_numpy(x) if isinstance(x, np.ndarray) else x
-        if t.dtype != dt:
-            t = t.to(dt)
-        if t.is_cuda:
-            return t
-        return t.pin_memory().to(dev, non_blocking=True)
-
-    labels_d, feats_d, image_d = up(labels, _I32), up(feats, _F32), up(image, _U8)
-    xs_d, ys_d, rop_d = up(xs, _I32), up(ys, _I32), up(region_of_point, _I32)
+    labels_d, feats_d, image_d = _stage(labels, _I32), _stage(feats, _F32), _stage(image, _U8)
+    xs_d, ys_d, rop_d = _stage(xs, _I32), _stage(ys, _I32), _stage(region_of_point, _I32)
     H, W = labels_d.shape
     if engine is None:
         engine = MergeEngine(H, W, n_regions, feats_d.shape[1], C=0 if image_d is None else image_d.shape[2],
                              n_points=feats_d.shape[0], device=labels_d.device)
     res = engine.run(labels_d, feats_d, tau, image=image_d, xs=xs_d, ys=ys_d, region_of_point=rop_d, max_rounds=max_rounds,
                      mlp=mlp)
-    if host:
-        res.labels = res.labels.cpu()
-        res.root = res.root.cpu()
-    return res
+    return _to_host_like(res, labels)
 
 
 def merge_scene_spectral(labels, image, *, n_regions, scale, shape=0.1, compactness=0.5, band_weights=None,
@@ -1002,28 +1019,14 @@ def merge_scene_spectral(labels, image, *, n_regions, scale, shape=0.1, compactn
     """Merge by spectral and shape heterogeneity end to end on one GPU (MergeEngine.run_spectral): label raster and
     uint8 [H, W, C] image -> merged label map, no embeddings.  Host (CPU / numpy) inputs are staged through pinned
     memory and the label map and roots come back on the host, as with merge_scene; CUDA inputs stay on the device."""
-    import numpy as np
-
     if image is None or str(image.dtype) not in ("uint8", "torch.uint8") or len(image.shape) != 3 or image.shape[2] < 1 \
             or len(labels.shape) != 2 or tuple(image.shape[:2]) != tuple(labels.shape):
         raise ValueError("merge_scene_spectral needs labels [H, W] and the image as uint8 [H, W, C >= 1]")
     _spectral_params(image.shape[2], shape, compactness, band_weights, scale)
-    host = not (isinstance(labels, torch.Tensor) and labels.is_cuda)
-    dev = torch.device("cuda", torch.cuda.current_device())
-
-    def up(x, dt):
-        t = torch.from_numpy(np.ascontiguousarray(x)) if isinstance(x, np.ndarray) else x
-        if t.dtype != dt:
-            t = t.to(dt)
-        return t if t.is_cuda else t.pin_memory().to(dev, non_blocking=True)
-
-    labels_d, image_d = up(labels, _I32), up(image, _U8)
+    labels_d, image_d = _stage(labels, _I32), _stage(image, _U8)
     H, W = labels_d.shape
     if engine is None:
         engine = MergeEngine(H, W, n_regions, 0, C=image_d.shape[2], n_points=0, device=labels_d.device)
     res = engine.run_spectral(labels_d, image_d, scale, shape=shape, compactness=compactness, band_weights=band_weights,
                               max_rounds=max_rounds)
-    if host:
-        res.labels = res.labels.cpu()
-        res.root = res.root.cpu()
-    return res
+    return _to_host_like(res, labels)

@@ -270,17 +270,12 @@ class ShardedMergeEngine:
     def _read_headers(self, gathered, after_enqueue=None):
         """The round's one host read-back: the slot headers of all ranks ([count, pad, 8 flags] each) and this rank's
         engine counters.  after_enqueue() runs between the enqueue of the copies and the wait for them."""
-        e = self.eng
         self.hdr_dev.copy_(gathered[:, :80])                       # one strided copy of the headers, then one to the host
         self.host_fflags.copy_(self.hdr_dev.view(torch.int64).view(self.world, 10), non_blocking=True)
-        e.host_counts.copy_(e.counts, non_blocking=True)
-        e.done.record()
-        if after_enqueue is not None:
-            after_enqueue()
-        e.done.synchronize()
-        return self.host_fflags.tolist(), e.host_counts.tolist()
+        c = self.eng._read_counts(after_enqueue)
+        return self.host_fflags.tolist(), c
 
-    def _pre_exchange(self, tau, mlp, do_unions, first_round, buf):
+    def _pre_exchange(self, rule, do_unions, first_round, buf):
         """Selection of the round, its local unions and the ONE exchange of the round -> gathered frontier slots.
 
         The union-find of the round is prepared BEFORE anyone knows whether the round takes place: local unions, then the
@@ -289,10 +284,10 @@ class ShardedMergeEngine:
         (Nothing selected anywhere: no unions, no pairs.)"""
         from .raster import _p, _stream
         e, L, s = self.eng, self.eng.L, _stream()
-        R, cap, n_edges = e.R, e.cap, e.counts[0:1]
-        e._select(tau, mlp)
+        R, cap = e.R, e.cap
+        rule.select(e)
         if do_unions:
-            L.check(L.dm_uf_union(_p(e.parent), _p(e.keys), _p(e.selected), _p(n_edges), cap, s), "dm_uf_union")
+            L.check(L.dm_uf_union(_p(e.parent), _p(e.keys), _p(e.selected), _p(e.n_edges), cap, s), "dm_uf_union")
             L.check(L.dm_uf_compress(_p(e.parent), R, s), "dm_uf_compress")
             L.check(L.dm_shard_frontier_pairs(_p(e.parent), _p(e.alive), _p(self.mask), self.rank, R, _p(self.fslot),
                                               self.row_cap, s), "dm_shard_frontier_pairs")
@@ -309,7 +304,7 @@ class ShardedMergeEngine:
         L.check(L.dm_slots_word_max(_p(fg), self.world, self.fslot_bytes, 16, _p(self.any_selected), s), "dm_slots_word_max")
         return fg
 
-    def _dist_round_body(self, tau, mlp, do_unions, fg):
+    def _dist_round_body(self, rule, do_unions, fg):
         """One round between two read-backs: unions from everybody's frontier pairs, rows of the components that grew
         across a tile border, merged statistics, re-keyed tile edge list, means / scores of what changed, and the next
         round's selection + exchange."""
@@ -329,19 +324,19 @@ class ShardedMergeEngine:
         L.check(L.dm_shard_plan(_p(e.parent), _p(e.alive), _p(self.mask_old), _p(self.mask), _p(self.grew), self.rank, R,
                                 _p(self.send), _p(self.seen_comp), s), "dm_shard_plan")
         self._exchange_rows(self.send, add=False, buf=1)
-        e._apply_and_rescore(mlp, self.seen_comp)          # embedding sums only of the components this rank sees
-        return self._pre_exchange(tau, mlp, do_unions, False, 1)
+        rule.merge_and_rescore(e, self.seen_comp)          # embedding sums only of the components this rank sees
+        return self._pre_exchange(rule, do_unions, False, 1)
 
-    def _dist_round(self, tau, mlp, do_unions):
+    def _dist_round(self, rule, do_unions):
         """The round body; one CUDA graph launch when every exchange in it is a kernel of this library (peer stores /
         peer all-reduce over symmetric memory + signal-pad barriers): collective calls cannot be captured."""
         # the body reads the gathered pairs of the previous exchange: buffer 0 after the head, buffer 1 after a body
         src = self._last_fg
-        body = lambda: self._dist_round_body(tau, mlp, do_unions, src)
+        body = lambda: self._dist_round_body(rule, do_unions, src)
         if self.peer_rows is None:
             self._last_fg = body()
         else:
-            self._last_fg = self.eng._graph_launch(body, tau, mlp, bool(do_unions), src.data_ptr())
+            self._last_fg = self.eng._graph_launch(body, rule, bool(do_unions), src.data_ptr())
         return self._last_fg
 
     def run(self, labels_tile, feats_local, tau, *, image_tile=None, xs_local=None, ys_local_rel=None, max_rounds=64,
@@ -356,8 +351,9 @@ class ShardedMergeEngine:
 
         mlp (a PackedMLP, replicated on every rank): the tcgen05 pair-MLP scores every live tile edge every round and an edge
         is selected when argmax(o) == 1 (Nets.py:28-35) instead of L2 distance < tau -- as MergeEngine.run(mlp=...) does."""
-        from .raster import MergeResult, _p, _stream
+        from .raster import _EDGES, _MERGED, MergeResult, _EmbeddingRule, _p, _stream
         e, L, dist, grp = self.eng, self.eng.L, self.dist, self.group
+        rule = _EmbeddingRule(tau, mlp)
         R, D, cap = e.R, e.D, e.cap
         if not hasattr(self, "mask"):
             self._alloc_dist()
@@ -369,7 +365,6 @@ class ShardedMergeEngine:
         e.pool_id_range = True
         with torch.cuda.device(e.dev):
             s = _stream()
-            n_edges = e.counts[0:1]
             # (1) tile pass: fused RAG + band pooling; e.keys / e.blen = the tile's own edge list,
             #     e.perim = border + incident boundary lengths of THIS tile (a partial, like area and the band sums)
             #     (the tile's point pooling only needs the labels: it runs beside the raster pass on the engine's side stream)
@@ -380,7 +375,7 @@ class ShardedMergeEngine:
             e._rag(labels_tile, image_tile, self.rows_own, self.rank == 0, self.rank == self.world - 1)
             # (2) which ranks see which region
             self.seen.zero_()
-            L.check(L.dm_mark_endpoints(_p(e.keys), _p(n_edges), cap, R, _p(self.seen), s), "dm_mark_endpoints")
+            L.check(L.dm_mark_endpoints(_p(e.keys), _p(e.n_edges), cap, R, _p(self.seen), s), "dm_mark_endpoints")
             # (3) pooled embeddings: per-tile partial sums; counts replicated, rows of regions seen by two ranks exchanged
             cur.wait_stream(e.side)
             L.check(L.dm_shard_seen(_p(e.area), _p(self.seen), _p(e.cnt), self.rank, R, _p(self.mask_cnt), _p(self.cnt_local), s),
@@ -393,18 +388,17 @@ class ShardedMergeEngine:
             L.check(L.dm_shard_frontier(_p(self.mask_cnt), _p(self.cnt_local), R, _p(e.cnt), _p(self.send), s), "dm_shard_frontier")
             self._exchange_rows(self.send, add=True, buf=0)
             # (4) merge loop on the tile's edges with the replicated parent array
-            e._merge_init(mlp)
+            rule.prepare(e)
+            e._merge_init()
             L.check(L.dm_region_mean(_p(e.sum), _p(e.cnt), R, D, _p(e.mean), _p(e.norm2), _p(self.seen), s), "dm_region_mean")
-            e._score(mlp, None)
+            rule.score(e, None)
             rounds = merges = 0
-            fg = self._last_fg = self._pre_exchange(tau, mlp, max_rounds > 0, True, 0)
+            fg = self._last_fg = self._pre_exchange(rule, max_rounds > 0, True, 0)
             # (5) tile-local relabel with the replicated root LUT: enqueued behind every exchange, right after the copies the
             #     host waits for, and gated on the device by "no rank selected an edge" -- when the loop ends it is already
             #     running, when it goes on the kernel returns at once
-            def gated_relabel():
-                L.check(L.dm_relabel_gated(_p(labels_tile), self.rows_own, self.W, labels_tile.stride(0), _p(e.parent), R,
-                                           _p(e.out), self.W, None if rounds == max_rounds else _p(self.any_selected), s),
-                        "dm_relabel_gated")
+            gated_relabel = lambda: e._relabel_gated(labels_tile, self.rows_own,
+                                                     None if rounds == max_rounds else self.any_selected)
             while True:
                 hf, c = self._read_headers(fg, gated_relabel)
                 f = [max(int(h[2 + k]) for h in hf) for k in range(8)]     # every rank sees every rank's flags: all act alike
@@ -414,21 +408,21 @@ class ShardedMergeEngine:
                     raise RuntimeError("tile edge list overflow / pipeline error (capacity %d, needed %d)" % (cap, f[6]))
                 if f[2] != 0 or any(int(h[0]) > self.row_cap for h in hf):
                     raise RuntimeError("row exchange slot overflow (row_cap %d)" % self.row_cap)
-                merges += int(c[5])
+                merges += int(c[_MERGED])
                 if f[0] == 0 or rounds == max_rounds:
                     break
                 rounds += 1
-                fg = self._dist_round(tau, mlp, rounds < max_rounds)
-            Ef = int(e.host_counts[0])
+                fg = self._dist_round(rule, rounds < max_rounds)
+            Ef = int(e.host_counts[_EDGES])
             if gather_outputs:
                 # per-tile partials -> global statistics; tile edge lists -> the global final edge list
                 allreduce_sum_(e.stats, dist, grp)                  # area | border | band sums | perimeter in one buffer
-                nmax = e.counts[0:1].clone()
+                nmax = e.n_edges.clone()
                 dist.all_reduce(nmax, op=MAX, group=grp)
                 m = max(1, int(nmax.item()))                        # (the gathered form may afford this host round trip)
                 gk = all_gather_slots(e.keys[:m], dist, grp)
                 gl = all_gather_slots(e.blen[:m], dist, grp)
-                gc = all_gather_slots(e.counts[0:1], dist, grp)
+                gc = all_gather_slots(e.n_edges, dist, grp)
                 tot = self.world * m
                 out_k = torch.empty(tot, dtype=torch.int64, device=e.dev)
                 out_l = torch.empty(tot, dtype=torch.int32, device=e.dev)

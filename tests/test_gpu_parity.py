@@ -514,6 +514,11 @@ def test_merge_scene_end_to_end_bit_exact(cuda, H, W, R, C):
     host = merge_scene(sc["labels"], sc["feats"], 0.5, n_regions=sc["n_regions"], image=sc["image"] if C else None,
                        region_of_point=sc["region_of_point"])
     assert not host.labels.is_cuda and np.array_equal(host.labels.numpy(), want["labels"])
+    # numpy views with negative strides (the same contents, reversed twice) are staged like contiguous arrays
+    flip = lambda a: np.flipud(np.ascontiguousarray(np.flipud(a)))
+    rev = merge_scene(flip(sc["labels"]), flip(sc["feats"]), 0.5, n_regions=sc["n_regions"],
+                      image=flip(sc["image"]) if C else None, region_of_point=flip(sc["region_of_point"]))
+    assert np.array_equal(rev.labels.numpy(), want["labels"]) and np.array_equal(rev.root.numpy(), want["root"])
 
 
 def test_relabel_and_compact(cuda):

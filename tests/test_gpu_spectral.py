@@ -260,7 +260,8 @@ def test_full_size_configs1_against_the_oracles(cuda):
 
 def test_determinism_and_shared_buffers_with_the_l2_loop(cuda):
     """Two spectral runs on one engine are bit-equal (the second replays the captured round graphs), and the L2 loop on
-    the same engine equals its oracle before and after them."""
+    the same engine equals its oracle before and after them.  The round graph is captured once per criterion and
+    parameters: runs that repeat them replay it."""
     from deepmerge_b200 import MergeEngine
     sc = o.synth_scene(512, 640, 2000, C=4)
     n = sc["n_regions"]
@@ -274,6 +275,8 @@ def test_determinism_and_shared_buffers_with_the_l2_loop(cuda):
         assert np.array_equal(r.labels.cpu().numpy(), l2["labels"]) and np.array_equal(u64(r.edge_keys), l2["keys"])
 
     run_l2()
+    run_l2()
+    assert l2["rounds"] >= 1 and len(eng._graphs) == 1
     want = so.merge_scene_spectral(sc["labels"], sc["image"], n, 30.0)
     runs = []
     for _ in range(2):
@@ -281,8 +284,9 @@ def test_determinism_and_shared_buffers_with_the_l2_loop(cuda):
         assert_same_run(r, want, want["labels"])
         runs.append((r.labels.clone(), r.scores.clone(), r.root.clone()))
     assert all(torch.equal(x, y) for x, y in zip(*runs))
-    assert want["rounds"] > 2 and eng.use_graphs
+    assert want["rounds"] > 2 and eng.use_graphs and len(eng._graphs) == 2
     run_l2()
+    assert len(eng._graphs) == 2
 
 
 def test_quality_on_the_synthetic_scene(cuda):
