@@ -1,5 +1,6 @@
 // Polygonizer: label raster -> closed rings of pixel-corner vertices, one set per region (dm_polygonize in
-// include/deepmerge_b200.h).  The per-side rule lives in polygon_core.cuh.
+// include/deepmerge_b200.h).  The per-side rule lives in polygon_core.cuh; the mask pass, the dense index and the
+// pointer jumping in chain.cuh, which the boundary-line tracer (lines.cu) shares.
 //
 // 1. mask_kernel    one pass over the labels: a 4-bit mask of boundary sides per pixel (8 pixels per uint32), one side
 //                   count per 32-pixel word of a row, the exact total and the label range check.
@@ -14,26 +15,22 @@
 // 5. starts_kernel  one ring per start side, listed with its start vertex; sort_pairs orders the list by start vertex
 //                   (radix), then stably by region (bucket + rank), whose CSR offsets are region_rings.
 // 6. vertex_kernel  corners scattered to ring offset + rank, ring areas as the sum of x * dy over the vertical sides.
-#include "common.cuh"
+#include "chain.cuh"
 #include "polygon_core.cuh"
 #include "prims.cuh"
 
 namespace dm {
 namespace poly {
 using namespace polycore;
+using namespace chain;
 
-constexpr int NT = 256;
-constexpr int MAX_PASSES = 64;
 constexpr uint8_t CORNER = 4;   // flags: bits 0-1 side / direction, bit 2 head vertex is a corner
 
-__device__ __forceinline__ uint64_t ld_relaxed(const uint64_t* p) {
-    uint64_t v;
-    asm volatile("ld.relaxed.gpu.global.u64 %0, [%1];" : "=l"(v) : "l"(p) : "memory");
-    return v;
-}
-__device__ __forceinline__ void st_relaxed(uint64_t* p, uint64_t v) {
-    asm volatile("st.relaxed.gpu.global.u64 [%0], %1;" ::"l"(p), "l"(v) : "memory");
-}
+struct SideMask {
+    static __device__ __forceinline__ unsigned mask(const int32_t* L, int64_t H, int64_t W, int64_t ld, int64_t x, int64_t y) {
+        return side_mask(L, H, W, ld, x, y);
+    }
+};
 
 struct Ws {
     uint32_t *masks, *wcnt, *wbase;
@@ -72,49 +69,6 @@ size_t carve(Ws& w, void* base, int64_t H, int64_t W, int64_t n_regions, int64_t
     return c.used();
 }
 
-__device__ __forceinline__ bool failed(const int64_t* counts) { return *(volatile const int64_t*)(counts + 3) != 0; }
-
-__global__ void __launch_bounds__(NT) mask_kernel(const int32_t* __restrict__ L, int64_t H, int64_t W, int64_t ld,
-                                                  int64_t wpr, int64_t n_regions, uint32_t* __restrict__ masks,
-                                                  uint32_t* __restrict__ wcnt, int64_t* __restrict__ counts,
-                                                  int64_t* __restrict__ n_words_dev) {
-    const int lane = threadIdx.x & 31;
-    const int64_t n_words = H * wpr;
-    const int64_t warp0 = ((int64_t)blockIdx.x * NT + threadIdx.x) >> 5, nwarps = ((int64_t)gridDim.x * NT) >> 5;
-    if (blockIdx.x == 0 && threadIdx.x == 0) *n_words_dev = n_words;
-    unsigned long long total = 0;
-    bool bad = false;
-    for (int64_t w = warp0; w < n_words; w += nwarps) {
-        const int64_t y = w / wpr, x = (w - y * wpr) * 32 + lane;
-        unsigned m = 0;
-        if (x < W) {
-            bad |= L[y * ld + x] >= n_regions;
-            m = side_mask(L, H, W, ld, x, y);
-        }
-        unsigned v = m << (4 * (lane & 7));
-        v |= __shfl_xor_sync(0xffffffffu, v, 1);
-        v |= __shfl_xor_sync(0xffffffffu, v, 2);
-        v |= __shfl_xor_sync(0xffffffffu, v, 4);
-        if ((lane & 7) == 0) masks[w * 4 + (lane >> 3)] = v;
-        const unsigned c = __reduce_add_sync(0xffffffffu, (unsigned)__popc(m));
-        if (lane == 0) wcnt[w] = c;
-        total += c;
-    }
-    if (__any_sync(0xffffffffu, bad) && lane == 0) atomicExch((unsigned long long*)(counts + 3), 1ull);
-    if (lane == 0 && total) atomicAdd((unsigned long long*)(counts + 2), total);
-}
-
-// dense index of side s of pixel (x, y)
-__device__ __forceinline__ uint32_t dense_index(const uint32_t* masks, const uint32_t* wbase, int64_t wpr, int64_t x,
-                                                int64_t y, int s) {
-    const int64_t w = y * wpr + (x >> 5);
-    const int k = (int)(x & 31);
-    const uint32_t* m = masks + w * 4;
-    uint32_t i = wbase[w];
-    for (int j = 0; j < (k >> 3); ++j) i += __popc(m[j]);
-    return i + __popc(m[k >> 3] & ((1u << (4 * (k & 7) + s)) - 1u));
-}
-
 __global__ void __launch_bounds__(NT) emit_kernel(const int32_t* __restrict__ L, int64_t H, int64_t W, int64_t ld,
                                                   int64_t wpr, int64_t cap, const uint32_t* __restrict__ masks,
                                                   const uint32_t* __restrict__ wbase, int64_t* __restrict__ counts, Ws ws) {
@@ -151,34 +105,6 @@ __global__ void __launch_bounds__(NT) emit_kernel(const int32_t* __restrict__ L,
             ++i;
         }
     }
-}
-
-// One pointer-jumping pass, in place.  phase 0: value = minimum head vertex over the sides [i, pointer);
-// phase 1: value = corners over (i, pointer], the start side of every ring points at itself with value 0.
-// A word read while its owner rewrites it is an older or newer (value, pointer) pair, both of which hold the invariant.
-__global__ void __launch_bounds__(NT) jump_kernel(uint64_t* jw, const int64_t* __restrict__ counts, int* changed,
-                                                  int phase, int pass) {
-    if (failed(counts)) return;
-    int* ch_flags = changed + phase * MAX_PASSES;
-    if (pass > 0 && !ch_flags[pass - 1]) return;
-    const int64_t n = counts[2];
-    bool ch = false;
-    for (int64_t i = (int64_t)blockIdx.x * NT + threadIdx.x; i < n; i += (int64_t)gridDim.x * NT) {
-        const uint64_t w = ld_relaxed(jw + i);
-        const uint32_t p = (uint32_t)w;
-        const uint64_t t = ld_relaxed(jw + p);
-        uint64_t nw;
-        if (phase == 0) {
-            const uint64_t mn = min(w >> 32, t >> 32);
-            ch |= mn != (w >> 32);
-            nw = (mn << 32) | (uint32_t)t;
-        } else {
-            ch |= (uint32_t)t != p;
-            nw = (((w >> 32) + (t >> 32)) << 32) | (uint32_t)t;
-        }
-        st_relaxed(jw + i, nw);
-    }
-    if (__syncthreads_or(ch) && threadIdx.x == 0) ch_flags[pass] = 1;
 }
 
 // After phase 0: the side whose head is its ring's minimum vertex starts the ring.  The word becomes phase 1's.
@@ -245,12 +171,6 @@ __global__ void __launch_bounds__(NT) vertex_kernel(const int64_t* __restrict__ 
     }
 }
 
-int ceil_log2(int64_t x) {
-    int b = 0;
-    while (((int64_t)1 << b) < x) ++b;
-    return b;
-}
-
 }  // namespace poly
 }  // namespace dm
 
@@ -291,7 +211,7 @@ extern "C" int dm_polygonize(const int32_t* labels, int64_t H, int64_t W, int64_
     if (ring_cap) DM_CUDA(cudaMemsetAsync(ring_area, 0, (size_t)ring_cap * sizeof(int64_t), s));
     const unsigned g_words = grid_for(n_words * 32, poly::NT, 16), g_sides = grid_for(capacity, poly::NT, 16);
     const unsigned g_rings = grid_for(ring_cap + 1, poly::NT, 16);
-    DM_TRY(launch(poly::mask_kernel, g_words, poly::NT, 0, s, labels, H, W, ld, wpr, n_regions, w.masks, w.wcnt, counts,
+    DM_TRY(launch(poly::mask_kernel<poly::SideMask>, g_words, poly::NT, 0, s, labels, H, W, ld, wpr, n_regions, w.masks, w.wcnt, counts,
         w.n_words_dev));
     DM_TRY(prims::scan_exclusive_u32(w.wcnt, w.wbase, w.n_words_dev, n_words, nullptr, w.scan, s));
     DM_TRY(launch(poly::emit_kernel, g_words, poly::NT, 0, s, labels, H, W, ld, wpr, capacity, w.masks, w.wbase, counts, w));

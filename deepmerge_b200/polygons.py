@@ -1,5 +1,6 @@
-"""Label raster -> polygons (dm_polygonize): the way back from a merged label map to one polygon per segment, as the
-reference's tile.shp holds them.  shapefile.write_polygonized writes the result."""
+"""Label raster -> polygons (dm_polygonize) and boundary lines (dm_lines): the way back from a merged label map to one
+polygon per segment, as the reference's tile.shp holds them, and to one polyline per shared boundary, as its lines.shp
+holds them.  shapefile.write_polygonized and shapefile.write_boundary_lines write the results."""
 from __future__ import annotations
 
 from dataclasses import dataclass
@@ -106,3 +107,78 @@ def polygonize(labels: torch.Tensor, n_regions: int, *, capacity=None) -> Polygo
             break
     k, v = int(c[0]), int(c[1])
     return Polygons(ring_region[:k], ring_offsets[:k + 1], ring_area[:k], vertices[:v], region_rings, int(c[2]))
+
+
+@dataclass
+class Lines:
+    """Boundary lines in canonical order (include/deepmerge_b200.h, dm_lines): line k separates the values
+    line_left[k] (-1: nodata or outside) and line_right[k] (>= 0, the larger), which lie on its left and right (pixel
+    coordinates, y down), and has the vertices vertices[line_offsets[k]:line_offsets[k + 1]] (start, corners, end; a
+    closed line repeats its start) and line_length[k] unit segments."""
+    line_left: torch.Tensor      # int32 [n_lines]
+    line_right: torch.Tensor     # int32 [n_lines]
+    line_length: torch.Tensor    # int64 [n_lines]
+    line_offsets: torch.Tensor   # int64 [n_lines + 1]
+    vertices: torch.Tensor       # int32 [n_vertices, 2]
+    boundary_segments: int
+
+    @property
+    def n_lines(self):
+        return self.line_left.shape[0]
+
+    def shapes(self, geotransform):
+        """-> one float64 [n, 2] polyline per line in map coordinates X = gt0 + x gt1, Y = gt3 + y gt5, with line_right
+        on the right of the direction of travel in (X, Y) too: a mirroring transform (gt1 gt5 > 0) reverses the vertex
+        order.  North-up geotransforms only."""
+        gt = [float(v) for v in geotransform]
+        if gt[2] != 0.0 or gt[4] != 0.0 or gt[1] == 0.0 or gt[5] == 0.0:
+            raise ValueError("Lines.shapes needs a north-up geotransform")
+        off = self.line_offsets.cpu().numpy()
+        v = self.vertices.cpu().numpy().astype(np.float64)
+        xy = np.stack([gt[0] + v[:, 0] * gt[1], gt[3] + v[:, 1] * gt[5]], axis=1)
+        flip = gt[1] * gt[5] > 0
+        return [xy[off[k]:off[k + 1]][::-1 if flip else 1] for k in range(len(off) - 1)]
+
+
+def default_line_capacity(n_regions, H, W):
+    return int(min(2 * H * W + H + W, max(1 << 16, 4 * (H + W) + 128 * n_regions), _MAX_CAPACITY))
+
+
+def boundary_lines(labels: torch.Tensor, n_regions: int, *, capacity=None) -> Lines:
+    """Boundary lines of an int32 label raster [H, W] on the GPU (strided row views accepted); negative labels are
+    nodata: one polyline per maximal chain of pixel sides between two values, ending where three or more boundaries
+    meet; see Lines for the layout.  `capacity` bounds the boundary segments; when it is too small the call is repeated
+    once with the exact count."""
+    L = lib()
+    _need_cuda(labels)
+    labels = _labels_2d(labels)
+    H, W = labels.shape
+    n_regions = int(n_regions)
+    dev = labels.device
+    ld = labels.stride(0) if H > 1 else W          # the row stride of a tensor with one row or none is arbitrary
+    cap = default_line_capacity(n_regions, H, W) if capacity is None else int(capacity)
+    with torch.cuda.device(dev):
+        for attempt in range(2):
+            left = torch.empty(max(cap, 1), dtype=_I32, device=dev)
+            right = torch.empty(max(cap, 1), dtype=_I32, device=dev)
+            length = torch.empty(max(cap, 1), dtype=_I64, device=dev)
+            offsets = torch.empty(cap + 1, dtype=_I64, device=dev)
+            vertices = torch.empty((max(2 * cap, 1), 2), dtype=_I32, device=dev)
+            counts = torch.zeros(4, dtype=_I64, device=dev)
+            ws_bytes = L.dm_lines_workspace_bytes(H, W, cap)
+            ws = torch.empty(max(ws_bytes, 1), dtype=_U8, device=dev)
+            L.check(L.dm_lines(_p(labels), H, W, ld, n_regions, cap, _p(left), _p(right), _p(length), _p(offsets),
+                               _p(vertices), _p(counts), _p(ws), ws_bytes, _stream()), "dm_lines")
+            c = counts.tolist()
+            if c[3] == 1:
+                raise ValueError("labels contain ids >= n_regions")
+            if c[3] == 2 and attempt == 0:
+                if c[2] > _MAX_CAPACITY:
+                    raise ValueError("the raster has %d boundary segments, more than 2^31 - 1" % c[2])
+                cap = int(c[2])
+                continue
+            if c[3] != 0:
+                raise RuntimeError("dm_lines: status %d" % c[3])
+            break
+    k, v = int(c[0]), int(c[1])
+    return Lines(left[:k], right[:k], length[:k], offsets[:k + 1], vertices[:v], int(c[2]))

@@ -21,6 +21,8 @@ the .dbf attribute table (dBase III, fixed-width ASCII records) and, for the poi
                   so the reference-shaped classes (deepmerge_b200.MyUtils2.PolygonConnectPointDataset) run on
                   real files when `osgeo` is not installed
   write_dbf / write_point_shp   writers (tests, and exporting a raster-derived RAG for GIS tools)
+  read_polygons / read_polylines, write_polygonized / write_boundary_lines   polygon and line geometry: the
+                  reference's tile.shp and lines.shp, read back or made from a label raster
 
 Conventions follow the OGR "ESRI Shapefile" driver: FID = record index, trailing blanks of strings
 are stripped, N fields without decimals are integers, blank / '*' filled numbers are null (None),
@@ -513,54 +515,53 @@ def Open(path, update=0):
 _POLY_TYPES = (5, 15, 25)           # Polygon, PolygonZ, PolygonM
 
 
-def read_polygons(path):
-    """-> list (one entry per record, FID order) of lists of rings, each ring a float64 [k, 2] array of (X, Y);
-    null shapes give an empty list.  Outer rings and holes are not distinguished: filling uses the even-odd rule."""
+def _read_multipart(path, types, kind):
     raw, st = _shp_header(path)
-    if st not in _POLY_TYPES:
-        raise ValueError("{0} is not a polygon shapefile (shape type {1})".format(path, st))
+    if st not in types:
+        raise ValueError("{0} is not a {1} shapefile (shape type {2})".format(path, kind, st))
     out = []
     off, end = 100, len(raw)
     while off + 8 <= end:
         (clen,) = struct.unpack_from(">i", raw, off + 4)
         body = off + 8
-        rings = []
-        if body + 44 <= end and struct.unpack_from("<i", raw, body)[0] in _POLY_TYPES:
+        parts_xy = []
+        if body + 44 <= end and struct.unpack_from("<i", raw, body)[0] in types:
             n_parts, n_points = struct.unpack_from("<ii", raw, body + 36)
             parts = list(struct.unpack_from("<%di" % n_parts, raw, body + 44)) + [n_points]
             pts = np.frombuffer(raw, "<f8", 2 * n_points, body + 44 + 4 * n_parts).reshape(n_points, 2)
-            rings = [pts[parts[i]:parts[i + 1]].copy() for i in range(n_parts)]
-        out.append(rings)
+            parts_xy = [pts[parts[i]:parts[i + 1]].copy() for i in range(n_parts)]
+        out.append(parts_xy)
         off = body + 2 * clen
     return out
 
 
-def write_polygon_shp(path, polygons):
-    """Polygon .shp + .shx; `polygons` = list of lists of rings ([k, 2] arrays, closed or not)."""
-    def closed(r):
-        r = np.asarray(r, np.float64).reshape(-1, 2)
-        return r if len(r) and np.array_equal(r[0], r[-1]) else np.concatenate([r, r[:1]])
+def read_polygons(path):
+    """-> list (one entry per record, FID order) of lists of rings, each ring a float64 [k, 2] array of (X, Y);
+    null shapes give an empty list.  Outer rings and holes are not distinguished: filling uses the even-odd rule."""
+    return _read_multipart(path, _POLY_TYPES, "polygon")
 
-    polys = [[closed(r) for r in rings] for rings in polygons]
-    allpts = np.concatenate([r for rings in polys for r in rings]) if any(polys) else np.zeros((1, 2))
+
+def _write_multipart(path, shape_type, records):
+    """.shp + .shx of a multi-part shape type: `records` = list of lists of parts ([k, 2] float64 arrays)."""
+    allpts = np.concatenate([p for parts in records for p in parts]) if any(records) else np.zeros((1, 2))
     bbox = (allpts[:, 0].min(), allpts[:, 1].min(), allpts[:, 0].max(), allpts[:, 1].max())
 
     def header(file_words):
         h = bytearray(100)
         struct.pack_into(">i", h, 0, 9994)
         struct.pack_into(">i", h, 24, file_words)
-        struct.pack_into("<ii", h, 28, 1000, 5)
+        struct.pack_into("<ii", h, 28, 1000, shape_type)
         struct.pack_into("<dddd", h, 36, *bbox)
         return bytes(h)
 
     recs, idx = bytearray(), bytearray()
-    for i, rings in enumerate(polys):
-        if rings:
-            pts = np.concatenate(rings)
-            starts = np.cumsum([0] + [len(r) for r in rings[:-1]])
-            content = struct.pack("<i4dii", 5, pts[:, 0].min(), pts[:, 1].min(), pts[:, 0].max(), pts[:, 1].max(),
-                                  len(rings), len(pts))
-            content += struct.pack("<%di" % len(rings), *starts.tolist()) + np.ascontiguousarray(pts, "<f8").tobytes()
+    for i, parts in enumerate(records):
+        if parts:
+            pts = np.concatenate(parts)
+            starts = np.cumsum([0] + [len(r) for r in parts[:-1]])
+            content = struct.pack("<i4dii", shape_type, pts[:, 0].min(), pts[:, 1].min(), pts[:, 0].max(),
+                                  pts[:, 1].max(), len(parts), len(pts))
+            content += struct.pack("<%di" % len(parts), *starts.tolist()) + np.ascontiguousarray(pts, "<f8").tobytes()
         else:
             content = struct.pack("<i", 0)
         idx += struct.pack(">ii", (100 + len(recs)) // 2, len(content) // 2)
@@ -570,6 +571,29 @@ def write_polygon_shp(path, polygons):
         f.write(header((100 + len(recs)) // 2) + bytes(recs))
     with open(base + ".shx", "wb") as f:
         f.write(header((100 + len(idx)) // 2) + bytes(idx))
+
+
+def write_polygon_shp(path, polygons):
+    """Polygon .shp + .shx; `polygons` = list of lists of rings ([k, 2] arrays, closed or not)."""
+    def closed(r):
+        r = np.asarray(r, np.float64).reshape(-1, 2)
+        return r if len(r) and np.array_equal(r[0], r[-1]) else np.concatenate([r, r[:1]])
+
+    _write_multipart(path, 5, [[closed(r) for r in rings] for rings in polygons])
+
+
+_LINE_TYPES = (3, 13, 23)           # PolyLine, PolyLineZ, PolyLineM
+
+
+def read_polylines(path):
+    """-> list (one entry per record, FID order) of lists of parts, each a float64 [k, 2] array of (X, Y); null
+    shapes give an empty list."""
+    return _read_multipart(path, _LINE_TYPES, "polyline")
+
+
+def write_polyline_shp(path, lines):
+    """PolyLine .shp + .shx with one single-part record per line ([k, 2] array of (X, Y), k >= 2)."""
+    _write_multipart(path, 3, [[np.asarray(v, np.float64).reshape(-1, 2)] for v in lines])
 
 
 def rasterize_polygons(polygons, geotransform, height, width, nodata=-1, ids=None):
@@ -649,3 +673,29 @@ def write_polygonized(path, polys, geotransform, columns=None):
         fields.append(FieldDefn(name, "N", 18, 0) if np.issubdtype(a.dtype, np.integer) else FieldDefn(name, OFTReal))
         cols[name] = a
     write_dbf(base + ".dbf", fields, cols)
+
+
+def write_boundary_lines(path, lines, geotransform):
+    """Write the boundary lines of a label raster (deepmerge_b200.boundary_lines -> Lines) as the reference's lines.shp:
+    one polyline record per line in canonical order with the attributes LEFT_FID / RIGHT_FID, the record index in the
+    polygon file that write_polygonized makes from the same raster of the region on the left / right of the line in map
+    coordinates (-1: nodata or outside the image), and LENGTH (pixel sides).  Every region with a pixel has a boundary,
+    so the regions present are the ids found on the lines, and a region's record index is the rank of its id among
+    them.  PolygonConnectPointDataset, score_layers and test_for_shp read the pair of files as they read the
+    reference's."""
+    shapes = lines.shapes(geotransform)
+    base = path[:-4] if path.lower().endswith(".shp") else path
+    write_polyline_shp(base + ".shp", shapes)
+    left = lines.line_left.cpu().numpy().astype(np.int64)
+    right = lines.line_right.cpu().numpy().astype(np.int64)
+    ids = np.unique(np.concatenate([left, right]))
+    ids = ids[ids >= 0]
+    fid = lambda v: np.where(v >= 0, np.searchsorted(ids, v), -1)
+    n = len(left)
+    fields = [FieldDefn("LEFT_FID", "N", 11, 0), FieldDefn("RIGHT_FID", "N", 11, 0), FieldDefn("LENGTH", "N", 18, 0)]
+    write_dbf(base + ".dbf", fields, records=np.full((n, 1 + 11 + 11 + 18), ord(" "), np.uint8))
+    t = DbfTable(base + ".dbf", update=True)
+    t.set_column("LEFT_FID", fid(left))
+    t.set_column("RIGHT_FID", fid(right))
+    t.set_column("LENGTH", lines.line_length.cpu().numpy().astype(np.int64))
+    t.flush()

@@ -476,6 +476,42 @@ int dm_polygonize(const int32_t* labels, int64_t H, int64_t W, int64_t ld, int64
                   int64_t* region_rings, int64_t* counts, void* ws, size_t ws_bytes, dm_stream_t stream);
 
 /* ----------------------------------------------------------------------------------- *
+ * Boundary lines of a label raster: the other half of the vector round trip, the reference's lines.shp (one polyline
+ * per shared boundary with LEFT_FID / RIGHT_FID, MyUtils2.py:155-193; its scores are written back onto these features,
+ * ExtractFeatures.py:181-186, 217-219).  Not part of the merge step.
+ *
+ * Pixel coordinates, y down; vertex (x, y) has 0 <= x <= W, 0 <= y <= H.  Every pixel has a value: its label when >= 0,
+ * else -1; positions outside the image have value -1.
+ *  - Boundary segment: a unit side between two 4-adjacent positions whose values differ (either may be outside the
+ *    image, so sides on the image border count; two nodata pixels never form one).
+ *  - Degree of a vertex: the number of boundary segments meeting there (0, 2, 3 or 4).  A node is a vertex of degree
+ *    >= 3: three or four distinct values around it, or a saddle (two values on the diagonals of the 2 x 2 block).
+ *  - Line: a maximal chain of boundary segments joined at vertices of degree 2.  An open line runs from a node to a
+ *    node (possibly the same one); a closed line is a cycle without a node (an island inside one region, a region that
+ *    fills the image, against -1).
+ *  - Orientation: every segment is travelled with the larger of its two values on its right ("right" as in
+ *    dm_polygonize: moving east, right is +y).  Along a line the same two values stay on the same sides, so
+ *    line_right = the larger value >= 0 and line_left = the smaller, which may be -1.
+ *  - Vertices of a line: the start, every corner, then the end, int32 (x, y).  A closed line starts at its smallest
+ *    vertex in (y, x) order (a corner) and repeats it at the end.
+ *  - Canonical order: lines ordered by (start y, start x, direction of the first segment: 0 E, 1 S, 2 W, 3 N), a
+ *    total order.  Two regions that share several disjoint pieces of boundary get one line per piece.
+ * Outputs (device, caller-owned), for capacity C:
+ *    line_left, line_right int32 [C]    line_length int64 [C] (unit segments)    line_offsets int64 [C + 1]
+ *    vertices int32 [2 C, 2] (a line has at most length + 1 vertices, so vertices <= segments + lines <= 2 C; a
+ *             raster of single-pixel checkers reaches it)
+ *    counts int64 [4]: [0] lines, [1] vertices, [2] boundary segments found (exact, also above capacity), [3] status:
+ *           0 ok, 1 a label >= n_regions, 2 capacity exceeded (outputs invalid; retry with capacity >= counts[2]).
+ * capacity bounds the boundary segments, < 2^31.  (H + 1) (W + 1) <= 2^32.  labels int32 [H, ld], ld >= W.  The
+ * workspace grows with H W / 4 bytes and the capacity.  The empty raster writes zero counts (when the outputs are given)
+ * and returns 0.
+ * ----------------------------------------------------------------------------------- */
+size_t dm_lines_workspace_bytes(int64_t H, int64_t W, int64_t capacity);
+int dm_lines(const int32_t* labels, int64_t H, int64_t W, int64_t ld, int64_t n_regions, int64_t capacity,
+             int32_t* line_left, int32_t* line_right, int64_t* line_length, int64_t* line_offsets, int32_t* vertices,
+             int64_t* counts, void* ws, size_t ws_bytes, dm_stream_t stream);
+
+/* ----------------------------------------------------------------------------------- *
  * R11 Contrastive pair loss forward + backward (Losses.py:34-38):
  *     d = sum_k (a-b)^2 ; L = mean(flag*d + (1-flag)*relu(margin-d)).
  *     loss fp32 [1]; grad_a, grad_b fp32 [B,D] (nullable).  flag int64 as collated.
