@@ -1,6 +1,7 @@
 // Boundary-line tracer: label raster -> one polyline per maximal chain of boundary segments between nodes, with the
-// values on its left and right (dm_lines in include/deepmerge_b200.h).  The per-vertex rule lives in lines_core.cuh;
-// the mask pass, the dense index and the pointer jumping in chain.cuh, shared with the polygonizer (polygon.cu).
+// values on its left and right (dm_lines in include/deepmerge_b200.h).  The per-vertex arithmetic lives in
+// lines_core.cuh.  Steps 1 to 5 are the kernels and the launch sequence (chain::trace) of chain.cuh, shared with the
+// polygonizer (polygon.cu); SegmentRule is their per-segment part.
 //
 // 1. mask_kernel    one pass over the labels: a 4-bit mask of the segments each pixel owns, counts per word, the
 //                   label range check.
@@ -29,20 +30,8 @@ constexpr uint8_t EMIT = 4;        // the head vertex is a vertex of the line (a
 constexpr uint8_t NODE_HEAD = 8;
 constexpr uint8_t NODE_TAIL = 16;
 
-struct OwnedMask {
-    static __device__ __forceinline__ unsigned mask(const int32_t* L, int64_t H, int64_t W, int64_t ld, int64_t x, int64_t y) {
-        return owned_mask(L, H, W, ld, x, y);
-    }
-};
-
-struct Ws {
-    uint32_t *masks, *wcnt, *wbase;
-    void* scan;
-    int64_t* n_words_dev;
-    int* changed;                       // [2][MAX_PASSES]: pass k of phase f changed a word
-    uint32_t *hv, *nxt, *line_of;       // per segment: head vertex y (W+1) + x, successor, line ended by the segment
-    uint8_t* flags;
-    uint64_t* jw;                       // per segment: the pointer-jumping word (value << 32 | pointer)
+struct Ws : Front {
+    uint32_t* line_of;                  // per segment: line ended by the segment
     uint64_t* lkeys;                    // per line: start vertex << 32 | direction of the first segment
     uint32_t *lvals, *vcount, *offs;    // per line: first segment, vertices, vertex offset
     void* sort;
@@ -50,18 +39,8 @@ struct Ws {
 
 size_t carve(Ws& w, void* base, int64_t H, int64_t W, int64_t cap) {
     Carver c(base);
-    const int64_t n_words = H * ceil_div(W, 32);
-    w.masks = c.take<uint32_t>((size_t)n_words * 4);
-    w.wcnt = c.take<uint32_t>((size_t)n_words);
-    w.wbase = c.take<uint32_t>((size_t)n_words);
-    w.scan = c.take<char>(prims::scan_ws_bytes(imax64(n_words, cap)));
-    w.n_words_dev = c.take<int64_t>(1);
-    w.changed = c.take<int>(2 * MAX_PASSES);
-    w.hv = c.take<uint32_t>((size_t)cap);
-    w.nxt = c.take<uint32_t>((size_t)cap);
+    carve_front(w, c, H, W, cap, cap);
     w.line_of = c.take<uint32_t>((size_t)cap);
-    w.flags = c.take<uint8_t>((size_t)cap);
-    w.jw = c.take<uint64_t>((size_t)cap);
     w.lkeys = c.take<uint64_t>((size_t)cap);
     w.lvals = c.take<uint32_t>((size_t)cap);
     w.vcount = c.take<uint32_t>((size_t)cap);
@@ -74,58 +53,39 @@ size_t carve(Ws& w, void* base, int64_t H, int64_t W, int64_t cap) {
 // last two vertices of the last vertex row (when (H + 1) (W + 1) = 2^32), and no cycle has its smallest vertex there.
 __device__ __forceinline__ uint64_t vertex_key(uint32_t hv) { return hv == 0xffffffffu ? hv : (uint64_t)hv + 1; }
 
-__global__ void __launch_bounds__(NT) emit_kernel(const int32_t* __restrict__ L, int64_t H, int64_t W, int64_t ld,
-                                                  int64_t wpr, int64_t cap, const uint32_t* __restrict__ masks,
-                                                  const uint32_t* __restrict__ wbase, int64_t* __restrict__ counts, Ws ws) {
-    if (failed(counts)) return;
-    if (counts[2] > cap) {
-        if (blockIdx.x == 0 && threadIdx.x == 0) counts[3] = 2;
-        return;
-    }
-    const int lane = threadIdx.x & 31;
-    const int64_t n_words = H * wpr;
-    const int64_t warp0 = ((int64_t)blockIdx.x * NT + threadIdx.x) >> 5, nwarps = ((int64_t)gridDim.x * NT) >> 5;
-    for (int64_t w = warp0; w < n_words; w += nwarps) {
-        const int64_t y = w / wpr, x = (w - y * wpr) * 32 + lane;
-        const unsigned m = (masks[w * 4 + (lane >> 3)] >> (4 * (lane & 7))) & 15u;
-        if (!__any_sync(0xffffffffu, m)) continue;
-        const unsigned c = __popc(m);
-        unsigned inc = c;
-#pragma unroll
-        for (int o = 1; o < 32; o <<= 1) {
-            const unsigned t = __shfl_up_sync(0xffffffffu, inc, o);
-            if (lane >= o) inc += t;
-        }
-        uint32_t i = wbase[w] + inc - c;
-        for (int b = 0; b < 4; ++b) {
-            if (!((m >> b) & 1u)) continue;
-            const Seg s = orient(L, H, W, ld, x, y, b);
-            const int64_t hx = s.x + step_x(s.d), hy = s.y + step_y(s.d);
-            const Next q = next_at(L, H, W, ld, hx, hy, s.d);
-            uint32_t j = i;
-            if (!q.node) {
-                const Owner o = owner_of(H, W, hx, hy, q.d);
-                j = dense_index(masks, wbase, wpr, o.x, o.y, o.b);
-            }
-            const uint32_t hv = (uint32_t)(hy * (W + 1) + hx);
-            uint8_t f = (uint8_t)s.d;
-            if (q.node || q.d != s.d) f |= EMIT;
-            if (q.node) f |= NODE_HEAD;
-            if (node_arms(arms(L, H, W, ld, s.x, s.y))) f |= NODE_TAIL;
-            ws.hv[i] = hv;
-            ws.nxt[i] = j;
-            ws.flags[i] = f;
-            ws.jw[i] = ((q.node ? 0 : vertex_key(hv)) << 32) | j;
-            ++i;
-        }
-    }
-}
+struct SegmentRule {
+    using Ws = lines::Ws;
 
-// After phase 0: list the lines and turn every word into phase 1's.
-__global__ void __launch_bounds__(NT) starts_kernel(int64_t* __restrict__ counts, int64_t W, int64_t cap, Ws ws) {
-    if (failed(counts)) return;
-    const int64_t n = counts[2];
-    for (int64_t i = (int64_t)blockIdx.x * NT + threadIdx.x; i < n; i += (int64_t)gridDim.x * NT) {
+    static __device__ __forceinline__ unsigned mask(const int32_t* L, int64_t H, int64_t W, int64_t ld, int64_t x, int64_t y) {
+        return owned_mask(L, H, W, ld, x, y);
+    }
+
+    // segment b of pixel (x, y): orientation, head vertex, flags and the dense index of its successor at the head; a
+    // segment whose head is a node points at itself
+    static __device__ __forceinline__ void emit(const int32_t* L, int64_t H, int64_t W, int64_t ld, int64_t wpr,
+                                                const uint32_t* masks, const uint32_t* wbase, int64_t x, int64_t y,
+                                                int b, uint32_t i, const Ws& ws) {
+        const Seg s = orient(L, H, W, ld, x, y, b);
+        const int64_t hx = s.x + step_x(s.d), hy = s.y + step_y(s.d);
+        const Next q = next_at(L, H, W, ld, hx, hy, s.d);
+        uint32_t j = i;
+        if (!q.node) {
+            const Owner o = owner_of(H, W, hx, hy, q.d);
+            j = dense_index(masks, wbase, wpr, o.x, o.y, o.b);
+        }
+        const uint32_t hv = (uint32_t)(hy * (W + 1) + hx);
+        uint8_t f = (uint8_t)s.d;
+        if (q.node || q.d != s.d) f |= EMIT;
+        if (q.node) f |= NODE_HEAD;
+        if (node_arms(arms(L, H, W, ld, s.x, s.y))) f |= NODE_TAIL;
+        ws.hv[i] = hv;
+        ws.nxt[i] = j;
+        ws.flags[i] = f;
+        ws.jw[i] = ((q.node ? 0 : vertex_key(hv)) << 32) | j;
+    }
+
+    // list the line segment i starts, if any, and turn its word into phase 1's
+    static __device__ __forceinline__ void start(int64_t* counts, int64_t W, int64_t cap, const Ws& ws, int64_t i) {
         const uint32_t hv = ws.hv[i], j = ws.nxt[i];
         const uint8_t f = ws.flags[i];
         const bool anchor = (ws.jw[i] >> 32) == vertex_key(hv);   // its head is its cycle's smallest vertex
@@ -149,7 +109,7 @@ __global__ void __launch_bounds__(NT) starts_kernel(int64_t* __restrict__ counts
         }
         ws.jw[i] = anchor || (f & NODE_HEAD) ? (uint64_t)i : ((uint64_t)((ws.flags[j] & EMIT) ? 1 : 0) << 32) | j;
     }
-}
+};
 
 // per line in final order: values, length cleared, vertex count (start + emitting segments from the first to the end)
 __global__ void __launch_bounds__(NT) info_kernel(const int32_t* __restrict__ L, int64_t H, int64_t W, int64_t ld,
@@ -207,12 +167,8 @@ __global__ void __launch_bounds__(NT) vertex_kernel(const int64_t* __restrict__ 
 
 using namespace dm;
 
-static bool lines_extent_ok(int64_t H, int64_t W) {
-    return H >= 0 && W >= 0 && H < (1ll << 31) && W < (1ll << 31) && (H + 1) * (W + 1) <= (1ll << 32);
-}
-
 extern "C" size_t dm_lines_workspace_bytes(int64_t H, int64_t W, int64_t capacity) {
-    if (!lines_extent_ok(H, W) || capacity < 0 || capacity >= (1ll << 31)) return 0;
+    if (!chain::extent_ok(H, W, capacity)) return 0;
     lines::Ws w;
     return lines::carve(w, nullptr, H, W, capacity);
 }
@@ -220,44 +176,22 @@ extern "C" size_t dm_lines_workspace_bytes(int64_t H, int64_t W, int64_t capacit
 extern "C" int dm_lines(const int32_t* labels, int64_t H, int64_t W, int64_t ld, int64_t n_regions, int64_t capacity,
                         int32_t* line_left, int32_t* line_right, int64_t* line_length, int64_t* line_offsets,
                         int32_t* vertices, int64_t* counts, void* ws, size_t ws_bytes, dm_stream_t stream) {
-    if (!lines_extent_ok(H, W) || ld < W || n_regions < 0 || n_regions >= (1ll << 31) || capacity < 0 ||
-        capacity >= (1ll << 31))
-        return DM_ERR_BAD_ARG;
+    if (!chain::args_ok(H, W, ld, n_regions, capacity)) return DM_ERR_BAD_ARG;
     cudaStream_t s = S(stream);
-    if (H == 0 || W == 0) {
-        if (counts) DM_CUDA(cudaMemsetAsync(counts, 0, 4 * sizeof(int64_t), s));
-        if (line_offsets) DM_CUDA(cudaMemsetAsync(line_offsets, 0, sizeof(int64_t), s));
-        return DM_OK;
-    }
+    if (H == 0 || W == 0) return chain::clear_empty(counts, line_offsets, s);
     if (!labels || !line_offsets || !counts || !ws ||
         (capacity > 0 && (!line_left || !line_right || !line_length || !vertices)))
         return DM_ERR_BAD_ARG;
     if (ws_bytes < dm_lines_workspace_bytes(H, W, capacity)) return DM_ERR_WORKSPACE;
     lines::Ws w;
     lines::carve(w, ws, H, W, capacity);
-    const int64_t wpr = ceil_div(W, 32), n_words = H * wpr;
-    DM_CUDA(cudaMemsetAsync(counts, 0, 4 * sizeof(int64_t), s));
-    DM_CUDA(cudaMemsetAsync(w.changed, 0, 2 * chain::MAX_PASSES * sizeof(int), s));
-    const unsigned g_words = grid_for(n_words * 32, chain::NT, 16), g_segs = grid_for(capacity + 1, chain::NT, 16);
-    DM_TRY(launch(chain::mask_kernel<lines::OwnedMask>, g_words, chain::NT, 0, s, labels, H, W, ld, wpr, n_regions,
-                  w.masks, w.wcnt, counts, w.n_words_dev));
-    DM_TRY(prims::scan_exclusive_u32(w.wcnt, w.wbase, w.n_words_dev, n_words, nullptr, w.scan, s));
-    DM_TRY(launch(lines::emit_kernel, g_words, chain::NT, 0, s, labels, H, W, ld, wpr, capacity, w.masks, w.wbase, counts,
-                  w));
-    const int passes = chain::ceil_log2(capacity) + 1;
-    for (int phase = 0; phase < 2; ++phase) {
-        for (int k = 0; k < passes; ++k) {
-            DM_TRY(launch(chain::jump_kernel, g_segs, chain::NT, 0, s, w.jw, counts, w.changed, phase, k));
-        }
-        if (phase == 0) {
-            DM_TRY(launch(lines::starts_kernel, g_segs, chain::NT, 0, s, counts, W, capacity, w));
-        }
-    }
+    DM_TRY(chain::trace<lines::SegmentRule>(labels, H, W, ld, n_regions, capacity, counts, w, s));
+    const unsigned g_lines = grid_for(capacity + 1, chain::NT, 16);
     // lines by start vertex (high half), then by the direction of their first segment (low half)
     const int vb = bits_for((H + 1) * (W + 1));
     DM_TRY(prims::sort_pairs(w.lkeys, w.lvals, counts, capacity, vb, 2 * vb, w.sort, s));
-    DM_TRY(launch(lines::info_kernel, g_segs, chain::NT, 0, s, labels, H, W, ld, counts, line_left, line_right,
+    DM_TRY(launch(lines::info_kernel, g_lines, chain::NT, 0, s, labels, H, W, ld, counts, line_left, line_right,
                   line_length, w));
     DM_TRY(prims::scan_exclusive_u32(w.vcount, w.offs, counts, capacity, counts + 1, w.scan, s));
-    return launch(lines::vertex_kernel, g_segs, chain::NT, 0, s, counts, W, w, vertices, line_offsets, line_length);
+    return launch(lines::vertex_kernel, g_lines, chain::NT, 0, s, counts, W, w, vertices, line_offsets, line_length);
 }

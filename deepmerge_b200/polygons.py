@@ -14,6 +14,51 @@ from .raster import _I32, _I64, _U8, _labels_2d, _need_cuda, _p, _stream
 _MAX_CAPACITY = (1 << 31) - 1
 
 
+def _trace(labels, n_regions, capacity, default_capacity, outputs, entry, workspace_bytes, elements):
+    """Runs the library's tracer `entry` (dm_polygonize or dm_lines, whose arguments are labels, H, W, ld, n_regions,
+    capacity, the output buffers, counts, workspace, stream) -> (counts as a list, the output buffers).
+    outputs(cap, device) allocates the buffers for a capacity of cap boundary elements (`elements` names them);
+    workspace_bytes(lib, H, W, n_regions, cap) is the tracer's workspace query.  When the capacity is too small the call
+    is repeated once with the exact count."""
+    L = lib()
+    _need_cuda(labels)
+    labels = _labels_2d(labels)
+    H, W = labels.shape
+    n_regions = int(n_regions)
+    dev = labels.device
+    ld = labels.stride(0) if H > 1 else W          # the row stride of a tensor with one row or none is arbitrary
+    cap = default_capacity(n_regions, H, W) if capacity is None else int(capacity)
+    with torch.cuda.device(dev):
+        for attempt in range(2):
+            outs = outputs(cap, dev)
+            counts = torch.zeros(4, dtype=_I64, device=dev)
+            ws_bytes = workspace_bytes(L, H, W, n_regions, cap)
+            ws = torch.empty(max(ws_bytes, 1), dtype=_U8, device=dev)
+            L.check(getattr(L, entry)(_p(labels), H, W, ld, n_regions, cap, *[_p(t) for t in outs], _p(counts), _p(ws),
+                                      ws_bytes, _stream()), entry)
+            c = counts.tolist()
+            if c[3] == 1:
+                raise ValueError("labels contain ids >= n_regions")
+            if c[3] == 2 and attempt == 0:
+                if c[2] > _MAX_CAPACITY:
+                    raise ValueError("the raster has %d %s, more than 2^31 - 1" % (c[2], elements))
+                cap = int(c[2])
+                continue
+            if c[3] != 0:
+                raise RuntimeError("%s: status %d" % (entry, c[3]))
+            return c, outs
+
+
+def _map_xy(shapes, geotransform):
+    """-> (float64 [n, 2] map coordinates X = gt0 + x gt1, Y = gt3 + y gt5 of shapes.vertices, whether the transform
+    mirrors: gt1 gt5 > 0).  North-up geotransforms only."""
+    gt = [float(v) for v in geotransform]
+    if gt[2] != 0.0 or gt[4] != 0.0 or gt[1] == 0.0 or gt[5] == 0.0:
+        raise ValueError("%s.shapes needs a north-up geotransform" % type(shapes).__name__)
+    v = shapes.vertices.cpu().numpy().astype(np.float64)
+    return np.stack([gt[0] + v[:, 0] * gt[1], gt[3] + v[:, 1] * gt[5]], axis=1), gt[1] * gt[5] > 0
+
+
 @dataclass
 class Polygons:
     """Rings of every region present, in canonical order (include/deepmerge_b200.h, dm_polygonize): ring k of
@@ -35,16 +80,11 @@ class Polygons:
         """-> (region_ids int64 [k], rings_per_region): for every region present, ascending, its rings as float64
         [n + 1, 2] closed rings in map coordinates X = gt0 + x gt1, Y = gt3 + y gt5, outer rings clockwise and holes
         counter-clockwise in (X, Y) as the shapefile specification requires.  North-up geotransforms only."""
-        gt = [float(v) for v in geotransform]
-        if gt[2] != 0.0 or gt[4] != 0.0 or gt[1] == 0.0 or gt[5] == 0.0:
-            raise ValueError("Polygons.shapes needs a north-up geotransform")
-        rr = self.region_rings.cpu().numpy()
-        off = self.ring_offsets.cpu().numpy()
-        v = self.vertices.cpu().numpy().astype(np.float64)
-        xy = np.stack([gt[0] + v[:, 0] * gt[1], gt[3] + v[:, 1] * gt[5]], axis=1)
         # outer rings have positive area in pixel coordinates; in (X, Y) the sign is multiplied by that of gt1 gt5, and
         # clockwise means negative there
-        flip = gt[1] * gt[5] > 0
+        xy, flip = _map_xy(self, geotransform)
+        rr = self.region_rings.cpu().numpy()
+        off = self.ring_offsets.cpu().numpy()
         ids = np.flatnonzero(np.diff(rr) > 0)
         out = []
         for r in ids:
@@ -72,39 +112,17 @@ def polygonize(labels: torch.Tensor, n_regions: int, *, capacity=None) -> Polygo
     """Rings of every region of an int32 label raster [H, W] on the GPU (strided row views accepted); negative labels
     are nodata.  Regions are 4-connected; see Polygons for the layout.  `capacity` bounds the boundary sides; when it
     is too small the call is repeated once with the exact count."""
-    L = lib()
-    _need_cuda(labels)
-    labels = _labels_2d(labels)
-    H, W = labels.shape
-    n_regions = int(n_regions)
-    dev = labels.device
-    ld = labels.stride(0) if H > 1 else W          # the row stride of a tensor with one row or none is arbitrary
-    cap = default_capacity(n_regions, H, W) if capacity is None else int(capacity)
-    with torch.cuda.device(dev):
-        for attempt in range(2):
-            ring_cap = cap // 4
-            ring_region = torch.empty(max(ring_cap, 1), dtype=_I32, device=dev)
-            ring_offsets = torch.empty(ring_cap + 1, dtype=_I64, device=dev)
-            ring_area = torch.empty(max(ring_cap, 1), dtype=_I64, device=dev)
-            vertices = torch.empty((max(cap, 1), 2), dtype=_I32, device=dev)
-            region_rings = torch.empty(n_regions + 1, dtype=_I64, device=dev)
-            counts = torch.zeros(4, dtype=_I64, device=dev)
-            ws_bytes = L.dm_polygonize_workspace_bytes(H, W, n_regions, cap)
-            ws = torch.empty(max(ws_bytes, 1), dtype=_U8, device=dev)
-            L.check(L.dm_polygonize(_p(labels), H, W, ld, n_regions, cap, _p(ring_region), _p(ring_offsets),
-                                    _p(ring_area), _p(vertices), _p(region_rings), _p(counts), _p(ws), ws_bytes,
-                                    _stream()), "dm_polygonize")
-            c = counts.tolist()
-            if c[3] == 1:
-                raise ValueError("labels contain ids >= n_regions")
-            if c[3] == 2 and attempt == 0:
-                if c[2] > _MAX_CAPACITY:
-                    raise ValueError("the raster has %d boundary sides, more than 2^31 - 1" % c[2])
-                cap = int(c[2])
-                continue
-            if c[3] != 0:
-                raise RuntimeError("dm_polygonize: status %d" % c[3])
-            break
+    def outputs(cap, dev):
+        ring_cap = cap // 4
+        return (torch.empty(max(ring_cap, 1), dtype=_I32, device=dev),       # ring_region
+                torch.empty(ring_cap + 1, dtype=_I64, device=dev),           # ring_offsets
+                torch.empty(max(ring_cap, 1), dtype=_I64, device=dev),       # ring_area
+                torch.empty((max(cap, 1), 2), dtype=_I32, device=dev),       # vertices
+                torch.empty(int(n_regions) + 1, dtype=_I64, device=dev))     # region_rings
+
+    c, (ring_region, ring_offsets, ring_area, vertices, region_rings) = _trace(
+        labels, n_regions, capacity, default_capacity, outputs, "dm_polygonize",
+        lambda L, H, W, R, cap: L.dm_polygonize_workspace_bytes(H, W, R, cap), "boundary sides")
     k, v = int(c[0]), int(c[1])
     return Polygons(ring_region[:k], ring_offsets[:k + 1], ring_area[:k], vertices[:v], region_rings, int(c[2]))
 
@@ -130,13 +148,8 @@ class Lines:
         """-> one float64 [n, 2] polyline per line in map coordinates X = gt0 + x gt1, Y = gt3 + y gt5, with line_right
         on the right of the direction of travel in (X, Y) too: a mirroring transform (gt1 gt5 > 0) reverses the vertex
         order.  North-up geotransforms only."""
-        gt = [float(v) for v in geotransform]
-        if gt[2] != 0.0 or gt[4] != 0.0 or gt[1] == 0.0 or gt[5] == 0.0:
-            raise ValueError("Lines.shapes needs a north-up geotransform")
+        xy, flip = _map_xy(self, geotransform)
         off = self.line_offsets.cpu().numpy()
-        v = self.vertices.cpu().numpy().astype(np.float64)
-        xy = np.stack([gt[0] + v[:, 0] * gt[1], gt[3] + v[:, 1] * gt[5]], axis=1)
-        flip = gt[1] * gt[5] > 0
         return [xy[off[k]:off[k + 1]][::-1 if flip else 1] for k in range(len(off) - 1)]
 
 
@@ -149,36 +162,15 @@ def boundary_lines(labels: torch.Tensor, n_regions: int, *, capacity=None) -> Li
     nodata: one polyline per maximal chain of pixel sides between two values, ending where three or more boundaries
     meet; see Lines for the layout.  `capacity` bounds the boundary segments; when it is too small the call is repeated
     once with the exact count."""
-    L = lib()
-    _need_cuda(labels)
-    labels = _labels_2d(labels)
-    H, W = labels.shape
-    n_regions = int(n_regions)
-    dev = labels.device
-    ld = labels.stride(0) if H > 1 else W          # the row stride of a tensor with one row or none is arbitrary
-    cap = default_line_capacity(n_regions, H, W) if capacity is None else int(capacity)
-    with torch.cuda.device(dev):
-        for attempt in range(2):
-            left = torch.empty(max(cap, 1), dtype=_I32, device=dev)
-            right = torch.empty(max(cap, 1), dtype=_I32, device=dev)
-            length = torch.empty(max(cap, 1), dtype=_I64, device=dev)
-            offsets = torch.empty(cap + 1, dtype=_I64, device=dev)
-            vertices = torch.empty((max(2 * cap, 1), 2), dtype=_I32, device=dev)
-            counts = torch.zeros(4, dtype=_I64, device=dev)
-            ws_bytes = L.dm_lines_workspace_bytes(H, W, cap)
-            ws = torch.empty(max(ws_bytes, 1), dtype=_U8, device=dev)
-            L.check(L.dm_lines(_p(labels), H, W, ld, n_regions, cap, _p(left), _p(right), _p(length), _p(offsets),
-                               _p(vertices), _p(counts), _p(ws), ws_bytes, _stream()), "dm_lines")
-            c = counts.tolist()
-            if c[3] == 1:
-                raise ValueError("labels contain ids >= n_regions")
-            if c[3] == 2 and attempt == 0:
-                if c[2] > _MAX_CAPACITY:
-                    raise ValueError("the raster has %d boundary segments, more than 2^31 - 1" % c[2])
-                cap = int(c[2])
-                continue
-            if c[3] != 0:
-                raise RuntimeError("dm_lines: status %d" % c[3])
-            break
+    def outputs(cap, dev):
+        return (torch.empty(max(cap, 1), dtype=_I32, device=dev),            # left
+                torch.empty(max(cap, 1), dtype=_I32, device=dev),            # right
+                torch.empty(max(cap, 1), dtype=_I64, device=dev),            # length
+                torch.empty(cap + 1, dtype=_I64, device=dev),                # offsets
+                torch.empty((max(2 * cap, 1), 2), dtype=_I32, device=dev))   # vertices
+
+    c, (left, right, length, offsets, vertices) = _trace(
+        labels, n_regions, capacity, default_line_capacity, outputs, "dm_lines",
+        lambda L, H, W, R, cap: L.dm_lines_workspace_bytes(H, W, cap), "boundary segments")
     k, v = int(c[0]), int(c[1])
     return Lines(left[:k], right[:k], length[:k], offsets[:k + 1], vertices[:v], int(c[2]))

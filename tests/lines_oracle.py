@@ -1,38 +1,16 @@
 """Loader of tests/lines_oracle.c, the sequential boundary-line tracer the tests and tools/time_lines.py compare dm_lines
-against.  TEST INFRASTRUCTURE ONLY.  The library is compiled with gcc into a temporary directory once per process, so
-the source tree is never written."""
+against.  TEST INFRASTRUCTURE ONLY.  c_oracle.load builds it."""
 from __future__ import annotations
 
-import atexit
 import ctypes
-import os
-import shutil
-import subprocess
-import tempfile
 
-HERE = os.path.dirname(os.path.abspath(__file__))
-SRC = os.path.join(HERE, "lines_oracle.c")
-
-_LIB = None
+from c_oracle import load
 
 
 def lib():
-    global _LIB
-    if _LIB is None:
-        d = tempfile.mkdtemp(prefix="lines_oracle_")
-        atexit.register(shutil.rmtree, d, True)
-        so = os.path.join(d, "liblines_oracle.so")
-        r = subprocess.run(["gcc", "-O2", "-std=c99", "-shared", "-fPIC", "-o", so, SRC], capture_output=True, text=True)
-        if r.returncode != 0:
-            raise RuntimeError("gcc failed on lines_oracle.c:\n" + r.stderr)
-        L = ctypes.CDLL(so)
-        p, i64, i = ctypes.c_void_p, ctypes.c_int64, ctypes.c_int
-        L.dmo_line_segments.restype = i64
-        L.dmo_line_segments.argtypes = [p, i64, i64, p]
-        L.dmo_lines.restype = i
-        L.dmo_lines.argtypes = [p, i64, i64, i64, p, p, p, p, p, p]
-        _LIB = L
-    return _LIB
+    p, i64, i = ctypes.c_void_p, ctypes.c_int64, ctypes.c_int
+    return load("lines_oracle", {"dmo_line_segments": (i64, [p, i64, i64, p]),
+                                 "dmo_lines": (i, [p, i64, i64, i64, p, p, p, p, p, p])})
 
 
 def n_segments(L):

@@ -1,38 +1,16 @@
 """Loader of tests/polygon_oracle.c, the sequential polygonizer the tests and tools/time_polygonize.py compare
-dm_polygonize against.  TEST INFRASTRUCTURE ONLY.  The library is compiled with gcc into a temporary directory once
-per process, so the source tree is never written."""
+dm_polygonize against.  TEST INFRASTRUCTURE ONLY.  c_oracle.load builds it."""
 from __future__ import annotations
 
-import atexit
 import ctypes
-import os
-import shutil
-import subprocess
-import tempfile
 
-HERE = os.path.dirname(os.path.abspath(__file__))
-SRC = os.path.join(HERE, "polygon_oracle.c")
-
-_LIB = None
+from c_oracle import load
 
 
 def lib():
-    global _LIB
-    if _LIB is None:
-        d = tempfile.mkdtemp(prefix="polygon_oracle_")
-        atexit.register(shutil.rmtree, d, True)
-        so = os.path.join(d, "libpolygon_oracle.so")
-        r = subprocess.run(["gcc", "-O2", "-std=c99", "-shared", "-fPIC", "-o", so, SRC], capture_output=True, text=True)
-        if r.returncode != 0:
-            raise RuntimeError("gcc failed on polygon_oracle.c:\n" + r.stderr)
-        L = ctypes.CDLL(so)
-        p, i64, i = ctypes.c_void_p, ctypes.c_int64, ctypes.c_int
-        L.dmo_poly_successor.restype = i
-        L.dmo_poly_successor.argtypes = [p, i64, i64, i64, i64, i, p]
-        L.dmo_polygonize.restype = i
-        L.dmo_polygonize.argtypes = [p, i64, i64, i64, p, p, p, p, p, p]
-        _LIB = L
-    return _LIB
+    p, i64, i = ctypes.c_void_p, ctypes.c_int64, ctypes.c_int
+    return load("polygon_oracle", {"dmo_poly_successor": (i, [p, i64, i64, i64, i64, i, p]),
+                                   "dmo_polygonize": (i, [p, i64, i64, i64, p, p, p, p, p, p])})
 
 
 def polygonize(labels, n_regions):

@@ -5,7 +5,8 @@ rasters with nodata against what shares no code with it: the boundary segments a
 orientation rule, the canonical order, and the boundary lengths and perimeters of oracle_np.build_rag.  The shapefile
 writer is checked by a round trip that pairs the line file with write_polygonized's polygon file.
 deepmerge_b200/csrc/lines_core.cuh (the kernels' per-vertex rule) is compiled with g++ and checked against the oracle
-on every 2 x 2 configuration.  The ABI rejects bad arguments without CUDA and before it enqueues anything."""
+on every 2 x 2 configuration.  The ABI rejects bad arguments without CUDA and before it enqueues anything (the checks
+of tests/tracer_abi.py, which test_polygonize_cpu runs on dm_polygonize)."""
 import ctypes
 import itertools
 import os
@@ -16,6 +17,7 @@ import pytest
 
 import lines_oracle as lo
 import polygon_oracle as po
+import tracer_abi
 from oracle import oracle_np as o
 from test_polygonize_cpu import CASES as POLY_CASES
 
@@ -266,68 +268,11 @@ def test_core_rule_on_every_2x2_block(core):
 # ---- ABI without CUDA -----------------------------------------------------------------------------------------------
 
 def test_abi_rejects_bad_arguments_without_cuda():
-    from deepmerge_b200 import _lib
-    L = _lib.lib()
-    bad = _lib.DM_ERR_BAD_ARG
-    f = L.dm_lines
-    nul = [None] * 6
-    assert f(None, 4, 4, 4, 3, 64, *nul, None, 0, None) == bad                  # null pointers with work to do
-    assert f(None, -1, 4, 4, 3, 64, *nul, None, 0, None) == bad                 # negative extent
-    assert f(None, 4, -1, 4, 3, 64, *nul, None, 0, None) == bad
-    assert f(None, 4, 4, 3, 3, 64, *nul, None, 0, None) == bad                  # ld < W
-    assert f(None, 4, 4, 4, 3, 1 << 31, *nul, None, 0, None) == bad             # capacity >= 2^31
-    assert f(None, 4, 4, 4, 3, -1, *nul, None, 0, None) == bad                  # negative capacity
-    assert f(None, 4, 4, 4, -1, 64, *nul, None, 0, None) == bad                 # negative region count
-    assert f(None, 1 << 20, 1 << 20, 1 << 20, 3, 64, *nul, None, 0, None) == bad    # more than 2^32 vertices
-    assert f(None, 0, 4, 4, 3, 64, *nul, None, 0, None) == 0                    # empty raster
-    assert f(None, 4, 0, 0, 3, 64, *nul, None, 0, None) == 0
-    assert L.dm_lines_workspace_bytes(64, 64, -1) == 0
-    assert 0 < L.dm_lines_workspace_bytes(64, 64, 1000) < L.dm_lines_workspace_bytes(64, 64, 100000)
-    assert L.dm_lines_workspace_bytes(1024, 1024, 1000) >= 1024 * 1024 // 2     # 4 bits of segments per pixel
+    tracer_abi.check_rejects_bad_arguments("dm_lines")
 
 
 def test_no_work_is_enqueued_before_an_argument_error():
-    """dm_lines checks every argument, the workspace size included, before it enqueues anything: a call that returns
-    DM_ERR_BAD_ARG or DM_ERR_WORKSPACE has launched no kernel and written no output."""
-    import torch
-    from deepmerge_b200 import _lib
-    L = _lib.lib()
-    cuda = torch.cuda.is_available()
-    probes = []
-
-    def buf(nbytes):
-        # With CUDA: device memory holding a sentinel of its own, which must survive the call.  Without: an address
-        # that nothing may dereference -- every CUDA call fails there first (DM_ERR_CUDA), so a bad-argument result
-        # shows that no CUDA call was made.
-        if not cuda:
-            return 16
-        t = torch.full((nbytes,), 0x41 + len(probes), dtype=torch.uint8, device="cuda")
-        probes.append((t, t.clone()))
-        return t.data_ptr()
-
-    bad, short = _lib.DM_ERR_BAD_ARG, _lib.DM_ERR_WORKSPACE
-    R, cap, H, W = 10, 64, 4, 4
-    ws = L.dm_lines_workspace_bytes(H, W, cap)
-
-    def outs():             # left, right, length, offsets, vertices, counts
-        return buf(4 * cap), buf(4 * cap), buf(8 * cap), buf(8 * cap + 8), buf(16 * cap), buf(32)
-
-    cases = [
-        ("labels", bad, lambda: L.dm_lines(None, H, W, W, R, cap, *outs(), buf(ws), ws, None)),
-        ("vertices", bad, lambda: L.dm_lines(buf(4 * H * W), H, W, W, R, cap, *outs()[:4], None, buf(32), buf(ws), ws,
-                                             None)),
-        ("workspace pointer", bad, lambda: L.dm_lines(buf(4 * H * W), H, W, W, R, cap, *outs(), None, ws, None)),
-        ("ld", bad, lambda: L.dm_lines(buf(4 * H * W), H, W, W - 1, R, cap, *outs(), buf(ws), ws, None)),
-        ("workspace", short, lambda: L.dm_lines(buf(4 * H * W), H, W, W, R, cap, *outs(), buf(ws), ws - 1, None)),
-    ]
-    for name, want, call in cases:
-        del probes[:]
-        n0 = L.dm_launch_count()
-        assert call() == want, name
-        assert L.dm_launch_count() == n0, name
-        if cuda:
-            torch.cuda.synchronize()
-            assert all(torch.equal(t, t0) for t, t0 in probes), name
+    tracer_abi.check_no_work_before_an_argument_error("dm_lines")
 
 
 def test_boundary_lines_refuses_cpu_tensors():

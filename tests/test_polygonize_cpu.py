@@ -4,7 +4,7 @@ The sequential tracer of tests/polygon_oracle.c (dmo_polygonize) is checked on h
 what shares no code with it: the round trip through the shapefile writer / reader and rasterize_polygons, the pixel counts and the
 perimeters of oracle_np.build_rag.  deepmerge_b200/csrc/polygon_core.cuh (the kernels' per-side rule) is compiled with
 g++ and checked against the oracle's successor rule on every 2 x 2 configuration.  The ABI rejects bad arguments without
-CUDA."""
+CUDA and before it enqueues anything (the checks of tests/tracer_abi.py, which test_lines_cpu runs on dm_lines)."""
 import ctypes
 import itertools
 import os
@@ -14,6 +14,7 @@ import numpy as np
 import pytest
 
 import polygon_oracle as po
+import tracer_abi
 from oracle import oracle_np as o
 
 HERE = os.path.dirname(os.path.abspath(__file__))
@@ -247,24 +248,11 @@ def test_core_successor_rule_on_every_2x2_block(core):
 # ---- ABI without CUDA -----------------------------------------------------------------------------------------------
 
 def test_abi_rejects_bad_arguments_without_cuda():
-    from deepmerge_b200 import _lib
-    _lib.lib()
-    L = _lib.lib()
-    bad = _lib.DM_ERR_BAD_ARG
-    f = L.dm_polygonize
-    nul = [None] * 6
-    assert f(None, 4, 4, 4, 3, 64, *nul, None, 0, None) == bad                  # null pointers with work to do
-    assert f(None, -1, 4, 4, 3, 64, *nul, None, 0, None) == bad                 # negative extent
-    assert f(None, 4, -1, 4, 3, 64, *nul, None, 0, None) == bad
-    assert f(None, 4, 4, 3, 3, 64, *nul, None, 0, None) == bad                  # ld < W
-    assert f(None, 4, 4, 4, 3, 1 << 31, *nul, None, 0, None) == bad             # capacity >= 2^31
-    assert f(None, 4, 4, 4, -1, 64, *nul, None, 0, None) == bad                 # negative region count
-    assert f(None, 1 << 20, 1 << 20, 1 << 20, 3, 64, *nul, None, 0, None) == bad    # more than 2^32 vertices
-    assert f(None, 0, 4, 4, 3, 64, *nul, None, 0, None) == 0                    # empty raster
-    assert f(None, 4, 0, 0, 3, 64, *nul, None, 0, None) == 0
-    assert 0 < L.dm_polygonize_workspace_bytes(64, 64, 10, 1000) < L.dm_polygonize_workspace_bytes(64, 64, 10, 100000)
-    assert L.dm_polygonize_workspace_bytes(1024, 1024, 10, 1000) >= 1024 * 1024 // 2     # 4 bits of sides per pixel
-    assert L.dm_polygonize_workspace_bytes(64, 64, 1 << 22, 1000) > L.dm_polygonize_workspace_bytes(64, 64, 10, 1000)
+    tracer_abi.check_rejects_bad_arguments("dm_polygonize")
+
+
+def test_no_work_is_enqueued_before_an_argument_error():
+    tracer_abi.check_no_work_before_an_argument_error("dm_polygonize")
 
 
 def test_polygonize_refuses_cpu_tensors():
