@@ -8,6 +8,6 @@ from .raster import (RAG, MergeEngine, MergeResult, build_rag, compact_roots, cs
                      merge_edge_lists, merge_graph, merge_scene, points_region, pool_bands, pool_dense, pool_points,
                      pool_points_csr, region_mean, relabel, score_l2, PackedMLP, score_mlp, mlp_forward, pool_boundary, ScenePipeline,
                      score_spectral, merge_scene_spectral)
-from .polygons import Lines, Polygons, boundary_lines, polygonize  # noqa: F401
+from .polygons import Lines, Polygons, boundary_lines, polygonize, rasterize  # noqa: F401
 
 __version__ = "0.1.0"

@@ -20,7 +20,8 @@ SYNTH_LIB_PATH = os.path.join(HERE, "libdeepmerge_b200_synth.so")
 DM_OK, DM_ERR_BAD_ARG, DM_ERR_WORKSPACE, DM_ERR_CUDA, DM_ERR_UNSUPPORTED, DM_ERR_CAPACITY = 0, -1, -2, -3, -4, -5
 
 _SCALARS = {
-    "int": ctypes.c_int, "int64_t": ctypes.c_int64, "uint32_t": ctypes.c_uint32, "float": ctypes.c_float,
+    "int": ctypes.c_int, "int64_t": ctypes.c_int64, "int32_t": ctypes.c_int32, "uint32_t": ctypes.c_uint32,
+    "float": ctypes.c_float, "double": ctypes.c_double,
     "size_t": ctypes.c_size_t, "dm_stream_t": ctypes.c_void_p, "void": None,
 }
 

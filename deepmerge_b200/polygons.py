@@ -1,6 +1,7 @@
 """Label raster -> polygons (dm_polygonize) and boundary lines (dm_lines): the way back from a merged label map to one
 polygon per segment, as the reference's tile.shp holds them, and to one polyline per shared boundary, as its lines.shp
-holds them.  shapefile.write_polygonized and shapefile.write_boundary_lines write the results."""
+holds them.  shapefile.write_polygonized and shapefile.write_boundary_lines write the results.  Polygons -> label raster
+(dm_rasterize): the way in, from the polygons shapefile.read_polygons / read_polygon_rings read."""
 from __future__ import annotations
 
 from dataclasses import dataclass
@@ -10,6 +11,7 @@ import torch
 
 from ._lib import lib
 from .raster import _I32, _I64, _U8, _labels_2d, _need_cuda, _p, _stream
+from .shapefile import PolygonRings
 
 _MAX_CAPACITY = (1 << 31) - 1
 
@@ -174,3 +176,83 @@ def boundary_lines(labels: torch.Tensor, n_regions: int, *, capacity=None) -> Li
         lambda L, H, W, R, cap: L.dm_lines_workspace_bytes(H, W, cap), "boundary segments")
     k, v = int(c[0]), int(c[1])
     return Lines(left[:k], right[:k], length[:k], offsets[:k + 1], vertices[:v], int(c[2]))
+
+
+def _flat_rings(polygons, dev):
+    """(xy float64 [n, 2], ring_offsets int64 [k + 1], ring_record int32 [k], n_records) on dev from PolygonRings (used in
+    place when its arrays are already such tensors on dev) or from a list of records, each a list of [n, 2] rings."""
+    if isinstance(polygons, PolygonRings):
+        xy, off, rec, n_records = polygons
+    else:
+        rings = [np.asarray(r, np.float64).reshape(-1, 2) for rings in polygons for r in rings]
+        n_records = len(polygons)
+        xy = np.concatenate(rings) if rings else np.zeros((0, 2))
+        off = np.zeros(len(rings) + 1, np.int64)
+        np.cumsum([len(r) for r in rings], out=off[1:])
+        rec = np.repeat(np.arange(n_records, dtype=np.int32), [len(r) for r in polygons])
+    t = lambda a, dt: torch.as_tensor(a).to(device=dev, dtype=dt).contiguous()    # noqa: E731  (no copy when it fits)
+    xy, off, rec = t(xy, torch.float64), t(off, _I64), t(rec, _I32)
+    if xy.dim() != 2 or xy.shape[1] != 2 or off.dim() != 1 or rec.dim() != 1 or off.shape[0] != rec.shape[0] + 1:
+        raise ValueError("rings: xy must be [n, 2] and ring_offsets one longer than ring_record")
+    return xy, off, rec, int(n_records)
+
+
+def default_raster_capacity(n_vertices, H):
+    return int(min(max(1 << 16, 2 * n_vertices + 2 * H), _MAX_CAPACITY))
+
+
+def rasterize(polygons, geotransform, height, width, *, nodata=-1, ids=None, capacity=None, device=None) -> torch.Tensor:
+    """int32 [height, width] label raster on the GPU, bit for bit shapefile.rasterize_polygons: a pixel takes ids[fid]
+    (default: fid) of the last polygon whose even-odd fill contains its centre, and nodata where there is none.
+    `polygons` is what shapefile.read_polygons returns (one list of rings per record) or shapefile.PolygonRings, whose
+    arrays may already be CUDA tensors.  North-up geotransforms only.  A non-finite coordinate raises ValueError.
+    `capacity` bounds the row crossings of all segments; when it is too small the call is repeated once with the exact
+    count."""
+    L = lib()
+    gt = [float(v) for v in geotransform]
+    if gt[2] != 0.0 or gt[4] != 0.0 or gt[1] == 0.0 or gt[5] == 0.0:
+        raise ValueError("rasterize needs a north-up geotransform")
+    H, W, nodata = int(height), int(width), int(nodata)
+    if H < 0 or W < 0:
+        raise ValueError("negative raster size")
+    if not -(1 << 31) <= nodata < (1 << 31):
+        raise ValueError("nodata must fit int32")
+    if device is None:
+        first = getattr(polygons, "xy", None)
+        device = first.device if isinstance(first, torch.Tensor) and first.is_cuda else torch.device("cuda")
+    dev = torch.device(device)
+    if dev.type != "cuda":
+        raise ValueError("deepmerge_b200 kernels need CUDA tensors (there is no CPU path)")
+    with torch.cuda.device(dev):
+        xy, off, rec, n_records = _flat_rings(polygons, dev)
+        if ids is not None:
+            ids = torch.as_tensor(ids)
+            if ids.dtype.is_floating_point or ids.dtype.is_complex or ids.dtype == torch.bool or ids.dim() != 1:
+                raise ValueError("ids must be a 1-D integer array")
+            if ids.shape[0] < n_records:
+                raise ValueError("ids has %d entries for %d records" % (ids.shape[0], n_records))
+            if ids.numel() and (int(ids.min()) < -(1 << 31) or int(ids.max()) >= (1 << 31)):
+                raise ValueError("ids must fit int32")
+            ids = ids.to(device=dev, dtype=_I32).contiguous()
+        n_v, n_rings = xy.shape[0], rec.shape[0]
+        cap = default_raster_capacity(n_v, H) if capacity is None else int(capacity)
+        out = torch.empty((H, W), dtype=_I32, device=dev)
+        for attempt in range(2):
+            counts = torch.zeros(4, dtype=_I64, device=dev)
+            ws_bytes = L.dm_rasterize_workspace_bytes(n_v, n_records, cap)
+            ws = torch.empty(max(ws_bytes, 1), dtype=_U8, device=dev)
+            L.check(L.dm_rasterize(_p(xy), n_v, _p(off), _p(rec), n_rings, n_records, gt[0], gt[1], gt[3], gt[5], _p(ids),
+                                   nodata, H, W, W, cap, _p(out), _p(counts), _p(ws), ws_bytes, _stream()), "dm_rasterize")
+            c = counts.tolist()
+            if c[3] == 1:
+                raise ValueError("rasterize: a coordinate is not finite, or a crossing overflows float64")
+            if c[3] == 4:
+                raise ValueError("rasterize: a ring offset or ring record is out of range")
+            if c[3] == 2 and attempt == 0:
+                if c[2] > _MAX_CAPACITY:
+                    raise ValueError("the polygons cross %d rows, more than 2^31 - 1" % c[2])
+                cap = int(c[2])
+                continue
+            if c[3] != 0:
+                raise RuntimeError("dm_rasterize: status %d" % c[3])
+            return out

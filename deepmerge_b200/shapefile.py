@@ -23,6 +23,7 @@ the .dbf attribute table (dBase III, fixed-width ASCII records) and, for the poi
   write_dbf / write_point_shp   writers (tests, and exporting a raster-derived RAG for GIS tools)
   read_polygons / read_polylines, write_polygonized / write_boundary_lines   polygon and line geometry: the
                   reference's tile.shp and lines.shp, read back or made from a label raster
+  read_polygon_rings   the polygons of a file as flat arrays (PolygonRings), what deepmerge_b200.rasterize takes
 
 Conventions follow the OGR "ESRI Shapefile" driver: FID = record index, trailing blanks of strings
 are stripped, N fields without decimals are integers, blank / '*' filled numbers are null (None),
@@ -33,6 +34,7 @@ from __future__ import annotations
 import datetime
 import os
 import struct
+from typing import NamedTuple
 
 import numpy as np
 
@@ -515,24 +517,98 @@ def Open(path, update=0):
 _POLY_TYPES = (5, 15, 25)           # Polygon, PolygonZ, PolygonM
 
 
-def _read_multipart(path, types, kind):
+class PolygonRings(NamedTuple):
+    """Every ring of a polygon file in one flat form: ring k has the vertices xy[ring_offsets[k]:ring_offsets[k + 1]]
+    and belongs to record ring_record[k]; records are numbered in FID order, and a null record has no ring but counts in
+    n_records.  deepmerge_b200.rasterize takes it as it is (numpy arrays or tensors)."""
+    xy: np.ndarray              # float64 [n_vertices, 2] of (X, Y)
+    ring_offsets: np.ndarray    # int64 [n_rings + 1]
+    ring_record: np.ndarray     # int32 [n_rings]
+    n_records: int
+
+
+def _take(raw, dtype, pos):
+    """The little-endian values of `dtype` at the byte offsets `pos` of raw (any alignment)."""
+    dt = np.dtype(dtype)
+    out = np.empty(len(pos), dt)
+    align = pos % dt.itemsize
+    for a in np.flatnonzero(np.bincount(align, minlength=dt.itemsize)).tolist():
+        words = np.frombuffer(raw, dt, (len(raw) - a) // dt.itemsize, a)
+        m = align == a
+        out[m] = words[(pos[m] - a) // dt.itemsize]
+    return out
+
+
+def _record_offsets(path, raw):
+    """Byte offsets of the record headers in the .shp bytes `raw`: from the .shx index when there is one, else by walking
+    the record headers."""
+    shx = (path[:-4] if path.lower().endswith(".shp") else path) + ".shx"
+    try:
+        with open(shx, "rb") as f:
+            idx = f.read()
+    except OSError:
+        idx = None
+    if idx is not None and len(idx) >= 100 and struct.unpack_from(">i", idx, 0)[0] == 9994:
+        return 2 * np.frombuffer(idx, ">i4", (len(idx) - 100) // 8 * 2, 100)[0::2].astype(np.int64)
+    offs = []
+    off, end = 100, len(raw)
+    while off + 8 <= end:
+        offs.append(off)
+        off += 8 + 2 * max(0, struct.unpack_from(">i", raw, off + 4)[0])
+    return np.asarray(offs, np.int64)
+
+
+def _read_flat(path, types, kind):
+    """-> (xy, part offsets, part record, n_records) of a multi-part file of `types`; records of another shape type,
+    null shapes, records without parts and records cut off by the end of the file have no parts."""
     raw, st = _shp_header(path)
     if st not in types:
         raise ValueError("{0} is not a {1} shapefile (shape type {2})".format(path, kind, st))
-    out = []
-    off, end = 100, len(raw)
-    while off + 8 <= end:
-        (clen,) = struct.unpack_from(">i", raw, off + 4)
-        body = off + 8
-        parts_xy = []
-        if body + 44 <= end and struct.unpack_from("<i", raw, body)[0] in types:
-            n_parts, n_points = struct.unpack_from("<ii", raw, body + 36)
-            parts = list(struct.unpack_from("<%di" % n_parts, raw, body + 44)) + [n_points]
-            pts = np.frombuffer(raw, "<f8", 2 * n_points, body + 44 + 4 * n_parts).reshape(n_points, 2)
-            parts_xy = [pts[parts[i]:parts[i + 1]].copy() for i in range(n_parts)]
-        out.append(parts_xy)
-        off = body + 2 * clen
+    body = _record_offsets(path, raw) + 8
+    n_records = len(body)
+    ok = body + 44 <= len(raw)
+    ok[ok] = np.isin(_take(raw, "<i4", body[ok]), types)
+    ok[ok] = _take(raw, "<i4", body[ok] + 36) > 0
+    rec = np.flatnonzero(ok)
+    body = body[ok]
+    n_parts = _take(raw, "<i4", body + 36).astype(np.int64)
+    n_points = _take(raw, "<i4", body + 40).astype(np.int64)
+    pts_at = body + 44 + 4 * n_parts                                        # byte offset of each record's points
+    if (n_points < 0).any() or (pts_at + 16 * n_points > len(raw)).any():
+        raise ValueError("{0}: corrupt or truncated record".format(path))
+    part_rec = np.repeat(np.arange(len(body)), n_parts)
+    part_first = np.concatenate([[0], np.cumsum(n_parts)])[:-1].astype(np.int64)
+    j = np.arange(len(part_rec)) - np.repeat(part_first, n_parts)
+    start = _take(raw, "<i4", body[part_rec] + 44 + 4 * j).astype(np.int64)
+    # the parts of a record split its points: the first starts at 0, none goes back or past the end
+    step = np.diff(np.append(start, 0))
+    step[part_first + n_parts - 1] = n_points - start[part_first + n_parts - 1]
+    if (start[part_first] != 0).any() or (step < 0).any():
+        raise ValueError("{0}: corrupt or truncated record".format(path))
+    v_first = np.concatenate([[0], np.cumsum(n_points)]).astype(np.int64)  # first vertex of each record
+    mv = memoryview(raw)                                                    # one copy of every record's point block
+    xy = np.frombuffer(bytearray().join([mv[p:p + 16 * n] for p, n in zip(pts_at.tolist(), n_points.tolist())]),
+                       "<f8").reshape(-1, 2)
+    offsets = np.append(v_first[part_rec] + start, v_first[-1])
+    return xy, offsets, rec[part_rec].astype(np.int32), n_records
+
+
+def _read_multipart(path, types, kind):
+    xy, off, rec, n = _read_flat(path, types, kind)
+    parts = np.split(xy, off[1:-1]) if len(rec) else []
+    out = [[] for _ in range(n)]
+    for r, p in zip(rec.tolist(), parts):
+        out[r].append(p)
     return out
+
+
+def read_polygon_rings(path) -> PolygonRings:
+    """-> PolygonRings of a Polygon / PolygonZ / PolygonM file (X and Y only): the flat form of read_polygons, with no
+    Python work per ring or vertex (the points are copied in one join of a slice per record).  The record offsets come
+    from the .shx index, or from walking the record headers of the .shp when it has none.  A record whose parts do not
+    split its points (the first part starting at 0, none going back) or that runs past the end of the file raises
+    ValueError."""
+    return PolygonRings(*_read_flat(path, _POLY_TYPES, "polygon"))
 
 
 def read_polygons(path):

@@ -512,6 +512,40 @@ int dm_lines(const int32_t* labels, int64_t H, int64_t W, int64_t ld, int64_t n_
              int64_t* counts, void* ws, size_t ws_bytes, dm_stream_t stream);
 
 /* ----------------------------------------------------------------------------------- *
+ * Rasterize polygons: the way in of the vector round trip, from the segment polygons of the reference's tile.shp to the
+ * label raster the merge starts from.  The contract of shapefile.rasterize_polygons, bit for bit.  Not part of the merge
+ * step.
+ *
+ * Input (device): vertices xy float64 [n_vertices, 2] of (X, Y) in map coordinates; ring k has the vertices
+ * [ring_offsets[k], ring_offsets[k + 1]) (int64 [n_rings + 1], non-decreasing, within [0, n_vertices]) and belongs to
+ * record ring_record[k] (int32 [n_rings], in [0, n_records)).  Records are the polygons, in FID order.
+ *  - Pixel coordinates: px = (X - gt0) / gt1, py = (Y - gt3) / gt5, fp64, subtract then divide; north-up transforms only
+ *    (the caller rejects rotated ones), gt1 != 0, gt5 != 0, either may be negative.
+ *  - Rings: a ring of fewer than 3 vertices is skipped.  A ring whose first and last pixel coordinates differ is closed
+ *    by a segment from its last vertex back to its first; an explicitly closed ring gets none.
+ *  - Crossings: segment (x0, y0) -> (x1, y1) crosses row r (0 <= r < H, yc = r + 0.5) iff (y0 <= yc) != (y1 <= yc),
+ *    at xi = x0 + ((yc - y0) (x1 - x0)) / (y1 - y0), each operation rounded once (no fused multiply-add), in column
+ *    clip(ceil(xi - 0.5), 0, W).
+ *  - Fill: the crossings of one (record, row) sorted by column, paired (1st, 2nd), (3rd, 4th), ..., fill the columns
+ *    [c_a, c_b): the even-odd rule over all rings of the record, so holes stay empty and self-intersections alternate.
+ *  - Value: a pixel gets ids[fid] of the largest record index fid whose fill covers it (ids null: fid itself), a pixel
+ *    that none covers gets nodata.  labels int32 [H, ld] (ld >= W), row-pitched; the columns in [W, ld) are not written.
+ * counts int64 [4]: [0] spans painted, [1] pixels painted (the sum of the span lengths, overlaps counted again),
+ *   [2] crossings found (exact, also above capacity), [3] status: 0 ok, 1 a non-finite pixel coordinate in a ring of 3 or
+ *   more vertices, or a crossing x that overflows fp64, 2 capacity exceeded (retry with capacity >= counts[2]), 3 internal
+ *   pairing error, 4 a ring offset or ring record out of range.  labels are valid only with status 0.
+ * capacity bounds the crossings, < 2^31; n_vertices, n_rings, n_records < 2^31; (H + 1) (W + 1) <= 2^32.  The workspace
+ * grows with 8 bytes per vertex and the capacity (keys and their sort by record, whose per-record arrays grow with
+ * n_records).  No H W workspace.  The empty raster writes zero counts (when given) and returns 0; no rings or no vertices
+ * fill labels with nodata.
+ * ----------------------------------------------------------------------------------- */
+size_t dm_rasterize_workspace_bytes(int64_t n_vertices, int64_t n_records, int64_t capacity);
+int dm_rasterize(const double* xy, int64_t n_vertices, const int64_t* ring_offsets, const int32_t* ring_record,
+                 int64_t n_rings, int64_t n_records, double gt0, double gt1, double gt3, double gt5, const int32_t* ids,
+                 int32_t nodata, int64_t H, int64_t W, int64_t ld, int64_t capacity, int32_t* labels, int64_t* counts,
+                 void* ws, size_t ws_bytes, dm_stream_t stream);
+
+/* ----------------------------------------------------------------------------------- *
  * R11 Contrastive pair loss forward + backward (Losses.py:34-38):
  *     d = sum_k (a-b)^2 ; L = mean(flag*d + (1-flag)*relu(margin-d)).
  *     loss fp32 [1]; grad_a, grad_b fp32 [B,D] (nullable).  flag int64 as collated.
