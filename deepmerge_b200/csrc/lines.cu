@@ -16,9 +16,13 @@
 // 6. sort_pairs     lines by (start vertex, first direction) (radix); info_kernel: per line its values, vertex count
 //                   and the line of its end segment; scan -> vertex offsets.
 // 7. vertex_kernel  start vertices and emitted head vertices scattered to line offset + rank, lengths counted.
+// dm_lines_simplified writes the vertices of step 7 to its workspace and simplifies them (simplify.cuh) into the output.
+#include <cmath>
+
 #include "chain.cuh"
 #include "lines_core.cuh"
 #include "prims.cuh"
+#include "simplify.cuh"
 
 namespace dm {
 namespace lines {
@@ -37,8 +41,7 @@ struct Ws : Front {
     void* sort;
 };
 
-size_t carve(Ws& w, void* base, int64_t H, int64_t W, int64_t cap) {
-    Carver c(base);
+void take(Ws& w, Carver& c, int64_t H, int64_t W, int64_t cap) {
     carve_front(w, c, H, W, cap, cap);
     w.line_of = c.take<uint32_t>((size_t)cap);
     w.lkeys = c.take<uint64_t>((size_t)cap);
@@ -46,6 +49,19 @@ size_t carve(Ws& w, void* base, int64_t H, int64_t W, int64_t cap) {
     w.vcount = c.take<uint32_t>((size_t)cap);
     w.offs = c.take<uint32_t>((size_t)cap);
     w.sort = c.take<char>(prims::ws_bytes(cap, false));
+}
+
+size_t carve(Ws& w, void* base, int64_t H, int64_t W, int64_t cap) {
+    Carver c(base);
+    take(w, c, H, W, cap);
+    return c.used();
+}
+
+// dm_lines_simplified: the tracer's workspace, then the simplifier's with the unsimplified lines (2 cap vertices).
+size_t carve_simplified(Ws& w, simplify::Ws& sw, void* base, int64_t H, int64_t W, int64_t cap) {
+    Carver c(base);
+    take(w, c, H, W, cap);
+    simplify::carve(sw, c, 2 * cap, cap, false);
     return c.used();
 }
 
@@ -173,6 +189,26 @@ extern "C" size_t dm_lines_workspace_bytes(int64_t H, int64_t W, int64_t capacit
     return lines::carve(w, nullptr, H, W, capacity);
 }
 
+namespace dm {
+namespace lines {
+
+// The back half of both entry points after the trace: the lines' sort, info and vertices.
+int finish(const int32_t* labels, int64_t H, int64_t W, int64_t ld, int64_t capacity, int32_t* line_left,
+           int32_t* line_right, int64_t* line_length, int64_t* line_offsets, int32_t* vertices, int64_t* counts,
+           Ws& w, cudaStream_t s) {
+    const unsigned g_lines = grid_for(capacity + 1, chain::NT, 16);
+    // lines by start vertex (high half), then by the direction of their first segment (low half)
+    const int vb = bits_for((H + 1) * (W + 1));
+    DM_TRY(prims::sort_pairs(w.lkeys, w.lvals, counts, capacity, vb, 2 * vb, w.sort, s));
+    DM_TRY(launch(lines::info_kernel, g_lines, chain::NT, 0, s, labels, H, W, ld, counts, line_left, line_right,
+                  line_length, w));
+    DM_TRY(prims::scan_exclusive_u32(w.vcount, w.offs, counts, capacity, counts + 1, w.scan, s));
+    return launch(lines::vertex_kernel, g_lines, chain::NT, 0, s, counts, W, w, vertices, line_offsets, line_length);
+}
+
+}  // namespace lines
+}  // namespace dm
+
 extern "C" int dm_lines(const int32_t* labels, int64_t H, int64_t W, int64_t ld, int64_t n_regions, int64_t capacity,
                         int32_t* line_left, int32_t* line_right, int64_t* line_length, int64_t* line_offsets,
                         int32_t* vertices, int64_t* counts, void* ws, size_t ws_bytes, dm_stream_t stream) {
@@ -186,12 +222,36 @@ extern "C" int dm_lines(const int32_t* labels, int64_t H, int64_t W, int64_t ld,
     lines::Ws w;
     lines::carve(w, ws, H, W, capacity);
     DM_TRY(chain::trace<lines::SegmentRule>(labels, H, W, ld, n_regions, capacity, counts, w, s));
-    const unsigned g_lines = grid_for(capacity + 1, chain::NT, 16);
-    // lines by start vertex (high half), then by the direction of their first segment (low half)
-    const int vb = bits_for((H + 1) * (W + 1));
-    DM_TRY(prims::sort_pairs(w.lkeys, w.lvals, counts, capacity, vb, 2 * vb, w.sort, s));
-    DM_TRY(launch(lines::info_kernel, g_lines, chain::NT, 0, s, labels, H, W, ld, counts, line_left, line_right,
-                  line_length, w));
-    DM_TRY(prims::scan_exclusive_u32(w.vcount, w.offs, counts, capacity, counts + 1, w.scan, s));
-    return launch(lines::vertex_kernel, g_lines, chain::NT, 0, s, counts, W, w, vertices, line_offsets, line_length);
+    return lines::finish(labels, H, W, ld, capacity, line_left, line_right, line_length, line_offsets, vertices, counts,
+                         w, s);
+}
+
+extern "C" size_t dm_lines_simplified_workspace_bytes(int64_t H, int64_t W, int64_t capacity) {
+    if (!chain::extent_ok(H, W, capacity) || !simplify::extent_ok(H, W)) return 0;
+    lines::Ws w;
+    simplify::Ws sw;
+    return lines::carve_simplified(w, sw, nullptr, H, W, capacity);
+}
+
+extern "C" int dm_lines_simplified(const int32_t* labels, int64_t H, int64_t W, int64_t ld, int64_t n_regions,
+                                   int64_t capacity, double tolerance, int32_t* line_left, int32_t* line_right,
+                                   int64_t* line_length, int64_t* line_offsets, int32_t* vertices, int64_t* counts,
+                                   void* ws, size_t ws_bytes, dm_stream_t stream) {
+    if (!chain::args_ok(H, W, ld, n_regions, capacity) || !simplify::extent_ok(H, W) || !std::isfinite(tolerance) ||
+        tolerance < 0)
+        return DM_ERR_BAD_ARG;
+    cudaStream_t s = S(stream);
+    if (H == 0 || W == 0) return chain::clear_empty(counts, line_offsets, s);
+    if (!labels || !line_offsets || !counts || !ws ||
+        (capacity > 0 && (!line_left || !line_right || !line_length || !vertices)))
+        return DM_ERR_BAD_ARG;
+    if (ws_bytes < dm_lines_simplified_workspace_bytes(H, W, capacity)) return DM_ERR_WORKSPACE;
+    lines::Ws w;
+    simplify::Ws sw;
+    lines::carve_simplified(w, sw, ws, H, W, capacity);
+    DM_TRY(chain::trace<lines::SegmentRule>(labels, H, W, ld, n_regions, capacity, counts, w, s));
+    DM_TRY(lines::finish(labels, H, W, ld, capacity, line_left, line_right, line_length, sw.in.off, sw.in.v, counts, w,
+                         s));
+    return simplify::run(counts, H, W, simpcore::quantize_tolerance(tolerance, H, W), 2 * capacity, capacity, sw,
+                         vertices, line_offsets, s);
 }

@@ -13,16 +13,24 @@
 // 5. starts_kernel  one ring per start side, listed with its start vertex; sort_pairs orders the list by start vertex
 //                   (radix), then stably by region (bucket + rank), whose CSR offsets are region_rings.
 // 6. vertex_kernel  corners scattered to ring offset + rank, ring areas as the sum of x * dy over the vertical sides.
+// dm_polygonize_simplified traces with NodeSideRule, which also emits (and flags) the head vertices that are nodes in
+// the sense of dm_lines, writes the rings of step 6 to its workspace and simplifies them (simplify.cuh) into the output.
+#include <cmath>
+#include <type_traits>
+
 #include "chain.cuh"
+#include "lines_core.cuh"
 #include "polygon_core.cuh"
 #include "prims.cuh"
+#include "simplify.cuh"
 
 namespace dm {
 namespace poly {
 using namespace polycore;
 using namespace chain;
 
-constexpr uint8_t CORNER = 4;   // flags: bits 0-1 side / direction, bit 2 head vertex is a corner
+constexpr uint8_t CORNER = 4;   // flags: bits 0-1 side / direction, bit 2 head vertex is a vertex of the ring
+constexpr uint8_t NODE = 8;     // NodeSideRule: the head vertex is a node
 
 struct Ws : Front {
     uint32_t* ring_of;                  // per side: ring of a start side
@@ -32,8 +40,7 @@ struct Ws : Front {
     void* sort;
 };
 
-size_t carve(Ws& w, void* base, int64_t H, int64_t W, int64_t n_regions, int64_t cap) {
-    Carver c(base);
+void take(Ws& w, Carver& c, int64_t H, int64_t W, int64_t n_regions, int64_t cap) {
     const int64_t ring_cap = cap / 4;
     carve_front(w, c, H, W, cap, ring_cap);
     w.ring_of = c.take<uint32_t>((size_t)cap);
@@ -43,6 +50,19 @@ size_t carve(Ws& w, void* base, int64_t H, int64_t W, int64_t n_regions, int64_t
     w.ccount = c.take<uint32_t>((size_t)ring_cap);
     w.offs = c.take<uint32_t>((size_t)ring_cap);
     w.sort = c.take<char>(prims::ws_bytes(ring_cap, false, n_regions + 1));
+}
+
+size_t carve(Ws& w, void* base, int64_t H, int64_t W, int64_t n_regions, int64_t cap) {
+    Carver c(base);
+    take(w, c, H, W, n_regions, cap);
+    return c.used();
+}
+
+// dm_polygonize_simplified: the tracer's workspace, then the simplifier's with the unsimplified rings (cap vertices).
+size_t carve_simplified(Ws& w, simplify::Ws& sw, void* base, int64_t H, int64_t W, int64_t n_regions, int64_t cap) {
+    Carver c(base);
+    take(w, c, H, W, n_regions, cap);
+    simplify::carve(sw, c, cap, cap / 4, true);
     return c.used();
 }
 
@@ -84,6 +104,16 @@ struct SideRule {
     }
 };
 
+// SideRule with every head vertex that is a node (linecore::node_arms) made a ring vertex and flagged NODE.
+struct NodeSideRule : SideRule {
+    static __device__ __forceinline__ void emit(const int32_t* L, int64_t H, int64_t W, int64_t ld, int64_t wpr,
+                                                const uint32_t* masks, const uint32_t* wbase, int64_t x, int64_t y,
+                                                int s, uint32_t i, const Ws& ws) {
+        SideRule::emit(L, H, W, ld, wpr, masks, wbase, x, y, s, i, ws);
+        if (linecore::node_arms(linecore::arms(L, H, W, ld, head_x(x, s), head_y(y, s)))) ws.flags[i] |= CORNER | NODE;
+    }
+};
+
 __global__ void __launch_bounds__(NT) region_keys_kernel(const int64_t* __restrict__ counts, Ws ws) {
     const int64_t n = counts[0];
     for (int64_t r = (int64_t)blockIdx.x * NT + threadIdx.x; r < n; r += (int64_t)gridDim.x * NT)
@@ -102,9 +132,11 @@ __global__ void __launch_bounds__(NT) ring_info_kernel(const int64_t* __restrict
     }
 }
 
+// node (NodeSideRule only): per vertex, whether it is a node
+template <bool Nodes>
 __global__ void __launch_bounds__(NT) vertex_kernel(const int64_t* __restrict__ counts, int64_t W, Ws ws,
                                                     int32_t* __restrict__ vertices, int64_t* __restrict__ ring_offsets,
-                                                    int64_t* __restrict__ ring_area) {
+                                                    int64_t* __restrict__ ring_area, uint8_t* __restrict__ node) {
     const int64_t n_rings = counts[0];
     const int64_t gtid = (int64_t)blockIdx.x * NT + threadIdx.x, gstride = (int64_t)gridDim.x * NT;
     for (int64_t r = gtid; r <= n_rings; r += gstride) ring_offsets[r] = r < n_rings ? (int64_t)ws.offs[r] : counts[1];
@@ -121,11 +153,34 @@ __global__ void __launch_bounds__(NT) vertex_kernel(const int64_t* __restrict__ 
             const int64_t pos = (int64_t)ws.offs[r] + rank;
             vertices[2 * pos] = (int32_t)hx;
             vertices[2 * pos + 1] = (int32_t)hy;
+            if (Nodes) node[pos] = (f & NODE) ? 1 : 0;
         }
         // shoelace area = sum of x dy: south sides (direction 1) add x, north sides (3) subtract it
         if ((f & 3) == 1) atomicAdd((unsigned long long*)(ring_area + r), (unsigned long long)hx);
         else if ((f & 3) == 3) atomicAdd((unsigned long long*)(ring_area + r), (unsigned long long)(-hx));
     }
+}
+
+// The whole tracer on workspace w, with rule SideRule or NodeSideRule; node receives NodeSideRule's node flags.
+template <class Rule>
+int polygonize(const int32_t* labels, int64_t H, int64_t W, int64_t ld, int64_t n_regions, int64_t capacity,
+               int32_t* ring_region, int64_t* ring_offsets, int64_t* ring_area, int32_t* vertices,
+               int64_t* region_rings, int64_t* counts, uint8_t* node, Ws& w, cudaStream_t s) {
+    const int64_t ring_cap = capacity / 4;
+    if (ring_cap) DM_CUDA(cudaMemsetAsync(ring_area, 0, (size_t)ring_cap * sizeof(int64_t), s));
+    DM_TRY(chain::trace<Rule>(labels, H, W, ld, n_regions, capacity, counts, w, s));
+    const unsigned g_sides = grid_for(capacity, poly::NT, 16), g_rings = grid_for(ring_cap + 1, poly::NT, 16);
+    // rings in raster order of their start vertex, then stably by region
+    DM_TRY(prims::sort_pairs(w.rkeys, w.rvals, counts, ring_cap, bits_for((H + 1) * (W + 1)), bits_for((H + 1) * (W + 1)),
+                             w.sort, s));
+    DM_TRY(launch(poly::region_keys_kernel, g_rings, poly::NT, 0, s, counts, w));
+    const int rb = bits_for(n_regions + 1);
+    DM_TRY(prims::sort_pairs(w.rkeys, w.rvals, counts, ring_cap, rb, rb, w.sort, s, n_regions + 1, region_rings, nullptr));
+    if (ring_cap == 0) DM_CUDA(cudaMemsetAsync(region_rings, 0, (size_t)(n_regions + 1) * sizeof(int64_t), s));
+    DM_TRY(launch(poly::ring_info_kernel, g_rings, poly::NT, 0, s, counts, ring_region, w));
+    DM_TRY(prims::scan_exclusive_u32(w.ccount, w.offs, counts, ring_cap, counts + 1, w.scan, s));
+    return launch(vertex_kernel<std::is_same<Rule, NodeSideRule>::value>, imax64(g_sides, g_rings), NT, 0, s, counts, W,
+                  w, vertices, ring_offsets, ring_area, node);
 }
 
 }  // namespace poly
@@ -155,19 +210,39 @@ extern "C" int dm_polygonize(const int32_t* labels, int64_t H, int64_t W, int64_
     if (ws_bytes < dm_polygonize_workspace_bytes(H, W, n_regions, capacity)) return DM_ERR_WORKSPACE;
     poly::Ws w;
     poly::carve(w, ws, H, W, n_regions, capacity);
-    const int64_t ring_cap = capacity / 4;
-    if (ring_cap) DM_CUDA(cudaMemsetAsync(ring_area, 0, (size_t)ring_cap * sizeof(int64_t), s));
-    DM_TRY(chain::trace<poly::SideRule>(labels, H, W, ld, n_regions, capacity, counts, w, s));
-    const unsigned g_sides = grid_for(capacity, poly::NT, 16), g_rings = grid_for(ring_cap + 1, poly::NT, 16);
-    // rings in raster order of their start vertex, then stably by region
-    DM_TRY(prims::sort_pairs(w.rkeys, w.rvals, counts, ring_cap, bits_for((H + 1) * (W + 1)), bits_for((H + 1) * (W + 1)),
-                             w.sort, s));
-    DM_TRY(launch(poly::region_keys_kernel, g_rings, poly::NT, 0, s, counts, w));
-    const int rb = bits_for(n_regions + 1);
-    DM_TRY(prims::sort_pairs(w.rkeys, w.rvals, counts, ring_cap, rb, rb, w.sort, s, n_regions + 1, region_rings, nullptr));
-    if (ring_cap == 0) DM_CUDA(cudaMemsetAsync(region_rings, 0, (size_t)(n_regions + 1) * sizeof(int64_t), s));
-    DM_TRY(launch(poly::ring_info_kernel, g_rings, poly::NT, 0, s, counts, ring_region, w));
-    DM_TRY(prims::scan_exclusive_u32(w.ccount, w.offs, counts, ring_cap, counts + 1, w.scan, s));
-    return launch(poly::vertex_kernel, imax64(g_sides, g_rings), poly::NT, 0, s, counts, W, w, vertices, ring_offsets,
-        ring_area);
+    return poly::polygonize<poly::SideRule>(labels, H, W, ld, n_regions, capacity, ring_region, ring_offsets, ring_area,
+                                            vertices, region_rings, counts, nullptr, w, s);
+}
+
+extern "C" size_t dm_polygonize_simplified_workspace_bytes(int64_t H, int64_t W, int64_t n_regions, int64_t capacity) {
+    if (!chain::extent_ok(H, W, capacity) || !simplify::extent_ok(H, W) || n_regions < 0) return 0;
+    poly::Ws w;
+    simplify::Ws sw;
+    return poly::carve_simplified(w, sw, nullptr, H, W, n_regions, capacity);
+}
+
+extern "C" int dm_polygonize_simplified(const int32_t* labels, int64_t H, int64_t W, int64_t ld, int64_t n_regions,
+                                        int64_t capacity, double tolerance, int32_t* ring_region, int64_t* ring_offsets,
+                                        int64_t* ring_area, int32_t* vertices, int64_t* region_rings, int64_t* counts,
+                                        void* ws, size_t ws_bytes, dm_stream_t stream) {
+    if (!chain::args_ok(H, W, ld, n_regions, capacity) || !simplify::extent_ok(H, W) || !std::isfinite(tolerance) ||
+        tolerance < 0)
+        return DM_ERR_BAD_ARG;
+    cudaStream_t s = S(stream);
+    if (H == 0 || W == 0) {
+        DM_TRY(chain::clear_empty(counts, ring_offsets, s));
+        if (region_rings) DM_CUDA(cudaMemsetAsync(region_rings, 0, (size_t)(n_regions + 1) * sizeof(int64_t), s));
+        return DM_OK;
+    }
+    if (!labels || !ring_offsets || !region_rings || !counts || !ws || (capacity > 0 && !vertices) ||
+        (capacity >= 4 && (!ring_region || !ring_area)))
+        return DM_ERR_BAD_ARG;
+    if (ws_bytes < dm_polygonize_simplified_workspace_bytes(H, W, n_regions, capacity)) return DM_ERR_WORKSPACE;
+    poly::Ws w;
+    simplify::Ws sw;
+    poly::carve_simplified(w, sw, ws, H, W, n_regions, capacity);
+    DM_TRY(poly::polygonize<poly::NodeSideRule>(labels, H, W, ld, n_regions, capacity, ring_region, sw.in.off,
+                                                ring_area, sw.in.v, region_rings, counts, sw.in.node, w, s));
+    return simplify::run(counts, H, W, simpcore::quantize_tolerance(tolerance, H, W), capacity, capacity / 4, sw,
+                         vertices, ring_offsets, s);
 }

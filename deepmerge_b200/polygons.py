@@ -4,6 +4,7 @@ holds them.  shapefile.write_polygonized and shapefile.write_boundary_lines writ
 (dm_rasterize): the way in, from the polygons shapefile.read_polygons / read_polygon_rings read."""
 from __future__ import annotations
 
+import math
 from dataclasses import dataclass
 
 import numpy as np
@@ -16,9 +17,20 @@ from .shapefile import PolygonRings
 _MAX_CAPACITY = (1 << 31) - 1
 
 
-def _trace(labels, n_regions, capacity, default_capacity, outputs, entry, workspace_bytes, elements):
+def _tolerance(tolerance):
+    """() for the unsimplified tracer, else (tolerance,): the extra argument of its _simplified entry point."""
+    if tolerance is None:
+        return ()
+    t = float(tolerance)
+    if not math.isfinite(t) or t < 0:
+        raise ValueError("tolerance must be finite and >= 0, got %r" % (tolerance,))
+    return (t,)
+
+
+def _trace(labels, n_regions, capacity, default_capacity, outputs, entry, workspace_bytes, elements, extra=()):
     """Runs the library's tracer `entry` (dm_polygonize or dm_lines, whose arguments are labels, H, W, ld, n_regions,
-    capacity, the output buffers, counts, workspace, stream) -> (counts as a list, the output buffers).
+    capacity, the output buffers, counts, workspace, stream; their _simplified forms take `extra`, the tolerance, after
+    capacity) -> (counts as a list, the output buffers).
     outputs(cap, device) allocates the buffers for a capacity of cap boundary elements (`elements` names them);
     workspace_bytes(lib, H, W, n_regions, cap) is the tracer's workspace query.  When the capacity is too small the call
     is repeated once with the exact count."""
@@ -36,8 +48,8 @@ def _trace(labels, n_regions, capacity, default_capacity, outputs, entry, worksp
             counts = torch.zeros(4, dtype=_I64, device=dev)
             ws_bytes = workspace_bytes(L, H, W, n_regions, cap)
             ws = torch.empty(max(ws_bytes, 1), dtype=_U8, device=dev)
-            L.check(getattr(L, entry)(_p(labels), H, W, ld, n_regions, cap, *[_p(t) for t in outs], _p(counts), _p(ws),
-                                      ws_bytes, _stream()), entry)
+            L.check(getattr(L, entry)(_p(labels), H, W, ld, n_regions, cap, *extra, *[_p(t) for t in outs], _p(counts),
+                                      _p(ws), ws_bytes, _stream()), entry)
             c = counts.tolist()
             if c[3] == 1:
                 raise ValueError("labels contain ids >= n_regions")
@@ -110,10 +122,18 @@ def default_capacity(n_regions, H, W):
     return int(min(4 * H * W, max(1 << 16, 8 * (H + W) + 256 * n_regions), _MAX_CAPACITY))
 
 
-def polygonize(labels: torch.Tensor, n_regions: int, *, capacity=None) -> Polygons:
+def polygonize(labels: torch.Tensor, n_regions: int, *, tolerance=None, capacity=None) -> Polygons:
     """Rings of every region of an int32 label raster [H, W] on the GPU (strided row views accepted); negative labels
     are nodata.  Regions are 4-connected; see Polygons for the layout.  `capacity` bounds the boundary sides; when it
-    is too small the call is repeated once with the exact count."""
+    is too small the call is repeated once with the exact count.
+
+    tolerance (pixels, finite, >= 0): Douglas-Peucker simplification (dm_polygonize_simplified in
+    include/deepmerge_b200.h) that keeps every shared boundary identical on both of its sides and the same as
+    boundary_lines(..., tolerance=) gives it: nodes, the image border and the start of a ring without nodes are kept,
+    and no ring drops below 3 vertices.  Vertices stay pixel corners; a ring may then hold a vertex where it does not
+    turn (a node).  ring_area stays the pixel count.  For a tolerance in map units: tolerance = metres / |gt1|.
+    W and H must be below 2^26.  None: corners only, as without simplification."""
+    extra = _tolerance(tolerance)
     def outputs(cap, dev):
         ring_cap = cap // 4
         return (torch.empty(max(ring_cap, 1), dtype=_I32, device=dev),       # ring_region
@@ -122,9 +142,10 @@ def polygonize(labels: torch.Tensor, n_regions: int, *, capacity=None) -> Polygo
                 torch.empty((max(cap, 1), 2), dtype=_I32, device=dev),       # vertices
                 torch.empty(int(n_regions) + 1, dtype=_I64, device=dev))     # region_rings
 
+    entry = "dm_polygonize_simplified" if extra else "dm_polygonize"
     c, (ring_region, ring_offsets, ring_area, vertices, region_rings) = _trace(
-        labels, n_regions, capacity, default_capacity, outputs, "dm_polygonize",
-        lambda L, H, W, R, cap: L.dm_polygonize_workspace_bytes(H, W, R, cap), "boundary sides")
+        labels, n_regions, capacity, default_capacity, outputs, entry,
+        lambda L, H, W, R, cap: getattr(L, entry + "_workspace_bytes")(H, W, R, cap), "boundary sides", extra)
     k, v = int(c[0]), int(c[1])
     return Polygons(ring_region[:k], ring_offsets[:k + 1], ring_area[:k], vertices[:v], region_rings, int(c[2]))
 
@@ -159,11 +180,17 @@ def default_line_capacity(n_regions, H, W):
     return int(min(2 * H * W + H + W, max(1 << 16, 4 * (H + W) + 128 * n_regions), _MAX_CAPACITY))
 
 
-def boundary_lines(labels: torch.Tensor, n_regions: int, *, capacity=None) -> Lines:
+def boundary_lines(labels: torch.Tensor, n_regions: int, *, tolerance=None, capacity=None) -> Lines:
     """Boundary lines of an int32 label raster [H, W] on the GPU (strided row views accepted); negative labels are
     nodata: one polyline per maximal chain of pixel sides between two values, ending where three or more boundaries
     meet; see Lines for the layout.  `capacity` bounds the boundary segments; when it is too small the call is repeated
-    once with the exact count."""
+    once with the exact count.
+
+    tolerance (pixels, finite, >= 0): Douglas-Peucker simplification (dm_lines_simplified in include/deepmerge_b200.h),
+    the same on every line as polygonize(..., tolerance=) applies to the rings on both of its sides.  A line keeps its
+    ends and its vertices on the image border; line_length stays the number of unit segments.  For a tolerance in map
+    units: tolerance = metres / |gt1|.  W and H must be below 2^26.  None: every corner, as without simplification."""
+    extra = _tolerance(tolerance)
     def outputs(cap, dev):
         return (torch.empty(max(cap, 1), dtype=_I32, device=dev),            # left
                 torch.empty(max(cap, 1), dtype=_I32, device=dev),            # right
@@ -171,9 +198,10 @@ def boundary_lines(labels: torch.Tensor, n_regions: int, *, capacity=None) -> Li
                 torch.empty(cap + 1, dtype=_I64, device=dev),                # offsets
                 torch.empty((max(2 * cap, 1), 2), dtype=_I32, device=dev))   # vertices
 
+    entry = "dm_lines_simplified" if extra else "dm_lines"
     c, (left, right, length, offsets, vertices) = _trace(
-        labels, n_regions, capacity, default_line_capacity, outputs, "dm_lines",
-        lambda L, H, W, R, cap: L.dm_lines_workspace_bytes(H, W, cap), "boundary segments")
+        labels, n_regions, capacity, default_line_capacity, outputs, entry,
+        lambda L, H, W, R, cap: getattr(L, entry + "_workspace_bytes")(H, W, cap), "boundary segments", extra)
     k, v = int(c[0]), int(c[1])
     return Lines(left[:k], right[:k], length[:k], offsets[:k + 1], vertices[:v], int(c[2]))
 

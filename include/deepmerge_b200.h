@@ -512,6 +512,48 @@ int dm_lines(const int32_t* labels, int64_t H, int64_t W, int64_t ld, int64_t n_
              int64_t* counts, void* ws, size_t ws_bytes, dm_stream_t stream);
 
 /* ----------------------------------------------------------------------------------- *
+ * Simplified rings and lines: dm_polygonize / dm_lines followed by Douglas-Peucker with tolerance t (pixels, finite,
+ * >= 0; anything else is DM_ERR_BAD_ARG before any launch), applied so that every shared boundary is simplified the
+ * same way on both of its sides.  Vertices stay integer pixel corners: simplification only drops vertices.
+ *  - Chains: every line of dm_lines, and every ring of dm_polygonize with its nodes (vertices of degree >= 3 as in
+ *    dm_lines) added as vertices where it does not turn.  A ring piece between two consecutive nodes has the vertices
+ *    of one line, forward when the region is line_right, reversed when it is line_left.
+ *  - Anchors, always kept: every node; the ends of every open line; every vertex on the image border (x in {0, W} or
+ *    y in {0, H}); and, in a chain with no node, its start vertex (its smallest vertex in (y, x) order).
+ *  - Pieces: from one anchor to the next along the chain; a closed chain with one anchor is one piece from it back to
+ *    itself.
+ *  - d(P): the exact Euclidean distance of an interior vertex P of an interval A..B to the segment AB (to A when
+ *    A = B).  The top vertex of an interval is its interior vertex of largest d; ties go to the position k nearest the
+ *    middle (the smallest |2k - n| for positions 0..n), then to the smaller vertex index y (W + 1) + x.  The rule is
+ *    symmetric under reversal, which is what makes both sides of a boundary agree.
+ *  - Douglas-Peucker: an interval keeps its top vertex when d(top) > t, and then recurses on both halves.  Guard,
+ *    whatever t: the top vertex of every piece with interior vertices is kept, and for a piece with A = B the top
+ *    vertices of both halves too, so every simplified ring keeps at least 3 distinct vertices.
+ *  - Exact: t is rounded once to a multiple of 2^-10 px (to nearest) and clamped to W + H; every decision compares
+ *    128-bit integers, the same on host and device.  This needs W, H < 2^26: larger rasters are DM_ERR_BAD_ARG.
+ *  - Consequences: the kept set for t2 >= t1 is a subset of the one for t1; every dropped vertex lies within t of the
+ *    output segment that replaced it; with no nodata the doubled signed areas of all simplified rings sum to 2 H W.
+ *    Simplified lines may cross each other at large t: the output shares its boundaries but is not repaired into a
+ *    valid planar layer.
+ * Outputs: the arrays of dm_polygonize / dm_lines, with the same sizes and canonical order.  A line keeps its start and
+ * end; a ring starts at its first kept vertex at or after the unsimplified ring's start.  ring_area stays the signed
+ * pixel area of the unsimplified ring, line_length the number of unit segments, counts[1] is the number of kept
+ * vertices.  Simplified rings may hold vertices where the direction does not change (nodes): "corners only" and the
+ * alternating axes of dm_polygonize do not apply to them.  The workspace adds about 40 bytes per unsimplified vertex
+ * (capacity for rings, 2 capacity for lines).
+ * ----------------------------------------------------------------------------------- */
+size_t dm_polygonize_simplified_workspace_bytes(int64_t H, int64_t W, int64_t n_regions, int64_t capacity);
+int dm_polygonize_simplified(const int32_t* labels, int64_t H, int64_t W, int64_t ld, int64_t n_regions,
+                             int64_t capacity, double tolerance, int32_t* ring_region, int64_t* ring_offsets,
+                             int64_t* ring_area, int32_t* vertices, int64_t* region_rings, int64_t* counts, void* ws,
+                             size_t ws_bytes, dm_stream_t stream);
+size_t dm_lines_simplified_workspace_bytes(int64_t H, int64_t W, int64_t capacity);
+int dm_lines_simplified(const int32_t* labels, int64_t H, int64_t W, int64_t ld, int64_t n_regions, int64_t capacity,
+                        double tolerance, int32_t* line_left, int32_t* line_right, int64_t* line_length,
+                        int64_t* line_offsets, int32_t* vertices, int64_t* counts, void* ws, size_t ws_bytes,
+                        dm_stream_t stream);
+
+/* ----------------------------------------------------------------------------------- *
  * Rasterize polygons: the way in of the vector round trip, from the segment polygons of the reference's tile.shp to the
  * label raster the merge starts from.  The contract of shapefile.rasterize_polygons, bit for bit.  Not part of the merge
  * step.
